@@ -281,6 +281,37 @@ def group_arrays(haps):
     return (np.asarray([h[0] for h in haps], dtype=np.uint64), np.asarray([h[1] for h in haps], dtype=np.uint8))
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, pi, theta, res, world):
+    """--dump-outputs: what the timed call computed in its last step, for comparing two builds output for output.
+    pi.npy / theta.npy: the per-site tracks of both groups ([2, sites] float64).  A track has no value (NaN) at a
+    masked or uncallable site; the dump keeps every array finite so that two dumps compare element by element:
+    pi_defined.npy / theta_defined.npy ([2, sites] float32) hold 1 where the track has a value and 0 where it is
+    NaN, and the track holds 0 there.  Beyond DUMP_BYTES a fixed seeded sample of sites, whose indices go to
+    site_index.npy.  region_totals.npy: per group [segregating sites, sum of pi, uncallable sites] ([2, 3] float64,
+    exact below 2**53); with N > 1 also merged_region_totals.npy, the totals after the exchange between the ranks."""
+    os.makedirs(out_dir, exist_ok=True)
+    n_groups, V = pi.shape
+    keep = (DUMP_BYTES - (1 << 20)) // (2 * n_groups * (8 + 4) + 8)  # tracks, flags, index per site; 1 MB for the rest
+    if V > keep:
+        idx = np.sort(np.random.default_rng(0).choice(V, keep, replace=False))
+        pi, theta = pi[:, idx], theta[:, idx]
+        np.save(os.path.join(out_dir, "site_index.npy"), idx.astype(np.float64))
+    for name, track in (("pi", pi), ("theta", theta)):
+        undefined = np.isnan(track)
+        np.save(os.path.join(out_dir, name + ".npy"), np.where(undefined, 0.0, track))
+        np.save(os.path.join(out_dir, name + "_defined.npy"), (~undefined).astype(np.float32))
+    totals = {"region_totals": (res.last_seg, res.last_pi_sum, res.last_unc)}
+    if world > 1:
+        totals["merged_region_totals"] = (res.merged_seg, res.merged_pi_sum, res.merged_unc)
+    for name, (seg, pi_sum, unc) in totals.items():
+        arr = np.array([[seg[k], pi_sum[k], unc[k]] for k in range(n_groups)], dtype=np.float64)
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+    log(f"wrote the last timed step's outputs to {out_dir}")
+
+
 def load_peaks():
     try:
         peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))
@@ -444,14 +475,21 @@ def run_ours(args):
         _lib.check(L.fm_comm_connect(comm, handles.ctypes.data))
         dist.barrier()
     warm = max(args.warmup, 3)
-    _lib.check(L.fm_bench_diversity(garr, 2, 1, mask.ctypes.data, mask.size // 2, warm, comm, C.byref(res)))
+    _lib.check(L.fm_bench_diversity(garr, 2, 1, mask.ctypes.data, mask.size // 2, warm, comm, C.byref(res), None,
+                                    None))
+    # the timed call copies its last step's tracks into these device buffers once its timed region has ended
+    last_pi = last_th = None
+    if args.dump_outputs and rank == 0:
+        last_pi = torch.empty((2, V), dtype=torch.float64, device=device)
+        last_th = torch.empty_like(last_pi)
     if world > 1:
         dist.barrier()
     torch.cuda.synchronize()
     with ClockSampler(local) as clocks:
         wall0 = time.perf_counter()
         _lib.check(L.fm_bench_diversity(garr, 2, 1, mask.ctypes.data, mask.size // 2, args.steps, comm,
-                                        C.byref(res)))
+                                        C.byref(res), None if last_pi is None else last_pi.data_ptr(),
+                                        None if last_th is None else last_th.data_ptr()))
         dev_ms = res.step_ms_avg * args.steps
         torch.cuda.synchronize()
         wall1 = time.perf_counter()
@@ -466,7 +504,10 @@ def run_ours(args):
         t_keep = time.perf_counter()
         while len(clocks.samples) < timed_samples + 8 and time.perf_counter() - t_keep < 4.0:
             _lib.check(L.fm_bench_diversity(garr, 2, 1, mask.ctypes.data, mask.size // 2, 200, None,
-                                            C.byref(_lib.BenchResult())))
+                                            C.byref(_lib.BenchResult()), None, None))
+    if last_pi is not None:
+        dump_outputs(args.dump_outputs, last_pi.cpu().numpy(), last_th.cpu().numpy(), res, world)
+        del last_pi, last_th
     tmax = torch.tensor([dev_ms], dtype=torch.float64, device=device)
     if world > 1:
         dist.all_reduce(tmax, op=dist.ReduceOp.MAX)
@@ -526,7 +567,7 @@ def run_ours(args):
             sizes = (C.c_size_t * 2)(len(g0), len(g1))
             _lib.check(L.fm_groups_create(m, idx.ctypes.data, side.ctypes.data, sizes, 2, hs))
             r = _lib.BenchResult()
-            _lib.check(L.fm_bench_diversity(hs, 2, 1, mask.ctypes.data, mask.size // 2, 1, None, C.byref(r)))
+            _lib.check(L.fm_bench_diversity(hs, 2, 1, mask.ctypes.data, mask.size // 2, 1, None, C.byref(r), None, None))
             for h in hs:
                 L.fm_group_release(C.c_void_p(h))
         one()
@@ -809,6 +850,8 @@ def main():
     ap.add_argument("--skip-parity", action="store_true")
     ap.add_argument("--skip-from-u8", action="store_true")
     ap.add_argument("--skip-configs", action="store_true", help="skip configs 1/3/4/5 and the strong-scaling block")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the per-site tracks and region totals of the last timed step as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

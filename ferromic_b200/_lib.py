@@ -170,7 +170,8 @@ def lib() -> C.CDLL:
     L.fm_vcf_batch_release.argtypes = [vp]
     L.fm_synth_fill.argtypes = [vp, vp, sz, sz, sz, u64, u64, vp, dbl, dbl]
     L.fm_timings_get.argtypes = [C.POINTER(Timings)]
-    L.fm_bench_diversity.argtypes = [C.POINTER(vp), sz, C.c_int, vp, sz, C.c_int, vp, C.POINTER(BenchResult)]
+    L.fm_bench_diversity.argtypes = [C.POINTER(vp), sz, C.c_int, vp, sz, C.c_int, vp, C.POINTER(BenchResult), vp,
+                                     vp]
     L.fm_comm_create.argtypes = [C.c_int, C.c_int, C.POINTER(vp)]
     L.fm_comm_export.argtypes = [vp, vp]
     L.fm_comm_connect.argtypes = [vp, vp]

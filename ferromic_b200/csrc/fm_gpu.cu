@@ -5417,9 +5417,11 @@ void launch_reduce(const double *pd, int nd, const uint32_t *pu, int nu, const f
 }  // namespace
 
 fm_status fm_bench_diversity(fm_group *const *groups, size_t n_groups, int mode, const int64_t *mask_iv,
-                             size_t n_mask, int iterations, fm_comm *comm, fm_bench_result *out) {
+                             size_t n_mask, int iterations, fm_comm *comm, fm_bench_result *out, double *last_pi,
+                             double *last_theta) {
     return guarded([&] {
         if (!groups || !n_groups || !out || iterations < 1) fail(FM_ERR_INVALID_ARG, "bad argument");
+        if ((last_pi || last_theta) && mode != 1) fail(FM_ERR_INVALID_ARG, "per-site tracks need mode 1");
         require_device();
         std::memset(out, 0, sizeof(*out));
         fm_matrix *m = groups[0]->m;
@@ -5620,6 +5622,15 @@ fm_status fm_bench_diversity(fm_group *const *groups, size_t n_groups, int mode,
         out->step_ms_avg = total / (float)iterations;
         out->plane_ms_avg = spans.empty() ? 0.f : plane / (float)spans.size();
         out->plane_bytes_per_step = bytes;
+        // the tracks are written by every step into the same buffers: after the last one they hold its results
+        for (size_t i = 0; i < n_groups && V; ++i) {
+            if (last_pi)
+                CK(cudaMemcpyAsync(last_pi + i * V, pg[i].pi.p, (size_t)V * sizeof(double), cudaMemcpyDefault, stream()));
+            if (last_theta)
+                CK(cudaMemcpyAsync(last_theta + i * V, pg[i].theta.p, (size_t)V * sizeof(double), cudaMemcpyDefault,
+                                   stream()));
+        }
+        if (last_pi || last_theta) CK(cudaStreamSynchronize(stream()));
         // region totals of the LAST timed step (parity check of the run: bench.py compares them with the public
         // call and, for N > 1, the exchanged totals with a rank-ordered sum of every rank's local ones)
         const int pl = (iterations - 1) & 1;

@@ -547,7 +547,9 @@ fm_status fm_timings_get(fm_timings *out);
  * and folds the per-batch partials on device.  Timing uses CUDA events on the launching stream:
  * step_ms_avg brackets all `iterations` steps, plane_ms_avg is the mean duration of one
  * plane-pass launch (events around every launch).  With a communicator every step ends with the
- * fused fold + peer exchange of the groups' region totals (S, sum pi, uncallable sites). */
+ * fused fold + peer exchange of the groups' region totals (S, sum pi, uncallable sites).
+ * Mode 1 only: non-null last_pi / last_theta (host or device memory, [n_groups][V] doubles)
+ * receive the per-site tracks of the last timed step, copied after the timed region. */
 typedef struct {
     float step_ms_avg;
     float plane_ms_avg;
@@ -566,7 +568,8 @@ typedef struct {
 } fm_bench_result;
 fm_status fm_bench_diversity(fm_group *const *groups, size_t n_groups, int mode,
                              const int64_t *mask_iv_or_null, size_t n_mask, int iterations,
-                             fm_comm *comm_or_null, fm_bench_result *out);
+                             fm_comm *comm_or_null, fm_bench_result *out, double *last_pi_or_null,
+                             double *last_theta_or_null);
 /* Same for the fused two-group Hudson pass (K3). */
 fm_status fm_bench_hudson(fm_group *g1, fm_group *g2, int iterations, fm_bench_result *out);
 

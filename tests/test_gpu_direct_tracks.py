@@ -91,6 +91,39 @@ def test_page_locked_outputs_equal_pageable_outputs_and_the_oracle(V):
         assert np.all(np.abs(a[ok] - b[ok]) <= 1e-9 * np.abs(b[ok]))
 
 
+def test_bench_hook_hands_back_the_tracks_of_its_last_step():
+    """fm_bench_diversity (mode 1, the timed loop of bench.py) copies the tracks of its last step into the caller's
+    arrays, host or device (bench.py --dump-outputs): the same bits as fm_per_site_diversity_multi for the same groups
+    and mask.  Mode 0 computes no tracks and refuses the arrays."""
+    import torch
+    from ferromic_b200 import _lib
+    from ferromic_b200.api import _Matrix
+    L = _lib.lib()
+    V = 70000
+    g, pos, pops = make_cohort(V, 40, n_pops=2, missing_rate=0.03, seed=2024)
+    miss = g < 0
+    alle = np.where(miss, 0, g).astype(np.uint8)
+    h1, h2 = both_sides(pops[0]), both_sides(pops[1])
+    mask = np.array([int(pos[50]), int(pos[90]), int(pos[V // 2]), int(pos[V // 2 + 500])], dtype=np.int64)
+    m = _Matrix(alle, miss, pos, max_allele=1, always_bitmap=True, ingest="packed")
+    groups = [m.group(h1), m.group(h2)]
+    p, pi, th = np.empty(V, dtype=np.int64), np.empty((2, V)), np.empty((2, V))
+    assert _multi(L, _lib, groups, (len(h1), len(h2)), pos, mask, p.ctypes.data, pi.ctypes.data, th.ctypes.data, V) == V
+    gh = (C.c_void_p * 2)(*[x.handle for x in groups])
+    h_pi, h_th = np.full((2, V), -7.0), np.full((2, V), -7.0)
+    d_pi = torch.full((2, V), -7.0, dtype=torch.float64, device="cuda")
+    d_th = torch.full_like(d_pi, -7.0)
+    for pi_ptr, th_ptr in ((h_pi.ctypes.data, h_th.ctypes.data), (d_pi.data_ptr(), d_th.data_ptr())):
+        _lib.check(L.fm_bench_diversity(gh, 2, 1, mask.ctypes.data, mask.size // 2, 3, None,
+                                        C.byref(_lib.BenchResult()), pi_ptr, th_ptr))
+    for got, ref in ((h_pi, pi), (h_th, th), (d_pi.cpu().numpy(), pi), (d_th.cpu().numpy(), th)):
+        assert np.array_equal(np.isnan(got), np.isnan(ref))
+        assert np.array_equal(got[~np.isnan(got)], ref[~np.isnan(ref)])
+    with pytest.raises(ValueError):
+        _lib.check(L.fm_bench_diversity(gh, 2, 0, None, 0, 1, None, C.byref(_lib.BenchResult()), h_pi.ctypes.data,
+                                        None))
+
+
 def test_single_group_call_and_cached_counts_route_with_page_locked_outputs():
     """fm_per_site_diversity (one group) forwards to the multi-group call; once the group's counts are cached the tracks
     come from the light kernel -- both must store into page-locked arrays like the plane pass does."""

@@ -61,7 +61,7 @@ def cfg1(L, dev, scale):
     arr = (C.c_void_p * 1)(g.value)
     res = _lib.BenchResult()
     for it in (50, 200):
-        _lib.check(L.fm_bench_diversity(arr, 1, 0, None, 0, it, None, C.byref(res)))
+        _lib.check(L.fm_bench_diversity(arr, 1, 0, None, 0, it, None, C.byref(res), None, None))
     line("cfg1 summary (S, pi, theta), one group, no bitmap", V, 2 * S, res.plane_ms_avg, res.group_bytes[0],
          {"step_ms": res.step_ms_avg, "note": "latency-sized: 62.6 MB per pass, resident in the 126 MB L2"})
     L.fm_group_release(g)
