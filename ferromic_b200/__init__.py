@@ -1,6 +1,6 @@
 """ferromic_b200 -- B200 (sm_100a) implementation of ferromic's per-site population-genetics
 estimators (segregating sites, pi, Watterson theta, per-site pi/theta tracks, Hudson FST/Dxy,
-Weir & Cockerham FST) behind the reference's own Python surface (`import ferromic_b200 as fm`).
+Weir & Cockerham FST, pairwise sample differences) behind the reference's own Python surface (`import ferromic_b200 as fm`).
 
 All estimator arithmetic runs in hand-written CUDA kernels through the C-ABI library
 `libferromic_gpu.so` (include/ferromic_gpu.h); there is no CPU fallback."""
@@ -20,6 +20,8 @@ from .api import (  # noqa: F401
     hudson_fst_sites,
     hudson_fst_with_sites,
     inversion_allele_frequency,
+    pairwise_difference_arrays,
+    pairwise_differences,
     nucleotide_diversity,
     per_site_diversity,
     per_site_diversity_arrays,

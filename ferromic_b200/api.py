@@ -870,6 +870,62 @@ def per_site_diversity(variants, haplotypes, region=None):  # lib.rs:1639-1665
     return [DiversitySite(int(p), float(a), float(b)) for p, a, b in zip(pos, pi, th)]
 
 
+def _pairwise(variants, sample_count, want_positions: bool):
+    """fm_pairwise_differences over the first sample_count samples: (differences, comparable, pair_start,
+    positions) as condensed arrays in pair order (0,1), (0,2), ..., (1,2), ...; the last two are None unless
+    want_positions."""
+    n = int(sample_count)
+    if n < 0:
+        raise ValueError("sample_count must not be negative")
+    vs = _parse_variants(variants)
+    n_pairs = n * (n - 1) // 2
+    diff = np.zeros(n_pairs, dtype=np.uint32)
+    comp = np.zeros(n_pairs, dtype=np.uint32)
+    if n_pairs == 0:
+        empty = (np.zeros(1, dtype=np.uint64), np.zeros(0, dtype=np.int64)) if want_positions else (None, None)
+        return (diff, comp) + empty
+    # samples beyond a variant's genotype list are None
+    m = _sparse_matrix(vs, max(n, vs.n_samples))
+    L = lib()
+    total = C.c_size_t()
+    if not want_positions:
+        check(L.fm_pairwise_differences(m.handle, n, _ptr(diff), _ptr(comp), None, None, 0, C.byref(total)))
+        return diff, comp, None, None
+    start = np.zeros(n_pairs + 1, dtype=np.uint64)
+    pos = np.zeros(1, dtype=np.int64)
+    st = L.fm_pairwise_differences(m.handle, n, _ptr(diff), _ptr(comp), _ptr(start), _ptr(pos), 0, C.byref(total))
+    if st == _lib.FM_ERR_INVALID_ARG and total.value > 0:
+        pos = np.zeros(total.value, dtype=np.int64)  # the first call reported the size: retry
+        st = L.fm_pairwise_differences(m.handle, n, _ptr(diff), _ptr(comp), _ptr(start), _ptr(pos), pos.size,
+                                       C.byref(total))
+    check(st)
+    return diff, comp, start, pos[:total.value]
+
+
+def pairwise_difference_arrays(variants, sample_count):
+    """Array form of calculate_pairwise_differences (stats.rs:4106-4231): (differences, comparable) as
+    condensed u32 arrays of the n (n - 1) / 2 sample pairs in scipy.spatial.distance.pdist order.  comparable
+    counts the variants where neither genotype is None, differences those of them where the genotypes differ
+    as ordered vectors."""
+    diff, comp, _, _ = _pairwise(variants, sample_count, False)
+    return diff, comp
+
+
+def pairwise_differences(variants, sample_count):  # stats.rs:4106-4231
+    """[((i, j), difference_count, differing_positions), ...] for every sample pair i < j of
+    0 .. sample_count-1; positions are the variants' own (0-based) positions in site order."""
+    diff, _, start, pos = _pairwise(variants, sample_count, True)
+    n = int(sample_count)
+    pos = pos.tolist()
+    start = start.tolist()
+    out, k = [], 0
+    for i in range(n):
+        for j in range(i + 1, n):
+            out.append(((i, j), int(diff[k]), pos[start[k]:start[k + 1]]))
+            k += 1
+    return out
+
+
 def _opt(value: float, some: int, bit: int):
     return value if (some >> bit) & 1 else None
 

@@ -8,6 +8,7 @@
 #include "fm_multi.cuh"
 #include "fm_falsta.cuh"
 #include "fm_vcf.cuh"
+#include "fm_pairwise.cuh"
 
 #include <nvtx3/nvToolsExt.h>
 
@@ -5369,6 +5370,139 @@ fm_status fm_vcf_batch_release(fm_vcf_batch *b) {
     if (b->d_order) dev_free(b->d_order);
     delete b;
     return FM_OK;
+}
+
+// ------------------------------------------------------------------------------------ pairwise differences
+fm_status fm_pairwise_differences(fm_matrix *m, size_t n_samples, uint32_t *differences, uint32_t *comparable,
+                                  uint64_t *pair_start, int64_t *positions, size_t positions_capacity,
+                                  size_t *n_positions_out) {
+    return guarded([&] {
+        FM_NVTX("fm_pairwise_differences (transpose + pair bit-GEMM)");
+        require_device();
+        if (!m) fail(FM_ERR_INVALID_ARG, "matrix is NULL");
+        if (n_samples > m->S) fail(FM_ERR_INVALID_ARG, "n_samples exceeds the matrix's sample count");
+        if (m->ploidy < 1 || m->ploidy > 2)
+            fail(FM_ERR_UNSUPPORTED, "pairwise differences support ploidy 1 and 2 on the GPU path");
+        if (m->streamed && !m->packed)
+            fail(FM_ERR_UNSUPPORTED, "pairwise differences need resident rows: this matrix was streamed as u8 rows");
+        uint32_t n_bits = 1;
+        while ((1u << n_bits) <= m->plane_max_allele) ++n_bits;
+        if (n_bits > 4)
+            fail(FM_ERR_UNSUPPORTED, "more than 16 distinct allele values (or allele indices above 15 on a streamed / "
+                                     "device-owned matrix) are not supported on the GPU path");
+        if (n_samples >= (1u << 21)) fail(FM_ERR_UNSUPPORTED, "more than 2^21 samples per pairwise call");
+        const uint64_t n_pairs = n_samples < 2 ? 0 : (uint64_t)n_samples * (n_samples - 1) / 2;
+        if (n_pairs && !differences) fail(FM_ERR_INVALID_ARG, "differences is NULL");
+        if (n_pairs == 0) {
+            if (pair_start) pair_start[0] = 0;
+            if (n_positions_out) *n_positions_out = 0;
+            return;
+        }
+        set_dev(m);
+        const uint32_t PL = (uint32_t)m->ploidy, S = (uint32_t)n_samples, V = (uint32_t)m->V;
+        const bool hc = m->has_missing;
+        const uint32_t n_words = (V + 31) / 32, n_chunks = (n_words + fm::kPwKT - 1) / fm::kPwKT;
+        fm::PwLayout L{(S + fm::kPwBlk - 1) / fm::kPwBlk, (hc ? PL : 0u) + PL * (m->packed ? 1u : n_bits)};
+        const size_t plane_words = (size_t)n_chunks * L.n_blk * L.tile_words();
+        DevBuf<uint32_t> d_planes(std::max<size_t>(plane_words, 4));
+        DevBuf<uint32_t> d_diff(n_pairs), d_comp(comparable ? n_pairs : 0);
+
+        // 1. transpose into K-tiled sample-major planes
+        Timer tm;
+        tm.start();
+        if (plane_words) {
+            CK(cudaMemsetAsync(d_planes.p, 0, plane_words * 4, stream()));
+            const uint64_t tasks = m->packed ? (uint64_t)n_words * ((S * PL + 31) / 32) : (uint64_t)n_words * ((S + 31) / 32);
+            const uint32_t grid = (uint32_t)std::min<uint64_t>((tasks + 7) / 8, 64ull * sm_count(m->device));
+            if (m->packed) {
+                const uint32_t n_cell_words = (S * PL + 31) / 32;
+                if (PL == 1)
+                    fm::fm_k_sample_planes_packed<1><<<grid, 256, 0, stream()>>>(m->d_abits, m->d_cbits, m->rw, V, S, n_words,
+                                                                                n_cell_words, L, d_planes.p);
+                else
+                    fm::fm_k_sample_planes_packed<2><<<grid, 256, 0, stream()>>>(m->d_abits, m->d_cbits, m->rw, V, S, n_words,
+                                                                                n_cell_words, L, d_planes.p);
+            } else {
+                const uint32_t miss_mode = !hc ? 0u : (m->in_band ? 2u : 1u);
+                auto run = [&](auto kern) {
+                    kern<<<grid, 256, 0, stream()>>>(m->d_data, m->d_missing, miss_mode, m->d_lut, V, S, (uint64_t)m->stride,
+                                                     n_words, L, d_planes.p);
+                };
+                const uint32_t form = (PL - 1) * 4 + (n_bits - 1);  // one instantiation per (ploidy, allele bits)
+                switch (form) {
+                    case 0: run(fm::fm_k_sample_planes<1, 1>); break;
+                    case 1: run(fm::fm_k_sample_planes<1, 2>); break;
+                    case 2: run(fm::fm_k_sample_planes<1, 3>); break;
+                    case 3: run(fm::fm_k_sample_planes<1, 4>); break;
+                    case 4: run(fm::fm_k_sample_planes<2, 1>); break;
+                    case 5: run(fm::fm_k_sample_planes<2, 2>); break;
+                    case 6: run(fm::fm_k_sample_planes<2, 3>); break;
+                    default: run(fm::fm_k_sample_planes<2, 4>); break;
+                }
+            }
+            CK(cudaGetLastError());
+            g_launches++;
+        }
+        tm.stop();
+        t_tim.repack_ms += tm.ms();
+
+        // 2. upper-triangle bit-GEMM over sample pairs
+        const uint64_t n_tiles = (uint64_t)L.n_blk * (L.n_blk + 1) / 2;
+        const size_t smem = (size_t)fm::kPwStages * 2 * L.tile_words() * 4 + 2 * fm::kPwStages * 8;
+        auto kern = hc ? fm::fm_k_pairwise_counts<true> : fm::fm_k_pairwise_counts<false>;
+        CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        Timer tk;
+        tk.start();
+        kern<<<(uint32_t)n_tiles, (fm::kPwConsumerWarps + 1) * 32, smem, stream()>>>(d_planes.p, L, n_chunks, S, V, d_diff.p,
+                                                                                    comparable ? d_comp.p : nullptr);
+        CK(cudaGetLastError());
+        g_launches++;
+        tk.stop();
+        t_tim.stats_ms += tk.ms();
+        t_tim.stats_launches++;
+        d_diff.download(differences, n_pairs);
+        if (comparable) d_comp.download(comparable, n_pairs);
+
+        // 3. positions: exclusive scan of the counts, then one warp per pair
+        if (pair_start || positions) {
+            DevBuf<uint64_t> d_start(n_pairs + 1);
+            thrust::transform_iterator<fm::U32ToU64, const uint32_t *> diff64(d_diff.p, fm::U32ToU64());
+            size_t tmp_bytes = 0;
+            CK(cub::DeviceScan::InclusiveSum(nullptr, tmp_bytes, diff64, d_start.p + 1, (int64_t)n_pairs, stream()));
+            DevBuf<uint8_t> d_tmp(std::max<size_t>(tmp_bytes, 16));
+            CK(cudaMemsetAsync(d_start.p, 0, 8, stream()));
+            CK(cub::DeviceScan::InclusiveSum(d_tmp.p, tmp_bytes, diff64, d_start.p + 1, (int64_t)n_pairs, stream()));
+            uint64_t total = 0;
+            CK(cudaMemcpyAsync(&total, d_start.p + n_pairs, 8, cudaMemcpyDeviceToHost, stream()));
+            if (pair_start) d_start.download(pair_start, n_pairs + 1);
+            CK(cudaStreamSynchronize(stream()));
+            if (n_positions_out) *n_positions_out = (size_t)total;
+            if (positions) {
+                if (total > positions_capacity)
+                    fail(FM_ERR_INVALID_ARG, "positions capacity too small: *n_positions_out holds the number needed");
+                if (total) {
+                    if ((n_pairs + 7) / 8 >= (1ull << 31)) fail(FM_ERR_UNSUPPORTED, "too many pairs for a positions call");
+                    DevBuf<int64_t> d_out(total);
+                    const uint32_t blocks = (uint32_t)((n_pairs + 7) / 8);
+                    if (hc)
+                        fm::fm_k_pairwise_positions<true><<<blocks, 256, 0, stream()>>>(d_planes.p, L, n_words, S, n_pairs,
+                                                                                        d_start.p, m->d_pos, d_out.p);
+                    else
+                        fm::fm_k_pairwise_positions<false><<<blocks, 256, 0, stream()>>>(d_planes.p, L, n_words, S, n_pairs,
+                                                                                         d_start.p, m->d_pos, d_out.p);
+                    CK(cudaGetLastError());
+                    g_launches++;
+                    d_out.download(positions, total);
+                }
+            }
+        } else if (n_positions_out) {
+            CK(cudaStreamSynchronize(stream()));
+            uint64_t total = 0;
+            for (uint64_t i = 0; i < n_pairs; ++i) total += differences[i];
+            *n_positions_out = (size_t)total;
+        }
+        CK(cudaStreamSynchronize(stream()));
+    });
 }
 
 // ------------------------------------------------------------------------------------ synthetic cohorts

@@ -519,6 +519,25 @@ fm_status fm_vcf_batch_matrix(const fm_vcf_batch *b, int pass_only, fm_matrix **
 fm_status fm_vcf_batch_matrix_packed(const fm_vcf_batch *b, int pass_only, fm_matrix **out);
 fm_status fm_vcf_batch_release(fm_vcf_batch *b);
 
+/* ---- pairwise genotype differences (calculate_pairwise_differences, stats.rs:4106-4231) ----
+ * For every pair of the first n_samples samples (n_samples <= the matrix's sample count), i < j in the order
+ * (0,1), (0,2), ..., (1,2), ... (scipy.spatial.distance.pdist order, n_pairs = n_samples (n_samples - 1) / 2):
+ *   comparable[p]  = #variants where neither genotype is None,
+ *   differences[p] = #of those where the genotypes differ as whole ordered vectors (phase and length count),
+ *   positions      = the 0-based positions of those variants, pair after pair, each pair's in site order;
+ *                    pair p's run is positions[pair_start[p] .. pair_start[p + 1]).
+ * A sample's genotype is the run of its leading called cells (side 0, side 1); it is None when cell 0 is missing --
+ * the inverse of from_variants, so every matrix form has an answer (u8 with bitmap / in-band / no missingness, rank
+ * LUT, resident packed rows).  Ploidy 1 or 2.  Outputs are host arrays: differences [n_pairs] (required),
+ * comparable [n_pairs], pair_start [n_pairs + 1] and positions [positions_capacity] may be NULL; *n_positions_out
+ * (may be NULL) receives the total number of differences.  Positions are requested by positions != NULL; when
+ * positions_capacity is too small the counts, pair_start and *n_positions_out are written and the call returns
+ * FM_ERR_INVALID_ARG so that the caller can retry.  The output grows with the number of differences: positions are
+ * meant for small inputs.  FM_ERR_UNSUPPORTED for a matrix streamed as u8 rows (no resident rows) and ploidy > 2. */
+fm_status fm_pairwise_differences(fm_matrix *m, size_t n_samples, uint32_t *differences, uint32_t *comparable_or_null,
+                                  uint64_t *pair_start_or_null /* [n_pairs+1] */, int64_t *positions_or_null,
+                                  size_t positions_capacity, size_t *n_positions_out);
+
 /* ---- synthetic cohorts for benchmarks and full-size parity tests ----
  * Fills a device-resident u8 matrix (reference layout) and, when d_missing != NULL, its packed
  * missing bitmap with a counter-based generator: entry (site, column) is a pure integer function

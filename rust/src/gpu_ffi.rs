@@ -75,6 +75,12 @@ extern "C" {
         n_sites: *mut usize) -> c_int;
     pub fn fm_adjusted_sequence_length(region_start: i64, region_end: i64, allow: *const i64,
         n_allow: usize, mask: *const i64, n_mask: usize, out: *mut i64) -> c_int;
+    // calculate_pairwise_differences (stats.rs:4106-4231): condensed pair order (0,1), (0,2), ..., (1,2), ...;
+    // positions != NULL requests the differing positions (FM_ERR_INVALID_ARG + *n_positions_out when the capacity
+    // is too small)
+    pub fn fm_pairwise_differences(m: *mut fm_matrix, n_samples: usize, differences: *mut u32,
+        comparable: *mut u32, pair_start: *mut u64, positions: *mut i64, positions_capacity: usize,
+        n_positions_out: *mut usize) -> c_int;
     // shard-mergeable window totals + finishers (multi-GPU, windows)
     pub fn fm_group_window_sums(g: *mut fm_group, windows: *const i64, n_windows: usize,
         n_variants: *mut u64, seg_sites: *mut u64, pi_sum: *mut f64, uncallable_lt2: *mut u64) -> c_int;
