@@ -662,15 +662,18 @@ struct fm_group {
     uint32_t n = 0;   // haplotype capacity
     uint32_t wq = 0;  // uint4 per plane row
     uint4 *d_allele = nullptr;
-    uint4 *d_called = nullptr;
+    uint4 *d_called = nullptr;  // multi-allelic groups of a matrix with missing data (fm_k_allele_counts needs allele 0)
     // tail layout (biallelic plane groups written by the compress plans): wq counts the FULL 16-byte words of a row,
-    // the last n % 128 haplotypes live in tw u32 words per row in d_tail_a / d_tail_c (fm_kernels.cuh GroupPlanes)
+    // the last n % 128 haplotypes live in tw u32 words per row in d_tail_a (fm_kernels.cuh GroupPlanes)
     uint32_t tw = 0;
-    uint32_t *d_tail_a = nullptr, *d_tail_c = nullptr;
+    uint32_t *d_tail_a = nullptr;
+    // biallelic plane groups of a matrix with missing data: K1 writes d_cnt (the called count of every site) when it
+    // repacks the rows, in place of a called plane; d_cnt is then an input of the plane pass, not a cache of it
+    bool cnt_in = false;
     double *d_tab = nullptr;   // 3 x (n+1) doubles: 1/k, k/(k-1), 1/H_{k-1}
     uint32_t *d_off = nullptr; // device copy of `off` (K1)
     std::mutex mu;
-    bool have_counts = false;
+    bool have_counts = false;       // d_alt (and d_cnt) hold the counts of every site
     uint32_t *d_alt = nullptr, *d_cnt = nullptr;
     uint32_t n_bits = 1;            // allele bitplanes (1 = biallelic; 2..4 = multi-allelic matrix)
     uint32_t *d_acount = nullptr;   // multi-allelic: cached per-allele counts [V][1 << n_bits]
@@ -712,11 +715,9 @@ uint32_t env_u32(const char *name, uint32_t dflt) {
 
 fm::PassGeom make_geom(const fm_group *const *gs, int ng, uint32_t v_lo, uint32_t v_hi) {
     fm::PassGeom G{};
-    uint32_t row_bytes = 0, planes = 0, max_wq = 0;
+    uint32_t row_bytes = 0, max_wq = 0;
     for (int i = 0; i < ng; ++i) {
-        const uint32_t p = gs[i]->d_called ? 2u : 1u;
-        row_bytes += gs[i]->wq * 16u * p;
-        planes += p;
+        row_bytes += gs[i]->wq * 16u;
         max_wq = std::max(max_wq, gs[i]->wq);
     }
     static const uint32_t step_target = env_u32("FM_STEP_BYTES", fm::kStepBytesTarget);
@@ -757,10 +758,10 @@ fm::PassGeom make_geom(const fm_group *const *gs, int ng, uint32_t v_lo, uint32_
         step_bytes = round_bytes * G.rounds;
     } else {
         if (row_bytes * 2 > warp_smem) {  // a single row does not fit twice: chunk its columns
-            G.cq = std::max(1u, step_goal / (16u * planes));
+            G.cq = std::max(1u, step_goal / (16u * (uint32_t)ng));
             G.n_chunks = (max_wq + G.cq - 1) / G.cq;
         }
-        step_bytes = G.cq * 16u * planes;
+        step_bytes = G.cq * 16u * (uint32_t)ng;
     }
     G.stage_bytes = (step_bytes + 127u) & ~127u;
     G.n_stages = std::min<uint32_t>(fm::kMaxStages, warp_smem / G.stage_bytes);
@@ -797,24 +798,14 @@ struct CounterPool {
 };
 thread_local CounterPool t_counters;
 
-template <int NG, int LG, bool HC>
+template <int NG, int LG>
 void launch_plane_pass_t(const fm::PassParams<NG> &P, uint32_t grid, size_t smem) {
-    CK(cudaFuncSetAttribute(fm::fm_k_plane_pass<NG, LG, HC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                            (int)smem));
-    fm::fm_k_plane_pass<NG, LG, HC><<<grid, P.geom.warps * 32, smem, stream()>>>(P);
+    CK(cudaFuncSetAttribute(fm::fm_k_plane_pass<NG, LG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    fm::fm_k_plane_pass<NG, LG><<<grid, P.geom.warps * 32, smem, stream()>>>(P);
 }
 
-template <int NG, bool HC>
-void launch_plane_pass_lg(const fm::PassParams<NG> &P, uint32_t grid, size_t smem) {
-    switch (P.geom.lps_log2) {
-        case 0: launch_plane_pass_t<NG, 0, HC>(P, grid, smem); break;
-        case 1: launch_plane_pass_t<NG, 1, HC>(P, grid, smem); break;
-        case 2: launch_plane_pass_t<NG, 2, HC>(P, grid, smem); break;
-        case 3: launch_plane_pass_t<NG, 3, HC>(P, grid, smem); break;
-        case 4: launch_plane_pass_t<NG, 4, HC>(P, grid, smem); break;
-        default: launch_plane_pass_t<NG, 5, HC>(P, grid, smem); break;
-    }
-}
+// bytes a plane pass reads for one group and site: allele row, tail words, called count
+uint64_t plane_site_bytes(const fm::GroupPlanes &g) { return g.wq * 16u + g.tw * 4u + (g.cnt ? 4u : 0u); }
 
 template <int NG>
 void launch_plane_pass(fm::PassParams<NG> P, int device) {
@@ -823,50 +814,47 @@ void launch_plane_pass(fm::PassParams<NG> P, int device) {
     const size_t smem = (size_t)P.geom.warps * P.geom.warp_smem_bytes;
     const uint32_t need = (P.geom.n_batches + P.geom.warps - 1) / P.geom.warps;
     const uint32_t grid = std::min<uint32_t>((uint32_t)sm_count(device), need);
-    bool hc = P.g[0].called != nullptr;
-    for (int g = 1; g < NG; ++g)
-        if ((P.g[g].called != nullptr) != hc) fail(FM_ERR_INVALID_ARG, "groups of one pass must share a matrix");
-    if (hc)
-        launch_plane_pass_lg<NG, true>(P, grid, smem);
-    else
-        launch_plane_pass_lg<NG, false>(P, grid, smem);
+    switch (P.geom.lps_log2) {
+        case 0: launch_plane_pass_t<NG, 0>(P, grid, smem); break;
+        case 1: launch_plane_pass_t<NG, 1>(P, grid, smem); break;
+        case 2: launch_plane_pass_t<NG, 2>(P, grid, smem); break;
+        case 3: launch_plane_pass_t<NG, 3>(P, grid, smem); break;
+        case 4: launch_plane_pass_t<NG, 4>(P, grid, smem); break;
+        default: launch_plane_pass_t<NG, 5>(P, grid, smem); break;
+    }
     CK(cudaGetLastError());
     g_launches++;
     t_tim.stats_launches++;
     uint64_t bytes = 0;
-    for (int g = 0; g < NG; ++g)
-        bytes += (uint64_t)(P.geom.v_hi - P.geom.v_lo) * (P.g[g].wq * 16u + P.g[g].tw * 4u) * (P.g[g].called ? 2u : 1u);
+    for (int g = 0; g < NG; ++g) bytes += (uint64_t)(P.geom.v_hi - P.geom.v_lo) * plane_site_bytes(P.g[g]);
     t_tim.stats_bytes = bytes;
 }
 
 fm::GroupPlanes planes_of(const fm_group *g);
 
 // Several groups of one matrix over one site range in ONE persistent launch (fm_k_plane_pass_seq).
-// Returns false when the groups cannot share a launch (column-chunked rows, mixed bitmap / no
-// bitmap, more than kMaxSeq groups): the caller then launches per group.
+// Returns false when the groups cannot share a launch (column-chunked rows, more than kMaxSeq
+// groups): the caller then launches per group.
 bool make_seq_params(fm_group *const *gs, size_t n, uint32_t v_lo, uint32_t v_hi, fm::SeqParams &P) {
     if (n < 2 || n > (size_t)fm::kMaxSeq) return false;
     static const uint32_t step_target = env_u32("FM_STEP_BYTES", fm::kStepBytesTarget);
     static const uint32_t disable = env_u32("FM_NO_SEQ", 0);
     if (disable) return false;
     const uint32_t warp_smem = fm::kWarpSmemBytes;
-    const bool hc = gs[0]->d_called != nullptr;
     uint32_t max_wq = 0;
     for (size_t i = 0; i < n; ++i) {
-        if (gs[i]->m != gs[0]->m || (gs[i]->d_called != nullptr) != hc || gs[i]->n_bits != 1 || gs[i]->count_only)
-            return false;
+        if (gs[i]->m != gs[0]->m || gs[i]->n_bits != 1 || gs[i]->count_only) return false;
         max_wq = std::max(max_wq, gs[i]->wq);
     }
     uint32_t lg = 0;
     while ((1u << lg) < std::min(max_wq, 8u)) ++lg;
-    const uint32_t planes = hc ? 2u : 1u;
-    while (lg < 5 && (uint64_t)max_wq * 16u * planes * (32u >> lg) * 2 > warp_smem) ++lg;
+    while (lg < 5 && (uint64_t)max_wq * 16u * (32u >> lg) * 2 > warp_smem) ++lg;
     if (lg >= 5) return false;
     P = fm::SeqParams{};
     P.n_seg = (uint32_t)n;
     uint32_t max_step = 0;
     for (size_t i = 0; i < n; ++i) {
-        const uint32_t round_bytes = gs[i]->wq * 16u * planes * (32u >> lg);
+        const uint32_t round_bytes = gs[i]->wq * 16u * (32u >> lg);
         uint32_t rounds = 1;
         while (rounds * 2 <= (1u << lg) && round_bytes * rounds * 2 <= step_target) rounds *= 2;
         P.seg[i].g = planes_of(gs[i]);
@@ -889,10 +877,10 @@ bool make_seq_params(fm_group *const *gs, size_t n, uint32_t v_lo, uint32_t v_hi
     return true;
 }
 
-template <int LG, bool HC>
+template <int LG>
 void launch_plane_pass_seq_t(const fm::SeqParams &P, uint32_t grid, size_t smem) {
-    CK(cudaFuncSetAttribute(fm::fm_k_plane_pass_seq<LG, HC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    fm::fm_k_plane_pass_seq<LG, HC><<<grid, fm::kWarpsPerCta * 32, smem, stream()>>>(P);
+    CK(cudaFuncSetAttribute(fm::fm_k_plane_pass_seq<LG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    fm::fm_k_plane_pass_seq<LG><<<grid, fm::kWarpsPerCta * 32, smem, stream()>>>(P);
 }
 
 void launch_plane_pass_seq(fm::SeqParams P, int device) {
@@ -901,11 +889,9 @@ void launch_plane_pass_seq(fm::SeqParams P, int device) {
     const size_t smem = (size_t)fm::kWarpsPerCta * P.geom.warp_smem_bytes;
     const uint32_t total = P.geom.n_batches * P.n_seg;
     const uint32_t grid = std::min<uint32_t>((uint32_t)sm_count(device), (total + fm::kWarpsPerCta - 1) / fm::kWarpsPerCta);
-    const bool hc = P.seg[0].g.called != nullptr;
-#define FM_SEQ_CASE(L)                                                   \
-    case L:                                                              \
-        if (hc) launch_plane_pass_seq_t<L, true>(P, grid, smem);         \
-        else launch_plane_pass_seq_t<L, false>(P, grid, smem);           \
+#define FM_SEQ_CASE(L)                                   \
+    case L:                                              \
+        launch_plane_pass_seq_t<L>(P, grid, smem);       \
         break;
     switch (P.geom.lps_log2) {
         FM_SEQ_CASE(0) FM_SEQ_CASE(1) FM_SEQ_CASE(2) FM_SEQ_CASE(3) FM_SEQ_CASE(4)
@@ -916,15 +902,14 @@ void launch_plane_pass_seq(fm::SeqParams P, int device) {
     g_launches++;
     t_tim.stats_launches++;
     uint64_t bytes = 0;
-    for (uint32_t i = 0; i < P.n_seg; ++i)
-        bytes += (uint64_t)(P.geom.v_hi - P.geom.v_lo) * (P.seg[i].g.wq * 16u + P.seg[i].g.tw * 4u) * (P.seg[i].g.called ? 2u : 1u);
+    for (uint32_t i = 0; i < P.n_seg; ++i) bytes += (uint64_t)(P.geom.v_hi - P.geom.v_lo) * plane_site_bytes(P.seg[i].g);
     t_tim.stats_bytes = bytes;
 }
 
 // fm_k_plane_pass_tab: an arbitrary list of plane segments (gpu = 1: independent (region, group) units;
 // gpu = 2: Hudson pairs over shared sites) in ONE persistent launch.  Fills rounds / b_lo of every segment,
 // uploads the descriptor table and launches.  Returns false when the segments cannot share a launch
-// (column-chunked rows, mixed bitmap / no bitmap): the caller then goes unit by unit.
+// (column-chunked rows): the caller then goes unit by unit.
 struct TabLaunch {
     DevBuf<fm::TabSeg> d_segs;
     DevBuf<uint32_t> d_prefix;
@@ -936,16 +921,11 @@ bool launch_plane_pass_tab(std::vector<fm::TabSeg> &segs, uint32_t gpu, const st
     if (segs.empty() || (gpu != 1 && gpu != 2) || segs.size() % gpu) return false;
     static const uint32_t step_target = env_u32("FM_STEP_BYTES", fm::kStepBytesTarget);
     const uint32_t warp_smem = fm::kWarpSmemBytes;
-    const bool hc = segs[0].g.called != nullptr;
     uint32_t max_wq = 0;
-    for (const fm::TabSeg &sg : segs) {
-        if ((sg.g.called != nullptr) != hc) return false;
-        max_wq = std::max(max_wq, sg.g.wq);
-    }
+    for (const fm::TabSeg &sg : segs) max_wq = std::max(max_wq, sg.g.wq);
     uint32_t lg = 0;
     while ((1u << lg) < std::min(max_wq, 8u)) ++lg;
-    const uint32_t planes = hc ? 2u : 1u;
-    while (lg < 5 && (uint64_t)max_wq * 16u * planes * (32u >> lg) * 2 > warp_smem) ++lg;
+    while (lg < 5 && (uint64_t)max_wq * 16u * (32u >> lg) * 2 > warp_smem) ++lg;
     if (lg >= 5) return false;
     const size_t n_units = segs.size() / gpu;
     uint32_t max_step = 0;
@@ -957,13 +937,13 @@ bool launch_plane_pass_tab(std::vector<fm::TabSeg> &segs, uint32_t gpu, const st
         for (uint32_t g = 0; g < gpu; ++g) {
             fm::TabSeg &sg = segs[u * gpu + g];
             if (sg.v_lo != s0.v_lo || sg.v_hi != s0.v_hi) return false;
-            const uint32_t round_bytes = sg.g.wq * 16u * planes * (32u >> lg);
+            const uint32_t round_bytes = sg.g.wq * 16u * (32u >> lg);
             uint32_t rounds = 1;
             while (rounds * 2 <= (1u << lg) && round_bytes * rounds * 2 <= step_target) rounds *= 2;
             sg.rounds = rounds;
             sg.b_lo = sg.v_lo / 32;
             max_step = std::max(max_step, round_bytes * rounds);
-            bytes += (uint64_t)(sg.v_hi - sg.v_lo) * (sg.g.wq * 16u + sg.g.tw * 4u) * planes;
+            bytes += (uint64_t)(sg.v_hi - sg.v_lo) * plane_site_bytes(sg.g);
         }
         keep.prefix[u] = (uint32_t)total;
         total += nb;
@@ -1013,22 +993,17 @@ bool launch_plane_pass_tab(std::vector<fm::TabSeg> &segs, uint32_t gpu, const st
                                              (uint32_t)((total * gpu + fm::kWarpsPerCta - 1) / fm::kWarpsPerCta));
     // the dynamic shared-memory limit is a per-device function attribute: set it once per (instantiation, device)
     static std::mutex attr_mu;
-    static bool attr_done[10][64] = {};
+    static bool attr_done[5][64] = {};
     auto once = [&](int slot, auto kern) {
         std::lock_guard<std::mutex> lk(attr_mu);
         if (device < 64 && attr_done[slot][device]) return;
         CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         if (device < 64) attr_done[slot][device] = true;
     };
-#define FM_TAB_CASE(L)                                                                                \
-    case L:                                                                                           \
-        if (hc) {                                                                                     \
-            once(2 * L, fm::fm_k_plane_pass_tab<L, true>);                                            \
-            fm::fm_k_plane_pass_tab<L, true><<<grid, fm::kWarpsPerCta * 32, smem, stream()>>>(P);     \
-        } else {                                                                                      \
-            once(2 * L + 1, fm::fm_k_plane_pass_tab<L, false>);                                       \
-            fm::fm_k_plane_pass_tab<L, false><<<grid, fm::kWarpsPerCta * 32, smem, stream()>>>(P);    \
-        }                                                                                             \
+#define FM_TAB_CASE(L)                                                                  \
+    case L:                                                                             \
+        once(L, fm::fm_k_plane_pass_tab<L>);                                            \
+        fm::fm_k_plane_pass_tab<L><<<grid, fm::kWarpsPerCta * 32, smem, stream()>>>(P); \
         break;
     switch (lg) {
         FM_TAB_CASE(0) FM_TAB_CASE(1) FM_TAB_CASE(2) FM_TAB_CASE(3) FM_TAB_CASE(4)
@@ -1075,7 +1050,17 @@ void set_tables(fm::DivEpilogue &e, const fm_group *g) {
 }
 
 fm::GroupPlanes planes_of(const fm_group *g) {
-    return fm::GroupPlanes{g->d_allele, g->d_called, g->wq, g->n, g->d_tail_a, g->d_tail_c, g->tw};
+    return fm::GroupPlanes{g->d_allele, g->cnt_in ? g->d_cnt : nullptr, g->wq, g->n, g->d_tail_a, g->tw};
+}
+
+// where a pass over all sites caches its called counts: nowhere when K1 already wrote them
+uint32_t *called_cache(fm_group *g) { return g->cnt_in ? nullptr : g->d_cnt; }
+
+// the cached-count arrays of a biallelic group (d_cnt exists from creation on when K1 fills it)
+void alloc_counts(fm_group *g) {
+    const size_t V = std::max<size_t>(g->m->V, 1);
+    if (!g->d_alt) g->d_alt = static_cast<uint32_t *>(dev_alloc(V * sizeof(uint32_t)));
+    if (!g->d_cnt) g->d_cnt = static_cast<uint32_t *>(dev_alloc(V * sizeof(uint32_t)));
 }
 
 // K5a: mask / filtered-position bit per site, one word per batch
@@ -1215,7 +1200,7 @@ DivResult run_diversity(fm_group *g, uint32_t v_lo, uint32_t v_hi, int pi_form, 
     } else {
         if (store_counts) {
             e.alt_out = g->d_alt;
-            e.called_out = g->d_cnt;
+            e.called_out = called_cache(g);
         }
         if (g->count_only) fail(FM_ERR_INVALID_ARG, "internal: a count-only group has no bitplanes to stream");
         fm::PassParams<1> P{};
@@ -1283,7 +1268,7 @@ bool run_diversity_multi(fm_group *const *gs, size_t n, uint32_t v_lo, uint32_t 
         e.part_u = part_u[i].p;
         if (store_counts) {  // cache the DensePopulationSummary arrays while the planes stream by
             e.alt_out = gs[i]->d_alt;
-            e.called_out = gs[i]->d_cnt;
+            e.called_out = called_cache(gs[i]);
         }
         P.seg[i].div = e;
     }
@@ -1308,10 +1293,7 @@ void ensure_counts(fm_group *g) {
     }
     set_dev(g->m);
     const size_t V = g->m->V;
-    if (!g->d_alt) {
-        g->d_alt = static_cast<uint32_t *>(dev_alloc(std::max<size_t>(V, 1) * sizeof(uint32_t)));
-        g->d_cnt = static_cast<uint32_t *>(dev_alloc(std::max<size_t>(V, 1) * sizeof(uint32_t)));
-    }
+    alloc_counts(g);
     DivResult r = run_diversity(g, 0, (uint32_t)V, FM_PIFORM_COUNTS, nullptr, nullptr, nullptr, 0,
                                 nullptr, 0, /*store_counts=*/true);
     g->seg = r.seg;
@@ -1741,9 +1723,9 @@ static size_t repack_warp_smem(const fm_matrix *m, uint32_t *row_buf_out, uint32
     // packed rows arrive as bit words: neither the u8 row nor the bitmap slice is staged
     const size_t row_buf = m->packed ? 0 : ((m->stride + 15) & ~(size_t)15) + 32;
     const size_t bit_buf = (!m->packed && m->has_missing && !m->in_band) ? ((m->stride + 63) / 64 + 2) * 8 : 0;
-    // full-row allele / called bit words + one group's two plane rows while they are assembled
-    // (+ 4 padding words per assembled row: the compress fragments or a zero into the word after the last one)
-    const size_t cnt_buf = 2 * ((m->stride + 31) / 32 + 1) * 4 + 2 * (((m->stride + 127) / 128) * 4 + 4) * 4;
+    // full-row allele / called bit words + one group's allele plane row while it is assembled
+    // (+ 4 padding words: the compress fragments or a zero into the word after the last one)
+    const size_t cnt_buf = 2 * ((m->stride + 31) / 32 + 1) * 4 + (((m->stride + 127) / 128) * 4 + 4) * 4;
     if (row_buf_out) *row_buf_out = (uint32_t)row_buf;
     if (bit_buf_out) *bit_buf_out = (uint32_t)bit_buf;
     return (row_buf + bit_buf + cnt_buf + 15) & ~(size_t)15;
@@ -1775,13 +1757,12 @@ static fm_group *alloc_group(fm_matrix *m, std::vector<uint32_t> &&off, bool cou
         {
             // tail layout when the padded last word would waste more than a quarter of itself and the group is
             // certain to be written by the compress plans (the only writer that knows the layout)
-            static const uint32_t no_tail = env_u32("FM_NO_TAIL", 0), no_plan = env_u32("FM_REPACK_BALLOT", 0),
-                                  v1 = env_u32("FM_REPACK_V1", 0);
+            static const uint32_t no_tail = env_u32("FM_NO_TAIL", 0);
             const uint32_t tail_bits = g->n % 128;
             const uint32_t tw = (tail_bits + 31) / 32;
-            // worth it when the row shrinks by at least 2 % (the tail words cost two extra loads per site in the
-            // epilogue: 2504 haplotypes = 19 words + 72 bits would save 4 of 320 bytes and run 3 % slower)
-            if (!no_tail && !no_plan && !v1 && n_bits == 1 && !g->count_only && row_fits_smem(m) && g->n >= 128 &&
+            // worth it when the row shrinks by at least 2 % (the tail words cost tw extra loads per site in the
+            // epilogue: 2504 haplotypes = 19 words + 72 bits would save 4 of 320 bytes and ran 3 % slower)
+            if (!no_tail && n_bits == 1 && !g->count_only && row_fits_smem(m) && g->n >= 128 &&
                 tail_bits != 0 && tail_bits <= 96 && (16u - 4u * tw) * 50u >= 16u * g->wq) {
                 g->wq = g->n / 128;
                 g->tw = tw;
@@ -1796,12 +1777,11 @@ static fm_group *alloc_group(fm_matrix *m, std::vector<uint32_t> &&off, bool cou
             g->d_cnt = static_cast<uint32_t *>(dev_alloc(std::max<size_t>(m->V, 1) * sizeof(uint32_t)));
         } else {
             g->d_allele = static_cast<uint4 *>(dev_alloc(plane_u4 * 16 * n_bits));
-            if (m->has_missing) g->d_called = static_cast<uint4 *>(dev_alloc(plane_u4 * 16));
-            if (g->tw) {
-                const size_t tail_words = std::max<size_t>(m->V, 1) * g->tw;
-                g->d_tail_a = static_cast<uint32_t *>(dev_alloc(tail_words * 4));
-                if (m->has_missing) g->d_tail_c = static_cast<uint32_t *>(dev_alloc(tail_words * 4));
-            }
+            // biallelic groups keep the called count per site instead of a called plane (K1 fills it)
+            g->cnt_in = m->has_missing && n_bits == 1;
+            if (g->cnt_in) g->d_cnt = static_cast<uint32_t *>(dev_alloc(std::max<size_t>(m->V, 1) * sizeof(uint32_t)));
+            else if (m->has_missing) g->d_called = static_cast<uint4 *>(dev_alloc(plane_u4 * 16));
+            if (g->tw) g->d_tail_a = static_cast<uint32_t *>(dev_alloc(std::max<size_t>(m->V, 1) * g->tw * 4));
         }
         // per-n tables: 1/n, n/(n-1) (stats.rs:2728-2732) and 1/H_{n-1} with the harmonic number
         // by forward summation exactly like stats.rs:4234-4240 / 4718-4719
@@ -1851,7 +1831,6 @@ struct RepackSet {  // device-resident descriptor tables of the groups one launc
         std::vector<uint32_t *> outs_a, outs_c;
         std::vector<uint32_t> plan;            // 8 words per entry
         std::vector<size_t> plan_at, plan_len;  // per plane group: first entry, entries (0 = no plan)
-        static const uint32_t no_plan = env_u32("FM_REPACK_BALLOT", 0);
         const bool staged = row_fits_smem(m);
         for (fm_group *g : gs) {
             if (g->count_only) {
@@ -1870,10 +1849,10 @@ struct RepackSet {  // device-resident descriptor tables of the groups one launc
                 h.push_back(fm::RepackGroup{g->d_off, g->n, g->wq, g->n_bits, reinterpret_cast<uint32_t *>(g->d_allele),
                                             reinterpret_cast<uint32_t *>(g->d_called),
                                             std::max<size_t>(m->V, 1) * g->wq * 4, nullptr, nullptr, nullptr, 0,
-                                            g->d_tail_a, g->d_tail_c, g->tw});
+                                            g->d_tail_a, g->tw, g->cnt_in ? g->d_cnt : nullptr});
                 plan_at.push_back(plan.size() / 8);
                 size_t ne = 0;
-                if (g->n_bits == 1 && ((staged && !no_plan) || m->packed)) {
+                if (g->n_bits == 1 && (staged || m->packed)) {
                     uint32_t pos = 0;
                     for (size_t k = 0; k < g->off.size(); ++ne) {  // offsets are sorted: one entry per row word
                         const uint32_t w = g->off[k] >> 5;
@@ -1900,7 +1879,7 @@ struct RepackSet {  // device-resident descriptor tables of the groups one launc
         }
         // every biallelic plane group takes the plan path when plans are in use -- also an empty group (no entries):
         // the direct and packed kernels compile without the ballot gathers
-        const bool plans_on = (staged && !no_plan) || m->packed;
+        const bool plans_on = staged || m->packed;
         bool any_bial = false;
         for (const fm::RepackGroup &rg : h) any_bial = any_bial || rg.n_bits == 1;
         if (plans_on && any_bial && plan.empty()) plan.resize(8, 0u);
@@ -1966,7 +1945,6 @@ static void launch_repack(const RepackSet &set, const uint8_t *data, size_t data
     const fm_matrix *m = gs[0]->m;
     uint32_t row_buf = 0, bit_buf = 0;
     uint32_t warp_smem = (uint32_t)repack_warp_smem(m, &row_buf, &bit_buf);
-    static const uint32_t force_v1 = env_u32("FM_REPACK_V1", 0);
     if (m->packed) {  // K1p: groups from the resident packed rows (data / missing are unused)
         if (warp_smem > repack_smem_limit(m))
             fail(FM_ERR_UNSUPPORTED, "packed rows wider than the repack kernel's shared-memory slice");
@@ -1992,7 +1970,7 @@ static void launch_repack(const RepackSet &set, const uint8_t *data, size_t data
         g_launches++;
         return;
     }
-    if (warp_smem <= 24 * 1024 && (!force_v1 || set.ct.n_groups)) {
+    if (warp_smem <= 24 * 1024) {
         // direct mode: nothing reads the raw bytes of the row after the full-row bit words are built
         static const uint32_t no_direct = env_u32("FM_REPACK_STAGED", 0);
         bool direct = !no_direct && set.need_row_bits && m->stride % 16 == 0 &&
@@ -2038,12 +2016,15 @@ static void launch_repack(const RepackSet &set, const uint8_t *data, size_t data
     for (const fm_group *g : set.plane_gs)
         if (g->tw) fail(FM_ERR_INVALID_ARG, "internal: a tail-layout group needs the plan path of the row-staged repack");
     for (const fm_group *g : set.plane_gs) {
+        // the kernel adds the called members of every row slice to d_cnt
+        if (g->cnt_in) CK(cudaMemsetAsync(g->d_cnt + v_lo, 0, (size_t)(v_hi - v_lo) * sizeof(uint32_t), st));
         const uint32_t blocks = (uint32_t)std::min<uint64_t>(
             (uint64_t)sm_count(m->device) * 8,
             std::max<uint64_t>(1, ((uint64_t)(v_hi - v_lo) * ((g->wq * 4 + 31) / 32) + 7) / 8));
         fm::fm_k_repack<<<blocks, 256, 0, st>>>(data, missing, m->stride, g->d_off, g->n, g->wq, v_base, word_base, v_lo,
                                                 v_hi, reinterpret_cast<uint32_t *>(g->d_allele),
-                                                reinterpret_cast<uint32_t *>(g->d_called), g->n_bits,
+                                                reinterpret_cast<uint32_t *>(g->d_called),
+                                                g->cnt_in ? g->d_cnt : nullptr, g->n_bits,
                                                 std::max<size_t>(m->V, 1) * g->wq * 4, m->in_band ? 1u : 0u, m->d_lut);
         CK(cudaGetLastError());
         g_launches++;
@@ -2181,7 +2162,6 @@ fm_status fm_group_release(fm_group *g) {
     dev_free(g->d_allele);
     dev_free(g->d_called);
     dev_free(g->d_tail_a);
-    dev_free(g->d_tail_c);
     dev_free(g->d_tab);
     dev_free(g->d_off);
     dev_free(g->d_alt);
@@ -2245,13 +2225,11 @@ static void summarize_groups(fm_group *const *groups, size_t n_groups) {
         order.erase(std::unique(order.begin(), order.end()), order.end());
         std::vector<std::unique_lock<std::mutex>> locks;
         for (fm_group *g : order) locks.emplace_back(g->mu);  // address order: no lock inversion
-        // classes of groups that can share a launch: biallelic planes, same bitmap presence
-        std::vector<fm_group *> todo[2];
+        // the groups that share a launch: biallelic planes whose counts are not cached yet
+        std::vector<fm_group *> gs;
         for (fm_group *g : order)
-            if (!g->have_counts && g->n_bits == 1 && !g->count_only && g->m->V > 0) todo[g->d_called ? 1 : 0].push_back(g);
-        for (int cls = 0; cls < 2; ++cls) {
-            std::vector<fm_group *> &gs = todo[cls];
-            if (gs.empty()) continue;
+            if (!g->have_counts && g->n_bits == 1 && !g->count_only && g->m->V > 0) gs.push_back(g);
+        if (!gs.empty()) {
             std::vector<fm::TabSeg> segs(gs.size());
             std::vector<size_t> part_off(gs.size());
             size_t total_b = 0;
@@ -2266,17 +2244,14 @@ static void summarize_groups(fm_group *const *groups, size_t n_groups) {
             for (size_t i = 0; i < gs.size(); ++i) {
                 fm_group *g = gs[i];
                 const uint32_t V = (uint32_t)g->m->V;
-                if (!g->d_alt) {
-                    g->d_alt = static_cast<uint32_t *>(dev_alloc((size_t)V * 4));
-                    g->d_cnt = static_cast<uint32_t *>(dev_alloc((size_t)V * 4));
-                }
+                alloc_counts(g);
                 fm::DivEpilogue de{};
                 set_tables(de, g);
                 de.pi_form = FM_PIFORM_COUNTS;
                 de.part_pi = ppi.p + part_off[i];
                 de.part_u = ppu.p + 2 * part_off[i];
                 de.alt_out = g->d_alt;
-                de.called_out = g->d_cnt;
+                de.called_out = called_cache(g);
                 segs[i] = fm::TabSeg{};
                 segs[i].g = planes_of(g);
                 segs[i].div = de;
@@ -2296,37 +2271,37 @@ static void summarize_groups(fm_group *const *groups, size_t n_groups) {
                 locks.clear();
                 for (fm_group *g : gs) ensure_counts(g);
                 for (fm_group *g : order) locks.emplace_back(g->mu);
-                continue;
-            }
-            DevBuf<uint4> d_ents(ents.size());
-            d_ents.upload(ents.data(), ents.size());
-            DevBuf<double> sd(ents.size());
-            DevBuf<uint64_t> su(ents.size() * 2);
-            fm::fm_k_reduce_partials_tab<<<(uint32_t)((ents.size() + 3) / 4), 128, 0, stream()>>>(
-                ppi.p, 1, ppu.p, 2, d_ents.p, (uint32_t)ents.size(), sd.p, su.p);
-            CK(cudaGetLastError());
-            g_launches++;
-            tm.stop();
-            std::vector<double> hd(ents.size());
-            std::vector<uint64_t> hu(ents.size() * 2);
-            sd.download(hd.data(), ents.size());
-            su.download(hu.data(), ents.size() * 2);
-            CK(cudaStreamSynchronize(stream()));
-            t_tim.stats_ms += tm.ms();
-            size_t e = 0;
-            for (size_t i = 0; i < gs.size(); ++i) {
-                const uint32_t nb = ((uint32_t)gs[i]->m->V + 31) / 32;
-                double pi = 0.0;
-                uint64_t sg = 0, un = 0;
-                for (uint32_t sb = 0; sb * fm::kSuperBatches < nb; ++sb, ++e) {  // fixed order, like finish_partials
-                    pi += hd[e];
-                    sg += hu[2 * e];
-                    un += hu[2 * e + 1];
+            } else {
+                DevBuf<uint4> d_ents(ents.size());
+                d_ents.upload(ents.data(), ents.size());
+                DevBuf<double> sd(ents.size());
+                DevBuf<uint64_t> su(ents.size() * 2);
+                fm::fm_k_reduce_partials_tab<<<(uint32_t)((ents.size() + 3) / 4), 128, 0, stream()>>>(
+                    ppi.p, 1, ppu.p, 2, d_ents.p, (uint32_t)ents.size(), sd.p, su.p);
+                CK(cudaGetLastError());
+                g_launches++;
+                tm.stop();
+                std::vector<double> hd(ents.size());
+                std::vector<uint64_t> hu(ents.size() * 2);
+                sd.download(hd.data(), ents.size());
+                su.download(hu.data(), ents.size() * 2);
+                CK(cudaStreamSynchronize(stream()));
+                t_tim.stats_ms += tm.ms();
+                size_t e = 0;
+                for (size_t i = 0; i < gs.size(); ++i) {
+                    const uint32_t nb = ((uint32_t)gs[i]->m->V + 31) / 32;
+                    double pi = 0.0;
+                    uint64_t sg = 0, un = 0;
+                    for (uint32_t sb = 0; sb * fm::kSuperBatches < nb; ++sb, ++e) {  // fixed order, like finish_partials
+                        pi += hd[e];
+                        sg += hu[2 * e];
+                        un += hu[2 * e + 1];
+                    }
+                    gs[i]->pi_sum = pi;
+                    gs[i]->seg = sg;
+                    gs[i]->unc = un;
+                    gs[i]->have_counts = true;
                 }
-                gs[i]->pi_sum = pi;
-                gs[i]->seg = sg;
-                gs[i]->unc = un;
-                gs[i]->have_counts = true;
             }
         }
         locks.clear();
@@ -3476,11 +3451,7 @@ fm_status fm_hudson_pair(fm_group *g1, fm_group *g2, int64_t L1, int64_t L2, int
             std::unique_lock<std::mutex> l1(g1->mu, std::defer_lock), l2(g2->mu, std::defer_lock);
             std::lock(l1, l2);
             if (!g1->have_counts && !g2->have_counts) {
-                for (fm_group *g : {g1, g2})
-                    if (!g->d_alt) {
-                        g->d_alt = static_cast<uint32_t *>(dev_alloc((size_t)V * 4));
-                        g->d_cnt = static_cast<uint32_t *>(dev_alloc((size_t)V * 4));
-                    }
+                for (fm_group *g : {g1, g2}) alloc_counts(g);
                 // ONE sweep of both groups' planes (fm_k_plane_pass_tab, pair units): every warp streams a batch of
                 // group 1, then the same batch of group 2, and evaluates the Hudson components in place -- the
                 // groups' counts and summary scalars are cached for later calls AND the Hudson partials (plus the
@@ -3499,7 +3470,7 @@ fm_status fm_hudson_pair(fm_group *g1, fm_group *g2, int64_t L1, int64_t L2, int
                     de.part_pi = ppi[k].p;
                     de.part_u = ppu[k].p;
                     de.alt_out = pair[k]->d_alt;
-                    de.called_out = pair[k]->d_cnt;
+                    de.called_out = called_cache(pair[k]);
                     segs[k] = fm::TabSeg{};
                     segs[k].g = planes_of(pair[k]);
                     segs[k].div = de;
@@ -5597,8 +5568,8 @@ fm_status fm_bench_diversity(fm_group *const *groups, size_t n_groups, int mode,
             e.pi_form = FM_PIFORM_COUNTS;
             e.part_pi = pg[i].part_pi[0].p;
             e.part_u = pg[i].part_u[0].p;
-            bytes += (uint64_t)V * (g->wq * 16u + g->tw * 4u) * (g->d_called ? 2u : 1u);
-            if (i < 8) out->group_bytes[i] = (uint64_t)V * (g->wq * 16u + g->tw * 4u) * (g->d_called ? 2u : 1u) + (mode == 1 ? (uint64_t)V * 16u : 0);
+            bytes += (uint64_t)V * plane_site_bytes(planes_of(g));
+            if (i < 8) out->group_bytes[i] = (uint64_t)V * plane_site_bytes(planes_of(g)) + (mode == 1 ? (uint64_t)V * 16u : 0);
             if (mode == 1) {
                 pg[i].pi.alloc(std::max<uint32_t>(V, 1));
                 pg[i].theta.alloc(std::max<uint32_t>(V, 1));
@@ -5849,8 +5820,7 @@ fm_status fm_bench_hudson(fm_group *g1, fm_group *g2, int iterations, fm_bench_r
         }
         out->step_ms_avg = total / (float)iterations;
         out->plane_ms_avg = plane / (float)spans.size();
-        out->plane_bytes_per_step = (uint64_t)V * 16u *
-                                    (g1->wq * (g1->d_called ? 2u : 1u) + g2->wq * (g2->d_called ? 2u : 1u));
+        out->plane_bytes_per_step = (uint64_t)V * (plane_site_bytes(P.g[0]) + plane_site_bytes(P.g[1]));
     });
 }
 

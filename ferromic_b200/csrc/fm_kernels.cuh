@@ -29,6 +29,18 @@ constexpr uint32_t kSchedStrideWords = 32;
 constexpr uint32_t kSuperBatches = 256;          // batches folded by fm_k_reduce_partials
 constexpr int kBatchRing = 8;                    // claimed-batch ring per warp (> kMaxStages)
 
+__device__ __forceinline__ double fm_warp_sum(double v) {
+    // fixed-shape butterfly: identical association for every batch
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
+__device__ __forceinline__ uint32_t fm_warp_sum_u(uint32_t v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
+
 // ------------------------------------------------------------------------------ K1 repack
 // One warp builds 32-bit words with __ballot_sync: lane j handles haplotype k = 32*w + j of
 // the group (offset table `off`, sorted/de-duplicated exactly like DenseMembership::build,
@@ -36,11 +48,14 @@ constexpr int kBatchRing = 8;                    // claimed-batch ring per warp 
 // when the matrix has no bitmap).  Words are written 32 at a time (one per lane, 128 B).
 // Plane row = wq uint4 = 4*wq words; padding bits are zero.  `data` starts at row v_base and
 // `missing` at bitmap word word_base, so a staged chunk of rows can be repacked in place.
+// Biallelic groups of a matrix with missing data keep no called plane (called == nullptr): the
+// row's called count is added to cnt[v] instead (zeroed by the caller; a row spans several warps).
 __global__ void __launch_bounds__(256)
 fm_k_repack(const uint8_t *__restrict__ data, const uint64_t *__restrict__ missing, size_t stride,
             const uint32_t *__restrict__ off, uint32_t n, uint32_t wq, uint32_t v_base, uint64_t word_base,
             uint32_t v_lo, uint32_t v_hi, uint32_t *__restrict__ allele, uint32_t *__restrict__ called,
-            uint32_t n_bits, size_t plane_stride_words, uint32_t in_band, const uint8_t *__restrict__ lut) {
+            uint32_t *__restrict__ cnt, uint32_t n_bits, size_t plane_stride_words, uint32_t in_band,
+            const uint8_t *__restrict__ lut) {
     const uint32_t lane = threadIdx.x & 31;
     const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const uint32_t nwarps = (gridDim.x * blockDim.x) >> 5;
@@ -94,6 +109,10 @@ fm_k_repack(const uint8_t *__restrict__ data, const uint64_t *__restrict__ missi
                 if (b < n_bits) allele[b * plane_stride_words + (size_t)v * words + w] = my_a[b];
             if (called) called[(size_t)v * words + w] = my_c;
         }
+        if (cnt) {  // warp-uniform
+            const uint32_t c = fm_warp_sum_u(w < words ? __popc(my_c) : 0u);
+            if (lane == 0 && c) atomicAdd(cnt + v, c);
+        }
     }
 }
 
@@ -107,7 +126,7 @@ fm_k_repack(const uint8_t *__restrict__ data, const uint64_t *__restrict__ missi
 struct RepackGroup {
     const uint32_t *off;       // sorted, de-duplicated column offsets (DenseMembership, stats.rs:1251-1284)
     uint32_t n, wq, n_bits;
-    uint32_t *allele, *called; // called == nullptr when the matrix has no bitmap
+    uint32_t *allele, *called; // called plane: multi-allelic groups of a matrix with missing data only
     size_t plane_stride_words; // distance between allele bit planes (multi-allelic groups)
     // count-only groups (the subpopulations of a W&C partition): no bitplanes are kept, the
     // per-site alt / called counts -- all K4 ever reads -- are produced straight from the staged row
@@ -120,9 +139,12 @@ struct RepackGroup {
     const uint4 *plan;
     uint32_t n_ent;
     // tail layout (plan path only): the plane row holds the wq FULL 16-byte words of the group; the remaining
-    // n % 128 haplotypes go to tw = ceil((n % 128) / 32) u32 words per row in separate arrays (tw == 0: padded rows)
-    uint32_t *tail_a, *tail_c;
+    // n % 128 haplotypes go to tw = ceil((n % 128) / 32) u32 words per row in a separate array (tw == 0: padded rows)
+    uint32_t *tail_a;
     uint32_t tw;
+    // biallelic groups of a matrix with missing data: the called count of every row (u32 [V]) in place of a
+    // called plane -- every consumer only ever reduces the group's called bits of a row to this one number
+    uint32_t *cnt;
 };
 
 __device__ __forceinline__ uint32_t fm_compress32(uint32_t x, const uint4 p0, const uint4 p1) {
@@ -228,8 +250,7 @@ fm_k_repack_rows(const uint8_t *__restrict__ data, size_t data_bytes, const uint
         const uint32_t rw = (uint32_t)((stride + 31) >> 5);
         uint32_t *arow = reinterpret_cast<uint32_t *>(rowb + row_buf_bytes + bit_buf_bytes);
         uint32_t *crow = arow + rw + 1;
-        uint32_t *outb = crow + rw + 1;  // 2 x out_cap words: one group's plane rows while they are assembled
-        const uint32_t out_cap = (uint32_t)((stride + 127) >> 7) * 4u + 4u;  // + one padding word (16-byte granule) per row
+        uint32_t *outb = crow + rw + 1;  // one group's allele plane row while it is assembled
         if (pk.a) {  // packed rows: the full-row bit words arrive ready-made
             const size_t r0 = (size_t)(v - v_base) * pk.rw;
             const uint32_t tail = (uint32_t)stride & 31u;
@@ -354,15 +375,14 @@ fm_k_repack_rows(const uint8_t *__restrict__ data, size_t data_bytes, const uint
             const RepackGroup G = groups[gi];
             const uint32_t words = G.wq * 4 + G.tw;  // tw != 0 only on the plan path
             if (G.n_bits == 1 && G.plan) {
-                uint32_t *oa = outb, *oc = outb + out_cap;
-                for (uint32_t i = lane; i < words; i += 32) {
-                    oa[i] = 0;
-                    oc[i] = 0;
-                }
+                uint32_t *oa = outb;
+                for (uint32_t i = lane; i < words; i += 32) oa[i] = 0;
                 __syncwarp();
+                uint32_t nc = 0;  // called members of this lane's entries
                 for (uint32_t e = lane; e < G.n_ent; e += 32) {
                     const uint4 p0 = __ldg(G.plan + 2 * e), p1 = __ldg(G.plan + 2 * e + 1);
                     const uint32_t cw = crow[p0.x];
+                    nc += __popc(cw & p0.y);
                     const uint32_t xa = fm_compress32(arow[p0.x] & cw, p0, p1);
                     const uint32_t sh = p0.z & 31u, wi = p0.z >> 5;
                     // straight-line: the fragment's low part and the part that spills into the next word (zero when
@@ -372,82 +392,20 @@ fm_k_repack_rows(const uint8_t *__restrict__ data, size_t data_bytes, const uint
                     // The word after the row's last one is padding (repack_warp_smem).
                     atomicOr(oa + wi, xa << sh);
                     atomicOr(oa + wi + 1, __funnelshift_l(xa, 0u, sh));
-                    if (G.called) {
-                        const uint32_t xc = fm_compress32(cw, p0, p1);
-                        atomicOr(oc + wi, xc << sh);
-                        atomicOr(oc + wi + 1, __funnelshift_l(xc, 0u, sh));
-                    }
+                }
+                if (G.cnt) {  // warp-uniform
+                    nc = fm_warp_sum_u(nc);
+                    if (lane == 0) G.cnt[v] = nc;
                 }
                 __syncwarp();
                 const uint32_t fw = G.wq * 4;
-                for (uint32_t i = lane; i < fw; i += 32) {
-                    const size_t o = (size_t)v * fw + i;
-                    G.allele[o] = oa[i];
-                    if (G.called) G.called[o] = oc[i];
-                }
-                if (lane < G.tw) {  // the row's last n % 128 haplotypes
-                    const size_t o = (size_t)v * G.tw + lane;
-                    G.tail_a[o] = oa[fw + lane];
-                    if (G.called) G.tail_c[o] = oc[fw + lane];
-                }
+                for (uint32_t i = lane; i < fw; i += 32) G.allele[(size_t)v * fw + i] = oa[i];
+                if (lane < G.tw) G.tail_a[(size_t)v * G.tw + lane] = oa[fw + lane];  // the row's last n % 128 haplotypes
                 __syncwarp();
                 continue;
             }
             if (MODE != 0) continue;  // direct / packed launches only carry plan groups (checked on the host)
-            if (G.n_bits == 1) {
-                // biallelic fast path: words whose 32 haplotypes all exist run a branch-free loop
-                // (one offset load, one bit test, one byte test, two ballots per word)
-                const uint32_t full_words = G.n >> 5;
-                for (uint32_t wb = 0; wb < words; wb += 32) {
-                    uint32_t my_a = 0, my_c = 0;
-                    const uint32_t lim = min(32u, words - wb);
-                    const uint32_t nfull = full_words > wb ? min(lim, full_words - wb) : 0u;
-                    const uint32_t *offp = G.off + (size_t)wb * 32 + lane;
-#pragma unroll 8
-                    for (uint32_t i = 0; i < nfull; ++i) {
-                        const uint32_t o = __ldg(offp + i * 32);
-                        const uint32_t cell = rb[o];
-                        uint32_t cbit = 1u;
-                        if (missing) {
-                            const uint32_t r = brel + o;
-                            cbit = ~(bits32[r >> 5] >> (r & 31u)) & 1u;
-                        } else if (in_band) {
-                            cbit = cell < 0x80u ? 1u : 0u;
-                        }
-                        const uint32_t abit = cbit & (cell != 0 ? 1u : 0u);
-                        const uint32_t wc = __ballot_sync(FULL, cbit);
-                        const uint32_t wa = __ballot_sync(FULL, abit);
-                        my_c = (i == lane) ? wc : my_c;
-                        my_a = (i == lane) ? wa : my_a;
-                    }
-                    for (uint32_t i = nfull; i < lim; ++i) {  // the partial word and the zero padding
-                        const uint32_t k = (wb + i) * 32 + lane;
-                        uint32_t cbit = 0u, abit = 0u;
-                        if (k < G.n) {
-                            const uint32_t o = __ldg(G.off + k);
-                            const uint32_t cell = rb[o];
-                            cbit = 1u;
-                            if (missing) {
-                                const uint32_t r = brel + o;
-                                cbit = ~(bits32[r >> 5] >> (r & 31u)) & 1u;
-                            } else if (in_band) {
-                                cbit = cell < 0x80u ? 1u : 0u;
-                            }
-                            abit = cbit & (cell != 0 ? 1u : 0u);
-                        }
-                        const uint32_t wc = __ballot_sync(FULL, cbit);
-                        const uint32_t wa = __ballot_sync(FULL, abit);
-                        my_c = (i == lane) ? wc : my_c;
-                        my_a = (i == lane) ? wa : my_a;
-                    }
-                    if (lane < lim) {
-                        const size_t o = (size_t)v * words + wb + lane;
-                        G.allele[o] = my_a;
-                        if (G.called) G.called[o] = my_c;
-                    }
-                }
-                continue;
-            }
+            if (G.n_bits == 1) continue;  // every biallelic group of a staged row takes its compress plan
             for (uint32_t wb = 0; wb < words; wb += 32) {  // multi-allelic: bit b of the allele index -> plane b
                 uint32_t my_a[4] = {0, 0, 0, 0}, my_c = 0;
                 const uint32_t lim = min(32u, words - wb);
@@ -643,40 +601,39 @@ fm_k_synth(uint8_t *__restrict__ data, uint64_t *__restrict__ missing, uint64_t 
 }
 
 // ------------------------------------------------------------------------------ plane pass
+// A biallelic group's plane pass input.  The allele plane is masked with "called" (allele bit = non-zero allele and
+// called), so alt = popc(allele row); the called count n comes from `cnt`, filled by K1 when the rows are repacked.
 struct GroupPlanes {
     const uint4 *allele;
-    const uint4 *called;  // nullptr => every member haplotype is called at every site
+    const uint32_t *cnt;  // [V] called members per site; nullptr => every member haplotype is called (n = cap)
     uint32_t wq;          // uint4 per row
     uint32_t cap;         // haplotype capacity (offsets.len())
-    // tail layout: the last cap % 128 haplotypes of every row live in tw u32 words per row (tail_a [V][tw], tail_c
-    // likewise) instead of a padded 16-byte word; the streaming pass reads them in the batch epilogue (lane = site).
+    // tail layout: the last cap % 128 haplotypes of every row live in tw u32 words per row (tail_a [V][tw]) instead
+    // of a padded 16-byte word; the streaming pass reads them in the batch epilogue (lane = site).
     // Cuts the padding of a 3463 + 1545 haplotype pair from 4.8 % of the plane bytes to 1 %.
-    const uint32_t *tail_a, *tail_c;
+    const uint32_t *tail_a;
     uint32_t tw;
 };
 
-// tail words of this lane's site, requested at the start of a batch and consumed in its epilogue
+// tail words and called count of this lane's site, requested at the start of a batch (one coalesced load per
+// array and warp) and consumed in its epilogue
 struct TailRegs {
-    uint32_t a[3], c[3];
+    uint32_t a[3], n;
 };
-__device__ __forceinline__ void fm_tail_load(const GroupPlanes &g, uint32_t v, uint32_t n_sites_total, bool hc, TailRegs &t) {
+__device__ __forceinline__ void fm_tail_load(const GroupPlanes &g, uint32_t v, uint32_t n_sites_total, TailRegs &t) {
 #pragma unroll
-    for (uint32_t k = 0; k < 3; ++k) {
-        t.a[k] = 0;
-        t.c[k] = 0;
-    }
-    if (g.tw && v < n_sites_total) {
+    for (uint32_t k = 0; k < 3; ++k) t.a[k] = 0;
+    t.n = g.cap;
+    if (v < n_sites_total) {
+        if (g.cnt) t.n = __ldg(g.cnt + v);
 #pragma unroll
         for (uint32_t k = 0; k < 3; ++k)
-            if (k < g.tw) {
-                t.a[k] = __ldg(g.tail_a + (size_t)v * g.tw + k);
-                if (hc) t.c[k] = __ldg(g.tail_c + (size_t)v * g.tw + k);
-            }
+            if (k < g.tw) t.a[k] = __ldg(g.tail_a + (size_t)v * g.tw + k);
     }
 }
-__device__ __forceinline__ void fm_tail_add(const TailRegs &t, uint32_t &alt, uint32_t &cnt, bool hc) {
+__device__ __forceinline__ void fm_tail_add(const TailRegs &t, uint32_t &alt, uint32_t &cnt) {
     alt += __popc(t.a[0]) + __popc(t.a[1]) + __popc(t.a[2]);
-    if (hc) cnt += __popc(t.c[0]) + __popc(t.c[1]) + __popc(t.c[2]);
+    cnt = t.n;
 }
 
 struct PassGeom {
@@ -746,18 +703,6 @@ __device__ __forceinline__ bool fm_in_sorted(const int64_t *a, uint32_t n, int64
             hi = mid;
     }
     return lo < n && a[lo] == x;
-}
-
-__device__ __forceinline__ double fm_warp_sum(double v) {
-    // fixed-shape butterfly: identical association for every batch
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-__device__ __forceinline__ uint32_t fm_warp_sum_u(uint32_t v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
 }
 
 // Mask / filtered-position lookup hoisted out of the streaming kernel: one bit per site
@@ -913,12 +858,12 @@ struct PassParams {
 };
 
 // Specialisations: NG groups, LG = log2(lanes per site) (LG == 5 is the column-chunked mode for
-// rows wider than a pipeline step), HC = planes carry a called bitplane.
+// rows wider than a pipeline step).
 //
 // Non-chunked geometry: a pipeline step holds `rounds` x SPS consecutive sites (SPS = 32/LPS);
 // in every round LPS consecutive lanes read consecutive uint4 of one row, so a quarter-warp
 // always touches one contiguous 128-byte span (bank-conflict free without padding).
-template <int NG, int LG, bool HC>
+template <int NG, int LG>
 __global__ void __launch_bounds__(kWarpsPerCta * 32, 1)
 fm_k_plane_pass(const __grid_constant__ PassParams<NG> P) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
@@ -928,7 +873,6 @@ fm_k_plane_pass(const __grid_constant__ PassParams<NG> P) {
     constexpr uint32_t LPS = 1u << LG;       // lanes per site
     constexpr uint32_t SPS = 32u >> LG;      // sites per round
     constexpr bool CHUNKED = (LG == 5);
-    constexpr uint32_t NPL = HC ? 2u : 1u;   // planes per group
     constexpr uint32_t FULL = 0xffffffffu;
 
     const uint32_t lane = threadIdx.x & 31;
@@ -995,7 +939,7 @@ fm_k_plane_pass(const __grid_constant__ PassParams<NG> P) {
             for (int g = 0; g < NG; ++g) {
                 const uint32_t w = P.g[g].wq;
                 bytes[g] = (v0 < n_sites_total && c0 < w) ? min(cq, w - c0) * 16u : 0u;
-                total += bytes[g] * NPL;
+                total += bytes[g];
             }
             if (total == 0) {
                 asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
@@ -1009,12 +953,8 @@ fm_k_plane_pass(const __grid_constant__ PassParams<NG> P) {
                     asm volatile(
                         "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::
                             "r"(dst), "l"(P.g[g].allele + src), "r"(bytes[g]), "r"(bar) : "memory");
-                    if constexpr (HC)
-                        asm volatile(
-                            "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::
-                                "r"(dst + cq * 16u), "l"(P.g[g].called + src), "r"(bytes[g]), "r"(bar) : "memory");
                 }
-                dst += cq * 16u * NPL;
+                dst += cq * 16u;
             }
         } else {
             const uint32_t v0 = b * 32 + k * step_sites;
@@ -1025,7 +965,7 @@ fm_k_plane_pass(const __grid_constant__ PassParams<NG> P) {
             }
             uint32_t total = 0;
 #pragma unroll
-            for (int g = 0; g < NG; ++g) total += nsites * wq16[g] * NPL;
+            for (int g = 0; g < NG; ++g) total += nsites * wq16[g];
             asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(total) : "memory");
 #pragma unroll
             for (int g = 0; g < NG; ++g) {
@@ -1036,13 +976,7 @@ fm_k_plane_pass(const __grid_constant__ PassParams<NG> P) {
                     "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::
                         "r"(dst), "l"(reinterpret_cast<const uint8_t *>(P.g[g].allele) + off), "r"(bytes), "r"(bar)
                     : "memory");
-                if constexpr (HC)
-                    asm volatile(
-                        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::
-                            "r"(dst + slot), "l"(reinterpret_cast<const uint8_t *>(P.g[g].called) + off), "r"(bytes),
-                        "r"(bar)
-                        : "memory");
-                dst += slot * NPL;
+                dst += slot;
             }
         }
     };
@@ -1068,11 +1002,10 @@ fm_k_plane_pass(const __grid_constant__ PassParams<NG> P) {
     for (uint32_t s = 0; s < n_stages; ++s) issue_next();
     __syncwarp();
 
-    // per-site totals of this lane's batch site; packed alt | called << 16 when HC (rows of the
-    // non-chunked modes hold < 65536 haplotypes), plain counts in chunked mode
-    uint32_t site_a[NG], site_c[NG], acc_a[NG], acc_c[NG];
+    // alt count of this lane's batch site
+    uint32_t site_a[NG], acc_a[NG];
 #pragma unroll
-    for (int g = 0; g < NG; ++g) site_a[g] = site_c[g] = acc_a[g] = acc_c[g] = 0;
+    for (int g = 0; g < NG; ++g) site_a[g] = acc_a[g] = 0;
 
     const uint32_t slot_in_round = lane >> LG;
     const uint32_t phase = lane & (LPS - 1);
@@ -1087,7 +1020,7 @@ fm_k_plane_pass(const __grid_constant__ PassParams<NG> P) {
 #pragma unroll
         for (int g = 0; g < NG; ++g) {
             plane_off[g] = acc;
-            acc += (CHUNKED ? cq * 16u : step_sites * wq16[g]) * NPL;
+            acc += CHUNKED ? cq * 16u : step_sites * wq16[g];
             const uint32_t w = P.g[g].wq;
             const uint32_t nit = (w + LPS - 1) / LPS;
             nit_full[g] = nit - 1;
@@ -1103,7 +1036,7 @@ fm_k_plane_pass(const __grid_constant__ PassParams<NG> P) {
         const uint32_t b = G.b_lo + bl;
         TailRegs tails[NG];
 #pragma unroll
-        for (int g = 0; g < NG; ++g) fm_tail_load(P.g[g], b * 32 + lane, n_sites_total, HC, tails[g]);
+        for (int g = 0; g < NG; ++g) fm_tail_load(P.g[g], b * 32 + lane, n_sites_total, tails[g]);
         for (uint32_t k = 0; k < spb; ++k) {
             {
                 const uint32_t bar = bar_base + 8u * stage;
@@ -1126,8 +1059,7 @@ fm_k_plane_pass(const __grid_constant__ PassParams<NG> P) {
                     for (int g = 0; g < NG; ++g) {
                         const uint32_t w16 = wq16[g];
                         const uint32_t ra = sbase + plane_off[g] + site_local * w16;
-                        const uint32_t pb = step_sites * w16;  // distance allele -> called plane
-                        uint32_t a = 0, c = 0;
+                        uint32_t a = 0;
                         if (live && !(G.debug & 2u)) {
                             // columns phase, phase+LPS, ...: the first nit-1 are inside the row for
                             // every lane, only the last one needs a bound check
@@ -1135,27 +1067,14 @@ fm_k_plane_pass(const __grid_constant__ PassParams<NG> P) {
                             const uint32_t nfull = nit_full[g];
 #pragma unroll 2
                             for (uint32_t j = 0; j < nfull; ++j) {
-                                const uint4 xa = fm_lds128(p);
-                                a += fm_popc4(xa);
-                                if constexpr (HC) {
-                                    const uint4 xc = fm_lds128(p + pb);
-                                    c += fm_popc4(xc);
-                                }
+                                a += fm_popc4(fm_lds128(p));
                                 p += LPS * 16u;
                             }
-                            if (phase < last_cols[g]) {
-                                const uint4 xa = fm_lds128(p);
-                                a += fm_popc4(xa);
-                                if constexpr (HC) {
-                                    const uint4 xc = fm_lds128(p + pb);
-                                    c += fm_popc4(xc);
-                                }
-                            }
+                            if (phase < last_cols[g]) a += fm_popc4(fm_lds128(p));
                         }
-                        uint32_t ac = HC ? (a | (c << 16)) : a;
 #pragma unroll
-                        for (uint32_t o = LPS >> 1; o > 0; o >>= 1) ac += __shfl_xor_sync(FULL, ac, o);
-                        const uint32_t t = __shfl_sync(FULL, ac, xfer_from);
+                        for (uint32_t o = LPS >> 1; o > 0; o >>= 1) a += __shfl_xor_sync(FULL, a, o);
+                        const uint32_t t = __shfl_sync(FULL, a, xfer_from);
                         if (xfer_round == k * rounds + r) site_a[g] = t;
                     }
                 };
@@ -1179,21 +1098,12 @@ fm_k_plane_pass(const __grid_constant__ PassParams<NG> P) {
                     const uint32_t ra = sbase + plane_off[g];
                     if (live) {
 #pragma unroll 2
-                        for (uint32_t u = lane * 16u; u < cols16; u += 512u) {
-                            acc_a[g] += fm_popc4(fm_lds128(ra + u));
-                            if constexpr (HC) acc_c[g] += fm_popc4(fm_lds128(ra + cq * 16u + u));
-                        }
+                        for (uint32_t u = lane * 16u; u < cols16; u += 512u) acc_a[g] += fm_popc4(fm_lds128(ra + u));
                     }
                     if (ck == n_chunks - 1) {
                         const uint32_t ta = fm_warp_sum_u(acc_a[g]);
-                        uint32_t tc = 0;
-                        if constexpr (HC) tc = fm_warp_sum_u(acc_c[g]);
-                        if (lane == site_in_batch) {
-                            site_a[g] = ta;
-                            site_c[g] = tc;
-                        }
+                        if (lane == site_in_batch) site_a[g] = ta;
                         acc_a[g] = 0;
-                        acc_c[g] = 0;
                     }
                 }
             }
@@ -1207,14 +1117,8 @@ fm_k_plane_pass(const __grid_constant__ PassParams<NG> P) {
             uint32_t alt[NG], cnt[NG];
 #pragma unroll
             for (int g = 0; g < NG; ++g) {
-                if constexpr (CHUNKED) {
-                    alt[g] = site_a[g];
-                    cnt[g] = HC ? site_c[g] : P.g[g].cap;
-                } else {
-                    alt[g] = HC ? (site_a[g] & 0xffffu) : site_a[g];
-                    cnt[g] = HC ? (site_a[g] >> 16) : P.g[g].cap;
-                }
-                fm_tail_add(tails[g], alt[g], cnt[g], HC);
+                alt[g] = site_a[g];
+                fm_tail_add(tails[g], alt[g], cnt[g]);
             }
             const uint32_t v = b * 32 + lane;
             const bool valid = (v >= G.v_lo) && (v < G.v_hi);
@@ -1277,7 +1181,7 @@ struct SeqParams {
     PassGeom geom;  // lps, n_stages, stage_bytes (max over groups), warps, site range, scheduler counters
 };
 
-template <int LG, bool HC>
+template <int LG>
 __global__ void __launch_bounds__(kWarpsPerCta * 32, 1)
 fm_k_plane_pass_seq(const __grid_constant__ SeqParams P) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
@@ -1286,7 +1190,6 @@ fm_k_plane_pass_seq(const __grid_constant__ SeqParams P) {
     static_assert(LG < 5, "column-chunked rows take the per-group kernel");
     constexpr uint32_t LPS = 1u << LG;
     constexpr uint32_t SPS = 32u >> LG;
-    constexpr uint32_t NPL = HC ? 2u : 1u;
     constexpr uint32_t FULL = 0xffffffffu;
 
     const uint32_t lane = threadIdx.x & 31;
@@ -1339,18 +1242,12 @@ fm_k_plane_pass_seq(const __grid_constant__ SeqParams P) {
             return;
         }
         const uint32_t bytes = nsites * iss_w16;
-        const uint32_t slot = iss_step_sites * iss_w16;
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes * NPL) : "memory");
+        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
         const size_t off = (size_t)v0 * iss_w16;
         const GroupPlanes &gp = P.seg[iss_seg].g;
         asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
                      "l"(reinterpret_cast<const uint8_t *>(gp.allele) + off), "r"(bytes), "r"(bar)
                      : "memory");
-        if constexpr (HC)
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                             dst + slot),
-                         "l"(reinterpret_cast<const uint8_t *>(gp.called) + off), "r"(bytes), "r"(bar)
-                         : "memory");
     };
     auto issue_next = [&]() {
         if (iss_k == iss_spb) {
@@ -1395,11 +1292,10 @@ fm_k_plane_pass_seq(const __grid_constant__ SeqParams P) {
         const uint32_t step_sites = SPS * rounds, spb = LPS / rounds;
         const uint32_t nit = (w + LPS - 1) / LPS;
         const uint32_t nfull = nit - 1, last_cols = w - nfull * LPS;
-        const uint32_t pb = step_sites * w16;  // distance allele -> called plane inside a stage
         const uint32_t b = G.b_lo + bl;
-        uint32_t site_ac = 0;
+        uint32_t site_a = 0;
         TailRegs tails;
-        fm_tail_load(S.g, b * 32 + lane, n_sites_total, HC, tails);
+        fm_tail_load(S.g, b * 32 + lane, n_sites_total, tails);
         for (uint32_t k = 0; k < spb; ++k) {
             {
                 const uint32_t bar = bar_base + 8u * stage;
@@ -1418,25 +1314,20 @@ fm_k_plane_pass_seq(const __grid_constant__ SeqParams P) {
                 const uint32_t site_local = r * SPS + slot_in_round;
                 const bool live = (v0 + site_local) < n_sites_total;
                 const uint32_t ra = sbase + site_local * w16;
-                uint32_t a = 0, c = 0;
+                uint32_t a = 0;
                 if (live) {
                     uint32_t p = ra + phase * 16u;
 #pragma unroll 2
                     for (uint32_t j = 0; j < nfull; ++j) {
                         a += fm_popc4(fm_lds128(p));
-                        if constexpr (HC) c += fm_popc4(fm_lds128(p + pb));
                         p += LPS * 16u;
                     }
-                    if (phase < last_cols) {
-                        a += fm_popc4(fm_lds128(p));
-                        if constexpr (HC) c += fm_popc4(fm_lds128(p + pb));
-                    }
+                    if (phase < last_cols) a += fm_popc4(fm_lds128(p));
                 }
-                uint32_t ac = HC ? (a | (c << 16)) : a;
 #pragma unroll
-                for (uint32_t o = LPS >> 1; o > 0; o >>= 1) ac += __shfl_xor_sync(FULL, ac, o);
-                const uint32_t t = __shfl_sync(FULL, ac, xfer_from);
-                if (xfer_round == k * rounds + r) site_ac = t;
+                for (uint32_t o = LPS >> 1; o > 0; o >>= 1) a += __shfl_xor_sync(FULL, a, o);
+                const uint32_t t = __shfl_sync(FULL, a, xfer_from);
+                if (xfer_round == k * rounds + r) site_a = t;
             };
             if (rounds == 1) {
                 round_body(0);
@@ -1453,9 +1344,8 @@ fm_k_plane_pass_seq(const __grid_constant__ SeqParams P) {
         }
         // ---- batch epilogue: lane i <-> site 32b + i
         {
-            uint32_t alt = HC ? (site_ac & 0xffffu) : site_ac;
-            uint32_t cnt = HC ? (site_ac >> 16) : S.g.cap;
-            fm_tail_add(tails, alt, cnt, HC);
+            uint32_t alt = site_a, cnt;
+            fm_tail_add(tails, alt, cnt);
             const uint32_t v = b * 32 + lane;
             const bool valid = (v >= G.v_lo) && (v < G.v_hi);
             double pi_part = 0.0;
@@ -1507,7 +1397,7 @@ struct TabParams {
     uint32_t inline_prefix[2];
 };
 
-template <int LG, bool HC>
+template <int LG>
 __global__ void __launch_bounds__(kWarpsPerCta * 32, 1)
 fm_k_plane_pass_tab(const __grid_constant__ TabParams P) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
@@ -1516,7 +1406,6 @@ fm_k_plane_pass_tab(const __grid_constant__ TabParams P) {
     static_assert(LG < 5, "column-chunked rows take the per-group kernel");
     constexpr uint32_t LPS = 1u << LG;
     constexpr uint32_t SPS = 32u >> LG;
-    constexpr uint32_t NPL = HC ? 2u : 1u;
     constexpr uint32_t FULL = 0xffffffffu;
 
     const uint32_t lane = threadIdx.x & 31;
@@ -1570,7 +1459,7 @@ fm_k_plane_pass_tab(const __grid_constant__ TabParams P) {
     // ---- issue side: context of the (unit batch, group) whose steps are being issued
     uint32_t iss_ring = 0, iss_k = 0, iss_spb = 0, iss_stage = 0, iss_batch = 0;
     uint32_t iss_w16 = 0, iss_step_sites = 1, iss_g = 0, iss_unit = 0, iss_b = 0, iss_nst = 0;
-    const uint4 *iss_allele = nullptr, *iss_called = nullptr;
+    const uint4 *iss_allele = nullptr;
     bool iss_live = false;
     auto load_iss_seg = [&]() {
         const TabSeg &S = segs[iss_unit * gpu + iss_g];
@@ -1579,7 +1468,6 @@ fm_k_plane_pass_tab(const __grid_constant__ TabParams P) {
         iss_spb = LPS / S.rounds;
         iss_nst = S.n_sites_total;
         iss_allele = S.g.allele;
-        iss_called = S.g.called;
     };
     auto issue = [&](uint32_t stage) {  // lane 0 only
         const uint32_t bar = bar_base + 8u * stage;
@@ -1591,17 +1479,11 @@ fm_k_plane_pass_tab(const __grid_constant__ TabParams P) {
             return;
         }
         const uint32_t bytes = nsites * iss_w16;
-        const uint32_t slot = iss_step_sites * iss_w16;
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes * NPL) : "memory");
+        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
         const size_t off = (size_t)v0 * iss_w16;
         asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
                      "l"(reinterpret_cast<const uint8_t *>(iss_allele) + off), "r"(bytes), "r"(bar)
                      : "memory");
-        if constexpr (HC)
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                             dst + slot),
-                         "l"(reinterpret_cast<const uint8_t *>(iss_called) + off), "r"(bytes), "r"(bar)
-                         : "memory");
     };
     auto issue_next = [&]() {
         if (iss_k == iss_spb) {
@@ -1654,14 +1536,13 @@ fm_k_plane_pass_tab(const __grid_constant__ TabParams P) {
             const uint32_t step_sites = SPS * rounds, spb = LPS / rounds;
             const uint32_t nit = (w + LPS - 1) / LPS;
             const uint32_t nfull = nit - 1, last_cols = w - nfull * LPS;
-            const uint32_t pb = step_sites * w16;
             const uint32_t nst = S.n_sites_total;
             b = S.b_lo + bl;
             u_vlo = S.v_lo;
             u_vhi = S.v_hi;
-            uint32_t site_ac = 0;
+            uint32_t site_a = 0;
             TailRegs tails;
-            fm_tail_load(S.g, b * 32 + lane, nst, HC, tails);
+            fm_tail_load(S.g, b * 32 + lane, nst, tails);
             for (uint32_t k = 0; k < spb; ++k) {
                 {
                     const uint32_t bar = bar_base + 8u * stage;
@@ -1680,25 +1561,20 @@ fm_k_plane_pass_tab(const __grid_constant__ TabParams P) {
                     const uint32_t site_local = r * SPS + slot_in_round;
                     const bool live = (v0 + site_local) < nst;
                     const uint32_t ra = sbase + site_local * w16;
-                    uint32_t a = 0, c = 0;
+                    uint32_t a = 0;
                     if (live) {
                         uint32_t p = ra + phase * 16u;
 #pragma unroll 2
                         for (uint32_t j = 0; j < nfull; ++j) {
                             a += fm_popc4(fm_lds128(p));
-                            if constexpr (HC) c += fm_popc4(fm_lds128(p + pb));
                             p += LPS * 16u;
                         }
-                        if (phase < last_cols) {
-                            a += fm_popc4(fm_lds128(p));
-                            if constexpr (HC) c += fm_popc4(fm_lds128(p + pb));
-                        }
+                        if (phase < last_cols) a += fm_popc4(fm_lds128(p));
                     }
-                    uint32_t ac = HC ? (a | (c << 16)) : a;
 #pragma unroll
-                    for (uint32_t o = LPS >> 1; o > 0; o >>= 1) ac += __shfl_xor_sync(FULL, ac, o);
-                    const uint32_t t = __shfl_sync(FULL, ac, xfer_from);
-                    if (xfer_round == k * rounds + r) site_ac = t;
+                    for (uint32_t o = LPS >> 1; o > 0; o >>= 1) a += __shfl_xor_sync(FULL, a, o);
+                    const uint32_t t = __shfl_sync(FULL, a, xfer_from);
+                    if (xfer_round == k * rounds + r) site_a = t;
                 };
                 if (rounds == 1) {
                     round_body(0);
@@ -1714,9 +1590,8 @@ fm_k_plane_pass_tab(const __grid_constant__ TabParams P) {
                 parity ^= (stage == 0);
             }
             // ---- group epilogue: lane i <-> site 32b + i (counts, summary partials, optional tracks)
-            uint32_t alt = HC ? (site_ac & 0xffffu) : site_ac;
-            uint32_t cnt = HC ? (site_ac >> 16) : S.g.cap;
-            fm_tail_add(tails, alt, cnt, HC);
+            uint32_t alt = site_a, cnt;
+            fm_tail_add(tails, alt, cnt);
             if (g == 0) {
                 alt_g0 = alt;
                 cnt_g0 = cnt;

@@ -574,9 +574,11 @@ typedef struct {
     float plane_ms_avg;
     uint64_t plane_launches;       /* plane-pass launches inside the timed region */
     uint64_t other_launches;       /* partial-reduction launches inside the timed region */
-    uint64_t plane_bytes_per_step; /* algorithmic bytes: plane rows read + per-site outputs written */
+    uint64_t plane_bytes_per_step; /* bytes a step moves: per group and site the allele plane row (16-byte words +
+                                    * tail words) and, with missing data, the 4-byte called count read, plus the
+                                    * 16 B of pi / theta tracks written (mode 1) */
     float group_ms_avg[8];         /* mean plane-pass duration per listed group (first 8) */
-    uint64_t group_bytes[8];       /* algorithmic bytes of one launch per listed group */
+    uint64_t group_bytes[8];       /* the same bytes for each listed group */
     float comm_ms_avg;             /* mean duration of the fused fold + peer exchange kernel (incl. waiting) */
     /* region totals of the last timed step, per listed group (first 8): this rank's, and -- with a
      * communicator -- the exchanged rank-ordered sums (parity check of the run) */

@@ -2,7 +2,7 @@
 """K1 (u8 rows -> group bitplanes) on a device-resident matrix: the two orientation groups of
 BASELINE configs[1] (every haplotype belongs to one of them) repacked by ONE launch through the
 streaming-ingest-free path (fm_group_create per group = one launch each) and timed by the library's
-own events (fm_timings.repack_ms).  Set FM_REPACK_BALLOT=1 for the ballot-gather version.
+own events (fm_timings.repack_ms).
 usage: bench_repack.py [sites]"""
 import ctypes as C
 import json
@@ -25,8 +25,7 @@ def main():
     S = 2504
     dev = torch.device("cuda:0")
     L = _lib.lib()
-    out = {"what": "K1 repack, two orientation groups covering all 5008 haplotypes", "sites": V,
-           "ballot_version": bool(int(os.environ.get("FM_REPACK_BALLOT", "0")))}
+    out = {"what": "K1 repack, two orientation groups covering all 5008 haplotypes", "sites": V}
     for missing in (0.01, 0.0):
         m, pos, keep = matrix(L, V, S, 1_002_504, dev, missing)
         rng = np.random.default_rng(3)
