@@ -179,7 +179,7 @@ def cfg1_batched(L, _lib, device, peak, scale, n_regions=64):
     alg = n_regions * V * H / 8.0  # no missing data: one allele bit per genotype
     return entry("configs[0] x %d regions" % n_regions,
                  "segregating sites + pi + theta inputs (dense summary) of %d regions of %d sites x %d haplotypes in ONE "
-                 "launch (fm_groups_summary_batch -> fm_k_plane_pass_tab), no missing data" % (n_regions, V, H),
+                 "launch (fm_groups_summary_batch -> fm_k_plane_pass_seq), no missing data" % (n_regions, V, H),
                  dev_ms, alg, peak, n_regions * V * H,
                  {"wall_ms": wall_ms, "one_call_per_region_wall_ms": serial_ms, "regions": n_regions,
                   "timing": "CUDA events around the pass + fold inside the library (fm_timings.stats_ms)"})

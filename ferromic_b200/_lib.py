@@ -74,7 +74,7 @@ EXPORTS = [
     "fm_comm_destroy", "fm_hudson_pair_sharded", "fm_falsta_track", "fm_falsta_tracks", "fm_falsta_format_value", "fm_vcf_parse", "fm_vcf_parse_device", "fm_vcf_batch_info",
     "fm_vcf_batch_variants", "fm_vcf_batch_genotypes", "fm_vcf_batch_positions", "fm_vcf_batch_errors", "fm_vcf_batch_matrix", "fm_vcf_batch_matrix_packed",
     "fm_vcf_batch_release", "fm_synth_fill", "fm_timings_reset", "fm_timings_get", "fm_bench_diversity",
-    "fm_bench_hudson", "fm_pairwise_differences",
+    "fm_pairwise_differences",
 ]
 
 _lib = None
@@ -180,7 +180,6 @@ def lib() -> C.CDLL:
     L.fm_comm_set_timeout_ms.argtypes = [vp, u64]
     L.fm_comm_destroy.argtypes = [vp]
     L.fm_hudson_pair_sharded.argtypes = [vp, vp, i64, sz, sz, vp, C.POINTER(HudsonOutcome), C.POINTER(HudsonSums)]
-    L.fm_bench_hudson.argtypes = [vp, vp, C.c_int, C.POINTER(BenchResult)]
     L.fm_pairwise_differences.argtypes = [vp, sz, vp, vp, vp, vp, sz, C.POINTER(sz)]
     for name in EXPORTS:
         fn = getattr(L, name)

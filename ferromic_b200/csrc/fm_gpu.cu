@@ -25,6 +25,7 @@
 #include <cstring>
 #include <limits>
 #include <map>
+#include <set>
 #include <memory>
 #include <mutex>
 #include <string>
@@ -713,64 +714,46 @@ uint32_t env_u32(const char *name, uint32_t dflt) {
     return x > 0 ? (uint32_t)x : dflt;
 }
 
-fm::PassGeom make_geom(const fm_group *const *gs, int ng, uint32_t v_lo, uint32_t v_hi) {
+// batches [b_lo, b_lo + n_batches) of the sites [v_lo, v_hi) (batch b = sites [32b, 32b+32))
+fm::PassGeom batch_range(uint32_t v_lo, uint32_t v_hi) {
     fm::PassGeom G{};
-    uint32_t row_bytes = 0, max_wq = 0;
-    for (int i = 0; i < ng; ++i) {
-        row_bytes += gs[i]->wq * 16u;
-        max_wq = std::max(max_wq, gs[i]->wq);
-    }
-    static const uint32_t step_target = env_u32("FM_STEP_BYTES", fm::kStepBytesTarget);
-    static const uint32_t base_warps = std::max(1u, std::min<uint32_t>(env_u32("FM_WARPS", fm::kWarpsPerCta), fm::kWarpsPerCta));
-    uint32_t warp_smem = (fm::kWarpsPerCta * fm::kWarpSmemBytes / base_warps) & ~127u;
-    static const uint32_t force_lg = env_u32("FM_FORCE_LG", 99);
-    G.warps = base_warps;
-    // rows wider than a warp's ring (biobank cohorts) are consumed in column chunks: fewer warps
-    // with deeper rings keep more bytes in flight per warp and amortise the per-step bookkeeping
-    static const uint32_t chunk_warps = std::min<uint32_t>(env_u32("FM_CHUNK_WARPS", 8), fm::kWarpsPerCta);
-    static const uint32_t chunk_step = env_u32("FM_CHUNK_STEP_BYTES", 14336);  // swept on B200: profiles/r01_sweep_chunked.txt
-    const bool chunked = (uint64_t)row_bytes * 2 > fm::kWarpSmemBytes;
-    uint32_t step_goal = step_target;
-    if (chunked) {
-        G.warps = chunk_warps;
-        warp_smem = (fm::kWarpsPerCta * fm::kWarpSmemBytes / chunk_warps) & ~127u;
-        step_goal = chunk_step;
-    }
-    G.warp_smem_bytes = warp_smem;
-    static const uint32_t dbg = env_u32("FM_DEBUG", 0);
-    G.debug = dbg;
-    // lanes per site: enough lanes to cover a row's uint4 columns (quarter-warps then read
-    // contiguous 128-byte spans), capped so that at least two pipeline stages fit.
-    uint32_t lg = 0;
-    while ((1u << lg) < std::min(max_wq, 8u)) ++lg;
-    if (force_lg <= 4) lg = force_lg;
-    while (lg < 5 && (uint64_t)row_bytes * (32u >> lg) * 2 > warp_smem) ++lg;
-    G.lps_log2 = lg;
-    G.lps = 1u << lg;
-    G.rounds = 1;
-    G.n_chunks = 1;
-    G.cq = max_wq;
-    uint32_t step_bytes;
-    if (lg < 5) {
-        // several rounds of (32/lps) sites per step while the step stays near the target size
-        const uint32_t round_bytes = row_bytes * (32u >> lg);
-        while (G.rounds * 2 <= G.lps && round_bytes * G.rounds * 2 <= step_target) G.rounds *= 2;
-        step_bytes = round_bytes * G.rounds;
-    } else {
-        if (row_bytes * 2 > warp_smem) {  // a single row does not fit twice: chunk its columns
-            G.cq = std::max(1u, step_goal / (16u * (uint32_t)ng));
-            G.n_chunks = (max_wq + G.cq - 1) / G.cq;
-        }
-        step_bytes = G.cq * 16u * (uint32_t)ng;
-    }
-    G.stage_bytes = (step_bytes + 127u) & ~127u;
-    G.n_stages = std::min<uint32_t>(fm::kMaxStages, warp_smem / G.stage_bytes);
-    if (G.n_stages < 2) fail(FM_ERR_INVALID_ARG, "internal: pipeline stage does not fit");
     G.v_lo = v_lo;
     G.v_hi = v_hi;
     G.b_lo = v_lo / 32;
     G.n_batches = v_hi > v_lo ? (v_hi + 31) / 32 - G.b_lo : 0;
-    G.n_sites_total = (uint32_t)gs[0]->m->V;
+    return G;
+}
+
+// Lanes per site (log2) of the row pass over rows of wq uint4: enough lanes to cover a row's uint4 columns
+// (quarter-warps then read contiguous 128-byte spans), raised until a step of 32 >> lg sites fits a warp's ring
+// twice.  5: the rows are too wide for the row pass and take the column-chunked pass.
+uint32_t row_lanes_log2(uint32_t wq) {
+    uint32_t lg = 0;
+    while ((1u << lg) < std::min(wq, 8u)) ++lg;
+    while (lg < 5 && (uint64_t)wq * 16u * (32u >> lg) * 2 > fm::kWarpSmemBytes) ++lg;
+    return lg;
+}
+
+// Geometry of the column-chunked pass over group g's rows (row_lanes_log2(g->wq) == 5).  Rows wider than a warp's
+// ring (biobank cohorts) are consumed in column chunks by fewer warps with deeper rings: more bytes in flight per
+// warp and the per-step bookkeeping amortised.
+fm::PassGeom make_geom(const fm_group *g, uint32_t v_lo, uint32_t v_hi) {
+    static const uint32_t chunk_warps = std::min<uint32_t>(env_u32("FM_CHUNK_WARPS", 8), fm::kWarpsPerCta);
+    static const uint32_t chunk_step = env_u32("FM_CHUNK_STEP_BYTES", 14336);  // swept on B200: profiles/r01_sweep_chunked.txt
+    fm::PassGeom G = batch_range(v_lo, v_hi);
+    const uint32_t row_bytes = g->wq * 16u;
+    G.warps = (uint64_t)row_bytes * 2 > fm::kWarpSmemBytes ? chunk_warps : fm::kWarpsPerCta;
+    G.warp_smem_bytes = (fm::kWarpsPerCta * fm::kWarpSmemBytes / G.warps) & ~127u;
+    G.cq = g->wq;
+    G.n_chunks = 1;
+    if ((uint64_t)row_bytes * 2 > G.warp_smem_bytes) {  // a single row does not fit twice: chunk its columns
+        G.cq = std::max(1u, chunk_step / 16u);
+        G.n_chunks = (g->wq + G.cq - 1) / G.cq;
+    }
+    G.stage_bytes = (G.cq * 16u + 127u) & ~127u;
+    G.n_stages = std::min<uint32_t>(fm::kMaxStages, G.warp_smem_bytes / G.stage_bytes);
+    if (G.n_stages < 2) fail(FM_ERR_INVALID_ARG, "internal: pipeline stage does not fit");
+    G.n_sites_total = (uint32_t)g->m->V;
     return G;
 }
 
@@ -798,223 +781,159 @@ struct CounterPool {
 };
 thread_local CounterPool t_counters;
 
-template <int NG, int LG>
-void launch_plane_pass_t(const fm::PassParams<NG> &P, uint32_t grid, size_t smem) {
-    CK(cudaFuncSetAttribute(fm::fm_k_plane_pass<NG, LG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    fm::fm_k_plane_pass<NG, LG><<<grid, P.geom.warps * 32, smem, stream()>>>(P);
-}
-
 // bytes a plane pass reads for one group and site: allele row, tail words, called count
 uint64_t plane_site_bytes(const fm::GroupPlanes &g) { return g.wq * 16u + g.tw * 4u + (g.cnt ? 4u : 0u); }
 
-template <int NG>
-void launch_plane_pass(fm::PassParams<NG> P, int device) {
-    if (P.geom.n_batches == 0) return;
+// Both plane passes use a whole SM's 224 KB of rings.  The dynamic shared-memory limit is a per-device function
+// attribute: set it once per (kernel, device).
+void allow_rings_once(const void *kern, int device) {
+    static std::mutex mu;
+    static std::set<std::pair<const void *, int>> done;
+    std::lock_guard<std::mutex> lk(mu);
+    if (!done.insert({kern, device}).second) return;
+    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(fm::kWarpsPerCta * fm::kWarpSmemBytes)));
+}
+
+void launch_chunked(fm::ChunkParams P, int device) {
+    const fm::PassGeom &G = P.geom;
+    if (G.n_batches == 0) return;
     P.geom.batch_counter = t_counters.take(device);
-    const size_t smem = (size_t)P.geom.warps * P.geom.warp_smem_bytes;
-    const uint32_t need = (P.geom.n_batches + P.geom.warps - 1) / P.geom.warps;
-    const uint32_t grid = std::min<uint32_t>((uint32_t)sm_count(device), need);
-    switch (P.geom.lps_log2) {
-        case 0: launch_plane_pass_t<NG, 0>(P, grid, smem); break;
-        case 1: launch_plane_pass_t<NG, 1>(P, grid, smem); break;
-        case 2: launch_plane_pass_t<NG, 2>(P, grid, smem); break;
-        case 3: launch_plane_pass_t<NG, 3>(P, grid, smem); break;
-        case 4: launch_plane_pass_t<NG, 4>(P, grid, smem); break;
-        default: launch_plane_pass_t<NG, 5>(P, grid, smem); break;
-    }
+    allow_rings_once(reinterpret_cast<const void *>(fm::fm_k_plane_pass_chunked), device);
+    const uint32_t grid = std::min<uint32_t>((uint32_t)sm_count(device), (G.n_batches + G.warps - 1) / G.warps);
+    fm::fm_k_plane_pass_chunked<<<grid, G.warps * 32, (size_t)G.warps * G.warp_smem_bytes, stream()>>>(P);
     CK(cudaGetLastError());
     g_launches++;
     t_tim.stats_launches++;
-    uint64_t bytes = 0;
-    for (int g = 0; g < NG; ++g) bytes += (uint64_t)(P.geom.v_hi - P.geom.v_lo) * plane_site_bytes(P.g[g]);
-    t_tim.stats_bytes = bytes;
+    t_tim.stats_bytes = (uint64_t)(G.v_hi - G.v_lo) * plane_site_bytes(P.g);
 }
 
 fm::GroupPlanes planes_of(const fm_group *g);
 
-// Several groups of one matrix over one site range in ONE persistent launch (fm_k_plane_pass_seq).
-// Returns false when the groups cannot share a launch (column-chunked rows, more than kMaxSeq
-// groups): the caller then launches per group.
-bool make_seq_params(fm_group *const *gs, size_t n, uint32_t v_lo, uint32_t v_hi, fm::SeqParams &P) {
-    if (n < 2 || n > (size_t)fm::kMaxSeq) return false;
-    static const uint32_t step_target = env_u32("FM_STEP_BYTES", fm::kStepBytesTarget);
-    static const uint32_t disable = env_u32("FM_NO_SEQ", 0);
-    if (disable) return false;
-    const uint32_t warp_smem = fm::kWarpSmemBytes;
-    uint32_t max_wq = 0;
-    for (size_t i = 0; i < n; ++i) {
-        if (gs[i]->m != gs[0]->m || gs[i]->n_bits != 1 || gs[i]->count_only) return false;
-        max_wq = std::max(max_wq, gs[i]->wq);
-    }
+// One launch of the row pass (fm_k_plane_pass_seq) over a list of segments (one per unit: independent (region, group)
+// units; pair units: Hudson pairs over shared sites), planned once and launchable any number of times.
+struct RowPlan {
+    fm::RowParams P{};
     uint32_t lg = 0;
-    while ((1u << lg) < std::min(max_wq, 8u)) ++lg;
-    while (lg < 5 && (uint64_t)max_wq * 16u * (32u >> lg) * 2 > warp_smem) ++lg;
-    if (lg >= 5) return false;
-    P = fm::SeqParams{};
-    P.n_seg = (uint32_t)n;
-    uint32_t max_step = 0;
-    for (size_t i = 0; i < n; ++i) {
-        const uint32_t round_bytes = gs[i]->wq * 16u * (32u >> lg);
-        uint32_t rounds = 1;
-        while (rounds * 2 <= (1u << lg) && round_bytes * rounds * 2 <= step_target) rounds *= 2;
-        P.seg[i].g = planes_of(gs[i]);
-        P.seg[i].rounds = rounds;
-        max_step = std::max(max_step, round_bytes * rounds);
-    }
-    fm::PassGeom &G = P.geom;
-    G.lps_log2 = lg;
-    G.lps = 1u << lg;
-    G.warps = fm::kWarpsPerCta;
-    G.warp_smem_bytes = warp_smem;
-    G.stage_bytes = (max_step + 127u) & ~127u;
-    G.n_stages = std::min<uint32_t>(fm::kMaxStages, warp_smem / G.stage_bytes);
-    if (G.n_stages < 2) return false;
-    G.v_lo = v_lo;
-    G.v_hi = v_hi;
-    G.b_lo = v_lo / 32;
-    G.n_batches = v_hi > v_lo ? (v_hi + 31) / 32 - G.b_lo : 0;  // per group
-    G.n_sites_total = (uint32_t)gs[0]->m->V;
-    return true;
-}
-
-template <int LG>
-void launch_plane_pass_seq_t(const fm::SeqParams &P, uint32_t grid, size_t smem) {
-    CK(cudaFuncSetAttribute(fm::fm_k_plane_pass_seq<LG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    fm::fm_k_plane_pass_seq<LG><<<grid, fm::kWarpsPerCta * 32, smem, stream()>>>(P);
-}
-
-void launch_plane_pass_seq(fm::SeqParams P, int device) {
-    if (P.geom.n_batches == 0) return;
-    P.geom.batch_counter = t_counters.take(device);
-    const size_t smem = (size_t)fm::kWarpsPerCta * P.geom.warp_smem_bytes;
-    const uint32_t total = P.geom.n_batches * P.n_seg;
-    const uint32_t grid = std::min<uint32_t>((uint32_t)sm_count(device), (total + fm::kWarpsPerCta - 1) / fm::kWarpsPerCta);
-#define FM_SEQ_CASE(L)                                   \
-    case L:                                              \
-        launch_plane_pass_seq_t<L>(P, grid, smem);       \
-        break;
-    switch (P.geom.lps_log2) {
-        FM_SEQ_CASE(0) FM_SEQ_CASE(1) FM_SEQ_CASE(2) FM_SEQ_CASE(3) FM_SEQ_CASE(4)
-        default: fail(FM_ERR_INVALID_ARG, "internal: bad sequential pass geometry");
-    }
-#undef FM_SEQ_CASE
-    CK(cudaGetLastError());
-    g_launches++;
-    t_tim.stats_launches++;
-    uint64_t bytes = 0;
-    for (uint32_t i = 0; i < P.n_seg; ++i) bytes += (uint64_t)(P.geom.v_hi - P.geom.v_lo) * plane_site_bytes(P.seg[i].g);
-    t_tim.stats_bytes = bytes;
-}
-
-// fm_k_plane_pass_tab: an arbitrary list of plane segments (gpu = 1: independent (region, group) units;
-// gpu = 2: Hudson pairs over shared sites) in ONE persistent launch.  Fills rounds / b_lo of every segment,
-// uploads the descriptor table and launches.  Returns false when the segments cannot share a launch
-// (column-chunked rows): the caller then goes unit by unit.
-struct TabLaunch {
-    DevBuf<fm::TabSeg> d_segs;
+    bool inline_table = false, pair = false;
+    uint64_t bytes = 0;  // plane bytes one launch reads
+    DevBuf<fm::RowSeg> d_segs;
     DevBuf<uint32_t> d_prefix;
-    DevBuf<fm::HudsonEpilogue> d_hud;
     std::vector<uint32_t> prefix;  // host copy: batches before unit u
 };
-bool launch_plane_pass_tab(std::vector<fm::TabSeg> &segs, uint32_t gpu, const std::vector<fm::HudsonEpilogue> *hud,
-                           int device, TabLaunch &keep) {
-    if (segs.empty() || (gpu != 1 && gpu != 2) || segs.size() % gpu) return false;
-    static const uint32_t step_target = env_u32("FM_STEP_BYTES", fm::kStepBytesTarget);
-    const uint32_t warp_smem = fm::kWarpSmemBytes;
-    uint32_t max_wq = 0;
-    for (const fm::TabSeg &sg : segs) max_wq = std::max(max_wq, sg.g.wq);
-    uint32_t lg = 0;
-    while ((1u << lg) < std::min(max_wq, 8u)) ++lg;
-    while (lg < 5 && (uint64_t)max_wq * 16u * (32u >> lg) * 2 > warp_smem) ++lg;
-    if (lg >= 5) return false;
+
+// Fills rounds / b_lo of every segment, the geometry and the unit prefix; up to kMaxSeq segments go into the kernel
+// parameters, a longer table is uploaded.  hud != nullptr: pair units (segments 2u and 2u + 1) with the Hudson
+// epilogue hud[u] each, at most kMaxSeq / 2 of them.  Returns false when the segments cannot share a launch
+// (column-chunked rows): the caller then goes unit by unit.
+bool plan_rows(std::vector<fm::RowSeg> &segs, const std::vector<fm::HudsonEpilogue> *hud, RowPlan &plan) {
+    const uint32_t gpu = hud ? 2u : 1u;  // segments per unit
+    if (segs.empty() || segs.size() % gpu) return false;
     const size_t n_units = segs.size() / gpu;
+    if (hud && (hud->size() != n_units || segs.size() > (size_t)fm::kMaxSeq))
+        fail(FM_ERR_INVALID_ARG, "internal: pair units take one Hudson epilogue each and travel in the parameters");
+    static const uint32_t step_target = env_u32("FM_STEP_BYTES", fm::kStepBytesTarget);
+    uint32_t max_wq = 0;
+    for (const fm::RowSeg &sg : segs) max_wq = std::max(max_wq, sg.g.wq);
+    const uint32_t lg = row_lanes_log2(max_wq);
+    if (lg >= 5) return false;
     uint32_t max_step = 0;
-    keep.prefix.assign(n_units + 1, 0);
-    uint64_t total = 0, bytes = 0;
+    plan.prefix.assign(n_units + 1, 0);
+    uint64_t total = 0;
+    plan.bytes = 0;
     for (size_t u = 0; u < n_units; ++u) {
-        fm::TabSeg &s0 = segs[u * gpu];
+        const fm::RowSeg &s0 = segs[u * gpu];
         const uint32_t nb = s0.v_hi > s0.v_lo ? (s0.v_hi + 31) / 32 - s0.v_lo / 32 : 0;
         for (uint32_t g = 0; g < gpu; ++g) {
-            fm::TabSeg &sg = segs[u * gpu + g];
+            fm::RowSeg &sg = segs[u * gpu + g];
             if (sg.v_lo != s0.v_lo || sg.v_hi != s0.v_hi) return false;
+            // several rounds of (32 >> lg) sites per step while the step stays near the target size
             const uint32_t round_bytes = sg.g.wq * 16u * (32u >> lg);
             uint32_t rounds = 1;
             while (rounds * 2 <= (1u << lg) && round_bytes * rounds * 2 <= step_target) rounds *= 2;
             sg.rounds = rounds;
             sg.b_lo = sg.v_lo / 32;
             max_step = std::max(max_step, round_bytes * rounds);
-            bytes += (uint64_t)(sg.v_hi - sg.v_lo) * plane_site_bytes(sg.g);
+            plan.bytes += (uint64_t)(sg.v_hi - sg.v_lo) * plane_site_bytes(sg.g);
         }
-        keep.prefix[u] = (uint32_t)total;
+        plan.prefix[u] = (uint32_t)total;
         total += nb;
         if (total >= (1ull << 31)) return false;
     }
-    keep.prefix[n_units] = (uint32_t)total;
-    if (total == 0) return true;
-    fm::TabParams P{};
+    plan.prefix[n_units] = (uint32_t)total;
+    fm::RowParams &P = plan.P;
+    P = fm::RowParams{};
     fm::PassGeom &G = P.geom;
-    G.lps_log2 = lg;
-    G.lps = 1u << lg;
     G.warps = fm::kWarpsPerCta;
-    G.warp_smem_bytes = warp_smem;
+    G.warp_smem_bytes = fm::kWarpSmemBytes;
     G.stage_bytes = (max_step + 127u) & ~127u;
-    G.n_stages = std::min<uint32_t>(fm::kMaxStages, warp_smem / G.stage_bytes);
+    G.n_stages = std::min<uint32_t>(fm::kMaxStages, G.warp_smem_bytes / G.stage_bytes);
     if (G.n_stages < 2) return false;
     G.n_batches = (uint32_t)total;
-    G.batch_counter = t_counters.take(device);
-    if (hud && hud->size() != n_units) fail(FM_ERR_INVALID_ARG, "internal: one Hudson epilogue per unit");
-    if (n_units == 1) {  // the whole table fits the kernel parameters
-        P.use_inline = 1;
-        for (uint32_t g = 0; g < gpu; ++g) P.inline_segs[g] = segs[g];
-        P.inline_prefix[0] = keep.prefix[0];
-        P.inline_prefix[1] = keep.prefix[1];
-        if (hud) {
-            P.has_inline_hud = 1;
-            P.inline_hud = (*hud)[0];
-        }
+    plan.lg = lg;
+    plan.pair = hud != nullptr;
+    plan.inline_table = segs.size() <= (size_t)fm::kMaxSeq;
+    if (plan.inline_table) {  // the whole table fits the kernel parameters
+        std::copy(segs.begin(), segs.end(), P.inline_segs);
+        std::copy(plan.prefix.begin(), plan.prefix.end(), P.inline_prefix);
+        if (hud) std::copy(hud->begin(), hud->end(), P.inline_hud);
     } else {
-        keep.d_segs.alloc(segs.size());
-        keep.d_segs.upload(segs.data(), segs.size());
-        keep.d_prefix.alloc(n_units + 1);
-        keep.d_prefix.upload(keep.prefix.data(), n_units + 1);
-        if (hud) {
-            keep.d_hud.alloc(n_units);
-            keep.d_hud.upload(hud->data(), n_units);
-            P.hud = keep.d_hud.p;
-        }
         // (pageable sources are staged by the driver before cudaMemcpyAsync returns: the host vectors may go away)
-        P.segs = keep.d_segs.p;
-        P.unit_prefix = keep.d_prefix.p;
+        plan.d_segs.alloc(segs.size());
+        plan.d_segs.upload(segs.data(), segs.size());
+        plan.d_prefix.alloc(n_units + 1);
+        plan.d_prefix.upload(plan.prefix.data(), n_units + 1);
+        P.segs = plan.d_segs.p;
+        P.unit_prefix = plan.d_prefix.p;
     }
     P.n_units = (uint32_t)n_units;
-    P.gpu = gpu;
-    const size_t smem = (size_t)fm::kWarpsPerCta * warp_smem;
-    const uint32_t grid = std::min<uint32_t>((uint32_t)sm_count(device),
-                                             (uint32_t)((total * gpu + fm::kWarpsPerCta - 1) / fm::kWarpsPerCta));
-    // the dynamic shared-memory limit is a per-device function attribute: set it once per (instantiation, device)
-    static std::mutex attr_mu;
-    static bool attr_done[5][64] = {};
-    auto once = [&](int slot, auto kern) {
-        std::lock_guard<std::mutex> lk(attr_mu);
-        if (device < 64 && attr_done[slot][device]) return;
-        CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        if (device < 64) attr_done[slot][device] = true;
-    };
-#define FM_TAB_CASE(L)                                                                  \
-    case L:                                                                             \
-        once(L, fm::fm_k_plane_pass_tab<L>);                                            \
-        fm::fm_k_plane_pass_tab<L><<<grid, fm::kWarpsPerCta * 32, smem, stream()>>>(P); \
-        break;
-    switch (lg) {
-        FM_TAB_CASE(0) FM_TAB_CASE(1) FM_TAB_CASE(2) FM_TAB_CASE(3) FM_TAB_CASE(4)
-        default: fail(FM_ERR_INVALID_ARG, "internal: bad table pass geometry");
+    return true;
+}
+
+template <int LG>
+void launch_rows_t(const RowPlan &plan, const fm::RowParams &P, uint32_t grid, int device) {
+    void (*kern)(fm::RowParams) = plan.pair           ? fm::fm_k_plane_pass_seq<LG, true, true>
+                                  : plan.inline_table ? fm::fm_k_plane_pass_seq<LG, true, false>
+                                                      : fm::fm_k_plane_pass_seq<LG, false, false>;
+    allow_rings_once(reinterpret_cast<const void *>(kern), device);
+    kern<<<grid, fm::kWarpsPerCta * 32, (size_t)fm::kWarpsPerCta * fm::kWarpSmemBytes, stream()>>>(P);
+}
+
+void launch_rows(const RowPlan &plan, int device) {
+    if (plan.P.geom.n_batches == 0) return;
+    fm::RowParams P = plan.P;
+    P.geom.batch_counter = t_counters.take(device);
+    const uint64_t warps_needed = (uint64_t)P.geom.n_batches * (plan.pair ? 2u : 1u);
+    const uint32_t grid = (uint32_t)std::min<uint64_t>(sm_count(device), (warps_needed + fm::kWarpsPerCta - 1) / fm::kWarpsPerCta);
+    switch (plan.lg) {
+        case 0: launch_rows_t<0>(plan, P, grid, device); break;
+        case 1: launch_rows_t<1>(plan, P, grid, device); break;
+        case 2: launch_rows_t<2>(plan, P, grid, device); break;
+        case 3: launch_rows_t<3>(plan, P, grid, device); break;
+        case 4: launch_rows_t<4>(plan, P, grid, device); break;
+        default: fail(FM_ERR_INVALID_ARG, "internal: bad row pass geometry");
     }
-#undef FM_TAB_CASE
     CK(cudaGetLastError());
     g_launches++;
     t_tim.stats_launches++;
-    t_tim.stats_bytes = bytes;
-    return true;
+    t_tim.stats_bytes = plan.bytes;
+}
+
+// super-batches [s_lo, s_lo + n_super) that fm_k_reduce_partials folds for the batches of G
+void super_range(const fm::PassGeom &G, uint32_t &s_lo, uint32_t &n_super) {
+    s_lo = G.b_lo / fm::kSuperBatches;
+    n_super = (G.b_lo + G.n_batches + fm::kSuperBatches - 1) / fm::kSuperBatches - s_lo;
+}
+
+// per-batch partials -> one row of nd doubles / nu u32 sums per super-batch, on the device
+void launch_reduce(const double *pd, int nd, const uint32_t *pu, int nu, const fm::PassGeom &G, double *sd,
+                   uint64_t *su, cudaStream_t st = nullptr) {
+    if (!st) st = stream();
+    uint32_t s_lo, n_super;
+    super_range(G, s_lo, n_super);
+    fm::fm_k_reduce_partials<<<(n_super + 3) / 4, 128, 0, st>>>(pd, nd, pu, nu, G.b_lo, G.n_batches,
+                                                                 s_lo, n_super, sd, su);
+    CK(cudaGetLastError());
+    g_launches++;
 }
 
 // reduce per-batch partials to per-super-batch on device, finish sequentially on the host
@@ -1023,14 +942,11 @@ void finish_partials(const double *d_pd, int nd, const uint32_t *d_pu, int nu, c
     for (int i = 0; i < nd; ++i) out_d[i] = 0.0;
     for (int i = 0; i < nu; ++i) out_u[i] = 0;
     if (G.n_batches == 0) return;
-    const uint32_t s_lo = G.b_lo / fm::kSuperBatches;
-    const uint32_t n_super = (G.b_lo + G.n_batches + fm::kSuperBatches - 1) / fm::kSuperBatches - s_lo;
+    uint32_t s_lo, n_super;
+    super_range(G, s_lo, n_super);
     DevBuf<double> sd((size_t)n_super * std::max(nd, 1));
     DevBuf<uint64_t> su((size_t)n_super * std::max(nu, 1));
-    fm::fm_k_reduce_partials<<<(n_super + 3) / 4, 128, 0, stream()>>>(
-        d_pd, nd, d_pu, nu, G.b_lo, G.n_batches, s_lo, n_super, sd.p, su.p);
-    CK(cudaGetLastError());
-    g_launches++;
+    launch_reduce(d_pd, nd, d_pu, nu, G, sd.p, su.p);
     std::vector<double> hd((size_t)n_super * std::max(nd, 1));
     std::vector<uint64_t> hu((size_t)n_super * std::max(nu, 1));
     sd.download(hd.data(), (size_t)n_super * nd);
@@ -1087,9 +1003,7 @@ void ensure_counts(fm_group *g);
 DivResult run_multi_diversity(fm_group *g, uint32_t v_lo, uint32_t v_hi, int form, double *d_pi, double *d_theta,
                               const int64_t *d_mask, uint32_t n_mask, const int64_t *d_filt, uint32_t n_filt) {
     DivResult r{0.0, 0, 0};
-    fm::PassGeom G{};
-    G.b_lo = v_lo / 32;
-    G.n_batches = v_hi > v_lo ? (v_hi + 31) / 32 - G.b_lo : 0;
+    const fm::PassGeom G = batch_range(v_lo, v_hi);
     if (G.n_batches == 0) return r;
     DevBuf<double> part_pi(G.n_batches);
     DevBuf<uint32_t> part_u((size_t)G.n_batches * 2);
@@ -1160,18 +1074,28 @@ void ensure_multi_counts_locked(fm_group *g) {
     g->pi_sum = r.pi_sum;
 }
 
+// segment of the row pass: group g over [v_lo, v_hi) into the diversity epilogue e
+fm::RowSeg div_seg(const fm_group *g, const fm::DivEpilogue &e, uint32_t v_lo, uint32_t v_hi) {
+    fm::RowSeg s{};
+    s.g = planes_of(g);
+    s.div = e;
+    s.v_lo = v_lo;
+    s.v_hi = v_hi;
+    s.n_sites_total = (uint32_t)g->m->V;
+    return s;
+}
+
 // Run the diversity statistics for sites [v_lo, v_hi): fused plane pass when counts are not
 // cached (optionally caching them when the range is the whole matrix), light kernel otherwise.
 DivResult run_diversity(fm_group *g, uint32_t v_lo, uint32_t v_hi, int pi_form, double *d_pi,
                         double *d_theta, const int64_t *d_mask, uint32_t n_mask, const int64_t *d_filt,
-                        uint32_t n_filt, bool store_counts, bool force_plane_pass = false) {
+                        uint32_t n_filt, bool store_counts) {
     if (g->n_bits > 1) {  // multi-allelic: always from the cached per-allele counts
         if (!g->have_counts) ensure_multi_counts_locked(g);
         return run_multi_diversity(g, v_lo, v_hi, pi_form == FM_PIFORM_COMPONENTS ? FM_MULTI_SPARSE : FM_MULTI_DENSE,
                                    d_pi, d_theta, d_mask, n_mask, d_filt, n_filt);
     }
-    const fm_group *gs[1] = {g};
-    fm::PassGeom G = make_geom(gs, 1, v_lo, v_hi);
+    const fm::PassGeom G = batch_range(v_lo, v_hi);
     DivResult r{0.0, 0, 0};
     if (G.n_batches == 0) return r;
     DevBuf<double> part_pi(G.n_batches);
@@ -1191,7 +1115,7 @@ DivResult run_diversity(fm_group *g, uint32_t v_lo, uint32_t v_hi, int pi_form, 
     e.pi_form = pi_form;
     e.part_pi = part_pi.p;
     e.part_u = part_u.p;
-    if (g->have_counts && !force_plane_pass) {
+    if (g->have_counts) {
         const uint32_t blocks = std::min<uint32_t>((G.n_batches + 7) / 8, 8u * sm_count(g->m->device));
         fm::fm_k_div_from_counts<<<blocks, 256, 0, stream()>>>(g->d_alt, g->d_cnt, e, v_lo, v_hi,
                                                                 G.b_lo, G.n_batches);
@@ -1203,11 +1127,12 @@ DivResult run_diversity(fm_group *g, uint32_t v_lo, uint32_t v_hi, int pi_form, 
             e.called_out = called_cache(g);
         }
         if (g->count_only) fail(FM_ERR_INVALID_ARG, "internal: a count-only group has no bitplanes to stream");
-        fm::PassParams<1> P{};
-        P.g[0] = planes_of(g);
-        P.geom = G;
-        P.div = e;
-        launch_plane_pass<1>(P, g->m->device);
+        std::vector<fm::RowSeg> segs{div_seg(g, e, v_lo, v_hi)};
+        RowPlan plan;
+        if (row_lanes_log2(g->wq) < 5 && plan_rows(segs, nullptr, plan))
+            launch_rows(plan, g->m->device);
+        else
+            launch_chunked(fm::ChunkParams{planes_of(g), make_geom(g, v_lo, v_hi), e}, g->m->device);
     }
     tm.stop();
     double od[1];
@@ -1224,37 +1149,34 @@ DivResult run_diversity(fm_group *g, uint32_t v_lo, uint32_t v_hi, int pi_form, 
     return r;
 }
 
-// Diversity statistics of several groups of one matrix over [v_lo, v_hi).  Groups whose counts
-// are not cached yet and whose rows fit the non-chunked geometry share ONE plane-pass launch
-// (fm_k_plane_pass_seq); everything else goes group by group through run_diversity.
+// Diversity statistics of several groups of one matrix over [v_lo, v_hi).  Groups whose counts are not cached yet
+// and whose rows fit the row pass share ONE launch of it (fm_k_plane_pass_seq); everything else goes group by group
+// through run_diversity.
 bool run_diversity_multi(fm_group *const *gs, size_t n, uint32_t v_lo, uint32_t v_hi, int pi_form,
                          double *const *d_pi, double *const *d_theta, const int64_t *d_mask, uint32_t n_mask,
                          const int64_t *d_filt, uint32_t n_filt, DivResult *out, bool store_counts = false,
                          Timer *ext_tm = nullptr) {
-    fm::SeqParams P{};
-    bool fuse = v_hi > v_lo;
-    for (size_t i = 0; i < n && fuse; ++i) fuse = !gs[i]->have_counts;
-    if (fuse) fuse = make_seq_params(gs, n, v_lo, v_hi, P);
-    if (!fuse) {
+    auto per_group = [&]() {
         for (size_t i = 0; i < n; ++i) {
             DivResult r = run_diversity(gs[i], v_lo, v_hi, pi_form, d_pi ? d_pi[i] : nullptr, d_theta ? d_theta[i] : nullptr,
                                         d_mask, n_mask, d_filt, n_filt, store_counts);
             if (out) out[i] = r;
         }
         return false;
-    }
-    const fm::PassGeom &G = P.geom;
+    };
+    bool fuse = v_hi > v_lo;
+    for (size_t i = 0; i < n && fuse; ++i)
+        fuse = !gs[i]->have_counts && gs[i]->m == gs[0]->m && gs[i]->n_bits == 1 && !gs[i]->count_only &&
+               row_lanes_log2(gs[i]->wq) < 5;
+    if (!fuse) return per_group();
+    const fm::PassGeom G = batch_range(v_lo, v_hi);
+    const bool tracks = d_pi != nullptr;
+    const bool use_flags = tracks && (d_mask || d_filt);
+    DevBuf<uint32_t> flags;
+    if (use_flags) flags.alloc(G.n_batches);
     std::vector<DevBuf<double>> part_pi(n);
     std::vector<DevBuf<uint32_t>> part_u(n);
-    DevBuf<uint32_t> flags;
-    Timer own_tm;
-    Timer &tm = ext_tm ? *ext_tm : own_tm;
-    tm.start();
-    const bool tracks = d_pi != nullptr;
-    if (tracks && (d_mask || d_filt)) {
-        flags.alloc(G.n_batches);
-        launch_site_flags(gs[0]->m, v_lo, v_hi, G.b_lo, G.n_batches, d_mask, n_mask, d_filt, n_filt, flags.p);
-    }
+    std::vector<fm::RowSeg> segs(n);
     for (size_t i = 0; i < n; ++i) {
         part_pi[i].alloc(G.n_batches);
         part_u[i].alloc((size_t)G.n_batches * 2);
@@ -1270,9 +1192,15 @@ bool run_diversity_multi(fm_group *const *gs, size_t n, uint32_t v_lo, uint32_t 
             e.alt_out = gs[i]->d_alt;
             e.called_out = called_cache(gs[i]);
         }
-        P.seg[i].div = e;
+        segs[i] = div_seg(gs[i], e, v_lo, v_hi);
     }
-    launch_plane_pass_seq(P, gs[0]->m->device);
+    RowPlan plan;
+    if (!plan_rows(segs, nullptr, plan)) return per_group();
+    Timer own_tm;
+    Timer &tm = ext_tm ? *ext_tm : own_tm;
+    tm.start();
+    if (use_flags) launch_site_flags(gs[0]->m, v_lo, v_hi, G.b_lo, G.n_batches, d_mask, n_mask, d_filt, n_filt, flags.p);
+    launch_rows(plan, gs[0]->m->device);
     tm.stop();
     for (size_t i = 0; i < n && out; ++i) {  // out == nullptr: the caller only wants the tracks
         double od[1];
@@ -1310,8 +1238,7 @@ struct HudsonTotals {
 // Hudson sums (and optional per-site outputs) for [v_lo, v_hi) from cached counts.
 HudsonTotals run_hudson_counts(fm_group *g1, fm_group *g2, uint32_t v_lo, uint32_t v_hi, int variant,
                                fm::HudsonEpilogue e) {
-    const fm_group *gs[2] = {g1, g2};
-    fm::PassGeom G = make_geom(gs, 2, v_lo, v_hi);
+    const fm::PassGeom G = batch_range(v_lo, v_hi);
     HudsonTotals t{0, 0, 0, 0, 0, 0, 0, 0};
     if (G.n_batches == 0) return t;
     DevBuf<double> pd((size_t)G.n_batches * 5);
@@ -2207,7 +2134,7 @@ fm_status fm_group_summary(fm_group *g, uint32_t *alt_out, uint32_t *called_out,
 
 // build_dense_population_summary for MANY groups -- normally one per region-sized matrix, the shape of the CLI's
 // loop over config entries (process.rs:2169 -> stats.rs:1367-1470) -- in one persistent launch: groups whose counts
-// are not cached yet become the units of one fm_k_plane_pass_tab pass (per LPS / bitmap class), their partials
+// are not cached yet become the units of one fm_k_plane_pass_seq launch, their partials
 // are folded by one kernel and come back in one copy.  Each group ends up exactly as after fm_group_summary.
 static void summarize_groups(fm_group *const *groups, size_t n_groups) {
     {
@@ -2230,7 +2157,7 @@ static void summarize_groups(fm_group *const *groups, size_t n_groups) {
         for (fm_group *g : order)
             if (!g->have_counts && g->n_bits == 1 && !g->count_only && g->m->V > 0) gs.push_back(g);
         if (!gs.empty()) {
-            std::vector<fm::TabSeg> segs(gs.size());
+            std::vector<fm::RowSeg> segs(gs.size());
             std::vector<size_t> part_off(gs.size());
             size_t total_b = 0;
             for (size_t i = 0; i < gs.size(); ++i) {
@@ -2252,26 +2179,22 @@ static void summarize_groups(fm_group *const *groups, size_t n_groups) {
                 de.part_u = ppu.p + 2 * part_off[i];
                 de.alt_out = g->d_alt;
                 de.called_out = called_cache(g);
-                segs[i] = fm::TabSeg{};
-                segs[i].g = planes_of(g);
-                segs[i].div = de;
-                segs[i].v_lo = 0;
-                segs[i].v_hi = V;
-                segs[i].n_sites_total = V;
+                segs[i] = div_seg(g, de, 0, V);
                 const uint32_t nb = (V + 31) / 32;
                 for (uint32_t sb = 0; sb * fm::kSuperBatches < nb; ++sb)
                     ents.push_back(make_uint4((uint32_t)part_off[i], 0u, nb, sb));
             }
             if (total_b >= (1ull << 31)) fail(FM_ERR_UNSUPPORTED, "too many sites for one batched summary call");
-            TabLaunch keep;
+            RowPlan plan;
             Timer tm;
             tm.start();
-            if (!launch_plane_pass_tab(segs, 1, nullptr, device, keep)) {
-                // rows wider than the table pass handles (column-chunked): one pass per group
+            if (!plan_rows(segs, nullptr, plan)) {
+                // rows wider than the row pass handles (column-chunked): one pass per group
                 locks.clear();
                 for (fm_group *g : gs) ensure_counts(g);
                 for (fm_group *g : order) locks.emplace_back(g->mu);
             } else {
+                launch_rows(plan, device);
                 DevBuf<uint4> d_ents(ents.size());
                 d_ents.upload(ents.data(), ents.size());
                 DevBuf<double> sd(ents.size());
@@ -2313,7 +2236,7 @@ static void summarize_groups(fm_group *const *groups, size_t n_groups) {
 fm_status fm_groups_summary_batch(fm_group *const *groups, size_t n_groups, uint64_t *seg_out, double *pi_sum_out,
                                   uint64_t *unc_out) {
     return guarded([&] {
-        FM_NVTX("fm_groups_summary_batch (table plane pass)");
+        FM_NVTX("fm_groups_summary_batch (row plane pass)");
         summarize_groups(groups, n_groups);
         for (size_t i = 0; i < n_groups; ++i) {
             const fm_group *g = groups[i];
@@ -3452,7 +3375,7 @@ fm_status fm_hudson_pair(fm_group *g1, fm_group *g2, int64_t L1, int64_t L2, int
             std::lock(l1, l2);
             if (!g1->have_counts && !g2->have_counts) {
                 for (fm_group *g : {g1, g2}) alloc_counts(g);
-                // ONE sweep of both groups' planes (fm_k_plane_pass_tab, pair units): every warp streams a batch of
+                // ONE sweep of both groups' planes (fm_k_plane_pass_seq, pair units): every warp streams a batch of
                 // group 1, then the same batch of group 2, and evaluates the Hudson components in place -- the
                 // groups' counts and summary scalars are cached for later calls AND the Hudson partials (plus the
                 // optional per-site values) come out of the same pass (stats.rs:3179-3278).
@@ -3460,7 +3383,7 @@ fm_status fm_hudson_pair(fm_group *g1, fm_group *g2, int64_t L1, int64_t L2, int
                 const uint32_t nb = (V + 31) / 32;
                 DevBuf<double> ppi[2], pd((size_t)nb * 5);
                 DevBuf<uint32_t> ppu[2], pu((size_t)nb * 3);
-                std::vector<fm::TabSeg> segs(2);
+                std::vector<fm::RowSeg> segs(2);
                 for (int k = 0; k < 2; ++k) {
                     ppi[k].alloc(nb);
                     ppu[k].alloc((size_t)nb * 2);
@@ -3471,28 +3394,21 @@ fm_status fm_hudson_pair(fm_group *g1, fm_group *g2, int64_t L1, int64_t L2, int
                     de.part_u = ppu[k].p;
                     de.alt_out = pair[k]->d_alt;
                     de.called_out = called_cache(pair[k]);
-                    segs[k] = fm::TabSeg{};
-                    segs[k].g = planes_of(pair[k]);
-                    segs[k].div = de;
-                    segs[k].v_lo = 0;
-                    segs[k].v_hi = V;
-                    segs[k].n_sites_total = V;
+                    segs[k] = div_seg(pair[k], de, 0, V);
                 }
                 fm::HudsonEpilogue he = e;
                 he.variant = site_variant;
                 he.part_d = pd.p;
                 he.part_u = pu.p;
                 std::vector<fm::HudsonEpilogue> hv{he};
-                TabLaunch keep;
+                RowPlan plan;
                 Timer tm;
                 tm.start();
-                static const uint32_t no_tab = env_u32("FM_NO_TAB", 0);
-                const bool ok = !no_tab && launch_plane_pass_tab(segs, 2, &hv, m->device, keep);
+                const bool ok = plan_rows(segs, &hv, plan);
+                if (ok) launch_rows(plan, m->device);
                 tm.stop();
                 if (ok) {
-                    fm::PassGeom G{};
-                    G.b_lo = 0;
-                    G.n_batches = nb;
+                    const fm::PassGeom G = batch_range(0, V);
                     for (int k = 0; k < 2; ++k) {
                         double od[1];
                         uint64_t ou[2];
@@ -3507,7 +3423,7 @@ fm_status fm_hudson_pair(fm_group *g1, fm_group *g2, int64_t L1, int64_t L2, int
                     finish_partials(pd.p, 5, pu.p, 3, G, od, ou);
                     main_t = HudsonTotals{od[0], od[1], od[2], od[3], od[4], ou[0], ou[1], ou[2]};
                     t_tim.stats_ms += tm.ms();
-                } else {  // rows too wide for the table pass: two streamed groups, then the light kernel
+                } else {  // rows too wide for the row pass: two chunked passes, then the light kernel
                     DivResult r[2];
                     run_diversity_multi(pair, 2, 0, V, FM_PIFORM_COUNTS, nullptr, nullptr, nullptr, 0, nullptr, 0, r, true);
                     for (int k = 0; k < 2; ++k) {
@@ -4402,13 +4318,8 @@ fm_status fm_comm_destroy(fm_comm *c) {
 }
 
 // ------------------------------------------------------------------------------------ sharded Hudson call
-namespace {
-void launch_reduce(const double *pd, int nd, const uint32_t *pu, int nu, const fm::PassGeom &G, double *sd,
-                   uint64_t *su, cudaStream_t st);
-}
-
 // One Hudson call over a cohort that is sharded by site range across the ranks of `comm` (SURVEY 8e, config 3):
-// every rank sweeps its own shard once (pair units of fm_k_plane_pass_tab, nothing cached, nothing written but
+// every rank sweeps its own shard once (pair units of fm_k_plane_pass_seq, nothing cached, nothing written but
 // the per-batch partials), folds the partials per super-batch, and the fold into region totals is fused with
 // the NVLink mailbox exchange; the rank-ordered merged totals come back in ONE small copy and are finished on
 // the host exactly like the single-GPU summaries path (stats.rs:3476-3566).  Three launches, one host sync.
@@ -4460,21 +4371,15 @@ fm_status fm_hudson_pair_sharded(fm_group *g1, fm_group *g2, int64_t sequence_le
         tm.start();
         if (V) {
             bool done = false;
-            TabLaunch keep;
             if (g1 != g2 && !g1->count_only && !g2->count_only && !(g1->have_counts && g2->have_counts)) {
-                std::vector<fm::TabSeg> segs(2);
-                fm_group *pair[2] = {g1, g2};
-                for (int k = 0; k < 2; ++k) {
-                    segs[k] = fm::TabSeg{};
-                    segs[k].g = planes_of(pair[k]);
-                    segs[k].v_lo = 0;
-                    segs[k].v_hi = V;
-                    segs[k].n_sites_total = V;
-                }
+                // no diversity epilogue (div.part_pi == nullptr): the Hudson partials are the only output
+                std::vector<fm::RowSeg> segs{div_seg(g1, fm::DivEpilogue{}, 0, V), div_seg(g2, fm::DivEpilogue{}, 0, V)};
                 std::vector<fm::HudsonEpilogue> hv{he};
-                done = launch_plane_pass_tab(segs, 2, &hv, m->device, keep);
+                RowPlan plan;
+                done = plan_rows(segs, &hv, plan);
+                if (done) launch_rows(plan, m->device);
             }
-            if (!done) {  // cached counts, count-only groups or rows wider than the table pass: from the counts
+            if (!done) {  // cached counts, count-only groups or rows wider than the row pass: from the counts
                 ensure_counts_pair(g1, g2);
                 const uint32_t blocks = std::min<uint32_t>((nb + 7) / 8, 8u * sm_count(m->device));
                 fm::fm_k_hudson_from_counts<<<blocks, 256, 0, stream()>>>(g1->d_alt, g1->d_cnt, g2->d_alt, g2->d_cnt, he, 0,
@@ -4482,14 +4387,9 @@ fm_status fm_hudson_pair_sharded(fm_group *g1, fm_group *g2, int64_t sequence_le
                 CK(cudaGetLastError());
                 g_launches++;
             }
-            fm::PassGeom G{};
-            G.b_lo = 0;
-            G.n_batches = nb;
             if (trace) CK(cudaEventRecord(te[1], stream()));
-            launch_reduce(pd.p, 5, pu.p, 3, G, sd.p, su.p, stream());
+            launch_reduce(pd.p, 5, pu.p, 3, batch_range(0, V), sd.p, su.p, stream());
             if (trace) CK(cudaEventRecord(te[2], stream()));
-            // `keep` (the descriptor table) goes back to the allocator here: the block carries an event on this
-            // stream, so a later owner waits for the pass -- no host synchronisation needed
         }
         unsigned long long w[8] = {};
         if (comm) {
@@ -5507,20 +5407,6 @@ fm_status fm_synth_fill(uint8_t *d_data, uint64_t *d_missing, size_t V, size_t S
 }
 
 // ------------------------------------------------------------------------------------ bench hooks
-namespace {
-
-void launch_reduce(const double *pd, int nd, const uint32_t *pu, int nu, const fm::PassGeom &G, double *sd,
-                   uint64_t *su, cudaStream_t st = nullptr) {
-    if (!st) st = stream();
-    const uint32_t s_lo = G.b_lo / fm::kSuperBatches;
-    const uint32_t n_super = (G.b_lo + G.n_batches + fm::kSuperBatches - 1) / fm::kSuperBatches - s_lo;
-    fm::fm_k_reduce_partials<<<(n_super + 3) / 4, 128, 0, st>>>(pd, nd, pu, nu, G.b_lo, G.n_batches,
-                                                                 s_lo, n_super, sd, su);
-    CK(cudaGetLastError());
-    g_launches++;
-}
-}  // namespace
-
 fm_status fm_bench_diversity(fm_group *const *groups, size_t n_groups, int mode, const int64_t *mask_iv,
                              size_t n_mask, int iterations, fm_comm *comm, fm_bench_result *out, double *last_pi,
                              double *last_theta) {
@@ -5533,7 +5419,6 @@ fm_status fm_bench_diversity(fm_group *const *groups, size_t n_groups, int mode,
         set_dev(m);
         const uint32_t V = (uint32_t)m->V;
         struct PerGroup {
-            fm::PassParams<1> P;
             DevBuf<double> part_pi[2], pi, theta, sd[2];  // batch / super-batch partials double-buffered by step
             DevBuf<uint32_t> part_u[2];                    // parity: reductions and exchange of step i overlap step i+1
             DevBuf<uint64_t> su[2];
@@ -5542,7 +5427,8 @@ fm_status fm_bench_diversity(fm_group *const *groups, size_t n_groups, int mode,
         DevBuf<int64_t> d_mask;
         DevBuf<uint32_t> d_flags, d_flags2;  // double-buffered by step parity
         std::vector<int64_t> merged;
-        const uint32_t nb_all = V ? (V + 31) / 32 : 0;
+        const fm::PassGeom G = batch_range(0, V);  // every group's batches
+        const uint32_t nb_all = G.n_batches;
         if (mode == 1 && mask_iv) {
             merge_intervals(mask_iv, n_mask, merged);
             d_mask.alloc(std::max<size_t>(merged.size(), 2));
@@ -5550,40 +5436,62 @@ fm_status fm_bench_diversity(fm_group *const *groups, size_t n_groups, int mode,
             d_flags.alloc(std::max<uint32_t>(nb_all, 1));
             d_flags2.alloc(std::max<uint32_t>(nb_all, 1));
         }
+        const bool use_flags = mode == 1 && mask_iv && nb_all;
+        uint32_t *flagbuf[2] = {d_flags.p, d_flags2.p};
+        // The plane launches of one step, one set per step parity: the groups whose rows fit the row pass in ONE
+        // launch of it (fm_k_plane_pass_seq), then one column-chunked launch per group with wider rows.
+        // launch_groups[l]: the groups whose partials launch l writes.
+        std::vector<std::vector<size_t>> launch_groups(1);
+        for (size_t i = 0; i < n_groups; ++i) {
+            if (row_lanes_log2(groups[i]->wq) < 5)
+                launch_groups[0].push_back(i);
+            else
+                launch_groups.push_back({i});
+        }
+        const bool rows = !launch_groups[0].empty();
+        if (!rows) launch_groups.erase(launch_groups.begin());
+        std::vector<fm::RowSeg> segs[2];
+        std::vector<fm::ChunkParams> chunked[2];
         uint64_t bytes = 0;
         for (size_t i = 0; i < n_groups; ++i) {
             fm_group *g = groups[i];
             if (g->m != m) fail(FM_ERR_INVALID_ARG, "groups must share one matrix");
-            const fm_group *gs[1] = {g};
-            fm::PassGeom G = make_geom(gs, 1, 0, V);
-            const size_t nb = std::max<uint32_t>(G.n_batches, 1);
+            const size_t nb = std::max<uint32_t>(nb_all, 1);
             for (int k = 0; k < 2; ++k) {
                 pg[i].part_pi[k].alloc(nb);
                 pg[i].part_u[k].alloc(nb * 2);
                 pg[i].sd[k].alloc(nb / fm::kSuperBatches + 2);
                 pg[i].su[k].alloc(2 * (nb / fm::kSuperBatches + 2));
             }
-            fm::DivEpilogue e{};
-            set_tables(e, g);
-            e.pi_form = FM_PIFORM_COUNTS;
-            e.part_pi = pg[i].part_pi[0].p;
-            e.part_u = pg[i].part_u[0].p;
             bytes += (uint64_t)V * plane_site_bytes(planes_of(g));
             if (i < 8) out->group_bytes[i] = (uint64_t)V * plane_site_bytes(planes_of(g)) + (mode == 1 ? (uint64_t)V * 16u : 0);
             if (mode == 1) {
                 pg[i].pi.alloc(std::max<uint32_t>(V, 1));
                 pg[i].theta.alloc(std::max<uint32_t>(V, 1));
-                e.pi_out = pg[i].pi.p;
-                e.theta_out = pg[i].theta.p;
-                e.pi_form = FM_PIFORM_COMPONENTS;
-                if (mask_iv) e.site_flags = d_flags.p;
                 bytes += (uint64_t)V * 16u;
             }
-            pg[i].P = fm::PassParams<1>{};
-            pg[i].P.g[0] = planes_of(g);
-            pg[i].P.geom = G;
-            pg[i].P.div = e;
+            for (int k = 0; k < 2; ++k) {
+                fm::DivEpilogue e{};
+                set_tables(e, g);
+                e.pi_form = FM_PIFORM_COUNTS;
+                e.part_pi = pg[i].part_pi[k].p;
+                e.part_u = pg[i].part_u[k].p;
+                if (mode == 1) {
+                    e.pi_out = pg[i].pi.p;
+                    e.theta_out = pg[i].theta.p;
+                    e.pi_form = FM_PIFORM_COMPONENTS;
+                    if (use_flags) e.site_flags = flagbuf[k];
+                }
+                if (row_lanes_log2(g->wq) < 5)
+                    segs[k].push_back(div_seg(g, e, 0, V));
+                else
+                    chunked[k].push_back(fm::ChunkParams{planes_of(g), make_geom(g, 0, V), e});
+            }
         }
+        RowPlan plan[2];
+        for (int k = 0; k < 2 && rows; ++k)
+            if (!plan_rows(segs[k], nullptr, plan[k])) fail(FM_ERR_INVALID_ARG, "internal: the groups do not fit one row pass");
+        const size_t n_launch = launch_groups.size();
         EventPairs evs;
         std::vector<std::pair<cudaEvent_t, cudaEvent_t>> spans, comm_spans;
         cudaEvent_t t0 = evs.next(), t1 = evs.next();
@@ -5599,12 +5507,7 @@ fm_status fm_bench_diversity(fm_group *const *groups, size_t n_groups, int mode,
         } side, xchg;  // side: mask lookup + reductions; xchg: the peer exchange (may wait for other ranks)
         CK(cudaStreamCreateWithFlags(&side.s, cudaStreamNonBlocking));
         if (comm) CK(cudaStreamCreateWithFlags(&xchg.s, cudaStreamNonBlocking));
-        const bool use_flags = mode == 1 && mask_iv && nb_all;
-        fm::SeqParams SP{};
-        const bool fused = make_seq_params(groups, n_groups, 0, V, SP);
-        uint32_t *flagbuf[2] = {d_flags.p, d_flags2.p};
         std::vector<cudaEvent_t> flags_ready(iterations, nullptr), side_done(iterations, nullptr);
-        std::vector<cudaEvent_t> reduced(n_groups, nullptr);  // last reduction of group i's per-batch partials
         auto ev = [&]() {
             cudaEvent_t e;
             CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
@@ -5628,65 +5531,37 @@ fm_status fm_bench_diversity(fm_group *const *groups, size_t n_groups, int mode,
             CK(cudaStreamWaitEvent(side.s, t0, 0));
             launch_flags(0);
         }
+        uint32_t s_lo = 0, n_super = 0;
+        super_range(G, s_lo, n_super);
         for (int it = 0; it < iterations; ++it) {
             const int pb = it & 1;
             // buffers of parity pb were last read by the side work of step it - 2
             if (it >= 2) CK(cudaStreamWaitEvent(stream(), side_done[it - 2], 0));
             if (use_flags) CK(cudaStreamWaitEvent(stream(), flags_ready[it], 0));
-            if (fused) {
-                // all groups in ONE persistent launch (fm_k_plane_pass_seq)
-                for (size_t i = 0; i < n_groups; ++i) {
-                    SP.seg[i].div = pg[i].P.div;
-                    SP.seg[i].div.part_pi = pg[i].part_pi[pb].p;
-                    SP.seg[i].div.part_u = pg[i].part_u[pb].p;
-                    if (use_flags) SP.seg[i].div.site_flags = flagbuf[pb];
-                }
-                if (use_flags && it + 1 < iterations) launch_flags(it + 1);  // next step's mask bits, under this pass
+            if (use_flags && it + 1 < iterations) launch_flags(it + 1);  // next step's mask bits, under this step's passes
+            for (size_t l = 0; l < n_launch; ++l) {
                 cudaEvent_t a = evs.next(), b = evs.next();
                 CK(cudaEventRecord(a, stream()));
-                launch_plane_pass_seq(SP, m->device);
+                if (rows && l == 0)
+                    launch_rows(plan[pb], m->device);
+                else
+                    launch_chunked(chunked[pb][l - (rows ? 1 : 0)], m->device);
                 CK(cudaEventRecord(b, stream()));
                 spans.emplace_back(a, b);
                 out->plane_launches++;
+                // side stream: reduce the partials of this launch's groups while the next pass streams
                 CK(cudaStreamWaitEvent(side.s, b, 0));
-                for (size_t i = 0; i < n_groups; ++i) {
-                    if (!pg[i].P.geom.n_batches) continue;
-                    launch_reduce(pg[i].part_pi[pb].p, 1, pg[i].part_u[pb].p, 2, pg[i].P.geom, pg[i].sd[pb].p,
-                                  pg[i].su[pb].p, side.s);
+                for (size_t i : launch_groups[l]) {
+                    if (!nb_all) break;
+                    launch_reduce(pg[i].part_pi[pb].p, 1, pg[i].part_u[pb].p, 2, G, pg[i].sd[pb].p, pg[i].su[pb].p,
+                                  side.s);
                     out->other_launches++;
-                    reduced[i] = ev();
-                    CK(cudaEventRecord(reduced[i], side.s));
                 }
-            } else
-            for (size_t i = 0; i < n_groups; ++i) {
-                if (use_flags) pg[i].P.div.site_flags = flagbuf[pb];
-                pg[i].P.div.part_pi = pg[i].part_pi[pb].p;
-                pg[i].P.div.part_u = pg[i].part_u[pb].p;
-                cudaEvent_t a = evs.next(), b = evs.next();
-                CK(cudaEventRecord(a, stream()));
-                launch_plane_pass<1>(pg[i].P, m->device);
-                CK(cudaEventRecord(b, stream()));
-                spans.emplace_back(a, b);
-                out->plane_launches++;
-                // side stream: reduce this group's partials while the next pass streams
-                CK(cudaStreamWaitEvent(side.s, b, 0));
-                if (pg[i].P.geom.n_batches) {
-                    launch_reduce(pg[i].part_pi[pb].p, 1, pg[i].part_u[pb].p, 2, pg[i].P.geom, pg[i].sd[pb].p,
-                                  pg[i].su[pb].p, side.s);
-                    out->other_launches++;
-                    reduced[i] = ev();
-                    CK(cudaEventRecord(reduced[i], side.s));
-                }
-                if (i == 0 && use_flags && it + 1 < iterations) launch_flags(it + 1);  // next step's mask bits
             }
             if (comm) {  // fold the region totals of every group and exchange them with all ranks
                 fm::CommFold folds[4];
                 uint32_t nf = 0, words = 0;
-                for (size_t i = 0; i < n_groups && nf < 4; ++i) {
-                    const fm::PassGeom &G = pg[i].P.geom;
-                    if (!G.n_batches) continue;
-                    const uint32_t s_lo = G.b_lo / fm::kSuperBatches;
-                    const uint32_t n_super = (G.b_lo + G.n_batches + fm::kSuperBatches - 1) / fm::kSuperBatches - s_lo;
+                for (size_t i = 0; i < n_groups && nf < 4 && nb_all; ++i) {
                     folds[nf++] = fm::CommFold{pg[i].sd[pb].p,
                                                reinterpret_cast<const unsigned long long *>(pg[i].su[pb].p), n_super, 1u,
                                                2u};
@@ -5715,7 +5590,7 @@ fm_status fm_bench_diversity(fm_group *const *groups, size_t n_groups, int mode,
             float t = 0.f;
             CK(cudaEventElapsedTime(&t, spans[si].first, spans[si].second));
             plane += t;
-            const size_t gi = fused ? 0 : si % n_groups;
+            const size_t gi = si % n_launch;
             if (gi < 8) out->group_ms_avg[gi] += t / (float)iterations;
         }
         if (comm) comm_check_status(comm);
@@ -5739,11 +5614,7 @@ fm_status fm_bench_diversity(fm_group *const *groups, size_t n_groups, int mode,
         // region totals of the LAST timed step (parity check of the run: bench.py compares them with the public
         // call and, for N > 1, the exchanged totals with a rank-ordered sum of every rank's local ones)
         const int pl = (iterations - 1) & 1;
-        for (size_t i = 0; i < n_groups && i < 8; ++i) {
-            const fm::PassGeom &G = pg[i].P.geom;
-            if (!G.n_batches) continue;
-            const uint32_t s_lo = G.b_lo / fm::kSuperBatches;
-            const uint32_t n_super = (G.b_lo + G.n_batches + fm::kSuperBatches - 1) / fm::kSuperBatches - s_lo;
+        for (size_t i = 0; i < n_groups && i < 8 && nb_all; ++i) {
             std::vector<double> hd(n_super);
             std::vector<uint64_t> hu((size_t)n_super * 2);
             pg[i].sd[pl].download(hd.data(), n_super);
@@ -5766,61 +5637,6 @@ fm_status fm_bench_diversity(fm_group *const *groups, size_t n_groups, int mode,
                 out->merged_unc[i] = w[3 * i + 2];
             }
         }
-    });
-}
-
-fm_status fm_bench_hudson(fm_group *g1, fm_group *g2, int iterations, fm_bench_result *out) {
-    return guarded([&] {
-        check_pair(g1, g2);
-        if (!out || iterations < 1) fail(FM_ERR_INVALID_ARG, "bad argument");
-        require_device();
-        std::memset(out, 0, sizeof(*out));
-        set_dev(g1->m);
-        const uint32_t V = (uint32_t)g1->m->V;
-        const fm_group *gs[2] = {g1, g2};
-        fm::PassGeom G = make_geom(gs, 2, 0, V);
-        const size_t nb = std::max<uint32_t>(G.n_batches, 1);
-        DevBuf<double> pd(nb * 5), sd(5 * (nb / fm::kSuperBatches + 2));
-        DevBuf<uint32_t> pu(nb * 3);
-        DevBuf<uint64_t> su(3 * (nb / fm::kSuperBatches + 2));
-        fm::HudsonEpilogue e{};
-        e.variant = dense_variant(g1->m);
-        e.part_d = pd.p;
-        e.part_u = pu.p;
-        fm::PassParams<2> P{};
-        P.g[0] = planes_of(g1);
-        P.g[1] = planes_of(g2);
-        P.geom = G;
-        P.hud = e;
-        EventPairs evs;
-        std::vector<std::pair<cudaEvent_t, cudaEvent_t>> spans;
-        cudaEvent_t t0 = evs.next(), t1 = evs.next();
-        CK(cudaStreamSynchronize(stream()));
-        CK(cudaEventRecord(t0, stream()));
-        for (int it = 0; it < iterations; ++it) {
-            cudaEvent_t a = evs.next(), b = evs.next();
-            CK(cudaEventRecord(a, stream()));
-            launch_plane_pass<2>(P, g1->m->device);
-            CK(cudaEventRecord(b, stream()));
-            spans.emplace_back(a, b);
-            out->plane_launches++;
-            if (G.n_batches) {
-                launch_reduce(pd.p, 5, pu.p, 3, G, sd.p, su.p);
-                out->other_launches++;
-            }
-        }
-        CK(cudaEventRecord(t1, stream()));
-        CK(cudaEventSynchronize(t1));
-        float total = 0.f, plane = 0.f;
-        CK(cudaEventElapsedTime(&total, t0, t1));
-        for (auto &sp : spans) {
-            float t = 0.f;
-            CK(cudaEventElapsedTime(&t, sp.first, sp.second));
-            plane += t;
-        }
-        out->step_ms_avg = total / (float)iterations;
-        out->plane_ms_avg = plane / (float)spans.size();
-        out->plane_bytes_per_step = (uint64_t)V * (plane_site_bytes(P.g[0]) + plane_site_bytes(P.g[1]));
     });
 }
 

@@ -1,11 +1,12 @@
 // fm_kernels.cuh -- sm_100a kernels of the per-site estimator path.
 //
-//   K1  fm_k_repack           u8 matrix (+ missing bitmap)  ->  per-group bitplanes
-//   K2  fm_k_plane_pass<1>    one group's planes  -> alt/called counts, pi/theta tracks, S, sum pi
-//   K3  fm_k_plane_pass<2>    two groups' planes  -> both counts + fused Hudson components
+//   K1  fm_k_repack              u8 matrix (+ missing bitmap)  ->  per-group bitplanes
+//   K2  fm_k_plane_pass_seq      a list of (group, site range) segments, one group or a Hudson pair per unit
+//                                -> alt/called counts, pi/theta tracks, S, sum pi (+ fused Hudson components)
+//   K2c fm_k_plane_pass_chunked  one group with rows wider than a warp's ring, streamed in column chunks
 //   K2'/K3' light kernels evaluating estimators from cached count arrays
-//   K5  fm_k_window_*         segmented (window) reductions
-//   fm_k_reduce_partials      deterministic second-level reduction of per-batch partials
+//   K5  fm_k_window_*            segmented (window) reductions
+//   fm_k_reduce_partials         deterministic second-level reduction of per-batch partials
 //
 // The plane pass is a persistent kernel: every warp owns a private ring of shared-memory
 // stages filled by 1-D TMA bulk copies (cp.async.bulk + mbarrier) and consumes them with
@@ -637,11 +638,8 @@ __device__ __forceinline__ void fm_tail_add(const TailRegs &t, uint32_t &alt, ui
 }
 
 struct PassGeom {
-    uint32_t lps;         // lanes per site: 1,2,4,...,32 (power of two)
-    uint32_t lps_log2;
-    uint32_t rounds;      // rounds of (32/lps) sites held by one pipeline step (power of two <= lps)
-    uint32_t n_chunks;    // column chunks per row (1 unless lps == 32)
-    uint32_t cq;          // chunk width in uint4 (chunked mode)
+    uint32_t n_chunks;    // column chunks per row (chunked pass)
+    uint32_t cq;          // chunk width in uint4 (chunked pass)
     uint32_t n_stages;    // pipeline depth of the per-warp ring (2..kMaxStages)
     uint32_t stage_bytes; // bytes reserved per stage (multiple of 128)
     uint32_t warp_smem_bytes;  // private staging ring of one warp (n_stages * stage_bytes <= this)
@@ -650,10 +648,9 @@ struct PassGeom {
     uint32_t b_lo, n_batches;  // global batch range (batch b = sites [32b, 32b+32))
     uint32_t n_sites_total;    // V (rows available in the planes)
     uint32_t *batch_counter;   // dynamic scheduler counters (zeroed before launch)
-    uint32_t debug;            // tuning only: bit0 skip epilogue, bit1 skip column loop
 };
 
-// Diversity epilogue (NG == 1): build_dense_population_summary (stats.rs:1367-1470) +
+// Diversity epilogue: build_dense_population_summary (stats.rs:1367-1470) +
 // calculate_per_site_diversity (stats.rs:4693-4750) fused.
 struct DivEpilogue {
     uint32_t *alt_out, *called_out;  // [V] or nullptr
@@ -670,9 +667,8 @@ struct DivEpilogue {
     uint32_t *part_u;                // [n_batches][2]: segregating sites, sites with called < 2
 };
 
-// Hudson epilogue (NG == 2).
+// Hudson epilogue of a pair of groups.
 struct HudsonEpilogue {
-    uint32_t *alt_out[2], *called_out[2];  // cached count arrays or nullptr
     int variant;                           // FM_HV_* (per-site form) or -1 for the summaries form
     double *fst, *dxy, *pi1, *pi2, *num, *den;  // per-site [v_hi - v_lo] or nullptr
     uint32_t *n1_out, *n2_out;
@@ -849,30 +845,143 @@ __device__ __forceinline__ void fm_hudson_contrib(const HudsonEpilogue &e, uint3
     }
 }
 
-template <int NG>
-struct PassParams {
-    GroupPlanes g[NG];
-    PassGeom geom;
-    DivEpilogue div;     // used when NG == 1
-    HudsonEpilogue hud;  // used when NG == 2
+// ------------------------------------------------------------------------------ plane pass: shared pieces
+// Both plane-pass kernels are persistent: every warp owns a private ring of n_stages shared-memory stages with one
+// mbarrier each.  Lane 0 fills a stage with one TMA bulk copy and the whole warp waits on its barrier phase.
+__device__ __forceinline__ void fm_ring_init(uint32_t bar_base, uint32_t n_stages, uint32_t lane) {
+    if (lane == 0) {
+        for (uint32_t s = 0; s < n_stages; ++s)
+            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_base + 8u * s));
+        fm_fence_mbar_init();
+    }
+    __syncwarp();
+}
+
+// lane 0: copy `bytes` from global memory into the stage at `dst`, completing on the stage's barrier `bar`;
+// bytes == 0 (a step past the last row) completes the phase with a plain arrive
+__device__ __forceinline__ void fm_ring_fill(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar) {
+    if (bytes == 0) {
+        asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
+        return;
+    }
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
+                 "l"(src), "r"(bytes), "r"(bar)
+                 : "memory");
+}
+
+__device__ __forceinline__ void fm_ring_wait(uint32_t bar, uint32_t parity) {
+    uint32_t ok;
+    do {
+        asm volatile(
+            "{\n\t.reg .pred p;\n\t"
+            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
+            "selp.u32 %0, 1, 0, p;\n\t}"
+            : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
+    } while (!ok);
+}
+
+// Dynamic batch scheduler of one warp.  The batch range [0, n_batches) is split over kSchedCounters counters; a
+// warp starts on its CTA's home range and steals from the others.  The issue side claims batches and the consume
+// side replays the same sequence from a small per-warp ring.  Partials are keyed by the batch index, so the
+// result does not depend on which warp processed which batch.  The atomic is fired one batch ahead so its round
+// trip never sits on the critical path.
+struct BatchScheduler {
+    uint32_t *counters;
+    uint32_t n_batches, j, tried, prefetched;
+    __device__ __forceinline__ BatchScheduler(uint32_t *c, uint32_t nb, uint32_t lane)
+        : counters(c), n_batches(nb), j(blockIdx.x % kSchedCounters), tried(0), prefetched(0) {
+        if (lane == 0) prefetched = atomicAdd(counters + j * kSchedStrideWords, 1u);
+    }
+    __device__ __forceinline__ uint32_t range_lo(uint32_t k) const {
+        return (uint32_t)(((uint64_t)n_batches * k) / kSchedCounters);
+    }
+    // next batch of the launch (warp-uniform), or 0xffffffff once every range is drained
+    __device__ __forceinline__ uint32_t claim(uint32_t lane) {
+        for (;;) {
+            const uint32_t idx = __shfl_sync(0xffffffffu, prefetched, 0);
+            const uint32_t lo = range_lo(j), hi = range_lo(j + 1);
+            if (idx < hi - lo) {  // fire the next claim on the same range, one batch ahead
+                if (lane == 0) prefetched = atomicAdd(counters + j * kSchedStrideWords, 1u);
+                return lo + idx;
+            }
+            if (++tried == kSchedCounters) return 0xffffffffu;
+            j = (j + 1 == kSchedCounters) ? 0 : j + 1;
+            if (lane == 0) prefetched = atomicAdd(counters + j * kSchedStrideWords, 1u);
+        }
+    }
 };
 
-// Specialisations: NG groups, LG = log2(lanes per site) (LG == 5 is the column-chunked mode for
-// rows wider than a pipeline step).
-//
-// Non-chunked geometry: a pipeline step holds `rounds` x SPS consecutive sites (SPS = 32/LPS);
-// in every round LPS consecutive lanes read consecutive uint4 of one row, so a quarter-warp
-// always touches one contiguous 128-byte span (bank-conflict free without padding).
-template <int NG, int LG>
+// Diversity epilogue of one batch, lane i <-> site v = 32b + i (all 32 lanes active): the per-site values of the
+// sites in [v_lo, v_hi), then the batch's partials at index bl.
+__device__ __forceinline__ void fm_div_batch(const DivEpilogue &e, uint32_t v, uint32_t v_lo, uint32_t v_hi,
+                                             uint32_t bl, uint32_t lane, uint32_t n, uint32_t alt) {
+    double pi_part = 0.0;
+    uint32_t seg = 0, unc = 0;
+    const uint32_t flags = e.site_flags ? __ldg(e.site_flags + bl) : 0u;
+    if (v >= v_lo && v < v_hi) fm_div_site(e, v, v_lo, n, alt, (flags >> lane) & 1u, pi_part, seg, unc);
+    const double s_pi = fm_warp_sum(pi_part);
+    const uint32_t s_u = fm_warp_sum_u(seg | (unc << 16));
+    if (lane == 0) {
+        e.part_pi[bl] = s_pi;
+        e.part_u[2 * bl] = s_u & 0xffffu;
+        e.part_u[2 * bl + 1] = s_u >> 16;
+    }
+}
+
+// ------------------------------------------------------------------------------ plane pass, rows
+// fm_k_plane_pass_seq: one persistent launch streams a LIST of plane segments.  A unit is one segment or, in the PAIR
+// instances, two segments over the same sites:
+//   * one segment per unit: independent (group, site range) units share one launch -- the groups of one per-site call, the
+//     per-region matrices the CLI builds one after the other (process.rs:2169), each with its own population --
+//     so many small passes stream at the rate of one large one, and the launch ramp-up and the end-of-kernel
+//     quantisation are paid once;
+//   * PAIR: a warp streams the batch of group 1, keeps its counts in registers, streams the same batch of
+//     group 2 and evaluates the Hudson components of the 32 sites in place (stats.rs:3179-3278 / 1554-1623) --
+//     both groups' counts and summary partials AND the Hudson partials from one sweep of the planes.
+// The batch index space is the concatenation of the units' batch ranges.  A step holds `rounds` x SPS consecutive
+// sites of one segment (SPS = 32/LPS sites per round); in every round LPS consecutive lanes read consecutive uint4
+// of one row, so a quarter-warp always touches one contiguous 128-byte span (bank-conflict free without padding).
+constexpr int kMaxSeq = 4;  // segments carried in the kernel parameters (no descriptor upload)
+
+struct RowSeg {
+    GroupPlanes g;
+    DivEpilogue div;          // div.part_pi == nullptr: no diversity epilogue
+    uint32_t rounds;          // rounds of (32/lps) sites per pipeline step for this segment's row width
+    uint32_t v_lo, v_hi;      // site range analysed
+    uint32_t b_lo;            // first batch of the range (v_lo / 32)
+    uint32_t n_sites_total;   // rows available in this segment's planes
+    uint32_t pad;
+};
+
+struct RowParams {
+    const RowSeg *segs;            // [n_units] (one segment per unit; the PAIR instances use the inline table only)
+    const uint32_t *unit_prefix;   // [n_units + 1]: batches of the units before u (unit u has prefix[u+1]-prefix[u])
+    uint32_t n_units;
+    PassGeom geom;                 // n_stages, stage_bytes, warp_smem_bytes, n_batches (whole launch), counters
+    // up to kMaxSeq segments travel in the kernel parameters themselves: a descriptor upload is three small H2D
+    // copies (~20 us of a 250 us sharded step).  The INLINE instances read these instead of the pointers above.
+    RowSeg inline_segs[kMaxSeq];
+    HudsonEpilogue inline_hud[kMaxSeq / 2];  // PAIR: one Hudson epilogue per unit
+    uint32_t inline_prefix[kMaxSeq + 1];
+};
+static_assert(sizeof(RowParams) <= 4096, "the row-pass parameters must fit the 4 KB kernel parameter space");
+
+// INLINE: the table is read from the kernel parameters.  Those reads compile to constant-bank loads, which keep
+// the per-batch segment lookups off the critical path; a pointer that may address either the parameters or global
+// memory makes every one of them a generic load (that form took 10 % longer per bench step on a B200:
+// profiles/r04_ab_one_table_variant.txt).  PAIR: two segments per unit and the Hudson epilogue; the one-segment
+// instances compile without them (the bench step and single groups run the smaller kernel).
+template <int LG, bool INLINE, bool PAIR>
 __global__ void __launch_bounds__(kWarpsPerCta * 32, 1)
-fm_k_plane_pass(const __grid_constant__ PassParams<NG> P) {
+fm_k_plane_pass_seq(const __grid_constant__ RowParams P) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t bars[kWarpsPerCta * kMaxStages];
     __shared__ uint32_t batch_ring[kWarpsPerCta * kBatchRing];
-
-    constexpr uint32_t LPS = 1u << LG;       // lanes per site
-    constexpr uint32_t SPS = 32u >> LG;      // sites per round
-    constexpr bool CHUNKED = (LG == 5);
+    static_assert(LG < 5, "column-chunked rows take fm_k_plane_pass_chunked");
+    static_assert(INLINE || !PAIR, "pair units travel in the kernel parameters");
+    constexpr uint32_t LPS = 1u << LG;
+    constexpr uint32_t SPS = 32u >> LG;
     constexpr uint32_t FULL = 0xffffffffu;
 
     const uint32_t lane = threadIdx.x & 31;
@@ -882,576 +991,26 @@ fm_k_plane_pass(const __grid_constant__ PassParams<NG> P) {
     const PassGeom &G = P.geom;
     const uint32_t n_stages = G.n_stages;
     const uint32_t stage_bytes = G.stage_bytes;
-    const uint32_t n_sites_total = G.n_sites_total;
-    const uint32_t n_batches = G.n_batches;
-    const uint32_t n_chunks = CHUNKED ? G.n_chunks : 1u;
-    const uint32_t cq = G.cq;
-    const uint32_t rounds = CHUNKED ? 1u : G.rounds;
-    const uint32_t step_sites = CHUNKED ? 1u : SPS * rounds;
-    const uint32_t spb = CHUNKED ? 32u * n_chunks : LPS / rounds;  // steps per batch
-
-    uint32_t wq16[NG];  // row bytes per plane
-#pragma unroll
-    for (int g = 0; g < NG; ++g) wq16[g] = P.g[g].wq * 16u;
-
-    const uint32_t smem_base = fm_smem_u32(smem_raw) + warp * G.warp_smem_bytes;
-    const uint32_t bar_base = fm_smem_u32(bars + warp * kMaxStages);
-    uint32_t *my_ring = batch_ring + warp * kBatchRing;
-    if (lane == 0) {
-        for (uint32_t s = 0; s < n_stages; ++s)
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_base + 8u * s));
-        fm_fence_mbar_init();
-    }
-    __syncwarp();
-
-    // ---- dynamic batch scheduler: the issue side claims batches, the consume side replays the
-    // same sequence from a small per-warp ring.  Partials are keyed by the batch index, so the
-    // result does not depend on which warp processed which batch.
-    // The atomic is fired one batch ahead so its round trip never sits on the critical path.
-    uint32_t sched_j = blockIdx.x % kSchedCounters, sched_tried = 0;
-    auto range_lo = [&](uint32_t j) { return (uint32_t)(((uint64_t)n_batches * j) / kSchedCounters); };
-    uint32_t prefetched = 0;
-    if (lane == 0) prefetched = atomicAdd(G.batch_counter + sched_j * kSchedStrideWords, 1u);
-    auto claim = [&]() -> uint32_t {
-        for (;;) {
-            const uint32_t idx = __shfl_sync(FULL, prefetched, 0);
-            const uint32_t lo = range_lo(sched_j), hi = range_lo(sched_j + 1);
-            if (idx < hi - lo) {  // fire the next claim on the same range, one batch ahead
-                if (lane == 0) prefetched = atomicAdd(G.batch_counter + sched_j * kSchedStrideWords, 1u);
-                return lo + idx;
-            }
-            if (++sched_tried == kSchedCounters) return 0xffffffffu;  // every range is drained
-            sched_j = (sched_j + 1 == kSchedCounters) ? 0 : sched_j + 1;
-            if (lane == 0) prefetched = atomicAdd(G.batch_counter + sched_j * kSchedStrideWords, 1u);
-        }
-    };
-
-    // issue the TMA bulk copies of step k of local batch `bl` into `stage` (lane 0 only)
-    auto issue = [&](uint32_t bl, uint32_t k, uint32_t stage) {
-        const uint32_t b = G.b_lo + bl;
-        const uint32_t bar = bar_base + 8u * stage;
-        uint32_t dst = smem_base + stage * stage_bytes;
-        if constexpr (CHUNKED) {
-            const uint32_t v0 = b * 32 + k / n_chunks;
-            const uint32_t c0 = (k % n_chunks) * cq;
-            uint32_t bytes[NG], total = 0;
-#pragma unroll
-            for (int g = 0; g < NG; ++g) {
-                const uint32_t w = P.g[g].wq;
-                bytes[g] = (v0 < n_sites_total && c0 < w) ? min(cq, w - c0) * 16u : 0u;
-                total += bytes[g];
-            }
-            if (total == 0) {
-                asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-                return;
-            }
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(total) : "memory");
-#pragma unroll
-            for (int g = 0; g < NG; ++g) {
-                if (bytes[g]) {
-                    const size_t src = (size_t)v0 * P.g[g].wq + c0;
-                    asm volatile(
-                        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::
-                            "r"(dst), "l"(P.g[g].allele + src), "r"(bytes[g]), "r"(bar) : "memory");
-                }
-                dst += cq * 16u;
-            }
-        } else {
-            const uint32_t v0 = b * 32 + k * step_sites;
-            const uint32_t nsites = (v0 < n_sites_total) ? min(step_sites, n_sites_total - v0) : 0u;
-            if (nsites == 0) {  // batch tail beyond V: complete the phase with a plain arrive
-                asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-                return;
-            }
-            uint32_t total = 0;
-#pragma unroll
-            for (int g = 0; g < NG; ++g) total += nsites * wq16[g];
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(total) : "memory");
-#pragma unroll
-            for (int g = 0; g < NG; ++g) {
-                const uint32_t bytes = nsites * wq16[g];
-                const uint32_t slot = step_sites * wq16[g];
-                const size_t off = (size_t)v0 * wq16[g];
-                asm volatile(
-                    "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::
-                        "r"(dst), "l"(reinterpret_cast<const uint8_t *>(P.g[g].allele) + off), "r"(bytes), "r"(bar)
-                    : "memory");
-                dst += slot;
-            }
-        }
-    };
-
-    // issue cursor (uniform across the warp)
-    uint32_t iss_ring = 0, iss_k = spb, iss_stage = 0, iss_batch = 0;
-    auto issue_next = [&]() {
-        if (iss_k == spb) {
-            if (iss_ring != 0 && iss_batch >= n_batches) return;  // scheduler drained
-            iss_batch = claim();
-            iss_k = 0;
-            if (lane == 0) my_ring[iss_ring & (kBatchRing - 1)] = iss_batch;
-            ++iss_ring;
-            if (iss_batch >= n_batches) {
-                iss_k = spb;
-                return;
-            }
-        }
-        if (lane == 0) issue(iss_batch, iss_k, iss_stage);
-        ++iss_k;
-        iss_stage = (iss_stage + 1 == n_stages) ? 0 : iss_stage + 1;
-    };
-    for (uint32_t s = 0; s < n_stages; ++s) issue_next();
-    __syncwarp();
-
-    // alt count of this lane's batch site
-    uint32_t site_a[NG], acc_a[NG];
-#pragma unroll
-    for (int g = 0; g < NG; ++g) site_a[g] = acc_a[g] = 0;
-
-    const uint32_t slot_in_round = lane >> LG;
-    const uint32_t phase = lane & (LPS - 1);
-    const uint32_t xfer_from = (lane & (SPS - 1)) << LG;          // source lane of the transpose
-    const uint32_t xfer_round = CHUNKED ? 0u : (lane >> (5 - LG));  // round whose sites land here
-
-    uint32_t plane_off[NG];  // byte offset of group g's allele plane inside a stage
-    uint32_t nit_full[NG];   // column iterations that are in range for every lane
-    uint32_t last_cols[NG];  // lanes (phases) that still have a column in the last iteration
-    {
-        uint32_t acc = 0;
-#pragma unroll
-        for (int g = 0; g < NG; ++g) {
-            plane_off[g] = acc;
-            acc += CHUNKED ? cq * 16u : step_sites * wq16[g];
-            const uint32_t w = P.g[g].wq;
-            const uint32_t nit = (w + LPS - 1) / LPS;
-            nit_full[g] = nit - 1;
-            last_cols[g] = w - (nit - 1) * LPS;
-        }
-    }
-
-    uint32_t con_ring = 0, stage = 0, parity = 0;
-    for (;;) {
-        const uint32_t bl = my_ring[con_ring & (kBatchRing - 1)];
-        ++con_ring;
-        if (bl >= n_batches) break;
-        const uint32_t b = G.b_lo + bl;
-        TailRegs tails[NG];
-#pragma unroll
-        for (int g = 0; g < NG; ++g) fm_tail_load(P.g[g], b * 32 + lane, n_sites_total, tails[g]);
-        for (uint32_t k = 0; k < spb; ++k) {
-            {
-                const uint32_t bar = bar_base + 8u * stage;
-                uint32_t ok;
-                do {
-                    asm volatile(
-                        "{\n\t.reg .pred p;\n\t"
-                        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-                        "selp.u32 %0, 1, 0, p;\n\t}"
-                        : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-                } while (!ok);
-            }
-            const uint32_t sbase = smem_base + stage * stage_bytes;
-            if constexpr (!CHUNKED) {
-                const uint32_t v0 = b * 32 + k * step_sites;
-                auto round_body = [&](uint32_t r) {
-                    const uint32_t site_local = r * SPS + slot_in_round;
-                    const bool live = (v0 + site_local) < n_sites_total;
-#pragma unroll
-                    for (int g = 0; g < NG; ++g) {
-                        const uint32_t w16 = wq16[g];
-                        const uint32_t ra = sbase + plane_off[g] + site_local * w16;
-                        uint32_t a = 0;
-                        if (live && !(G.debug & 2u)) {
-                            // columns phase, phase+LPS, ...: the first nit-1 are inside the row for
-                            // every lane, only the last one needs a bound check
-                            uint32_t p = ra + phase * 16u;
-                            const uint32_t nfull = nit_full[g];
-#pragma unroll 2
-                            for (uint32_t j = 0; j < nfull; ++j) {
-                                a += fm_popc4(fm_lds128(p));
-                                p += LPS * 16u;
-                            }
-                            if (phase < last_cols[g]) a += fm_popc4(fm_lds128(p));
-                        }
-#pragma unroll
-                        for (uint32_t o = LPS >> 1; o > 0; o >>= 1) a += __shfl_xor_sync(FULL, a, o);
-                        const uint32_t t = __shfl_sync(FULL, a, xfer_from);
-                        if (xfer_round == k * rounds + r) site_a[g] = t;
-                    }
-                };
-                if (rounds == 1) {
-                    round_body(0);
-                } else {
-                    for (uint32_t r = 0; r < rounds; r += 2) {  // rounds is a power of two
-                        round_body(r);
-                        round_body(r + 1);
-                    }
-                }
-            } else {
-                const uint32_t site_in_batch = k / n_chunks;
-                const uint32_t ck = k - site_in_batch * n_chunks;
-                const uint32_t c0 = ck * cq;
-                const bool live = (b * 32 + site_in_batch) < n_sites_total;
-#pragma unroll
-                for (int g = 0; g < NG; ++g) {
-                    const uint32_t w = P.g[g].wq;
-                    const uint32_t cols16 = (c0 < w) ? min(cq, w - c0) * 16u : 0u;
-                    const uint32_t ra = sbase + plane_off[g];
-                    if (live) {
-#pragma unroll 2
-                        for (uint32_t u = lane * 16u; u < cols16; u += 512u) acc_a[g] += fm_popc4(fm_lds128(ra + u));
-                    }
-                    if (ck == n_chunks - 1) {
-                        const uint32_t ta = fm_warp_sum_u(acc_a[g]);
-                        if (lane == site_in_batch) site_a[g] = ta;
-                        acc_a[g] = 0;
-                    }
-                }
-            }
-            __syncwarp();   // every lane is done reading this stage
-            issue_next();   // refill it with the step n_stages ahead
-            stage = (stage + 1 == n_stages) ? 0 : stage + 1;
-            parity ^= (stage == 0);
-        }
-        // ---- batch epilogue: lane i <-> site 32b + i, all 32 lanes active
-        {
-            uint32_t alt[NG], cnt[NG];
-#pragma unroll
-            for (int g = 0; g < NG; ++g) {
-                alt[g] = site_a[g];
-                fm_tail_add(tails[g], alt[g], cnt[g]);
-            }
-            const uint32_t v = b * 32 + lane;
-            const bool valid = (v >= G.v_lo) && (v < G.v_hi);
-            if constexpr (NG == 1) {
-                double pi_part = 0.0;
-                uint32_t seg = 0, unc = 0;
-                const uint32_t flags = P.div.site_flags ? __ldg(P.div.site_flags + bl) : 0u;
-                if (valid && !(G.debug & 1u))
-                    fm_div_site(P.div, v, G.v_lo, cnt[0], alt[0], (flags >> lane) & 1u, pi_part, seg, unc);
-                const double s_pi = fm_warp_sum(pi_part);
-                const uint32_t s_u = fm_warp_sum_u(seg | (unc << 16));
-                if (lane == 0) {
-                    P.div.part_pi[bl] = s_pi;
-                    P.div.part_u[2 * bl] = s_u & 0xffffu;
-                    P.div.part_u[2 * bl + 1] = s_u >> 16;
-                }
-            } else {
-                HudsonAcc acc{0.0, 0.0, 0.0, 0.0, 0.0, 0u, 0u, 0u};
-                if (valid) {
-                    fm_hudson_contrib(P.hud, v, G.v_lo, cnt[0], alt[0], cnt[1], alt[1], acc);
-#pragma unroll
-                    for (int g = 0; g < NG; ++g) {
-                        if (P.hud.alt_out[g]) P.hud.alt_out[g][v] = alt[g];
-                        if (P.hud.called_out[g]) P.hud.called_out[g][v] = cnt[g];
-                    }
-                }
-                const double r0 = fm_warp_sum(acc.num), r1 = fm_warp_sum(acc.den),
-                             r2 = fm_warp_sum(acc.dxy), r3 = fm_warp_sum(acc.pi1),
-                             r4 = fm_warp_sum(acc.pi2);
-                const uint32_t u01 = fm_warp_sum_u(acc.skipped | (acc.unc1 << 8) | (acc.unc2 << 16));
-                if (lane == 0) {
-                    double *pd = P.hud.part_d + (size_t)bl * 5;
-                    pd[0] = r0; pd[1] = r1; pd[2] = r2; pd[3] = r3; pd[4] = r4;
-                    uint32_t *pu = P.hud.part_u + (size_t)bl * 3;
-                    pu[0] = u01 & 0xffu; pu[1] = (u01 >> 8) & 0xffu; pu[2] = u01 >> 16;
-                }
-            }
-        }
-    }
-}
-
-// ------------------------------------------------------------------------------ plane pass, several groups
-// fm_k_plane_pass_seq: ONE persistent launch streams the planes of up to kMaxSeq groups one after
-// the other over the same site range (the two orientation groups of a per-site diversity call).
-// Same per-warp TMA rings, same dynamic scheduler and the same per-batch arithmetic as
-// fm_k_plane_pass<1>; the batch index space is the concatenation of the groups' batch ranges, so
-// the launch ramp-up and the end-of-kernel quantisation (a warp's last batch) are paid once, not
-// once per group, and the finer batches of the smallest group fill the tail.
-constexpr int kMaxSeq = 4;
-
-struct SeqGroup {
-    GroupPlanes g;
-    DivEpilogue div;
-    uint32_t rounds;  // rounds of (32/lps) sites per pipeline step for this group's row width
-};
-
-struct SeqParams {
-    SeqGroup seg[kMaxSeq];
-    uint32_t n_seg;
-    PassGeom geom;  // lps, n_stages, stage_bytes (max over groups), warps, site range, scheduler counters
-};
-
-template <int LG>
-__global__ void __launch_bounds__(kWarpsPerCta * 32, 1)
-fm_k_plane_pass_seq(const __grid_constant__ SeqParams P) {
-    extern __shared__ __align__(128) uint8_t smem_raw[];
-    __shared__ __align__(8) uint64_t bars[kWarpsPerCta * kMaxStages];
-    __shared__ uint32_t batch_ring[kWarpsPerCta * kBatchRing];
-    static_assert(LG < 5, "column-chunked rows take the per-group kernel");
-    constexpr uint32_t LPS = 1u << LG;
-    constexpr uint32_t SPS = 32u >> LG;
-    constexpr uint32_t FULL = 0xffffffffu;
-
-    const uint32_t lane = threadIdx.x & 31;
-    const uint32_t warp = __shfl_sync(FULL, threadIdx.x >> 5, 0);
-    const PassGeom &G = P.geom;
-    const uint32_t n_stages = G.n_stages;
-    const uint32_t stage_bytes = G.stage_bytes;
-    const uint32_t n_sites_total = G.n_sites_total;
-    const uint32_t nb_seg = G.n_batches;              // batches per group (same site range for all)
-    const uint32_t n_batches = nb_seg * P.n_seg;      // concatenated batch space
-
-    const uint32_t smem_base = fm_smem_u32(smem_raw) + warp * G.warp_smem_bytes;
-    const uint32_t bar_base = fm_smem_u32(bars + warp * kMaxStages);
-    uint32_t *my_ring = batch_ring + warp * kBatchRing;
-    if (lane == 0) {
-        for (uint32_t s = 0; s < n_stages; ++s)
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_base + 8u * s));
-        fm_fence_mbar_init();
-    }
-    __syncwarp();
-
-    uint32_t sched_j = blockIdx.x % kSchedCounters, sched_tried = 0;
-    auto range_lo = [&](uint32_t j) { return (uint32_t)(((uint64_t)n_batches * j) / kSchedCounters); };
-    uint32_t prefetched = 0;
-    if (lane == 0) prefetched = atomicAdd(G.batch_counter + sched_j * kSchedStrideWords, 1u);
-    auto claim = [&]() -> uint32_t {
-        for (;;) {
-            const uint32_t idx = __shfl_sync(FULL, prefetched, 0);
-            const uint32_t lo = range_lo(sched_j), hi = range_lo(sched_j + 1);
-            if (idx < hi - lo) {
-                if (lane == 0) prefetched = atomicAdd(G.batch_counter + sched_j * kSchedStrideWords, 1u);
-                return lo + idx;
-            }
-            if (++sched_tried == kSchedCounters) return 0xffffffffu;
-            sched_j = (sched_j + 1 == kSchedCounters) ? 0 : sched_j + 1;
-            if (lane == 0) prefetched = atomicAdd(G.batch_counter + sched_j * kSchedStrideWords, 1u);
-        }
-    };
-
-    // ---- issue side: per-group context of the batch being issued
-    uint32_t iss_ring = 0, iss_k = 0, iss_spb = 0, iss_stage = 0, iss_batch = 0;
-    uint32_t iss_w16 = 0, iss_step_sites = 1, iss_seg = 0, iss_lb = 0;
-    auto issue = [&](uint32_t stage) {  // lane 0 only: TMA bulk copies of step iss_k of batch iss_lb of group iss_seg
-        const uint32_t bar = bar_base + 8u * stage;
-        const uint32_t dst = smem_base + stage * stage_bytes;
-        const uint32_t v0 = (G.b_lo + iss_lb) * 32 + iss_k * iss_step_sites;
-        const uint32_t nsites = (v0 < n_sites_total) ? min(iss_step_sites, n_sites_total - v0) : 0u;
-        if (nsites == 0) {
-            asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-            return;
-        }
-        const uint32_t bytes = nsites * iss_w16;
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-        const size_t off = (size_t)v0 * iss_w16;
-        const GroupPlanes &gp = P.seg[iss_seg].g;
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
-                     "l"(reinterpret_cast<const uint8_t *>(gp.allele) + off), "r"(bytes), "r"(bar)
-                     : "memory");
-    };
-    auto issue_next = [&]() {
-        if (iss_k == iss_spb) {
-            if (iss_ring != 0 && iss_batch >= n_batches) return;  // scheduler drained
-            iss_batch = claim();
-            iss_k = 0;
-            if (lane == 0) my_ring[iss_ring & (kBatchRing - 1)] = iss_batch;
-            ++iss_ring;
-            if (iss_batch >= n_batches) {
-                iss_spb = 0;
-                return;
-            }
-            iss_seg = iss_batch / nb_seg;
-            iss_lb = iss_batch - iss_seg * nb_seg;
-            const uint32_t r = P.seg[iss_seg].rounds;
-            iss_w16 = P.seg[iss_seg].g.wq * 16u;
-            iss_step_sites = SPS * r;
-            iss_spb = LPS / r;
-        }
-        if (lane == 0) issue(iss_stage);
-        ++iss_k;
-        iss_stage = (iss_stage + 1 == n_stages) ? 0 : iss_stage + 1;
-    };
-    for (uint32_t s = 0; s < n_stages; ++s) issue_next();
-    __syncwarp();
-
-    const uint32_t slot_in_round = lane >> LG;
-    const uint32_t phase = lane & (LPS - 1);
-    const uint32_t xfer_from = (lane & (SPS - 1)) << LG;
-    const uint32_t xfer_round = lane >> (5 - LG);
-
-    uint32_t con_ring = 0, stage = 0, parity = 0;
-    for (;;) {
-        const uint32_t gb = my_ring[con_ring & (kBatchRing - 1)];
-        ++con_ring;
-        if (gb >= n_batches) break;
-        // ---- consume side: this batch's group
-        const uint32_t sg = gb / nb_seg;
-        const uint32_t bl = gb - sg * nb_seg;
-        const SeqGroup &S = P.seg[sg];
-        const uint32_t w = S.g.wq, w16 = w * 16u, rounds = S.rounds;
-        const uint32_t step_sites = SPS * rounds, spb = LPS / rounds;
-        const uint32_t nit = (w + LPS - 1) / LPS;
-        const uint32_t nfull = nit - 1, last_cols = w - nfull * LPS;
-        const uint32_t b = G.b_lo + bl;
-        uint32_t site_a = 0;
-        TailRegs tails;
-        fm_tail_load(S.g, b * 32 + lane, n_sites_total, tails);
-        for (uint32_t k = 0; k < spb; ++k) {
-            {
-                const uint32_t bar = bar_base + 8u * stage;
-                uint32_t ok;
-                do {
-                    asm volatile(
-                        "{\n\t.reg .pred p;\n\t"
-                        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-                        "selp.u32 %0, 1, 0, p;\n\t}"
-                        : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-                } while (!ok);
-            }
-            const uint32_t sbase = smem_base + stage * stage_bytes;
-            const uint32_t v0 = b * 32 + k * step_sites;
-            auto round_body = [&](uint32_t r) {
-                const uint32_t site_local = r * SPS + slot_in_round;
-                const bool live = (v0 + site_local) < n_sites_total;
-                const uint32_t ra = sbase + site_local * w16;
-                uint32_t a = 0;
-                if (live) {
-                    uint32_t p = ra + phase * 16u;
-#pragma unroll 2
-                    for (uint32_t j = 0; j < nfull; ++j) {
-                        a += fm_popc4(fm_lds128(p));
-                        p += LPS * 16u;
-                    }
-                    if (phase < last_cols) a += fm_popc4(fm_lds128(p));
-                }
-#pragma unroll
-                for (uint32_t o = LPS >> 1; o > 0; o >>= 1) a += __shfl_xor_sync(FULL, a, o);
-                const uint32_t t = __shfl_sync(FULL, a, xfer_from);
-                if (xfer_round == k * rounds + r) site_a = t;
-            };
-            if (rounds == 1) {
-                round_body(0);
-            } else {
-                for (uint32_t r = 0; r < rounds; r += 2) {
-                    round_body(r);
-                    round_body(r + 1);
-                }
-            }
-            __syncwarp();
-            issue_next();
-            stage = (stage + 1 == n_stages) ? 0 : stage + 1;
-            parity ^= (stage == 0);
-        }
-        // ---- batch epilogue: lane i <-> site 32b + i
-        {
-            uint32_t alt = site_a, cnt;
-            fm_tail_add(tails, alt, cnt);
-            const uint32_t v = b * 32 + lane;
-            const bool valid = (v >= G.v_lo) && (v < G.v_hi);
-            double pi_part = 0.0;
-            uint32_t seg = 0, unc = 0;
-            const uint32_t flags = S.div.site_flags ? __ldg(S.div.site_flags + bl) : 0u;
-            if (valid) fm_div_site(S.div, v, G.v_lo, cnt, alt, (flags >> lane) & 1u, pi_part, seg, unc);
-            const double s_pi = fm_warp_sum(pi_part);
-            const uint32_t s_u = fm_warp_sum_u(seg | (unc << 16));
-            if (lane == 0) {
-                S.div.part_pi[bl] = s_pi;
-                S.div.part_u[2 * bl] = s_u & 0xffffu;
-                S.div.part_u[2 * bl + 1] = s_u >> 16;
-            }
-        }
-    }
-}
-
-// ------------------------------------------------------------------------------ plane pass, segment table
-// fm_k_plane_pass_tab: the same persistent per-warp-ring pass over an arbitrary LIST of plane segments read
-// from a descriptor table in device memory.  Two uses:
-//   * unit = one segment: many (region, group) pairs -- e.g. the per-region matrices the CLI builds one after
-//     the other (process.rs:2169), each with its own population -- share ONE launch, so 64 small regions stream
-//     at the rate of one large one instead of paying 64 launches + ramp-ups (SURVEY 8d: cfg1 x 64);
-//   * unit = two segments over the same sites (gpu == 2): a warp streams the batch of group 1, keeps its
-//     counts in registers, streams the same batch of group 2 and evaluates the Hudson components of the 32
-//     sites in place (stats.rs:3179-3278 / 1554-1623) -- both groups' counts and summary partials AND the
-//     Hudson partials from one sweep of the planes, each group streamed with its own step geometry.
-struct TabSeg {
-    GroupPlanes g;
-    DivEpilogue div;
-    uint32_t rounds;          // rounds of (32/lps) sites per pipeline step for this segment's row width
-    uint32_t v_lo, v_hi;      // site range analysed
-    uint32_t b_lo;            // first batch of the range (v_lo / 32)
-    uint32_t n_sites_total;   // rows available in this segment's planes
-    uint32_t pad;
-};
-
-struct TabParams {
-    const TabSeg *segs;            // [n_units * gpu]
-    const uint32_t *unit_prefix;   // [n_units + 1]: batches of the units before u (unit u has prefix[u+1]-prefix[u])
-    uint32_t n_units, gpu;         // gpu = segments (groups) per unit: 1 or 2
-    const HudsonEpilogue *hud;     // [n_units] Hudson epilogues (gpu == 2) or nullptr
-    PassGeom geom;                 // lps, n_stages, stage_bytes, warps, warp_smem_bytes, n_batches (total), counters
-    // a single unit travels in the kernel parameters themselves (no descriptor upload: three small H2D copies
-    // are ~20 us of a 250 us sharded step); use_inline selects these instead of the pointers above
-    uint32_t use_inline, has_inline_hud;
-    TabSeg inline_segs[2];
-    HudsonEpilogue inline_hud;
-    uint32_t inline_prefix[2];
-};
-
-template <int LG>
-__global__ void __launch_bounds__(kWarpsPerCta * 32, 1)
-fm_k_plane_pass_tab(const __grid_constant__ TabParams P) {
-    extern __shared__ __align__(128) uint8_t smem_raw[];
-    __shared__ __align__(8) uint64_t bars[kWarpsPerCta * kMaxStages];
-    __shared__ uint32_t batch_ring[kWarpsPerCta * kBatchRing];
-    static_assert(LG < 5, "column-chunked rows take the per-group kernel");
-    constexpr uint32_t LPS = 1u << LG;
-    constexpr uint32_t SPS = 32u >> LG;
-    constexpr uint32_t FULL = 0xffffffffu;
-
-    const uint32_t lane = threadIdx.x & 31;
-    const uint32_t warp = __shfl_sync(FULL, threadIdx.x >> 5, 0);
-    const PassGeom &G = P.geom;
-    const uint32_t n_stages = G.n_stages;
-    const uint32_t stage_bytes = G.stage_bytes;
     const uint32_t n_batches = G.n_batches;  // whole launch
-    const uint32_t gpu = P.gpu;
-    const TabSeg *const segs = P.use_inline ? P.inline_segs : P.segs;
-    const uint32_t *const unit_prefix = P.use_inline ? P.inline_prefix : P.unit_prefix;
-    const HudsonEpilogue *const hud = P.use_inline ? (P.has_inline_hud ? &P.inline_hud : nullptr) : P.hud;
+    constexpr uint32_t gpu = PAIR ? 2u : 1u;  // segments per unit
+    auto seg = [&](uint32_t i) -> const RowSeg & {
+        if constexpr (INLINE) return P.inline_segs[i]; else return P.segs[i];
+    };
+    auto prefix = [&](uint32_t u) -> uint32_t {
+        if constexpr (INLINE) return P.inline_prefix[u]; else return P.unit_prefix[u];
+    };
 
     const uint32_t smem_base = fm_smem_u32(smem_raw) + warp * G.warp_smem_bytes;
     const uint32_t bar_base = fm_smem_u32(bars + warp * kMaxStages);
     uint32_t *my_ring = batch_ring + warp * kBatchRing;
-    if (lane == 0) {
-        for (uint32_t s = 0; s < n_stages; ++s)
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_base + 8u * s));
-        fm_fence_mbar_init();
-    }
-    __syncwarp();
-
-    uint32_t sched_j = blockIdx.x % kSchedCounters, sched_tried = 0;
-    auto range_lo = [&](uint32_t j) { return (uint32_t)(((uint64_t)n_batches * j) / kSchedCounters); };
-    uint32_t prefetched = 0;
-    if (lane == 0) prefetched = atomicAdd(G.batch_counter + sched_j * kSchedStrideWords, 1u);
-    auto claim = [&]() -> uint32_t {
-        for (;;) {
-            const uint32_t idx = __shfl_sync(FULL, prefetched, 0);
-            const uint32_t lo = range_lo(sched_j), hi = range_lo(sched_j + 1);
-            if (idx < hi - lo) {
-                if (lane == 0) prefetched = atomicAdd(G.batch_counter + sched_j * kSchedStrideWords, 1u);
-                return lo + idx;
-            }
-            if (++sched_tried == kSchedCounters) return 0xffffffffu;
-            sched_j = (sched_j + 1 == kSchedCounters) ? 0 : sched_j + 1;
-            if (lane == 0) prefetched = atomicAdd(G.batch_counter + sched_j * kSchedStrideWords, 1u);
-        }
-    };
+    fm_ring_init(bar_base, n_stages, lane);
+    BatchScheduler sched(G.batch_counter, n_batches, lane);
     // unit of a launch-wide batch index: last u with prefix[u] <= gb (warp-uniform)
     auto unit_of = [&](uint32_t gb) -> uint32_t {
         uint32_t lo = 0, hi = P.n_units;
         while (hi - lo > 1) {
             const uint32_t mid = (lo + hi) >> 1;
-            if (unit_prefix[mid] <= gb) lo = mid; else hi = mid;
+            if (prefix(mid) <= gb) lo = mid; else hi = mid;
         }
         return lo;
     };
@@ -1462,7 +1021,7 @@ fm_k_plane_pass_tab(const __grid_constant__ TabParams P) {
     const uint4 *iss_allele = nullptr;
     bool iss_live = false;
     auto load_iss_seg = [&]() {
-        const TabSeg &S = segs[iss_unit * gpu + iss_g];
+        const RowSeg &S = seg(iss_unit * gpu + iss_g);
         iss_w16 = S.g.wq * 16u;
         iss_step_sites = SPS * S.rounds;
         iss_spb = LPS / S.rounds;
@@ -1470,20 +1029,10 @@ fm_k_plane_pass_tab(const __grid_constant__ TabParams P) {
         iss_allele = S.g.allele;
     };
     auto issue = [&](uint32_t stage) {  // lane 0 only
-        const uint32_t bar = bar_base + 8u * stage;
-        const uint32_t dst = smem_base + stage * stage_bytes;
         const uint32_t v0 = iss_b * 32 + iss_k * iss_step_sites;
         const uint32_t nsites = (v0 < iss_nst) ? min(iss_step_sites, iss_nst - v0) : 0u;
-        if (nsites == 0) {
-            asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-            return;
-        }
-        const uint32_t bytes = nsites * iss_w16;
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-        const size_t off = (size_t)v0 * iss_w16;
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
-                     "l"(reinterpret_cast<const uint8_t *>(iss_allele) + off), "r"(bytes), "r"(bar)
-                     : "memory");
+        fm_ring_fill(smem_base + stage * stage_bytes, reinterpret_cast<const uint8_t *>(iss_allele) + (size_t)v0 * iss_w16,
+                     nsites * iss_w16, bar_base + 8u * stage);
     };
     auto issue_next = [&]() {
         if (iss_k == iss_spb) {
@@ -1493,7 +1042,7 @@ fm_k_plane_pass_tab(const __grid_constant__ TabParams P) {
                 load_iss_seg();
             } else {
                 if (iss_ring != 0 && iss_batch >= n_batches) return;  // scheduler drained
-                iss_batch = claim();
+                iss_batch = sched.claim(lane);
                 iss_k = 0;
                 if (lane == 0) my_ring[iss_ring & (kBatchRing - 1)] = iss_batch;
                 ++iss_ring;
@@ -1506,7 +1055,7 @@ fm_k_plane_pass_tab(const __grid_constant__ TabParams P) {
                 iss_unit = unit_of(iss_batch);
                 iss_g = 0;
                 load_iss_seg();
-                iss_b = segs[iss_unit * gpu].b_lo + (iss_batch - unit_prefix[iss_unit]);
+                iss_b = seg(iss_unit * gpu).b_lo + (iss_batch - prefix(iss_unit));
             }
         }
         if (lane == 0) issue(iss_stage);
@@ -1518,8 +1067,8 @@ fm_k_plane_pass_tab(const __grid_constant__ TabParams P) {
 
     const uint32_t slot_in_round = lane >> LG;
     const uint32_t phase = lane & (LPS - 1);
-    const uint32_t xfer_from = (lane & (SPS - 1)) << LG;
-    const uint32_t xfer_round = lane >> (5 - LG);
+    const uint32_t xfer_from = (lane & (SPS - 1)) << LG;  // source lane of the transpose
+    const uint32_t xfer_round = lane >> (5 - LG);         // round whose sites land here
 
     uint32_t con_ring = 0, stage = 0, parity = 0;
     for (;;) {
@@ -1527,34 +1076,26 @@ fm_k_plane_pass_tab(const __grid_constant__ TabParams P) {
         ++con_ring;
         if (gb >= n_batches) break;
         const uint32_t unit = unit_of(gb);
-        const uint32_t bl = gb - unit_prefix[unit];  // batch inside the unit's range
+        const uint32_t bl = gb - prefix(unit);  // batch inside the unit's range
         uint32_t alt_g0 = 0, cnt_g0 = 0, alt_g1 = 0, cnt_g1 = 0;
         uint32_t b = 0, u_vlo = 0, u_vhi = 0;
         for (uint32_t g = 0; g < gpu; ++g) {
-            const TabSeg &S = segs[unit * gpu + g];
+            const RowSeg &S = seg(unit * gpu + g);
             const uint32_t w = S.g.wq, w16 = w * 16u, rounds = S.rounds;
             const uint32_t step_sites = SPS * rounds, spb = LPS / rounds;
+            // columns phase, phase+LPS, ...: the first nit-1 are inside the row for every lane, only the last one
+            // needs a bound check
             const uint32_t nit = (w + LPS - 1) / LPS;
             const uint32_t nfull = nit - 1, last_cols = w - nfull * LPS;
             const uint32_t nst = S.n_sites_total;
             b = S.b_lo + bl;
             u_vlo = S.v_lo;
             u_vhi = S.v_hi;
-            uint32_t site_a = 0;
+            uint32_t site_a = 0;  // alt count of this lane's batch site
             TailRegs tails;
             fm_tail_load(S.g, b * 32 + lane, nst, tails);
             for (uint32_t k = 0; k < spb; ++k) {
-                {
-                    const uint32_t bar = bar_base + 8u * stage;
-                    uint32_t ok;
-                    do {
-                        asm volatile(
-                            "{\n\t.reg .pred p;\n\t"
-                            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-                            "selp.u32 %0, 1, 0, p;\n\t}"
-                            : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-                    } while (!ok);
-                }
+                fm_ring_wait(bar_base + 8u * stage, parity);
                 const uint32_t sbase = smem_base + stage * stage_bytes;
                 const uint32_t v0 = b * 32 + k * step_sites;
                 auto round_body = [&](uint32_t r) {
@@ -1579,13 +1120,13 @@ fm_k_plane_pass_tab(const __grid_constant__ TabParams P) {
                 if (rounds == 1) {
                     round_body(0);
                 } else {
-                    for (uint32_t r = 0; r < rounds; r += 2) {
+                    for (uint32_t r = 0; r < rounds; r += 2) {  // rounds is a power of two
                         round_body(r);
                         round_body(r + 1);
                     }
                 }
-                __syncwarp();
-                issue_next();
+                __syncwarp();   // every lane is done reading this stage
+                issue_next();   // refill it with the step n_stages ahead
                 stage = (stage + 1 == n_stages) ? 0 : stage + 1;
                 parity ^= (stage == 0);
             }
@@ -1599,24 +1140,10 @@ fm_k_plane_pass_tab(const __grid_constant__ TabParams P) {
                 alt_g1 = alt;
                 cnt_g1 = cnt;
             }
-            const uint32_t v = b * 32 + lane;
-            const bool valid = (v >= S.v_lo) && (v < S.v_hi);
-            if (S.div.part_pi) {
-                double pi_part = 0.0;
-                uint32_t seg = 0, unc = 0;
-                const uint32_t flags = S.div.site_flags ? __ldg(S.div.site_flags + bl) : 0u;
-                if (valid) fm_div_site(S.div, v, S.v_lo, cnt, alt, (flags >> lane) & 1u, pi_part, seg, unc);
-                const double s_pi = fm_warp_sum(pi_part);
-                const uint32_t s_u = fm_warp_sum_u(seg | (unc << 16));
-                if (lane == 0) {
-                    S.div.part_pi[bl] = s_pi;
-                    S.div.part_u[2 * bl] = s_u & 0xffffu;
-                    S.div.part_u[2 * bl + 1] = s_u >> 16;
-                }
-            }
+            if (S.div.part_pi) fm_div_batch(S.div, b * 32 + lane, S.v_lo, S.v_hi, bl, lane, cnt, alt);
         }
-        if (gpu == 2 && hud) {  // ---- Hudson components of the batch from both groups' counts
-            const HudsonEpilogue &H = hud[unit];
+        if constexpr (PAIR) {  // ---- Hudson components of the batch from both groups' counts
+            const HudsonEpilogue &H = P.inline_hud[unit];
             const uint32_t v = b * 32 + lane;
             HudsonAcc acc{0.0, 0.0, 0.0, 0.0, 0.0, 0u, 0u, 0u};
             if (v >= u_vlo && v < u_vhi) fm_hudson_contrib(H, v, u_vlo, cnt_g0, alt_g0, cnt_g1, alt_g1, acc);
@@ -1630,6 +1157,108 @@ fm_k_plane_pass_tab(const __grid_constant__ TabParams P) {
                 pu[0] = u01 & 0xffu; pu[1] = (u01 >> 8) & 0xffu; pu[2] = u01 >> 16;
             }
         }
+    }
+}
+
+// ------------------------------------------------------------------------------ plane pass, column chunks
+// fm_k_plane_pass_chunked: one group whose rows are too wide for two sites per warp ring (biobank cohorts).  A
+// pipeline step holds one column chunk of cq uint4 of one site's row (the whole row when it fits a stage: n_chunks
+// == 1); every lane popcounts its 16-byte columns of the chunk and the warp sums the row when its last chunk is in.
+struct ChunkParams {
+    GroupPlanes g;
+    PassGeom geom;
+    DivEpilogue div;
+};
+
+__global__ void __launch_bounds__(kWarpsPerCta * 32, 1)
+fm_k_plane_pass_chunked(const __grid_constant__ ChunkParams P) {
+    extern __shared__ __align__(128) uint8_t smem_raw[];
+    __shared__ __align__(8) uint64_t bars[kWarpsPerCta * kMaxStages];
+    __shared__ uint32_t batch_ring[kWarpsPerCta * kBatchRing];
+    constexpr uint32_t FULL = 0xffffffffu;
+
+    const uint32_t lane = threadIdx.x & 31;
+    const uint32_t warp = __shfl_sync(FULL, threadIdx.x >> 5, 0);
+    const PassGeom &G = P.geom;
+    const uint32_t n_stages = G.n_stages;
+    const uint32_t stage_bytes = G.stage_bytes;
+    const uint32_t n_sites_total = G.n_sites_total;
+    const uint32_t n_batches = G.n_batches;
+    const uint32_t n_chunks = G.n_chunks;
+    const uint32_t cq = G.cq;
+    const uint32_t spb = 32u * n_chunks;  // steps per batch
+    const uint32_t w = P.g.wq;
+
+    const uint32_t smem_base = fm_smem_u32(smem_raw) + warp * G.warp_smem_bytes;
+    const uint32_t bar_base = fm_smem_u32(bars + warp * kMaxStages);
+    uint32_t *my_ring = batch_ring + warp * kBatchRing;
+    fm_ring_init(bar_base, n_stages, lane);
+    BatchScheduler sched(G.batch_counter, n_batches, lane);
+
+    // issue the bulk copy of step k of local batch `bl` into `stage` (lane 0 only)
+    auto issue = [&](uint32_t bl, uint32_t k, uint32_t stage) {
+        const uint32_t v0 = (G.b_lo + bl) * 32 + k / n_chunks;
+        const uint32_t c0 = (k % n_chunks) * cq;
+        const uint32_t bytes = (v0 < n_sites_total && c0 < w) ? min(cq, w - c0) * 16u : 0u;
+        fm_ring_fill(smem_base + stage * stage_bytes, P.g.allele + ((size_t)v0 * w + c0), bytes, bar_base + 8u * stage);
+    };
+
+    // issue cursor (uniform across the warp)
+    uint32_t iss_ring = 0, iss_k = spb, iss_stage = 0, iss_batch = 0;
+    auto issue_next = [&]() {
+        if (iss_k == spb) {
+            if (iss_ring != 0 && iss_batch >= n_batches) return;  // scheduler drained
+            iss_batch = sched.claim(lane);
+            iss_k = 0;
+            if (lane == 0) my_ring[iss_ring & (kBatchRing - 1)] = iss_batch;
+            ++iss_ring;
+            if (iss_batch >= n_batches) {
+                iss_k = spb;
+                return;
+            }
+        }
+        if (lane == 0) issue(iss_batch, iss_k, iss_stage);
+        ++iss_k;
+        iss_stage = (iss_stage + 1 == n_stages) ? 0 : iss_stage + 1;
+    };
+    for (uint32_t s = 0; s < n_stages; ++s) issue_next();
+    __syncwarp();
+
+    uint32_t site_a = 0, acc_a = 0;  // alt count of this lane's batch site, running row sum of this lane's columns
+    uint32_t con_ring = 0, stage = 0, parity = 0;
+    for (;;) {
+        const uint32_t bl = my_ring[con_ring & (kBatchRing - 1)];
+        ++con_ring;
+        if (bl >= n_batches) break;
+        const uint32_t b = G.b_lo + bl;
+        TailRegs tails;
+        fm_tail_load(P.g, b * 32 + lane, n_sites_total, tails);
+        for (uint32_t k = 0; k < spb; ++k) {
+            fm_ring_wait(bar_base + 8u * stage, parity);
+            const uint32_t sbase = smem_base + stage * stage_bytes;
+            const uint32_t site_in_batch = k / n_chunks;
+            const uint32_t ck = k - site_in_batch * n_chunks;
+            const uint32_t c0 = ck * cq;
+            const bool live = (b * 32 + site_in_batch) < n_sites_total;
+            const uint32_t cols16 = (c0 < w) ? min(cq, w - c0) * 16u : 0u;
+            if (live) {
+#pragma unroll 2
+                for (uint32_t u = lane * 16u; u < cols16; u += 512u) acc_a += fm_popc4(fm_lds128(sbase + u));
+            }
+            if (ck == n_chunks - 1) {
+                const uint32_t ta = fm_warp_sum_u(acc_a);
+                if (lane == site_in_batch) site_a = ta;
+                acc_a = 0;
+            }
+            __syncwarp();   // every lane is done reading this stage
+            issue_next();   // refill it with the step n_stages ahead
+            stage = (stage + 1 == n_stages) ? 0 : stage + 1;
+            parity ^= (stage == 0);
+        }
+        // ---- batch epilogue: lane i <-> site 32b + i
+        uint32_t alt = site_a, cnt;
+        fm_tail_add(tails, alt, cnt);
+        fm_div_batch(P.div, b * 32 + lane, G.v_lo, G.v_hi, bl, lane, cnt, alt);
     }
 }
 
@@ -1721,7 +1350,7 @@ fm_k_reduce_partials(const double *__restrict__ pd, int nd, const uint32_t *__re
     }
 }
 
-// The same fold for many units at once (fm_k_plane_pass_tab launches): entry e = (first partial of the unit in
+// The same fold for many units at once (fm_k_plane_pass_seq launches): entry e = (first partial of the unit in
 // the shared partial arrays, the unit's first global batch, its batch count, the global super-batch index); one
 // warp per entry, the association of fm_k_reduce_partials -- a unit reduced here gives the bits it would give alone.
 __global__ void __launch_bounds__(128)

@@ -577,7 +577,8 @@ typedef struct {
     uint64_t plane_bytes_per_step; /* bytes a step moves: per group and site the allele plane row (16-byte words +
                                     * tail words) and, with missing data, the 4-byte called count read, plus the
                                     * 16 B of pi / theta tracks written (mode 1) */
-    float group_ms_avg[8];         /* mean plane-pass duration per listed group (first 8) */
+    float group_ms_avg[8];         /* mean duration of each plane-pass launch of a step (first 8): one launch for
+                                    * the groups whose rows fit the row pass, then one per group with wider rows */
     uint64_t group_bytes[8];       /* the same bytes for each listed group */
     float comm_ms_avg;             /* mean duration of the fused fold + peer exchange kernel (incl. waiting) */
     /* region totals of the last timed step, per listed group (first 8): this rank's, and -- with a
@@ -591,8 +592,6 @@ fm_status fm_bench_diversity(fm_group *const *groups, size_t n_groups, int mode,
                              const int64_t *mask_iv_or_null, size_t n_mask, int iterations,
                              fm_comm *comm_or_null, fm_bench_result *out, double *last_pi_or_null,
                              double *last_theta_or_null);
-/* Same for the fused two-group Hudson pass (K3). */
-fm_status fm_bench_hudson(fm_group *g1, fm_group *g2, int iterations, fm_bench_result *out);
 
 #ifdef __cplusplus
 }

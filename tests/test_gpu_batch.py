@@ -1,6 +1,6 @@
-"""fm_k_plane_pass_tab through its two entry points: fm_groups_summary_batch (many (matrix, group) units in one
-launch -- the CLI's per-region loop, process.rs:2169) and the fused first call of fm_hudson_pair (both groups'
-counts + Hudson partials from one sweep, stats.rs:3179-3278).  Everything must equal the one-at-a-time calls
+"""The segment table of the row pass (fm_k_plane_pass_seq) through its two entry points: fm_groups_summary_batch
+(many (matrix, group) units in one launch -- the CLI's per-region loop, process.rs:2169) and the fused first call of
+fm_hudson_pair (both groups' counts + Hudson partials from one sweep, stats.rs:3179-3278).  Everything must equal the one-at-a-time calls
 bit for bit, and the oracle."""
 import ctypes as C
 

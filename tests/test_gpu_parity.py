@@ -71,14 +71,30 @@ def test_summary_matches_oracle(n_samples, missing):
 
 
 def test_wide_rows_chunked_mode():
-    # > 12 KB per plane row forces the column-chunked path (lps == 32, n_chunks > 1)
-    g, pos, _ = make_cohort(70, 52000, missing_rate=0.01, seed=3)
-    vs, d, m = dense_pair(g, pos)
-    haps = both_sides(range(52000))
-    ref = orc.build_summary(d, haps)
-    got = m.group(haps).summary(want_arrays=True)
-    assert np.array_equal(got["alt"], ref.alt) and np.array_equal(got["called"], ref.called)
-    assert got["segregating_sites"] == ref.seg and close(got["pi_sum"], ref.pi_sum, 1e-12)
+    # plane rows wider than two sites per warp ring take the column-chunked pass: 52000 samples (13 KB rows) stream a
+    # whole row per stage, 60000 samples (15 KB rows) two column chunks per row
+    from ferromic_b200.api import _Variants
+    for n_samples in (52000, 60000):
+        g, pos, _ = make_cohort(70, n_samples, missing_rate=0.01, seed=3)
+        vs, d, m = dense_pair(g, pos)
+        haps = both_sides(range(n_samples))
+        ref = orc.build_summary(d, haps)
+        got = m.group(haps).summary(want_arrays=True)
+        assert np.array_equal(got["alt"], ref.alt) and np.array_equal(got["called"], ref.called)
+        assert got["segregating_sites"] == ref.seg and close(got["pi_sum"], ref.pi_sum, 1e-12)
+        # per-site pi / theta tracks of the chunked pass under a mask (sparse semantics: whole-sample missingness)
+        gs = g.copy()
+        gs[:, :, 1][gs[:, :, 0] < 0] = -1
+        gs[:, :, 0][gs[:, :, 1] < 0] = -1
+        svs, _ = orc.from_numpy(gs, pos)
+        region = (int(pos[3]), int(pos[66]))
+        mask = [(int(pos[10]), int(pos[20])), (int(pos[40]), int(pos[40]) + 1)]
+        rp, rpi, rth = orc.per_site_diversity(svs, haps, region, mask=mask)
+        gp, gpi, gth = fm().per_site_diversity_arrays(_Variants(svs.positions, svs.gt), haps, region, mask=mask)
+        assert np.array_equal(gp, rp)
+        assert np.isnan(gpi).sum() >= 10  # the masked sites
+        assert_arrays_close(gpi, rpi, 1e-12)
+        assert_arrays_close(gth, rth, 1e-12)
 
 
 @pytest.mark.parametrize("missing", [0.0, 0.15])
@@ -692,10 +708,12 @@ def test_inband_missing_equals_bitmap(max_allele):
 
 
 # ------------------------------------------------------------------ several groups in one launch
-@pytest.mark.parametrize("S,missing,n_groups", [(40, 0.1, 2), (700, 0.02, 3), (2504, 0.01, 2), (300, 0.0, 4)])
+@pytest.mark.parametrize("S,missing,n_groups", [(40, 0.1, 2), (700, 0.02, 3), (2504, 0.01, 2), (300, 0.0, 4),
+                                                (700, 0.02, 6)])
 def test_per_site_diversity_multi_equals_per_group_calls(S, missing, n_groups):
     """fm_per_site_diversity_multi streams every group's planes in ONE persistent launch
-    (fm_k_plane_pass_seq); per-site values must equal the per-group calls bit for bit."""
+    (fm_k_plane_pass_seq; more than four groups read their segment table from device memory); per-site values
+    must equal the per-group calls bit for bit."""
     import ctypes as C
     from ferromic_b200 import _lib
     from ferromic_b200.api import _Matrix

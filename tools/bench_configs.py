@@ -1,9 +1,9 @@
 #!/usr/bin/env python
 """Device-resident timing of the other BASELINE.json configs (bench.py measures configs[1]):
   cfg1  100k sites x 5008 haplotypes, one group, no bitmap: S + pi + theta (summary pass)
-  cfg3  Hudson FST/Dxy between two populations (fused two-group pass), sites per GPU of the 8-GPU shard
+  cfg3  Hudson FST/Dxy between two populations (first fm_hudson_pair call), sites per GPU of the 8-GPU shard
   cfg4  W&C over 26 subpopulations (27 count passes once, then K4 on cached counts)
-  cfg5  biobank shard: 200k haplotypes, 1% missing, two populations, 100 kb windows
+  cfg5  biobank shard: 200k haplotypes, 1% missing, two populations (column-chunked pass), 100 kb windows
 One JSON line per config on stdout.  usage: bench_configs.py [cfg1 cfg3 cfg4 cfg5] [--scale F]"""
 import ctypes as C
 import json
@@ -73,11 +73,6 @@ def cfg3(L, dev, scale):
     m, pos, keep = matrix(L, V, S, 10_002_504, dev, 0.0)
     g1 = group_handle(L, m, [(s, k) for s in range(S // 2) for k in (0, 1)])
     g2 = group_handle(L, m, [(s, k) for s in range(S // 2, S) for k in (0, 1)])
-    res = _lib.BenchResult()
-    for it in (5, 30):
-        _lib.check(L.fm_bench_hudson(g1, g2, it, C.byref(res)))
-    line("cfg3 Hudson per-site fused two-group kernel (NG=2; kept for reference, no longer the product path)", V, 2 * S, res.plane_ms_avg,
-         res.plane_bytes_per_step, {"step_ms": res.step_ms_avg})
     # the product path of fm_hudson_pair's first call: ONE sequential launch over both groups' planes
     # (counts + summary scalars cached) + the light Hudson kernel on the counts; device time by events
     o = _lib.HudsonOutcome()
@@ -97,7 +92,7 @@ def cfg3(L, dev, scale):
         L.fm_timings_get(C.byref(tim))
         if best is None or tim.stats_ms < best[0]:
             best = (tim.stats_ms, dt * 1e3, tim.kernel_launches)
-    plane_bytes = res.plane_bytes_per_step
+    plane_bytes = V * 2 * S // 8  # allele planes of both groups: one bit per haplotype and site
     print(json.dumps({"config": "cfg3 fm_hudson_pair first call (sequential count launch over both groups + light "
                                 "Hudson kernel + reductions)", "device_ms": best[0], "wall_ms": best[1],
                       "kernel_launches": best[2], "genotypes_per_s": V * 2 * S / (best[0] * 1e-3),
@@ -142,11 +137,13 @@ def cfg5(L, dev, scale):
     m, pos, keep = matrix(L, V, S, 2_100_000, dev, 0.01)
     g1 = group_handle(L, m, [(s, k) for s in range(S // 2) for k in (0, 1)])
     g2 = group_handle(L, m, [(s, k) for s in range(S // 2, S) for k in (0, 1)])
+    # the product's pass over rows this wide: the column-chunked kernel, one launch per group
+    arr = (C.c_void_p * 2)(g1.value, g2.value)
     res = _lib.BenchResult()
     for it in (3, 10):
-        _lib.check(L.fm_bench_hudson(g1, g2, it, C.byref(res)))
-    line("cfg5 biobank shard, 200k haplotypes, 1% missing, fused two-group pass (column-chunked rows)", V, 2 * S,
-         res.plane_ms_avg, res.plane_bytes_per_step, {"step_ms": res.step_ms_avg})
+        _lib.check(L.fm_bench_diversity(arr, 2, 0, None, 0, it, None, C.byref(res), None, None))
+    line("cfg5 biobank shard, 200k haplotypes, 1% missing, column-chunked pass (both groups, one launch each)", V, 2 * S,
+         res.group_ms_avg[0] + res.group_ms_avg[1], res.plane_bytes_per_step, {"step_ms": res.step_ms_avg})
     edges = np.arange(int(pos[0]), int(pos[-1]) + 1, 100_000, dtype=np.int64)
     ww = np.stack([edges, edges + 99_999], axis=1).reshape(-1).copy()
     n = len(edges)
