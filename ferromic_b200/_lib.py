@@ -57,7 +57,7 @@ class VcfInfo(C.Structure):
         "n_lines", "n_variants", "n_errors", "n_samples", "max_ploidy", "total_variants", "filtered_variants",
         "filtered_due_to_mask", "filtered_due_to_allow", "missing_data_variants", "low_gq_variants", "mnp_variants",
         "total_data_points", "missing_data_points", "n_positions_with_missing", "n_filtered_positions")] + [
-        ("h2d_ms", C.c_float), ("index_ms", C.c_float), ("parse_ms", C.c_float)]
+        ("h2d_ms", C.c_float), ("index_ms", C.c_float), ("parse_ms", C.c_float), ("inflate_ms", C.c_float)]
 
 
 EXPORTS = [
@@ -74,7 +74,7 @@ EXPORTS = [
     "fm_comm_destroy", "fm_hudson_pair_sharded", "fm_falsta_track", "fm_falsta_tracks", "fm_falsta_format_value", "fm_vcf_parse", "fm_vcf_parse_device", "fm_vcf_batch_info",
     "fm_vcf_batch_variants", "fm_vcf_batch_genotypes", "fm_vcf_batch_positions", "fm_vcf_batch_errors", "fm_vcf_batch_matrix", "fm_vcf_batch_matrix_packed",
     "fm_vcf_batch_release", "fm_synth_fill", "fm_timings_reset", "fm_timings_get", "fm_bench_diversity",
-    "fm_pairwise_differences",
+    "fm_pairwise_differences", "fm_bgzf_inflate", "fm_vcf_parse_bgzf",
 ]
 
 _lib = None
@@ -160,6 +160,9 @@ def lib() -> C.CDLL:
                                C.POINTER(vp)]
     L.fm_vcf_parse_device.argtypes = [vp, sz, C.c_char, C.c_char_p, vp, sz, vp, sz, u16, C.c_int, vp, sz, C.c_int, vp,
                                       sz, sz, C.POINTER(vp)]
+    L.fm_bgzf_inflate.argtypes = [vp, sz, vp, sz, C.POINTER(u64)]
+    L.fm_vcf_parse_bgzf.argtypes = [vp, sz, u64, C.c_char_p, vp, sz, vp, sz, u16, C.c_int, vp, sz, C.c_int, vp, sz, sz,
+                                    C.POINTER(vp)]
     L.fm_vcf_batch_info.argtypes = [vp, C.POINTER(VcfInfo)]
     L.fm_vcf_batch_variants.argtypes = [vp, vp, vp, vp, vp, vp, vp]
     L.fm_vcf_batch_genotypes.argtypes = [vp, vp]

@@ -9,6 +9,7 @@
 #include "fm_falsta.cuh"
 #include "fm_vcf.cuh"
 #include "fm_pairwise.cuh"
+#include "fm_bgzf.cuh"
 
 #include <nvtx3/nvToolsExt.h>
 
@@ -23,6 +24,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <limits>
 #include <map>
 #include <set>
@@ -4925,7 +4927,140 @@ struct VcfChunkGuard {  // frees chunk buffers on every exit path
     }
 };
 
+// Copies chunk after chunk to the device on a stream and a thread of its own while the calling thread consumes the
+// chunks that have arrived: wait(c) orders the calling stream after chunk c's copy.
+struct ChunkUploader {
+    size_t nc = 0;
+    std::vector<cudaEvent_t> ev;
+    cudaStream_t cs = nullptr;
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    std::atomic<size_t> recorded{0};
+    std::atomic<int> copy_err{0};
+    std::string copy_msg;
+    std::thread th;
+
+    void start(size_t n_chunks, std::function<void(size_t, cudaStream_t)> copy) {  // copy(c, stream) enqueues chunk c
+        nc = n_chunks;
+        ev.assign(nc, nullptr);
+        CK(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
+        CK(cudaEventCreate(&e0));
+        CK(cudaEventCreate(&e1));
+        for (auto &e : ev) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+        CK(cudaStreamSynchronize(stream()));  // a destination may be a recycled block still in use on this stream
+        const int dev = t_device;
+        th = std::thread([this, dev, copy] {
+            try {
+                CK(cudaSetDevice(dev));
+                CK(cudaEventRecord(e0, cs));
+                for (size_t c = 0; c < nc; ++c) {
+                    copy(c, cs);
+                    CK(cudaEventRecord(ev[c], cs));
+                    recorded.store(c + 1, std::memory_order_release);
+                }
+                CK(cudaEventRecord(e1, cs));
+                CK(cudaStreamSynchronize(cs));
+            } catch (const FmError &e) {
+                copy_msg = e.msg;
+                copy_err.store(e.code ? e.code : FM_ERR_CUDA);
+                recorded.store(nc, std::memory_order_release);
+            } catch (...) {  // nothing may escape a std::thread
+                copy_msg = "upload thread failed";
+                copy_err.store(FM_ERR_CUDA);
+                recorded.store(nc, std::memory_order_release);
+            }
+        });
+    }
+    bool wait(size_t c) {  // false: the upload failed (finish() reports it)
+        while (recorded.load(std::memory_order_acquire) <= c && !copy_err.load()) std::this_thread::yield();
+        if (copy_err.load()) return false;
+        CK(cudaStreamWaitEvent(stream(), ev[c], 0));
+        return true;
+    }
+    float finish() {  // joins the thread, throws its error; device time of all copies
+        th.join();
+        if (copy_err.load()) fail(copy_err.load(), copy_msg);
+        float ms = 0.f;
+        if (nc) CK(cudaEventElapsedTime(&ms, e0, e1));
+        return ms;
+    }
+    ~ChunkUploader() {
+        if (th.joinable()) th.join();
+        for (auto &e : ev)
+            if (e) cudaEventDestroy(e);
+        if (e0) cudaEventDestroy(e0);
+        if (e1) cudaEventDestroy(e1);
+        if (cs) cudaStreamDestroy(cs);
+    }
+};
+
+// ------------------------------------------------------------------------------------ BGZF inflate (fm_bgzf.cuh)
+std::vector<fm::BgzfMember> bgzf_members(const uint8_t *gz, size_t n) {
+    std::vector<fm::BgzfMember> mem;
+    const fm::BgzfWalkError e = fm::bgzf_walk(gz, n, mem);
+    const std::string where =
+        "BGZF member " + std::to_string(e.member) + " at byte offset " + std::to_string(e.offset) + ": " + e.what;
+    if (e.kind == fm::BGZF_WALK_NOT_BGZF)
+        fail(FM_ERR_UNSUPPORTED, where + " (the device decoder reads BGZF, as bgzip writes it: recompress with "
+                                         "bgzip, or inflate on the host and call fm_vcf_parse)");
+    if (e.kind != fm::BGZF_WALK_OK) fail(FM_ERR_PARSE, where);
+    return mem;
+}
+
+// Inflates members [m0, m0 + n) of `mem` (deflate data at d_in + in_off, table copy at d_mem) so that member m lands
+// at out + (mem[m].out_off - mem[m0].out_off).  d_first_bad: one word, set to ~0 here; the kernel lowers it.
+void bgzf_launch(const uint8_t *d_in, const std::vector<fm::BgzfMember> &mem, const fm::BgzfMember *d_mem, size_t m0,
+                 size_t n, uint8_t *out, int32_t *d_err, uint32_t *d_first_bad) {
+    CK(cudaMemsetAsync(d_first_bad, 0xff, 4, stream()));
+    const uint32_t blocks = (uint32_t)((n + fm::INFLATE_WARPS - 1) / fm::INFLATE_WARPS);
+    fm::fm_k_inflate_members<<<blocks, 32 * fm::INFLATE_WARPS, 0, stream()>>>(
+        d_in, d_mem + m0, (uint32_t)n, out, mem[m0].out_off, d_err + m0, d_first_bad);
+    CK(cudaGetLastError());
+    g_launches++;
+}
+
+// first_bad: the kernel's *d_first_bad after the launch over members m0..; throws FM_ERR_PARSE naming the member
+void bgzf_check(const std::vector<fm::BgzfMember> &mem, size_t m0, uint32_t first_bad, const int32_t *d_err) {
+    if (first_bad == ~0u) return;
+    const size_t m = m0 + first_bad;
+    int32_t code = 0;
+    CK(cudaMemcpy(&code, d_err + m, 4, cudaMemcpyDeviceToHost));
+    fail(FM_ERR_PARSE, "BGZF member " + std::to_string(m) + " at byte offset " + std::to_string(mem[m].off) + ": " +
+                           fm::bgzf_error_text(code));
+}
+
 }  // namespace
+
+fm_status fm_bgzf_inflate(const uint8_t *gz, size_t n_gz, uint8_t *out, size_t capacity, uint64_t *total_out) {
+    return guarded([&] {
+        FM_NVTX("fm_bgzf_inflate");
+        if (n_gz && !gz) fail(FM_ERR_INVALID_ARG, "gz is NULL");
+        if (capacity && !out) fail(FM_ERR_INVALID_ARG, "out is NULL");
+        require_device();
+        CK(cudaSetDevice(t_device));
+        const std::vector<fm::BgzfMember> mem = bgzf_members(gz, n_gz);
+        const uint64_t total = mem.empty() ? 0 : mem.back().out_off + mem.back().isize;
+        if (total_out) *total_out = total;
+        const uint64_t want = std::min<uint64_t>(capacity, total);
+        if (!want) return;
+        size_t m1 = 0;  // the members that cover [0, want)
+        while (m1 < mem.size() && mem[m1].out_off < want) ++m1;
+        const fm::BgzfMember &last = mem[m1 - 1];
+        DevBuf<uint8_t> d_in(last.in_off + last.in_len), d_out(last.out_off + last.isize);
+        DevBuf<fm::BgzfMember> d_mem(m1);
+        DevBuf<int32_t> d_err(m1);
+        DevBuf<uint32_t> d_first(1);
+        h2d(d_in.p, gz, d_in.n, stream());
+        d_mem.upload(mem.data(), m1);
+        CK(cudaMemsetAsync(d_err.p, 0, m1 * 4, stream()));
+        bgzf_launch(d_in.p, mem, d_mem.p, 0, m1, d_out.p, d_err.p, d_first.p);
+        uint32_t *h_first = reinterpret_cast<uint32_t *>(t_pinned.ensure(64));
+        CK(cudaMemcpyAsync(h_first, d_first.p, 4, cudaMemcpyDeviceToHost, stream()));
+        CK(cudaStreamSynchronize(stream()));
+        bgzf_check(mem, 0, *h_first, d_err.p);
+        CK(cudaMemcpyAsync(out, d_out.p, want, cudaMemcpyDeviceToHost, stream()));
+        CK(cudaStreamSynchronize(stream()));
+    });
+}
 
 fm_status fm_vcf_parse_device(const char *d_text, size_t n_bytes, char host_last_byte, const char *chr,
                               const int64_t *regions, size_t n_regions, const uint32_t *kept_col_indices,
@@ -4993,75 +5128,132 @@ fm_status fm_vcf_parse(const char *text, size_t n_bytes, const char *chr, const 
         DevBuf<uint8_t> d_text(std::max<size_t>(doff[nc], 64));
         VcfChunkGuard g;
         g.v.resize(nc);
-        const int dev = t_device;
-        std::vector<cudaEvent_t> ev(nc, nullptr);
-        std::atomic<size_t> recorded{0};
-        std::atomic<int> copy_err{0};
-        std::string copy_msg;
         float h2d_ms = 0.f;
-        cudaStream_t cs = nullptr;
-        cudaEvent_t e0 = nullptr, e1 = nullptr;
-        auto cleanup = [&] {
-            for (auto &e : ev)
-                if (e) cudaEventDestroy(e);
-            if (e0) cudaEventDestroy(e0);
-            if (e1) cudaEventDestroy(e1);
-            if (cs) cudaStreamDestroy(cs);
-        };
-        try {
-            CK(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
-            CK(cudaEventCreate(&e0));
-            CK(cudaEventCreate(&e1));
-            for (auto &e : ev) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-            CK(cudaStreamSynchronize(stream()));  // d_text may be a recycled block still in use on this stream
-            tr.mark("alloc + streams");
-            std::thread uploader([&] {
-                try {
-                    CK(cudaSetDevice(dev));
-                    CK(cudaEventRecord(e0, cs));
-                    for (size_t c = 0; c < nc; ++c) {
-                        const size_t nb = cut[c + 1] - cut[c], body = ((nb + 15) / 16) * 16;
-                        const size_t tail = body >= 16 ? body - 16 : 0;  // partial last word + padding read zero
-                        CK(cudaMemsetAsync(d_text.p + doff[c] + tail, 0, body + 32 - tail, cs));
-                        h2d(d_text.p + doff[c], text + cut[c], nb, cs);
-                        CK(cudaEventRecord(ev[c], cs));
-                        recorded.store(c + 1, std::memory_order_release);
-                    }
-                    CK(cudaEventRecord(e1, cs));
-                    CK(cudaStreamSynchronize(cs));
-                } catch (const FmError &e) {
-                    copy_msg = e.msg;
-                    copy_err.store(e.code ? e.code : FM_ERR_CUDA);
-                    recorded.store(nc, std::memory_order_release);
-                } catch (...) {  // nothing may escape a std::thread
-                    copy_msg = "upload thread failed";
-                    copy_err.store(FM_ERR_CUDA);
-                    recorded.store(nc, std::memory_order_release);
-                }
+        {
+            ChunkUploader up;
+            up.start(nc, [&](size_t c, cudaStream_t cs) {
+                const size_t nb = cut[c + 1] - cut[c], body = ((nb + 15) / 16) * 16;
+                const size_t tail = body >= 16 ? body - 16 : 0;  // partial last word + padding read zero
+                CK(cudaMemsetAsync(d_text.p + doff[c] + tail, 0, body + 32 - tail, cs));
+                h2d(d_text.p + doff[c], text + cut[c], nb, cs);
             });
-            try {
-                for (size_t c = 0; c < nc; ++c) {
-                    while (recorded.load(std::memory_order_acquire) <= c && !copy_err.load()) std::this_thread::yield();
-                    if (copy_err.load()) break;
-                    CK(cudaStreamWaitEvent(stream(), ev[c], 0));
-                    vcf_chunk(sh, d_text.p + doff[c], cut[c + 1] - cut[c], text[cut[c + 1] - 1], g.v[c]);
-                }
-            } catch (...) {
-                uploader.join();
-                throw;
-            }
+            tr.mark("alloc + streams");
+            for (size_t c = 0; c < nc && up.wait(c); ++c)
+                vcf_chunk(sh, d_text.p + doff[c], cut[c + 1] - cut[c], text[cut[c + 1] - 1], g.v[c]);
             tr.mark("chunks parsed");
-            uploader.join();
-            if (copy_err.load()) fail(copy_err.load(), copy_msg);
-            if (nc) CK(cudaEventElapsedTime(&h2d_ms, e0, e1));
-        } catch (...) {
-            cleanup();
-            throw;
+            h2d_ms = up.finish();
         }
-        cleanup();
         tr.mark("join + cleanup");
         t_tim.h2d_ms += h2d_ms;
         vcf_finish(sh, g.v, h2d_ms, out);
+        tr.mark("finish");
+    });
+}
+
+// BGZF: fm_vcf_parse with the uploader moving compressed members.  Chunks are runs of whole members of about the
+// same inflated size as fm_vcf_parse's text chunks; the compressed stream is resident, the inflated text rotates
+// through two buffers (vcf_chunk has finished with its text when it returns).  A chunk's parse range ends at its
+// last '\n'; the partial line after it moves to the front of the other buffer and the next chunk inflates behind it.
+fm_status fm_vcf_parse_bgzf(const uint8_t *gz, size_t n_gz, uint64_t data_offset, const char *chr,
+                            const int64_t *regions, size_t n_regions, const uint32_t *kept_col_indices, size_t n_kept,
+                            uint16_t min_gq, int allow_mode, const int64_t *allow, size_t n_allow, int mask_mode,
+                            const int64_t *mask, size_t n_mask, size_t max_ploidy, fm_vcf_batch **out) {
+    return guarded([&] {
+        FM_NVTX("fm_vcf_parse_bgzf");
+        if (!out) fail(FM_ERR_INVALID_ARG, "out is NULL");
+        *out = nullptr;
+        if (n_gz && !gz) fail(FM_ERR_INVALID_ARG, "gz is NULL");
+        require_device();
+        CK(cudaSetDevice(t_device));
+        VcfTrace tr;
+        VcfShared sh;
+        vcf_prepare(sh, chr, regions, n_regions, kept_col_indices, n_kept, min_gq, allow_mode, allow, n_allow, mask_mode,
+                    mask, n_mask, max_ploidy);
+        std::vector<fm::BgzfMember> mem = bgzf_members(gz, n_gz);
+        const uint64_t total = mem.empty() ? 0 : mem.back().out_off + mem.back().isize;
+        if (data_offset > total) fail(FM_ERR_INVALID_ARG, "data_offset lies past the end of the inflated stream");
+        size_t m0 = 0;  // first member holding data-section bytes
+        while (m0 < mem.size() && mem[m0].out_off + mem[m0].isize <= data_offset) ++m0;
+        size_t target = (size_t)env_u32_early("FM_VCF_CHUNK_MB", 64) << 20;
+        if (const uint32_t tb = env_u32_early("FM_VCF_CHUNK_BYTES", 0)) target = tb;  // tests: many tiny chunks
+        std::vector<size_t> mb{m0};  // chunk c = members [mb[c], mb[c + 1])
+        while (mb.back() < mem.size()) {
+            size_t m = mb.back();
+            uint64_t bytes = 0;
+            do bytes += mem[m++].isize;
+            while (m < mem.size() && bytes + mem[m].isize <= target);
+            mb.push_back(m);
+        }
+        const size_t nc = mb.size() - 1;
+        auto inflated = [&](size_t c) { return mem[mb[c + 1] - 1].out_off + mem[mb[c + 1] - 1].isize - mem[mb[c]].out_off; };
+        // the compressed members [m0, end) stay resident, indexed from the first one's deflate data
+        const uint64_t gz_base = nc ? mem[m0].in_off : 0;
+        DevBuf<uint8_t> d_gz(std::max<uint64_t>(nc ? mem.back().in_off + mem.back().in_len - gz_base : 0, 16));
+        for (size_t m = m0; m < mem.size(); ++m) mem[m].in_off -= gz_base;
+        DevBuf<fm::BgzfMember> d_mem(std::max<size_t>(mem.size(), 1));
+        DevBuf<int32_t> d_err(std::max<size_t>(mem.size(), 1));
+        DevBuf<uint32_t> d_state(4);  // first bad member, last '\n' + 1, last byte
+        d_mem.upload(mem.data(), mem.size());
+        CK(cudaMemsetAsync(d_err.p, 0, d_err.n * 4, stream()));
+        // text buffers: chunk c parses from tb[c & 1] + lead; the first chunk starts data_offset - out_off bytes into
+        // its first member, and inflates that far before an aligned start
+        const uint64_t skip0 = nc ? data_offset - mem[m0].out_off : 0, lead0 = (skip0 + 15) / 16 * 16;
+        DevBuf<uint8_t> tb[2];
+        auto ensure = [&](DevBuf<uint8_t> &b, uint64_t bytes) {
+            if (b.n < bytes + 64) b.alloc(bytes + bytes / 8 + 64);  // + the parse range's zero pad and 32 bytes
+        };
+        if (nc) ensure(tb[0], lead0 + inflated(0));
+        VcfChunkGuard g;
+        g.v.resize(nc);
+        float h2d_ms = 0.f, inflate_ms = 0.f;
+        tr.mark("prepare + member walk");
+        {
+            ChunkUploader up;
+            up.start(nc, [&](size_t c, cudaStream_t cs) {
+                const fm::BgzfMember &a = mem[mb[c]], &z = mem[mb[c + 1] - 1];
+                h2d(d_gz.p + a.in_off, gz + gz_base + a.in_off, z.in_off + z.in_len - a.in_off, cs);
+            });
+            uint64_t carry = 0;  // bytes of a partial line at the front of this chunk's buffer
+            for (size_t c = 0; c < nc && up.wait(c); ++c) {
+                const uint64_t skip = c ? 0 : skip0, len = carry + inflated(c) - skip;
+                if (len >= (1ull << 31)) fail(FM_ERR_UNSUPPORTED, "a single line run exceeds 2^31 bytes");
+                uint8_t *text = tb[c & 1].p + (c ? 0 : lead0);
+                Timer t;
+                t.start();
+                bgzf_launch(d_gz.p, mem, d_mem.p, mb[c], mb[c + 1] - mb[c], text + carry - skip, d_err.p, d_state.p);
+                t.stop();
+                CK(cudaMemsetAsync(d_state.p + 1, 0, 8, stream()));
+                const int sms = sm_count(t_device);
+                fm::fm_k_text_tail<<<(uint32_t)std::max<uint64_t>(std::min<uint64_t>((len + 255) / 256, 4ull * sms), 1),
+                                     256, 0, stream()>>>(text, (uint32_t)len, d_state.p + 1);
+                CK(cudaGetLastError());
+                g_launches++;
+                uint32_t *hs = reinterpret_cast<uint32_t *>(t_pinned.ensure(64));
+                CK(cudaMemcpyAsync(hs, d_state.p, 12, cudaMemcpyDeviceToHost, stream()));
+                CK(cudaStreamSynchronize(stream()));
+                const uint32_t first_bad = hs[0], last_nl = hs[1];
+                const char last_byte = (char)hs[2];
+                inflate_ms += t.ms();
+                bgzf_check(mem, mb[c], first_bad, d_err.p);
+                const bool final = c + 1 == nc;
+                const uint64_t n_parse = final ? len : last_nl, next_carry = len - n_parse;
+                if (!final) {
+                    ensure(tb[(c + 1) & 1], next_carry + inflated(c + 1));
+                    if (next_carry)
+                        CK(cudaMemcpyAsync(tb[(c + 1) & 1].p, text + n_parse, next_carry, cudaMemcpyDeviceToDevice,
+                                           stream()));
+                }
+                const uint64_t body = (n_parse + 15) / 16 * 16;  // zero to the 16-byte boundary and 32 bytes on
+                CK(cudaMemsetAsync(text + n_parse, 0, body + 32 - n_parse, stream()));
+                vcf_chunk(sh, text, n_parse, final ? last_byte : '\n', g.v[c]);
+                carry = next_carry;
+            }
+            tr.mark("chunks inflated + parsed");
+            h2d_ms = up.finish();
+        }
+        t_tim.h2d_ms += h2d_ms;
+        vcf_finish(sh, g.v, h2d_ms, out);
+        (*out)->info.inflate_ms = inflate_ms;
         tr.mark("finish");
     });
 }

@@ -5,7 +5,8 @@ header is consumed here like the reference does (sample names, exclusion set -> 
 indices, :4181-4215); the data lines -- `process_variant` for every line, the merge of line-local
 statistics, the (position, genotype bytes) sort -- run on the device through `fm_vcf_parse`.
 Genotypes stay on the device; `VcfBatch.matrix()` is `DenseGenotypeMatrix::from_variants` without
-a host round trip, ready for groups / partitions and the estimators."""
+a host round trip, ready for groups / partitions and the estimators.  BGZF input (`.vcf.gz`) is inflated
+on the device too (`process_vcf_bgzf`)."""
 from __future__ import annotations
 
 import ctypes as C
@@ -154,14 +155,8 @@ def _pairs(v) -> np.ndarray:
     return a
 
 
-def process_lines(text: bytes, chr_: str, regions: Sequence[Tuple[int, int]], kept_col_indices: Sequence[int],
-                  min_gq: int, allow_regions: Optional[Dict[str, Sequence[Tuple[int, int]]]] = None,
-                  mask_regions: Optional[Dict[str, Sequence[Tuple[int, int]]]] = None, max_ploidy: int = 2) -> VcfBatch:
-    """Data lines of a VCF (bytes, '\\n'-terminated) through the device parser.  regions are
-    ZeroBasedHalfOpen (start, end) pairs; allow / mask maps are keyed by chromosome name without
-    the chr prefix, as the reference's BED loaders store them."""
-    if isinstance(text, str):
-        text = text.encode()
+def _parse_args(chr_: str, regions, kept_col_indices, allow_regions, mask_regions):
+    """The arguments after `chr` that fm_vcf_parse and fm_vcf_parse_bgzf share (arrays kept alive by the caller)."""
     key = _normalize_chr(chr_)
 
     def mode(m):
@@ -173,20 +168,33 @@ def process_lines(text: bytes, chr_: str, regions: Sequence[Tuple[int, int]], ke
 
     am, av = mode(allow_regions)
     mm, mv = mode(mask_regions)
-    reg = _pairs(regions)
-    kept = np.ascontiguousarray(kept_col_indices, dtype=np.uint32)
+    return _pairs(regions), np.ascontiguousarray(kept_col_indices, dtype=np.uint32), am, av, mm, mv
+
+
+def _call_parse(fn, head, chr_, regions, kept_col_indices, min_gq, allow_regions, mask_regions, max_ploidy) -> VcfBatch:
+    reg, kept, am, av, mm, mv = _parse_args(chr_, regions, kept_col_indices, allow_regions, mask_regions)
     h = C.c_void_p()
     p = lambda a: a.ctypes.data_as(C.c_void_p)
-    check(lib().fm_vcf_parse(text, len(text), chr_.encode(), p(reg), len(reg), p(kept), len(kept), int(min_gq),
-                             am, p(av), len(av), mm, p(mv), len(mv), int(max_ploidy), C.byref(h)))
+    check(fn(*head, chr_.encode(), p(reg), len(reg), p(kept), len(kept), int(min_gq), am, p(av), len(av), mm, p(mv),
+             len(mv), int(max_ploidy), C.byref(h)))
     return VcfBatch(h, chr_, int(kept.max()) if len(kept) else -1)
 
 
-def process_vcf_text(text: bytes, chr_: str, regions, min_gq: int, allow_regions=None, mask_regions=None,
-                     exclusion_set: Iterable[str] = (), max_ploidy: int = 2) -> Tuple[VcfBatch, List[str]]:
-    """A whole (uncompressed) VCF text: header handled like process_vcf (:4181-4215), data lines on the GPU."""
+def process_lines(text: bytes, chr_: str, regions: Sequence[Tuple[int, int]], kept_col_indices: Sequence[int],
+                  min_gq: int, allow_regions: Optional[Dict[str, Sequence[Tuple[int, int]]]] = None,
+                  mask_regions: Optional[Dict[str, Sequence[Tuple[int, int]]]] = None, max_ploidy: int = 2) -> VcfBatch:
+    """Data lines of a VCF (bytes, '\\n'-terminated) through the device parser.  regions are
+    ZeroBasedHalfOpen (start, end) pairs; allow / mask maps are keyed by chromosome name without
+    the chr prefix, as the reference's BED loaders store them."""
     if isinstance(text, str):
         text = text.encode()
+    return _call_parse(lib().fm_vcf_parse, (text, len(text)), chr_, regions, kept_col_indices, min_gq, allow_regions,
+                       mask_regions, max_ploidy)
+
+
+def _scan_header(text: bytes, exclusion_set: Iterable[str]) -> Tuple[List[str], List[int], int]:
+    """Header lines like process_vcf (:4181-4215): (sample names, kept column indices, offset of the first data
+    line).  Raises when no sample remains."""
     off = 0
     names: List[str] = []
     kept: List[int] = []
@@ -202,7 +210,70 @@ def process_vcf_text(text: bytes, chr_: str, regions, min_gq: int, allow_regions
             break
     if not names:
         raise VcfParseError("No samples remain after applying exclusions")
+    return names, kept, off
+
+
+def process_vcf_text(text: bytes, chr_: str, regions, min_gq: int, allow_regions=None, mask_regions=None,
+                     exclusion_set: Iterable[str] = (), max_ploidy: int = 2) -> Tuple[VcfBatch, List[str]]:
+    """A whole (uncompressed) VCF text: header handled like process_vcf (:4181-4215), data lines on the GPU."""
+    if isinstance(text, str):
+        text = text.encode()
+    names, kept, off = _scan_header(text, exclusion_set)
     return process_lines(text[off:], chr_, regions, kept, min_gq, allow_regions, mask_regions, max_ploidy), names
+
+
+# ------------------------------------------------------------------------------- BGZF input (.vcf.gz)
+# bgzip / tabix write BGZF: independent gzip members of at most 64 KiB.  The device inflates them (fm_bgzf_inflate,
+# fm_vcf_parse_bgzf), so only the compressed bytes cross the bus.  `data` is bytes or any contiguous bytes-like
+# buffer (a numpy view of page-locked memory uploads without a bounce copy).
+def _gz_buffer(data):
+    if isinstance(data, bytes):
+        return data, len(data)
+    a = np.frombuffer(data, dtype=np.uint8)
+    return a.ctypes.data_as(C.c_void_p), a.size
+
+
+def _inflate_prefix(data, capacity: int) -> Tuple[bytes, int]:
+    """(first min(capacity, total) inflated bytes, total inflated size)."""
+    ptr, n = _gz_buffer(data)
+    total = C.c_uint64()
+    out = (C.c_uint8 * max(capacity, 1))()
+    check(lib().fm_bgzf_inflate(ptr, n, out, capacity, C.byref(total)))
+    return bytes(out)[:min(capacity, total.value)], total.value
+
+
+def bgzf_inflate(data) -> bytes:
+    """The whole inflated stream, decoded on the device."""
+    ptr, n = _gz_buffer(data)
+    total = C.c_uint64()
+    check(lib().fm_bgzf_inflate(ptr, n, None, 0, C.byref(total)))
+    return _inflate_prefix(data, total.value)[0]
+
+
+def read_bgzf_header(data) -> Tuple[bytes, int]:
+    """(header bytes up to and including the #CHROM line, offset of the first data line in the inflated stream).
+    Inflates a prefix, doubling it until the #CHROM line ends (or the stream does)."""
+    cap = 1 << 16
+    while True:
+        head, total = _inflate_prefix(data, cap)
+        at = 0 if head.startswith(b"#CHROM") else head.find(b"\n#CHROM") + 1
+        nl = head.find(b"\n", at) if at > 0 or head.startswith(b"#CHROM") else -1
+        if nl >= 0:
+            return head[:nl + 1], nl + 1
+        if len(head) >= total:
+            return head, len(head)
+        cap *= 2
+
+
+def process_vcf_bgzf(data, chr_: str, regions, min_gq: int, allow_regions=None, mask_regions=None,
+                     exclusion_set: Iterable[str] = (), max_ploidy: int = 2) -> Tuple[VcfBatch, List[str]]:
+    """process_vcf_text for a BGZF-compressed VCF (.vcf.gz as bgzip writes it): the same header rules, the same
+    VcfBatch; the members are inflated and parsed on the device."""
+    header, _ = read_bgzf_header(data)
+    names, kept, off = _scan_header(header, exclusion_set)
+    ptr, n = _gz_buffer(data)
+    return _call_parse(lib().fm_vcf_parse_bgzf, (ptr, n, off), chr_, regions, kept, min_gq, allow_regions,
+                       mask_regions, max_ploidy), names
 
 
 # ------------------------------------------------------------------------------- multi-GPU (SURVEY §8e)

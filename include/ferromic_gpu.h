@@ -484,6 +484,7 @@ typedef struct {
         missing_data_variants, low_gq_variants, mnp_variants, total_data_points, missing_data_points,
         n_positions_with_missing, n_filtered_positions;
     float h2d_ms, index_ms, parse_ms; /* device time of the upload, line index and the two parse kernels */
+    float inflate_ms;                 /* device time of the BGZF inflate kernels (fm_vcf_parse_bgzf; 0 otherwise) */
 } fm_vcf_info;
 fm_status fm_vcf_parse(const char *text, size_t n_bytes, const char *chr, const int64_t *regions,
                        size_t n_regions, const uint32_t *kept_col_indices, size_t n_kept, uint16_t min_gq,
@@ -497,6 +498,22 @@ fm_status fm_vcf_parse_device(const char *d_text, size_t n_bytes, char host_last
                               size_t n_kept, uint16_t min_gq, int allow_mode, const int64_t *allow,
                               size_t n_allow, int mask_mode, const int64_t *mask, size_t n_mask,
                               size_t max_ploidy, fm_vcf_batch **out);
+/* ---- BGZF input (the format bgzip / tabix write: independent gzip members of at most 64 KiB, each carrying its
+ * compressed size in a `BC` extra subfield) inflated on the device.  Every member's length and CRC32 are checked
+ * against its trailer.  A gzip stream without the BGZF header is FM_ERR_UNSUPPORTED (recompress with bgzip, or
+ * inflate on the host and call fm_vcf_parse); a truncated or inconsistent one is FM_ERR_PARSE naming the member
+ * and its byte offset. */
+/* Inflate the first min(capacity, total) bytes of a BGZF stream on the device into host memory; only the members
+ * covering them are decoded (header reads ask for a prefix).  *total_out = the whole stream's inflated size. */
+fm_status fm_bgzf_inflate(const uint8_t *gz, size_t n_gz, uint8_t *out, size_t capacity, uint64_t *total_out);
+/* fm_vcf_parse over the inflated stream from byte data_offset on (the first data line; header consumed by the
+ * caller): same arguments after `chr`, same batch, same statistics, same error lines.  Only compressed bytes cross
+ * the bus; FM_VCF_CHUNK_MB / FM_VCF_CHUNK_BYTES count inflated bytes. */
+fm_status fm_vcf_parse_bgzf(const uint8_t *gz, size_t n_gz, uint64_t data_offset, const char *chr,
+                            const int64_t *regions, size_t n_regions, const uint32_t *kept_col_indices,
+                            size_t n_kept, uint16_t min_gq, int allow_mode, const int64_t *allow, size_t n_allow,
+                            int mask_mode, const int64_t *mask, size_t n_mask, size_t max_ploidy,
+                            fm_vcf_batch **out);
 fm_status fm_vcf_batch_info(const fm_vcf_batch *b, fm_vcf_info *out);
 /* per-variant arrays in output order (any pointer may be NULL): 0-based position, flags
  * (1 mask | 2 allow | 4 low GQ | 8 missing, process.rs:785-789), the variant's own genotype stride,

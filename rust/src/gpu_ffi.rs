@@ -81,6 +81,12 @@ extern "C" {
     pub fn fm_pairwise_differences(m: *mut fm_matrix, n_samples: usize, differences: *mut u32,
         comparable: *mut u32, pair_start: *mut u64, positions: *mut i64, positions_capacity: usize,
         n_positions_out: *mut usize) -> c_int;
+    // BGZF (.vcf.gz as bgzip writes it) inflated on the device; fm_vcf_parse_bgzf parses from data_offset on
+    pub fn fm_bgzf_inflate(gz: *const u8, n_gz: usize, out: *mut u8, capacity: usize, total_out: *mut u64) -> c_int;
+    pub fn fm_vcf_parse_bgzf(gz: *const u8, n_gz: usize, data_offset: u64, chr: *const c_char, regions: *const i64,
+        n_regions: usize, kept_col_indices: *const u32, n_kept: usize, min_gq: u16, allow_mode: c_int,
+        allow: *const i64, n_allow: usize, mask_mode: c_int, mask: *const i64, n_mask: usize, max_ploidy: usize,
+        out: *mut *mut fm_vcf_batch) -> c_int;
     // shard-mergeable window totals + finishers (multi-GPU, windows)
     pub fn fm_group_window_sums(g: *mut fm_group, windows: *const i64, n_windows: usize,
         n_variants: *mut u64, seg_sites: *mut u64, pi_sum: *mut f64, uncallable_lt2: *mut u64) -> c_int;
