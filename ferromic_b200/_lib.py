@@ -14,6 +14,7 @@ FM_OK, FM_ERR_INVALID_REGION, FM_ERR_PARSE, FM_ERR_INVALID_ARG = 0, 1, 2, 3
 FM_ERR_CUDA, FM_ERR_UNSUPPORTED, FM_ERR_NO_DEVICE = 4, 5, 6
 FM_PI_SUMMARY, FM_PI_DENSE, FM_PI_SPARSE = 0, 1, 2
 FM_HUDSON_SUMMARIES, FM_HUDSON_DENSE, FM_HUDSON_SPARSE = 0, 1, 2
+FM_BGZF_EOF = 1
 
 
 class HudsonOutcome(C.Structure):
@@ -74,7 +75,8 @@ EXPORTS = [
     "fm_comm_destroy", "fm_hudson_pair_sharded", "fm_falsta_track", "fm_falsta_tracks", "fm_falsta_format_value", "fm_vcf_parse", "fm_vcf_parse_device", "fm_vcf_batch_info",
     "fm_vcf_batch_variants", "fm_vcf_batch_genotypes", "fm_vcf_batch_positions", "fm_vcf_batch_errors", "fm_vcf_batch_matrix", "fm_vcf_batch_matrix_packed",
     "fm_vcf_batch_release", "fm_synth_fill", "fm_timings_reset", "fm_timings_get", "fm_bench_diversity",
-    "fm_pairwise_differences", "fm_bgzf_inflate", "fm_vcf_parse_bgzf",
+    "fm_pairwise_differences", "fm_bgzf_inflate", "fm_vcf_parse_bgzf", "fm_bgzf_deflate_bound", "fm_bgzf_deflate",
+    "fm_falsta_tracks_bgzf",
 ]
 
 _lib = None
@@ -163,6 +165,9 @@ def lib() -> C.CDLL:
     L.fm_bgzf_inflate.argtypes = [vp, sz, vp, sz, C.POINTER(u64)]
     L.fm_vcf_parse_bgzf.argtypes = [vp, sz, u64, C.c_char_p, vp, sz, vp, sz, u16, C.c_int, vp, sz, C.c_int, vp, sz, sz,
                                     C.POINTER(vp)]
+    L.fm_bgzf_deflate_bound.argtypes = [sz, C.c_int, C.POINTER(sz)]
+    L.fm_bgzf_deflate.argtypes = [vp, sz, C.c_int, vp, sz, C.POINTER(sz)]
+    L.fm_falsta_tracks_bgzf.argtypes = [vp, vp, sz, sz, i64, i64, C.c_int, vp, vp, sz, C.POINTER(sz)]
     L.fm_vcf_batch_info.argtypes = [vp, C.POINTER(VcfInfo)]
     L.fm_vcf_batch_variants.argtypes = [vp, vp, vp, vp, vp, vp, vp]
     L.fm_vcf_batch_genotypes.argtypes = [vp, vp]

@@ -111,13 +111,14 @@ fm_k_falsta_lengths(const int *__restrict__ idx, const double *__restrict__ valu
 
 __global__ void __launch_bounds__(256)
 fm_k_falsta_write(const int *__restrict__ idx, const double *__restrict__ values, uint64_t n, uint64_t region_len,
-                  uint32_t n_tracks, int mode, const uint64_t *__restrict__ offs, char *__restrict__ out) {
+                  uint32_t n_tracks, int mode, const uint64_t *__restrict__ offs, char *__restrict__ out,
+                  const uint64_t *__restrict__ track_shift) {
     const uint64_t total = region_len * n_tracks;
     for (uint64_t g = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; g < total;
          g += (uint64_t)gridDim.x * blockDim.x) {
         const uint64_t t = g / region_len, j = g - t * region_len;
         const int i = idx[j];
-        char *dst = out + offs[g];
+        char *dst = out + offs[g] + (track_shift ? track_shift[t] : 0);
         uint32_t len;
         if (i >= 0) {
             char buf[56];
@@ -133,6 +134,21 @@ fm_k_falsta_write(const int *__restrict__ idx, const double *__restrict__ values
         }
         if (g + 1 < total) dst[len] = (j + 1 < region_len) ? ',' : '\n';
     }
+}
+
+// Headed text (fm_falsta_tracks_bgzf): heads[t] + line t + '\n' per track.  The lines were written with track t
+// shifted by track_shift[t] = the bytes of heads 0..t; block t copies heads[t] (bytes [head_off[t], head_off[t + 1])
+// of `heads`) in front of line t, whose first token the scan put at line_start[t] (unshifted).  The last block
+// closes the text with '\n' at out[end].
+__global__ void __launch_bounds__(128)
+fm_k_falsta_heads(const char *__restrict__ heads, const uint64_t *__restrict__ head_off,
+                  const uint64_t *__restrict__ line_start, const uint64_t *__restrict__ track_shift, uint32_t n_tracks,
+                  uint64_t end, char *__restrict__ out) {
+    const uint32_t t = blockIdx.x;
+    const uint64_t h0 = head_off[t], hn = head_off[t + 1] - h0;
+    char *dst = out + line_start[t] + track_shift[t] - hn;
+    for (uint64_t k = threadIdx.x; k < hn; k += blockDim.x) dst[k] = heads[h0 + k];
+    if (t + 1 == n_tracks && threadIdx.x == 0) out[end] = '\n';
 }
 
 }  // namespace fm

@@ -10,6 +10,7 @@
 #include "fm_vcf.cuh"
 #include "fm_pairwise.cuh"
 #include "fm_bgzf.cuh"
+#include "fm_deflate.cuh"
 
 #include <nvtx3/nvToolsExt.h>
 
@@ -4451,31 +4452,42 @@ fm_status fm_falsta_format_value(double value, int mode, char *buf, size_t capac
     return FM_OK;
 }
 
-fm_status fm_falsta_tracks(const int64_t *pos1, const double *values, size_t n, size_t n_tracks, int64_t region_start,
-                           int64_t region_end, int mode, char *out, size_t capacity, size_t *line_len,
-                           size_t *len_out) {
-    return guarded([&] {
-        FM_NVTX("fm_falsta_tracks");
-        if (!len_out) fail(FM_ERR_INVALID_ARG, "len_out is NULL");
-        *len_out = 0;
-        if (n_tracks == 0) return;
+namespace {
+// The FALSTA chain up to the scan: scatter -> token lengths -> 64-bit exclusive scan of the lengths.  starts[t] is
+// where line t begins in the unheaded text, starts[n_tracks] = total + 1; `write` then renders the text.
+struct FalstaChain {
+    size_t n = 0, n_tracks = 0;
+    int mode = 0;
+    uint64_t L = 0, T = 0, total = 0;
+    uint32_t blocks = 0;
+    DevBuf<int> d_idx;
+    DevBuf<uint32_t> d_len;
+    DevBuf<uint64_t> d_off;
+    DevBuf<int64_t> d_pos;
+    DevBuf<double> d_val;
+    std::vector<uint64_t> starts;
+
+    // argument checks of fm_falsta_tracks (n_tracks > 0)
+    static void check(const int64_t *pos1, const double *values, size_t n, size_t n_tracks, int mode) {
         if (n && (!pos1 || !values)) fail(FM_ERR_INVALID_ARG, "record arrays are NULL");
         if (mode != FM_FALSTA_DIVERSITY && mode != FM_FALSTA_FST) fail(FM_ERR_INVALID_ARG, "unknown track mode");
         if (n >= (1ull << 31)) fail(FM_ERR_UNSUPPORTED, "more than 2^31 records per track");
         if (n_tracks > 64) fail(FM_ERR_UNSUPPORTED, "more than 64 tracks per call");
-        require_device();
-        CK(cudaSetDevice(t_device));
+    }
+    FalstaChain(const int64_t *pos1, const double *values, size_t n_, size_t n_tracks_, int64_t region_start,
+                int64_t region_end, int mode_)
+        : n(n_), n_tracks(n_tracks_), mode(mode_) {
         // ZeroBasedHalfOpen::from_1based_inclusive (process.rs:193-206)
         int64_t s1 = region_start < 1 ? 1 : region_start;
         int64_t e1 = region_end < s1 ? s1 : region_end;
         const uint64_t rs = (uint64_t)(s1 - 1), re = (uint64_t)e1;
-        const uint64_t L = re - rs;  // >= 1 by construction
-        const uint64_t T = L * n_tracks;
-        DevBuf<int> d_idx(L);
-        DevBuf<uint32_t> d_len(T);
-        DevBuf<uint64_t> d_off(T);
-        DevBuf<int64_t> d_pos(std::max<size_t>(n, 1));
-        DevBuf<double> d_val(std::max<size_t>(n * n_tracks, 1));
+        L = re - rs;  // >= 1 by construction
+        T = L * n_tracks;
+        d_idx.alloc(L);
+        d_len.alloc(T);
+        d_off.alloc(T);
+        d_pos.alloc(std::max<size_t>(n, 1));
+        d_val.alloc(std::max<size_t>(n * n_tracks, 1));
         CK(cudaMemsetAsync(d_idx.p, 0xFF, L * sizeof(int), stream()));
         h2d(d_pos.p, pos1, n * 8, stream());
         h2d(d_val.p, values, n * n_tracks * 8, stream());
@@ -4486,11 +4498,10 @@ fm_status fm_falsta_tracks(const int64_t *pos1, const double *values, size_t n, 
             CK(cudaGetLastError());
             g_launches++;
         }
-        const uint32_t blocks = (uint32_t)std::min<uint64_t>((T + 255) / 256, 16ull * dev_sms);
+        blocks = (uint32_t)std::min<uint64_t>((T + 255) / 256, 16ull * dev_sms);
         // FM_FALSTA_TEST_INFLATE=k (length queries only) adds k bytes to every token length so that a test can push
         // the body past 4 GiB without a multi-gigabyte input
         const uint32_t inflate = env_u32("FM_FALSTA_TEST_INFLATE", 0);
-        if (inflate && out) fail(FM_ERR_INVALID_ARG, "FM_FALSTA_TEST_INFLATE is for length queries (out == NULL) only");
         fm::fm_k_falsta_lengths<<<blocks, 256, 0, stream()>>>(d_idx.p, d_val.p, n, L, (uint32_t)n_tracks, mode,
                                                                d_len.p, inflate);
         CK(cudaGetLastError());
@@ -4500,32 +4511,53 @@ fm_status fm_falsta_tracks(const int64_t *pos1, const double *values, size_t n, 
         // scan is given a u64 initial value.
         size_t tmp_bytes = 0;
         thrust::transform_iterator<fm::U32ToU64, const uint32_t *> len64(d_len.p, fm::U32ToU64());
-        CK(cub::DeviceScan::ExclusiveScan(nullptr, tmp_bytes, len64, d_off.p, cuda::std::plus<>(), (uint64_t)0, (int64_t)T,
-                                          stream()));
+        CK(cub::DeviceScan::ExclusiveScan(nullptr, tmp_bytes, len64, d_off.p, cuda::std::plus<>(), (uint64_t)0,
+                                          (int64_t)T, stream()));
         DevBuf<uint8_t> d_tmp(std::max<size_t>(tmp_bytes, 16));
-        CK(cub::DeviceScan::ExclusiveScan(d_tmp.p, tmp_bytes, len64, d_off.p, cuda::std::plus<>(), (uint64_t)0, (int64_t)T,
-                                          stream()));
+        CK(cub::DeviceScan::ExclusiveScan(d_tmp.p, tmp_bytes, len64, d_off.p, cuda::std::plus<>(), (uint64_t)0,
+                                          (int64_t)T, stream()));
         // line t starts at off[t*L]; the call ends at off[T-1] + len[T-1]
-        std::vector<uint64_t> starts(n_tracks + 1);
+        starts.assign(n_tracks + 1, 0);
         for (size_t t = 0; t < n_tracks; ++t)
             CK(cudaMemcpyAsync(&starts[t], d_off.p + t * L, 8, cudaMemcpyDeviceToHost, stream()));
         uint32_t last_len = 0;
         CK(cudaMemcpyAsync(&starts[n_tracks], d_off.p + (T - 1), 8, cudaMemcpyDeviceToHost, stream()));
         CK(cudaMemcpyAsync(&last_len, d_len.p + (T - 1), 4, cudaMemcpyDeviceToHost, stream()));
         CK(cudaStreamSynchronize(stream()));
-        const uint64_t total = starts[n_tracks] + last_len;
+        total = starts[n_tracks] + last_len;
         starts[n_tracks] = total + 1;  // as if a separator followed the last line too
-        if (line_len)
-            for (size_t t = 0; t < n_tracks; ++t) line_len[t] = (size_t)(starts[t + 1] - starts[t] - 1);
-        *len_out = (size_t)total;
-        if (!out) return;  // length query
-        if (total > capacity) fail(FM_ERR_INVALID_ARG, "output capacity too small for the track lines");
-        DevBuf<char> d_out(std::max<uint64_t>(total, 1));
+    }
+    void write(char *d_out, const uint64_t *d_shift) {
         fm::fm_k_falsta_write<<<blocks, 256, 0, stream()>>>(d_idx.p, d_val.p, n, L, (uint32_t)n_tracks, mode, d_off.p,
-                                                             d_out.p);
+                                                             d_out, d_shift);
         CK(cudaGetLastError());
         g_launches++;
-        CK(cudaMemcpyAsync(out, d_out.p, total, cudaMemcpyDeviceToHost, stream()));
+    }
+};
+}  // namespace
+
+fm_status fm_falsta_tracks(const int64_t *pos1, const double *values, size_t n, size_t n_tracks, int64_t region_start,
+                           int64_t region_end, int mode, char *out, size_t capacity, size_t *line_len,
+                           size_t *len_out) {
+    return guarded([&] {
+        FM_NVTX("fm_falsta_tracks");
+        if (!len_out) fail(FM_ERR_INVALID_ARG, "len_out is NULL");
+        *len_out = 0;
+        if (n_tracks == 0) return;
+        FalstaChain::check(pos1, values, n, n_tracks, mode);
+        require_device();
+        CK(cudaSetDevice(t_device));
+        if (env_u32("FM_FALSTA_TEST_INFLATE", 0) && out)
+            fail(FM_ERR_INVALID_ARG, "FM_FALSTA_TEST_INFLATE is for length queries (out == NULL) only");
+        FalstaChain c(pos1, values, n, n_tracks, region_start, region_end, mode);
+        if (line_len)
+            for (size_t t = 0; t < n_tracks; ++t) line_len[t] = (size_t)(c.starts[t + 1] - c.starts[t] - 1);
+        *len_out = (size_t)c.total;
+        if (!out) return;  // length query
+        if (c.total > capacity) fail(FM_ERR_INVALID_ARG, "output capacity too small for the track lines");
+        DevBuf<char> d_out(std::max<uint64_t>(c.total, 1));
+        c.write(d_out.p, nullptr);
+        CK(cudaMemcpyAsync(out, d_out.p, c.total, cudaMemcpyDeviceToHost, stream()));
         CK(cudaStreamSynchronize(stream()));
     });
 }
@@ -4533,6 +4565,142 @@ fm_status fm_falsta_tracks(const int64_t *pos1, const double *values, size_t n, 
 fm_status fm_falsta_track(const int64_t *pos1, const double *values, size_t n, int64_t region_start,
                           int64_t region_end, int mode, char *out, size_t capacity, size_t *len_out) {
     return fm_falsta_tracks(pos1, values, n, 1, region_start, region_end, mode, out, capacity, nullptr, len_out);
+}
+
+// ------------------------------------------------------------------------------------ BGZF deflate (fm_deflate.cuh)
+namespace {
+constexpr uint8_t kBgzfEof[28] = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 0x42, 0x43, 2, 0,
+                                  0x1b, 0, 3, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+constexpr uint64_t kDeflateBatch = 8192;  // members per launch: 512 MiB of slots, 1 GiB of distances
+
+// BGZF members of the device bytes d_in[0, n) into out[0, capacity) while they fit; returns the members' total size.
+// Per batch: fm_k_deflate_members writes each member to its 64 KiB slot, a scan of the sizes places them, and
+// fm_k_deflate_compact packs them so that only the members cross the bus.
+uint64_t bgzf_deflate_device(const uint8_t *d_in, uint64_t n, uint8_t *out, uint64_t capacity) {
+    const uint64_t n_mem = (n + fm::DEFL_BLOCK - 1) / fm::DEFL_BLOCK;
+    if (!n_mem) return 0;
+    const uint64_t batch = std::min(n_mem, kDeflateBatch);
+    CK(cudaFuncSetAttribute(fm::fm_k_deflate_members, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                            (int)sizeof(fm::DeflateShared)));
+    DevBuf<uint32_t> d_slots(batch * (fm::DEFL_SLOT / 4)), d_sizes(batch);
+    DevBuf<uint16_t> d_dist(batch * fm::DEFL_BLOCK);
+    DevBuf<uint64_t> d_offs(batch);
+    size_t tmp_bytes = 0;
+    thrust::transform_iterator<fm::U32ToU64, const uint32_t *> size64(d_sizes.p, fm::U32ToU64());
+    CK(cub::DeviceScan::ExclusiveScan(nullptr, tmp_bytes, size64, d_offs.p, cuda::std::plus<>(), (uint64_t)0,
+                                      (int64_t)batch, stream()));
+    DevBuf<uint8_t> d_tmp(std::max<size_t>(tmp_bytes, 16));
+    uint64_t total = 0;
+    for (uint64_t m0 = 0; m0 < n_mem; m0 += batch) {
+        const uint64_t k = std::min(batch, n_mem - m0), off = m0 * fm::DEFL_BLOCK;
+        const uint64_t bytes = std::min<uint64_t>(n - off, k * fm::DEFL_BLOCK);
+        fm::fm_k_deflate_members<<<(uint32_t)k, fm::DEFL_THREADS, sizeof(fm::DeflateShared), stream()>>>(
+            d_in + off, bytes, d_slots.p, d_dist.p, d_sizes.p);
+        CK(cudaGetLastError());
+        g_launches++;
+        CK(cub::DeviceScan::ExclusiveScan(d_tmp.p, tmp_bytes, size64, d_offs.p, cuda::std::plus<>(), (uint64_t)0,
+                                          (int64_t)k, stream()));
+        uint64_t last_off = 0;
+        uint32_t last_size = 0;
+        CK(cudaMemcpyAsync(&last_off, d_offs.p + (k - 1), 8, cudaMemcpyDeviceToHost, stream()));
+        CK(cudaMemcpyAsync(&last_size, d_sizes.p + (k - 1), 4, cudaMemcpyDeviceToHost, stream()));
+        CK(cudaStreamSynchronize(stream()));
+        const uint64_t part = last_off + last_size;
+        if (out && total + part <= capacity) {
+            DevBuf<uint8_t> d_packed(part);
+            fm::fm_k_deflate_compact<<<(uint32_t)k, 256, 0, stream()>>>(d_slots.p, d_sizes.p, d_offs.p, d_packed.p);
+            CK(cudaGetLastError());
+            g_launches++;
+            CK(cudaMemcpyAsync(out + total, d_packed.p, part, cudaMemcpyDeviceToHost, stream()));
+            CK(cudaStreamSynchronize(stream()));
+        }
+        total += part;
+    }
+    return total;
+}
+
+// Appends the EOF member to a stream of `total` bytes when asked; the result's length goes to *len_out, and a
+// capacity below it is FM_ERR_INVALID_ARG (the members were copied only if they fit).
+void bgzf_finish(int flags, uint64_t total, uint8_t *out, size_t capacity, size_t *len_out) {
+    const uint64_t need = total + ((flags & FM_BGZF_EOF) ? sizeof(kBgzfEof) : 0);
+    *len_out = (size_t)need;
+    if (need > capacity) fail(FM_ERR_INVALID_ARG, "output capacity too small for the BGZF stream (" +
+                                                      std::to_string(need) + " bytes needed)");
+    if (flags & FM_BGZF_EOF) std::memcpy(out + total, kBgzfEof, sizeof(kBgzfEof));
+}
+}  // namespace
+
+fm_status fm_bgzf_deflate_bound(size_t n, int flags, size_t *bound_out) {
+    return guarded([&] {  // host only: works without a CUDA device
+        if (!bound_out) fail(FM_ERR_INVALID_ARG, "bound_out is NULL");
+        if (flags & ~FM_BGZF_EOF) fail(FM_ERR_INVALID_ARG, "unknown flags");
+        const uint64_t members = (n + fm::DEFL_BLOCK - 1) / fm::DEFL_BLOCK;  // stored: 18 + 5 + bytes + 8 each
+        *bound_out = (size_t)(n + 31 * members + ((flags & FM_BGZF_EOF) ? sizeof(kBgzfEof) : 0));
+    });
+}
+
+fm_status fm_bgzf_deflate(const uint8_t *in, size_t n, int flags, uint8_t *out, size_t capacity, size_t *len_out) {
+    return guarded([&] {
+        FM_NVTX("fm_bgzf_deflate");
+        if (!len_out) fail(FM_ERR_INVALID_ARG, "len_out is NULL");
+        *len_out = 0;
+        if (n && !in) fail(FM_ERR_INVALID_ARG, "in is NULL");
+        if (capacity && !out) fail(FM_ERR_INVALID_ARG, "out is NULL");
+        if (flags & ~FM_BGZF_EOF) fail(FM_ERR_INVALID_ARG, "unknown flags");
+        require_device();
+        CK(cudaSetDevice(t_device));
+        uint64_t total = 0;
+        if (n) {
+            DevBuf<uint8_t> d_in(n);
+            h2d(d_in.p, in, n, stream());
+            total = bgzf_deflate_device(d_in.p, n, out, capacity);
+        }
+        bgzf_finish(flags, total, out, capacity, len_out);
+    });
+}
+
+fm_status fm_falsta_tracks_bgzf(const int64_t *pos1, const double *values, size_t n, size_t n_tracks,
+                                int64_t region_start, int64_t region_end, int mode, const char *const *heads,
+                                uint8_t *out, size_t capacity, size_t *len_out) {
+    return guarded([&] {
+        FM_NVTX("fm_falsta_tracks_bgzf");
+        if (!len_out) fail(FM_ERR_INVALID_ARG, "len_out is NULL");
+        *len_out = 0;
+        if (n_tracks == 0) return;
+        FalstaChain::check(pos1, values, n, n_tracks, mode);
+        if (!heads) fail(FM_ERR_INVALID_ARG, "heads is NULL");
+        if (capacity && !out) fail(FM_ERR_INVALID_ARG, "out is NULL");
+        // heads, then per track its byte count and the running shift of the lines: one upload
+        std::vector<uint64_t> meta(3 * n_tracks + 1, 0);  // head_off[T + 1], shift[T], line_start[T]
+        std::string blob;
+        for (size_t t = 0; t < n_tracks; ++t) {
+            if (!heads[t]) fail(FM_ERR_INVALID_ARG, "heads[" + std::to_string(t) + "] is NULL");
+            blob += heads[t];
+            meta[t + 1] = blob.size();
+            meta[n_tracks + 1 + t] = blob.size();
+        }
+        require_device();
+        CK(cudaSetDevice(t_device));
+        if (env_u32("FM_FALSTA_TEST_INFLATE", 0))
+            fail(FM_ERR_INVALID_ARG, "FM_FALSTA_TEST_INFLATE is for length queries of fm_falsta_tracks only");
+        FalstaChain c(pos1, values, n, n_tracks, region_start, region_end, mode);
+        for (size_t t = 0; t < n_tracks; ++t) meta[2 * n_tracks + 1 + t] = c.starts[t];
+        const uint64_t text = c.total + blob.size() + 1;  // heads + lines + the closing '\n'
+        DevBuf<uint64_t> d_meta(meta.size());
+        DevBuf<char> d_heads(std::max<size_t>(blob.size(), 1));
+        DevBuf<uint8_t> d_text(text);
+        d_meta.upload(meta.data(), meta.size());
+        if (!blob.empty()) h2d(d_heads.p, blob.data(), blob.size(), stream());
+        const uint64_t *d_shift = d_meta.p + n_tracks + 1;
+        c.write(reinterpret_cast<char *>(d_text.p), d_shift);
+        fm::fm_k_falsta_heads<<<(uint32_t)n_tracks, 128, 0, stream()>>>(d_heads.p, d_meta.p, d_shift + n_tracks,
+                                                                          d_shift, (uint32_t)n_tracks, text - 1,
+                                                                          reinterpret_cast<char *>(d_text.p));
+        CK(cudaGetLastError());
+        g_launches++;
+        const uint64_t total = bgzf_deflate_device(d_text.p, text, out, capacity);
+        bgzf_finish(0, total, out, capacity, len_out);
+    });
 }
 
 // ------------------------------------------------------------------------------------ VCF parse/filter stage

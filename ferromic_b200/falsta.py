@@ -4,7 +4,11 @@ Mirrors `append_diversity_falsta` / `append_fst_falsta` (process.rs:3740-4002): 
 same track order, same "omit a diversity track without records" rule, the same gzip-append file
 convention.  The track bodies -- region_len comma-joined tokens per line, the O(tracks x sites)
 string work of the reference -- are rendered on the device by `fm_falsta_tracks`
-(scatter -> token lengths -> exclusive scan -> write); the host only splices headers in."""
+(scatter -> token lengths -> exclusive scan -> write); the host only splices headers in.
+
+With `bgzf=True` a writer appends BGZF members instead of one gzip member per call: the device renders the headed
+text and deflates it (`fm_falsta_tracks_bgzf`), so the text never crosses the bus uncompressed and no host gzip pass
+runs.  The file decompresses to the same text; gzip.open, zcat and flate2's MultiGzDecoder read either form."""
 from __future__ import annotations
 
 import ctypes as C
@@ -71,6 +75,43 @@ def track_lines(pos1, values, region_start: int, region_end: int, mode: int) -> 
     return lines
 
 
+def _render_text(pos1, values, region_start: int, region_end: int, mode: int, heads: Sequence[str]) -> bytes:
+    """heads[t] + line t + '\n' for every track."""
+    lines = track_lines(pos1, values, region_start, region_end, mode)
+    return b"".join(h.encode() + line + b"\n" for h, line in zip(heads, lines))
+
+
+def _render_bgzf(pos1, values, region_start: int, region_end: int, mode: int, heads: Sequence[str]) -> bytes:
+    """What _render_text gives, as BGZF members (no EOF member) rendered and deflated on the device."""
+    pos1 = np.ascontiguousarray(pos1, dtype=np.int64)
+    values = np.ascontiguousarray(values, dtype=np.float64)
+    if values.ndim == 1:
+        values = values[None, :]
+    T, n = values.shape
+    if n != pos1.shape[0]:
+        raise ValueError("values and positions differ in length")
+    enc = [h.encode() for h in heads]
+    if len(enc) != T:
+        raise ValueError("one head per track")
+    c_heads = (C.c_char_p * T)(*enc)
+    L = lib()
+    s1 = max(region_start, 1)
+    region_len = max(region_end, s1) - s1 + 1
+    text = T * (3 * region_len + 26 * min(n, region_len)) + sum(map(len, enc)) + 16  # as in track_lines
+    bound = C.c_size_t(0)
+    check(L.fm_bgzf_deflate_bound(text, 0, C.byref(bound)))
+    out = _scratch(bound.value)
+    size = C.c_size_t(0)
+    args = (pos1.ctypes.data_as(C.c_void_p), values.ctypes.data_as(C.c_void_p), n, T, region_start, region_end, mode,
+            C.cast(c_heads, C.c_void_p))
+    st = L.fm_falsta_tracks_bgzf(*args, out.ctypes.data_as(C.c_void_p), bound.value, C.byref(size))
+    if st != 0 and size.value > bound.value:
+        out = _scratch(size.value)
+        st = L.fm_falsta_tracks_bgzf(*args, out.ctypes.data_as(C.c_void_p), size.value, C.byref(size))
+    check(st)
+    return out[: size.value].tobytes()
+
+
 def _in_region(pos1: np.ndarray, region_start: int, region_end: int) -> np.ndarray:
     # from_1based_inclusive + relative_position_1based_inclusive (process.rs:193-206, 314-321)
     s1 = max(region_start, 1)
@@ -82,6 +123,10 @@ def diversity_falsta_text(seqname: str, region_start: int, region_end: int,
                           per_site: Sequence[Tuple[int, float, float, int, bool]]) -> bytes:
     """Text `append_diversity_falsta` appends for one region (process.rs:3740-3806).
     per_site records: (pos_1based, pi, theta, group_id, is_filtered)."""
+    return _diversity(seqname, region_start, region_end, per_site, _render_text)
+
+
+def _diversity(seqname, region_start, region_end, per_site, render) -> bytes:
     if len(per_site) == 0:
         return b""
     pos = np.array([r[0] for r in per_site], dtype=np.int64)
@@ -92,21 +137,13 @@ def diversity_falsta_text(seqname: str, region_start: int, region_end: int,
     inside = _in_region(pos, region_start, region_end)
     out = []
     for g in sorted(set(gid.tolist())):  # BTreeSet<u8> order
-        rendered = {}
-        for is_filtered in (False, True):
+        for is_filtered, prefix in ((False, "unfiltered_"), (True, "filtered_")):  # pi then theta of each
             sel = (gid == g) & (flt == is_filtered)
             if not np.any(sel & inside):
                 continue  # `any` stays false: the track is omitted
-            rendered[is_filtered] = track_lines(pos[sel], np.stack([pi[sel], th[sel]]), region_start, region_end,
-                                                DIVERSITY)
-        for is_filtered, which, prefix in ((False, 0, "unfiltered_pi_"), (False, 1, "unfiltered_theta_"),
-                                           (True, 0, "filtered_pi_"), (True, 1, "filtered_theta_")):
-            if is_filtered not in rendered:
-                continue
-            head = f">{prefix}chr_{seqname}_start_{region_start}_end_{region_end}_group_{g}\n"
-            out.append(head.encode())
-            out.append(rendered[is_filtered][which])
-            out.append(b"\n")
+            heads = [f">{prefix}{stat}_chr_{seqname}_start_{region_start}_end_{region_end}_group_{g}\n"
+                     for stat in ("pi", "theta")]
+            out.append(render(pos[sel], np.stack([pi[sel], th[sel]]), region_start, region_end, DIVERSITY, heads))
     return b"".join(out)
 
 
@@ -117,6 +154,10 @@ def fst_falsta_text(seqname: str, region_start: int, region_end: int,
     wc_sites records: (position_1based, overall_fst, overall_numerator, overall_denominator,
     pairwise_fst, pairwise_numerator, pairwise_denominator) -- PerSiteWcOutput;
     hudson_sites records: (position_1based, fst, numerator, denominator)."""
+    return _fst(seqname, region_start, region_end, wc_sites, hudson_sites, _render_text)
+
+
+def _fst(seqname, region_start, region_end, wc_sites, hudson_sites, render) -> bytes:
     if len(wc_sites) == 0 and len(hudson_sites) == 0:
         return b""
     tail = f"chr_{seqname}_start_{region_start}_end_{region_end}\n"
@@ -125,11 +166,8 @@ def fst_falsta_text(seqname: str, region_start: int, region_end: int,
     def emit(records, heads):
         arr = np.array(records, dtype=np.float64).reshape(len(records), len(heads) + 1)
         pos = np.array([int(r[0]) for r in records], dtype=np.int64)
-        lines = track_lines(pos, np.ascontiguousarray(arr[:, 1:].T), region_start, region_end, FST)
-        for h, line in zip(heads, lines):
-            out.append((">" + h + tail).encode())
-            out.append(line)
-            out.append(b"\n")
+        out.append(render(pos, np.ascontiguousarray(arr[:, 1:].T), region_start, region_end, FST,
+                          [">" + h + tail for h in heads]))
 
     if len(wc_sites):
         emit(wc_sites, ("haplotype_overall_fst_summary_", "haplotype_overall_fst_numerator_",
@@ -176,17 +214,33 @@ def _append_gz(path, text: bytes) -> None:
         f.write(text)
 
 
-def append_diversity_falsta(path, seqname, region_start, region_end, per_site) -> None:
+def _append_bytes(path, members: bytes) -> None:
+    # BGZF members are complete gzip members already: a plain append
+    with open(path, "ab") as f:
+        f.write(members)
+
+
+def append_diversity_falsta(path, seqname, region_start, region_end, per_site, bgzf: bool = False) -> None:
     if len(per_site) == 0:  # process.rs:3745-3754: warns and returns before the file is opened
         return
-    _append_gz(path, diversity_falsta_text(seqname, region_start, region_end, per_site))
+    if bgzf:
+        _append_bytes(path, _diversity(seqname, region_start, region_end, per_site, _render_bgzf))
+    else:
+        _append_gz(path, diversity_falsta_text(seqname, region_start, region_end, per_site))
 
 
-def append_hudson_tsv(path, rows) -> None:
-    _append_gz(path, hudson_tsv_text(rows))
+def append_hudson_tsv(path, rows, bgzf: bool = False) -> None:
+    if bgzf:
+        from .vcf import bgzf_deflate
+        _append_bytes(path, bgzf_deflate(hudson_tsv_text(rows), eof=False))
+    else:
+        _append_gz(path, hudson_tsv_text(rows))
 
 
-def append_fst_falsta(path, seqname, region_start, region_end, wc_sites, hudson_sites) -> None:
+def append_fst_falsta(path, seqname, region_start, region_end, wc_sites, hudson_sites, bgzf: bool = False) -> None:
     if len(wc_sites) == 0 and len(hudson_sites) == 0:  # process.rs:3835-3837
         return
-    _append_gz(path, fst_falsta_text(seqname, region_start, region_end, wc_sites, hudson_sites))
+    if bgzf:
+        _append_bytes(path, _fst(seqname, region_start, region_end, wc_sites, hudson_sites, _render_bgzf))
+    else:
+        _append_gz(path, fst_falsta_text(seqname, region_start, region_end, wc_sites, hudson_sites))

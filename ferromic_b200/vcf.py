@@ -250,6 +250,19 @@ def bgzf_inflate(data) -> bytes:
     return _inflate_prefix(data, total.value)[0]
 
 
+def bgzf_deflate(data, eof: bool = True) -> bytes:
+    """`data` as a BGZF stream, compressed on the device: one member per 0xff00 bytes, as bgzip cuts them, and the
+    28-byte EOF member when `eof`.  gzip, zcat and bgzf_inflate read it; the bytes depend on `data` alone."""
+    ptr, n = _gz_buffer(data)
+    bound = C.c_size_t()
+    check(lib().fm_bgzf_deflate_bound(n, _lib.FM_BGZF_EOF if eof else 0, C.byref(bound)))
+    out = np.empty(max(bound.value, 1), dtype=np.uint8)
+    size = C.c_size_t()
+    check(lib().fm_bgzf_deflate(ptr, n, _lib.FM_BGZF_EOF if eof else 0, out.ctypes.data_as(C.c_void_p), bound.value,
+                                C.byref(size)))
+    return out[:size.value].tobytes()
+
+
 def read_bgzf_header(data) -> Tuple[bytes, int]:
     """(header bytes up to and including the #CHROM line, offset of the first data line in the inflated stream).
     Inflates a prefix, doubling it until the #CHROM line ends (or the stream does)."""

@@ -506,6 +506,22 @@ fm_status fm_vcf_parse_device(const char *d_text, size_t n_bytes, char host_last
 /* Inflate the first min(capacity, total) bytes of a BGZF stream on the device into host memory; only the members
  * covering them are decoded (header reads ask for a prefix).  *total_out = the whole stream's inflated size. */
 fm_status fm_bgzf_inflate(const uint8_t *gz, size_t n_gz, uint8_t *out, size_t capacity, uint64_t *total_out);
+/* ---- BGZF deflate (DESIGN §0 row f7) ----
+ * The device writes BGZF as bgzip cuts it: one member (gzip header with the `BC` subfield, one DEFLATE block,
+ * CRC32 + ISIZE) per 0xff00 input bytes, compressed independently; gzip, zcat, flate2's MultiGzDecoder and
+ * fm_bgzf_inflate read the result.  The bytes are a pure function of the input (not of the device or the schedule).
+ * n == 0 gives no data members; FM_BGZF_EOF appends the standard 28-byte empty member.  When `capacity` is too
+ * small the call returns FM_ERR_INVALID_ARG and *len_out still receives the exact length needed.
+ * fm_bgzf_deflate_bound is host-only: the worst case (every member stored) plus the EOF member when asked for. */
+#define FM_BGZF_EOF 1
+fm_status fm_bgzf_deflate_bound(size_t n, int flags, size_t *bound_out);
+fm_status fm_bgzf_deflate(const uint8_t *in, size_t n, int flags, uint8_t *out, size_t capacity, size_t *len_out);
+/* fm_falsta_tracks rendered as heads[t] + line t + '\n' for every track (the text a FALSTA writer appends) and
+ * deflated on the device: only the BGZF members (no EOF member) cross the bus.  Arguments and region clamping as in
+ * fm_falsta_tracks; heads[t] are NUL-terminated. */
+fm_status fm_falsta_tracks_bgzf(const int64_t *pos1, const double *values, size_t n, size_t n_tracks,
+                                int64_t region_start, int64_t region_end, int mode, const char *const *heads,
+                                uint8_t *out, size_t capacity, size_t *len_out);
 /* fm_vcf_parse over the inflated stream from byte data_offset on (the first data line; header consumed by the
  * caller): same arguments after `chr`, same batch, same statistics, same error lines.  Only compressed bytes cross
  * the bus; FM_VCF_CHUNK_MB / FM_VCF_CHUNK_BYTES count inflated bytes. */

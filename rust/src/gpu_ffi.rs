@@ -87,6 +87,14 @@ extern "C" {
         n_regions: usize, kept_col_indices: *const u32, n_kept: usize, min_gq: u16, allow_mode: c_int,
         allow: *const i64, n_allow: usize, mask_mode: c_int, mask: *const i64, n_mask: usize, max_ploidy: usize,
         out: *mut *mut fm_vcf_batch) -> c_int;
+    // BGZF written on the device: one member per 0xff00 input bytes (flags: FM_BGZF_EOF = 1 appends the EOF member);
+    // fm_falsta_tracks_bgzf renders heads[t] + track line t + '\n' per track and deflates it (no EOF member)
+    pub fn fm_bgzf_deflate_bound(n: usize, flags: c_int, bound_out: *mut usize) -> c_int;
+    pub fn fm_bgzf_deflate(input: *const u8, n: usize, flags: c_int, out: *mut u8, capacity: usize,
+        len_out: *mut usize) -> c_int;
+    pub fn fm_falsta_tracks_bgzf(pos1: *const i64, values: *const f64, n: usize, n_tracks: usize,
+        region_start: i64, region_end: i64, mode: c_int, heads: *const *const c_char, out: *mut u8,
+        capacity: usize, len_out: *mut usize) -> c_int;
     // shard-mergeable window totals + finishers (multi-GPU, windows)
     pub fn fm_group_window_sums(g: *mut fm_group, windows: *const i64, n_windows: usize,
         n_variants: *mut u64, seg_sites: *mut u64, pi_sum: *mut f64, uncallable_lt2: *mut u64) -> c_int;
