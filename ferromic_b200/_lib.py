@@ -61,6 +61,19 @@ class VcfInfo(C.Structure):
         ("h2d_ms", C.c_float), ("index_ms", C.c_float), ("parse_ms", C.c_float), ("inflate_ms", C.c_float)]
 
 
+class PcaParams(C.Structure):
+    _fields_ = [("k", C.c_uint32), ("oversampling", C.c_uint32), ("power_iterations", C.c_uint32),
+                ("min_maf", C.c_double), ("max_missing", C.c_double), ("seed", C.c_uint64), ("has_region", C.c_int),
+                ("region_start", C.c_int64), ("region_end", C.c_int64)]
+
+
+class PcaInfo(C.Structure):
+    _fields_ = [("n_haplotypes", C.c_uint64), ("n_sites", C.c_uint64), ("rank", C.c_uint64),
+                ("total_variance", C.c_double)] + [
+        (f, C.c_float) for f in ("stats_ms", "planes_ms", "zt_q_ms", "z_r_ms", "gram_ms", "small_ms", "total_ms")] + [
+        ("zt_q_launches", C.c_uint32), ("z_r_launches", C.c_uint32)]
+
+
 EXPORTS = [
     "fm_last_error", "fm_version", "fm_device_count", "fm_set_device", "fm_set_devices", "fm_get_devices", "fm_synchronize", "fm_trim_pool",
     "fm_matrix_create", "fm_matrix_create_inband", "fm_matrix_create_device", "fm_matrix_retain", "fm_matrix_release",
@@ -76,7 +89,7 @@ EXPORTS = [
     "fm_vcf_batch_variants", "fm_vcf_batch_genotypes", "fm_vcf_batch_positions", "fm_vcf_batch_errors", "fm_vcf_batch_matrix", "fm_vcf_batch_matrix_packed",
     "fm_vcf_batch_release", "fm_synth_fill", "fm_timings_reset", "fm_timings_get", "fm_bench_diversity",
     "fm_pairwise_differences", "fm_bgzf_inflate", "fm_vcf_parse_bgzf", "fm_bgzf_deflate_bound", "fm_bgzf_deflate",
-    "fm_falsta_tracks_bgzf",
+    "fm_falsta_tracks_bgzf", "fm_haplotype_pca",
 ]
 
 _lib = None
@@ -189,6 +202,8 @@ def lib() -> C.CDLL:
     L.fm_comm_destroy.argtypes = [vp]
     L.fm_hudson_pair_sharded.argtypes = [vp, vp, i64, sz, sz, vp, C.POINTER(HudsonOutcome), C.POINTER(HudsonSums)]
     L.fm_pairwise_differences.argtypes = [vp, sz, vp, vp, vp, vp, sz, C.POINTER(sz)]
+    L.fm_haplotype_pca.argtypes = [vp, vp, vp, sz, C.POINTER(PcaParams), vp, vp, vp, vp, vp, vp, sz,
+                                   C.POINTER(PcaInfo)]
     for name in EXPORTS:
         fn = getattr(L, name)
         if name not in ("fm_last_error", "fm_version"):

@@ -926,6 +926,86 @@ def pairwise_differences(variants, sample_count):  # stats.rs:4106-4231
     return out
 
 
+class HaplotypePcaResult:
+    """Top principal components of the standardized haplotype x site matrix (fm_haplotype_pca).  Rows follow
+    `haplotypes` ((sample, side), sorted and de-duplicated); columns of `loadings` follow `positions`."""
+    __slots__ = ("haplotypes", "scores", "singular_values", "explained_variance_ratio", "total_variance",
+                 "positions", "loadings")
+
+    def __init__(self, haplotypes, scores, singular_values, explained_variance_ratio, total_variance, positions,
+                 loadings):
+        self.haplotypes = haplotypes
+        self.scores = scores
+        self.singular_values = singular_values
+        self.explained_variance_ratio = explained_variance_ratio
+        self.total_variance = total_variance
+        self.positions = positions
+        self.loadings = loadings
+
+    def __repr__(self):
+        return (f"HaplotypePcaResult(n_haplotypes={len(self.haplotypes)}, n_sites={len(self.positions)}, "
+                f"singular_values={self.singular_values.tolist()})")
+
+
+def _matrix_pca(m: _Matrix, haplotypes, n_components=10, region=None, min_maf=0.0, max_missing=0.0, oversampling=10,
+                power_iterations=4, seed=0, loadings=False):
+    """fm_haplotype_pca on a device matrix: dict of offsets, scores, singular_values, explained_variance_ratio,
+    total_variance, kept (matrix rows), loadings and the call's info struct."""
+    for name, x in (("n_components", n_components), ("oversampling", oversampling),
+                    ("power_iterations", power_iterations)):
+        if int(x) < 0 or int(x) >= 2 ** 32:
+            raise ValueError(f"{name} must lie in [0, 2^32)")
+    idx = np.asarray([h[0] for h in haplotypes], dtype=np.uint64)
+    side = np.asarray([h[1] for h in haplotypes], dtype=np.uint8)
+    n_in = len(haplotypes)
+    k = int(n_components)
+    prm = _lib.PcaParams(k, int(oversampling), int(power_iterations), float(min_maf), float(max_missing),
+                         int(seed) & 0xFFFFFFFFFFFFFFFF, 0 if region is None else 1,
+                         0 if region is None else int(region[0]), 0 if region is None else int(region[1]))
+    info = _lib.PcaInfo()
+    off = np.zeros(max(n_in, 1), dtype=np.uint32)
+    scores = np.zeros(max(n_in * k, 1), dtype=np.float64)
+    sv = np.zeros(max(k, 1), dtype=np.float64)
+    evr = np.zeros(max(k, 1), dtype=np.float64)
+    cap = m.V
+    kept = np.zeros(max(cap, 1), dtype=np.uint64)
+    load = np.zeros(max(cap * k, 1), dtype=np.float64) if loadings else None
+    check(lib().fm_haplotype_pca(m.handle, _ptr(idx), _ptr(side), n_in, C.byref(prm), _ptr(off), _ptr(scores), _ptr(sv),
+                                 _ptr(evr), _ptr(kept), _ptr(load), cap, C.byref(info)))
+    n, M = int(info.n_haplotypes), int(info.n_sites)
+    return dict(offsets=off[:n].copy(), scores=scores[:n * k].reshape(n, k), singular_values=sv[:k],
+                explained_variance_ratio=evr[:k], total_variance=float(info.total_variance), kept=kept[:M].astype(np.int64),
+                loadings=None if load is None else load[:M * k].reshape(M, k), info=info)
+
+
+def haplotype_pca(variants, haplotypes=None, n_components=10, region=None, min_maf=0.0, max_missing=0.0,
+                  oversampling=10, power_iterations=4, seed=0, loadings=False) -> HaplotypePcaResult:
+    """Top `n_components` principal components of the standardized haplotype x site matrix, computed on the GPU by
+    randomized subspace iteration (definition in include/ferromic_gpu.h, fm_haplotype_pca).  haplotypes: (sample,
+    side) pairs, None = every cell of every sample; region: 0-based inclusive (start, end) over positions, None =
+    every variant.  Missing cells follow from_variants semantics and are mean-imputed (Z = 0)."""
+    vs = _parse_variants(variants)
+    if region is not None:
+        region = (int(region[0]), int(region[1]))
+        if region[1] < region[0]:
+            raise ValueError("region end must be greater than or equal to region start")
+    if vs.n_variants == 0 or vs.n_samples == 0:
+        raise ValueError("haplotype PCA needs at least one variant and one sample")
+    if haplotypes is None:
+        valid = np.logical_and.accumulate(vs.gt != MISSING, axis=2)
+        sides = min(2, max(1, int(valid.sum(axis=2).max())))
+        haps = [(s, h) for s in range(vs.n_samples) for h in range(sides)]
+    else:
+        haps = _parse_haplotypes(haplotypes)
+    m = _sparse_matrix(vs)
+    r = _matrix_pca(m, haps, n_components, region, min_maf, max_missing, oversampling, power_iterations, seed,
+                    loadings)
+    P = m.P
+    return HaplotypePcaResult([(int(o) // P, int(o) % P) for o in r["offsets"]], r["scores"], r["singular_values"],
+                              r["explained_variance_ratio"], r["total_variance"], vs.positions[r["kept"]],
+                              r["loadings"])
+
+
 def _opt(value: float, some: int, bit: int):
     return value if (some >> bit) & 1 else None
 

@@ -11,10 +11,13 @@
 #include "fm_pairwise.cuh"
 #include "fm_bgzf.cuh"
 #include "fm_deflate.cuh"
+#include "fm_pca.cuh"
 
 #include <nvtx3/nvToolsExt.h>
 
 #include <cub/device/device_scan.cuh>
+#include <cub/device/device_select.cuh>
+#include <thrust/iterator/counting_iterator.h>
 #include <thrust/iterator/transform_iterator.h>
 #include <cuda/std/functional>
 
@@ -5604,6 +5607,13 @@ fm_status fm_vcf_batch_release(fm_vcf_batch *b) {
 }
 
 // ------------------------------------------------------------------------------------ pairwise differences
+// The per-cell transposes of pairwise differences and haplotype PCA read resident rows of ploidy 1 or 2.
+static void require_cell_rows(const fm_matrix *m, const char *what) {
+    if (m->ploidy < 1 || m->ploidy > 2) fail(FM_ERR_UNSUPPORTED, std::string(what) + " support ploidy 1 and 2 on the GPU path");
+    if (m->streamed && !m->packed)
+        fail(FM_ERR_UNSUPPORTED, std::string(what) + " need resident rows: this matrix was streamed as u8 rows");
+}
+
 fm_status fm_pairwise_differences(fm_matrix *m, size_t n_samples, uint32_t *differences, uint32_t *comparable,
                                   uint64_t *pair_start, int64_t *positions, size_t positions_capacity,
                                   size_t *n_positions_out) {
@@ -5612,10 +5622,7 @@ fm_status fm_pairwise_differences(fm_matrix *m, size_t n_samples, uint32_t *diff
         require_device();
         if (!m) fail(FM_ERR_INVALID_ARG, "matrix is NULL");
         if (n_samples > m->S) fail(FM_ERR_INVALID_ARG, "n_samples exceeds the matrix's sample count");
-        if (m->ploidy < 1 || m->ploidy > 2)
-            fail(FM_ERR_UNSUPPORTED, "pairwise differences support ploidy 1 and 2 on the GPU path");
-        if (m->streamed && !m->packed)
-            fail(FM_ERR_UNSUPPORTED, "pairwise differences need resident rows: this matrix was streamed as u8 rows");
+        require_cell_rows(m, "pairwise differences");
         uint32_t n_bits = 1;
         while ((1u << n_bits) <= m->plane_max_allele) ++n_bits;
         if (n_bits > 4)
@@ -5733,6 +5740,320 @@ fm_status fm_pairwise_differences(fm_matrix *m, size_t n_samples, uint32_t *diff
             *n_positions_out = (size_t)total;
         }
         CK(cudaStreamSynchronize(stream()));
+    });
+}
+
+// ------------------------------------------------------------------------------------ haplotype PCA
+// Host steps of the subspace iteration: they act on n x l and l x l blocks (l <= 64) and stay in the library so that
+// the C ABI needs no linear-algebra package.
+
+// Householder QR of the n x l row-major block A; A is replaced by the explicit orthonormal factor Q = H_0 .. H_{l-1}
+// I[:, :l].  Stable at any condition number: a zero column gets no reflection and Q stays orthonormal.
+static void pca_orth(std::vector<double> &A, uint32_t n, uint32_t l) {
+    std::vector<double> V((size_t)n * l, 0.0), vn(l, 0.0);
+    for (uint32_t j = 0; j < l; ++j) {
+        double nrm = 0.0;
+        for (uint32_t i = j; i < n; ++i) nrm += A[(size_t)i * l + j] * A[(size_t)i * l + j];
+        nrm = std::sqrt(nrm);
+        if (nrm == 0.0) continue;
+        const double alpha = A[(size_t)j * l + j] >= 0.0 ? -nrm : nrm;
+        double v2 = 0.0;
+        for (uint32_t i = j; i < n; ++i) {
+            const double v = A[(size_t)i * l + j] - (i == j ? alpha : 0.0);
+            V[(size_t)i * l + j] = v;
+            v2 += v * v;
+        }
+        vn[j] = v2;
+        for (uint32_t c = j; c < l; ++c) {
+            double d = 0.0;
+            for (uint32_t i = j; i < n; ++i) d += V[(size_t)i * l + j] * A[(size_t)i * l + c];
+            const double f = 2.0 * d / v2;
+            for (uint32_t i = j; i < n; ++i) A[(size_t)i * l + c] -= f * V[(size_t)i * l + j];
+        }
+    }
+    std::fill(A.begin(), A.end(), 0.0);
+    for (uint32_t j = 0; j < l; ++j) A[(size_t)j * l + j] = 1.0;
+    for (uint32_t j = l; j-- > 0;) {
+        if (vn[j] == 0.0) continue;
+        for (uint32_t c = 0; c < l; ++c) {
+            double d = 0.0;
+            for (uint32_t i = j; i < n; ++i) d += V[(size_t)i * l + j] * A[(size_t)i * l + c];
+            const double f = 2.0 * d / vn[j];
+            for (uint32_t i = j; i < n; ++i) A[(size_t)i * l + c] -= f * V[(size_t)i * l + j];
+        }
+    }
+}
+
+// Cyclic Jacobi eigensolver of the symmetric l x l matrix C (row-major, destroyed): eigenvalues in descending order
+// (ties keep index order) and the matching unit eigenvectors as the columns of E.
+static void pca_eigh(std::vector<double> &C, uint32_t l, std::vector<double> &lam, std::vector<double> &E) {
+    std::vector<double> V((size_t)l * l, 0.0);
+    for (uint32_t i = 0; i < l; ++i) V[(size_t)i * l + i] = 1.0;
+    double total = 0.0;
+    for (double x : C) total += x * x;
+    for (int sweep = 0; sweep < 100; ++sweep) {
+        double off = 0.0;
+        for (uint32_t p = 0; p < l; ++p)
+            for (uint32_t q = p + 1; q < l; ++q) off += 2.0 * C[(size_t)p * l + q] * C[(size_t)p * l + q];
+        if (off <= 1e-32 * total || off == 0.0) break;
+        for (uint32_t p = 0; p < l; ++p)
+            for (uint32_t q = p + 1; q < l; ++q) {
+                const double apq = C[(size_t)p * l + q];
+                if (apq == 0.0) continue;
+                const double theta = (C[(size_t)q * l + q] - C[(size_t)p * l + p]) / (2.0 * apq);
+                const double t = (theta >= 0.0 ? 1.0 : -1.0) / (std::fabs(theta) + std::sqrt(theta * theta + 1.0));
+                const double c = 1.0 / std::sqrt(t * t + 1.0), s = t * c;
+                for (uint32_t r = 0; r < l; ++r) {  // C <- C J
+                    const double x = C[(size_t)r * l + p], y = C[(size_t)r * l + q];
+                    C[(size_t)r * l + p] = c * x - s * y;
+                    C[(size_t)r * l + q] = s * x + c * y;
+                }
+                for (uint32_t r = 0; r < l; ++r) {  // C <- J^T C
+                    const double x = C[(size_t)p * l + r], y = C[(size_t)q * l + r];
+                    C[(size_t)p * l + r] = c * x - s * y;
+                    C[(size_t)q * l + r] = s * x + c * y;
+                }
+                C[(size_t)p * l + q] = C[(size_t)q * l + p] = 0.0;
+                for (uint32_t r = 0; r < l; ++r) {  // V <- V J
+                    const double x = V[(size_t)r * l + p], y = V[(size_t)r * l + q];
+                    V[(size_t)r * l + p] = c * x - s * y;
+                    V[(size_t)r * l + q] = s * x + c * y;
+                }
+            }
+    }
+    std::vector<uint32_t> ord(l);
+    for (uint32_t i = 0; i < l; ++i) ord[i] = i;
+    std::stable_sort(ord.begin(), ord.end(), [&](uint32_t a, uint32_t b) { return C[(size_t)a * l + a] > C[(size_t)b * l + b]; });
+    lam.assign(l, 0.0);
+    E.assign((size_t)l * l, 0.0);
+    for (uint32_t c = 0; c < l; ++c) {
+        lam[c] = C[(size_t)ord[c] * l + ord[c]];
+        for (uint32_t r = 0; r < l; ++r) E[(size_t)r * l + c] = V[(size_t)r * l + ord[c]];
+    }
+}
+
+static double ms_since(std::chrono::steady_clock::time_point t0) {
+    return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+}
+
+fm_status fm_haplotype_pca(fm_matrix *m, const uint64_t *sample_idx, const uint8_t *side, size_t n_in,
+                           const fm_pca_params *prm, uint32_t *hap_off_out, double *scores, double *sv, double *evr,
+                           uint64_t *kept_out, double *loadings, size_t site_capacity, fm_pca_info *info) {
+    return guarded([&] {
+        FM_NVTX("fm_haplotype_pca");
+        const auto t_call = std::chrono::steady_clock::now();
+        require_device();
+        if (!m || !prm || !info) fail(FM_ERR_INVALID_ARG, "matrix, params or info is NULL");
+        std::memset(info, 0, sizeof(*info));
+        if (n_in && (!sample_idx || !side)) fail(FM_ERR_INVALID_ARG, "haplotype arrays are NULL");
+        require_cell_rows(m, "haplotype PCA calls");
+        set_dev(m);
+        const std::vector<uint32_t> off = membership_offsets(m, sample_idx, side, n_in);
+        const uint32_t n = (uint32_t)off.size();
+        uint32_t v_lo = 0, v_hi = (uint32_t)m->V;
+        if (prm->has_region) site_range(m, prm->region_start, prm->region_end, v_lo, v_hi);
+        const uint32_t R = v_hi - v_lo;
+        fm::PcaCells cells{m->d_data, m->d_missing, !m->has_missing ? 0u : (m->in_band ? 2u : 1u), (uint64_t)m->stride,
+                           m->packed ? m->d_abits : nullptr, m->packed ? m->d_cbits : nullptr, m->rw};
+
+        // 1. site statistics, kept-site list, per-site scales and T
+        DevBuf<uint32_t> d_off(std::max<uint32_t>(n, 1)), d_alt(std::max<uint32_t>(R, 1)), d_called(std::max<uint32_t>(R, 1)),
+            d_kept(std::max<uint32_t>(R, 1)), d_nsel(1), d_inc(1);
+        DevBuf<uint8_t> d_keep(std::max<uint32_t>(R, 1));
+        DevBuf<unsigned long long> d_total(1);
+        uint32_t M = 0, incomplete = 0;
+        unsigned long long T = 0;
+        DevBuf<double> d_u;
+        {
+            FM_NVTX("fm_haplotype_pca: site statistics");
+            Timer tm;
+            tm.start();
+            d_off.upload(off.data(), n);
+            if (n && R) {
+                fm::fm_k_pca_site_stats<<<(R + 7) / 8, 256, 0, stream()>>>(cells, d_off.p, n, v_lo, R, prm->min_maf,
+                                                                          prm->max_missing, d_alt.p, d_called.p, d_keep.p);
+                CK(cudaGetLastError());
+                g_launches++;
+                thrust::counting_iterator<uint32_t> rows(v_lo);
+                size_t tmp_bytes = 0;
+                CK(cub::DeviceSelect::Flagged(nullptr, tmp_bytes, rows, d_keep.p, d_kept.p, d_nsel.p, (int64_t)R, stream()));
+                DevBuf<uint8_t> d_tmp(std::max<size_t>(tmp_bytes, 16));
+                CK(cub::DeviceSelect::Flagged(d_tmp.p, tmp_bytes, rows, d_keep.p, d_kept.p, d_nsel.p, (int64_t)R, stream()));
+                CK(cudaMemcpyAsync(&M, d_nsel.p, 4, cudaMemcpyDeviceToHost, stream()));
+                CK(cudaStreamSynchronize(stream()));
+            }
+            d_u.alloc(2 * (size_t)std::max<uint32_t>(M, 1));
+            if (M) {
+                CK(cudaMemsetAsync(d_total.p, 0, 8, stream()));
+                CK(cudaMemsetAsync(d_inc.p, 0, 4, stream()));
+                fm::fm_k_pca_scales<<<(M + 255) / 256, 256, 0, stream()>>>(d_kept.p, M, v_lo, d_alt.p, d_called.p, n, d_u.p,
+                                                                         d_total.p, d_inc.p);
+                CK(cudaGetLastError());
+                g_launches++;
+                CK(cudaMemcpyAsync(&T, d_total.p, 8, cudaMemcpyDeviceToHost, stream()));
+                CK(cudaMemcpyAsync(&incomplete, d_inc.p, 4, cudaMemcpyDeviceToHost, stream()));
+            }
+            tm.stop();
+            info->stats_ms = tm.ms();
+        }
+        info->n_haplotypes = n;
+        info->n_sites = M;
+        info->total_variance = (double)T;
+        if (hap_off_out && n) std::memcpy(hap_off_out, off.data(), (size_t)n * 4);
+
+        // 2. arguments (every message names n and M)
+        const uint64_t k = prm->k;
+        const uint64_t l64 = std::min<uint64_t>(std::min<uint64_t>(k + prm->oversampling, n), M);
+        char where[96];
+        snprintf(where, sizeof(where), " (n = %u haplotypes, M = %u kept sites)", n, M);
+        if (!(prm->min_maf >= 0.0 && prm->min_maf <= 0.5)) fail(FM_ERR_INVALID_ARG, std::string("min_maf must lie in [0, 0.5]") + where);
+        if (!(prm->max_missing >= 0.0 && prm->max_missing < 1.0))
+            fail(FM_ERR_INVALID_ARG, std::string("max_missing must lie in [0, 1)") + where);
+        if (k == 0) fail(FM_ERR_INVALID_ARG, std::string("k must be at least 1") + where);
+        if (k > std::min<uint64_t>(n, M)) fail(FM_ERR_INVALID_ARG, std::string("k exceeds min(n, M)") + where);
+        if (l64 > fm::kPcaMaxRank)
+            fail(FM_ERR_INVALID_ARG, std::string("l = min(k + oversampling, n, M) exceeds 64") + where);
+        if ((kept_out || loadings) && M > site_capacity)
+            fail(FM_ERR_INVALID_ARG, std::string("site capacity too small: info->n_sites holds the number needed") + where);
+        if (!scores || !sv || !evr) fail(FM_ERR_INVALID_ARG, "scores, singular_values and explained_variance_ratio are required");
+        const uint32_t l = (uint32_t)l64;
+        info->rank = l;
+
+        // 3. haplotype-major planes of the kept sites (a called plane only when some kept site has a missing cell)
+        const bool hc = incomplete != 0;
+        const uint32_t n_words = (M + 31) / 32, n_chunks = (n_words + fm::kPwKT - 1) / fm::kPwKT;
+        const fm::PwLayout L{(n + fm::kPwBlk - 1) / fm::kPwBlk, hc ? 2u : 1u};
+        const size_t plane_words = (size_t)n_chunks * L.n_blk * L.tile_words();
+        DevBuf<uint32_t> d_planes(plane_words);
+        {
+            FM_NVTX("fm_haplotype_pca: planes");
+            Timer tm;
+            tm.start();
+            CK(cudaMemsetAsync(d_planes.p, 0, plane_words * 4, stream()));
+            const uint64_t tasks = (uint64_t)n_words * ((n + 31) / 32);
+            const uint32_t grid = (uint32_t)std::min<uint64_t>((tasks + 7) / 8, 64ull * sm_count(m->device));
+            fm::fm_k_pca_planes<<<grid, 256, 0, stream()>>>(cells, d_off.p, n, d_kept.p, M, n_words, L, d_planes.p);
+            CK(cudaGetLastError());
+            g_launches++;
+            tm.stop();
+            info->planes_ms = tm.ms();
+        }
+
+        // 4. products.  Z R: a CTA per (site slice, 256 haplotypes); the slicing depends on n and M only, so the
+        // summation order -- and the result -- is the same on every device.
+        const uint32_t n_cg = (l + fm::kPcaCols - 1) / fm::kPcaCols, lp = n_cg * fm::kPcaCols, threads = 64 * n_cg;
+        const uint32_t n_hb = (L.n_blk + fm::kPcaHapBlocks - 1) / fm::kPcaHapBlocks;
+        const uint32_t want_slices = std::max<uint32_t>(1, 1024 / n_hb);
+        const uint32_t cps = (n_chunks + want_slices - 1) / want_slices, n_slices = (n_chunks + cps - 1) / cps;
+        const size_t smem_a = (size_t)fm::kPwBlk * lp * 8 + (size_t)L.planes * fm::kPwKT * fm::kPcaWordPitch * 4;
+        const size_t smem_b = (size_t)fm::kPcaChunk * lp * 8 + (size_t)fm::kPcaChunk * 16 +
+                              (size_t)std::min(fm::kPcaHapBlocks, L.n_blk) * L.tile_words() * 4;
+        auto kern_a = hc ? fm::fm_k_pca_zt_q<true> : fm::fm_k_pca_zt_q<false>;
+        auto kern_b = hc ? fm::fm_k_pca_z_r<true> : fm::fm_k_pca_z_r<false>;
+        CK(cudaFuncSetAttribute(kern_a, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_a));
+        CK(cudaFuncSetAttribute(kern_b, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
+        DevBuf<double> d_Q((size_t)n * l), d_Y((size_t)n * l), d_W((size_t)M * l), d_part((size_t)n_slices * n * l);
+        std::vector<double> Qh((size_t)n * l);
+        auto z_r = [&](const double *Rm) {  // Y = Z R (R = G when null), then Qh = orth(Y)
+            {
+                FM_NVTX("fm_haplotype_pca: Z R");
+                Timer tm;
+                tm.start();
+                kern_b<<<dim3(n_slices, n_hb), threads, smem_b, stream()>>>(d_planes.p, L, d_u.p, Rm, d_kept.p, prm->seed, n,
+                                                                           M, l, n_chunks, cps, d_part.p);
+                CK(cudaGetLastError());
+                const uint64_t n_el = (uint64_t)n * l;
+                fm::fm_k_pca_fold<<<(uint32_t)((n_el + 255) / 256), 256, 0, stream()>>>(d_part.p, n_slices, n_el, d_Y.p);
+                CK(cudaGetLastError());
+                g_launches += 2;
+                tm.stop();
+                info->z_r_ms += tm.ms();
+                info->z_r_launches++;
+            }
+            FM_NVTX("fm_haplotype_pca: orth");
+            const auto t0 = std::chrono::steady_clock::now();
+            d_Y.download(Qh.data(), Qh.size());
+            CK(cudaStreamSynchronize(stream()));
+            pca_orth(Qh, n, l);
+            d_Q.upload(Qh.data(), Qh.size());
+            info->small_ms += (float)ms_since(t0);
+        };
+        auto zt_q = [&]() {  // W = Z^T Q
+            FM_NVTX("fm_haplotype_pca: Z^T Q");
+            Timer tm;
+            tm.start();
+            kern_a<<<n_chunks, threads, smem_a, stream()>>>(d_planes.p, L, d_u.p, d_Q.p, n, M, l, d_W.p);
+            CK(cudaGetLastError());
+            g_launches++;
+            tm.stop();
+            info->zt_q_ms += tm.ms();
+            info->zt_q_launches++;
+        };
+        z_r(nullptr);
+        for (uint32_t it = 0; it < prm->power_iterations; ++it) {
+            zt_q();
+            z_r(d_W.p);
+        }
+        zt_q();
+
+        // 5. C = W^T W (fixed-order partials folded on the host), eigenpairs, scores, loadings
+        constexpr uint32_t kGramCtas = 256;
+        std::vector<double> part((size_t)kGramCtas * l * l), Cm((size_t)l * l, 0.0);
+        {
+            FM_NVTX("fm_haplotype_pca: W^T W");
+            Timer tm;
+            tm.start();
+            DevBuf<double> d_gram((size_t)kGramCtas * l * l);
+            fm::fm_k_pca_gram<<<kGramCtas, 256, 0, stream()>>>(d_W.p, M, l, d_gram.p);
+            CK(cudaGetLastError());
+            g_launches++;
+            d_gram.download(part.data(), part.size());
+            tm.stop();
+            info->gram_ms = tm.ms();
+        }
+        const auto t0 = std::chrono::steady_clock::now();
+        for (uint32_t b = 0; b < kGramCtas; ++b)
+            for (size_t e = 0; e < (size_t)l * l; ++e) Cm[e] += part[(size_t)b * l * l + e];
+        std::vector<double> lam, E;
+        pca_eigh(Cm, l, lam, E);
+        std::vector<double> sig(k), sign(k, 1.0);
+        for (uint32_t c = 0; c < k; ++c) sig[c] = std::sqrt(std::max(lam[c], 0.0));
+        for (uint32_t c = 0; c < k; ++c) {
+            double best = -1.0;
+            for (uint32_t i = 0; i < n; ++i) {
+                double s = 0.0;
+                for (uint32_t a = 0; a < l; ++a) s += Qh[(size_t)i * l + a] * E[(size_t)a * l + c];
+                s *= sig[c];
+                scores[(size_t)i * k + c] = s;
+                if (std::fabs(s) > best) {
+                    best = std::fabs(s);
+                    sign[c] = s < 0.0 ? -1.0 : 1.0;
+                }
+            }
+            for (uint32_t i = 0; i < n; ++i) scores[(size_t)i * k + c] *= sign[c];
+            sv[c] = sig[c];
+            evr[c] = T ? sig[c] * sig[c] / (double)T : 0.0;
+        }
+        info->small_ms += (float)ms_since(t0);
+        if (kept_out && M) {
+            std::vector<uint32_t> kh(M);
+            d_kept.download(kh.data(), M);
+            CK(cudaStreamSynchronize(stream()));
+            for (uint32_t j = 0; j < M; ++j) kept_out[j] = kh[j];
+        }
+        if (loadings && M) {
+            std::vector<double> Wh((size_t)M * l);
+            d_W.download(Wh.data(), Wh.size());
+            CK(cudaStreamSynchronize(stream()));
+            for (uint32_t j = 0; j < M; ++j)
+                for (uint32_t c = 0; c < k; ++c) {
+                    double s = 0.0;
+                    for (uint32_t a = 0; a < l; ++a) s += Wh[(size_t)j * l + a] * E[(size_t)a * l + c];
+                    loadings[(size_t)j * k + c] = sign[c] * s / sig[c];
+                }
+        }
+        CK(cudaStreamSynchronize(stream()));
+        info->total_ms = (float)ms_since(t_call);
     });
 }
 

@@ -571,6 +571,52 @@ fm_status fm_pairwise_differences(fm_matrix *m, size_t n_samples, uint32_t *diff
                                   uint64_t *pair_start_or_null /* [n_pairs+1] */, int64_t *positions_or_null,
                                   size_t positions_capacity, size_t *n_positions_out);
 
+/* ---- haplotype PCA (this project's estimator; DESIGN.md §0 row f8, §3, §4 "Haplotype PCA") ----
+ * Top k principal components of the standardized haplotype x site matrix, by randomized subspace iteration
+ * (Halko, Martinsson & Tropp 2011, Alg. 4.4, re-orthonormalized on the haplotype side).  Not bit-compatible with
+ * the reference's pca.rs: the test matrix and the filters are defined here.
+ *   haplotypes  (sample_idx, side) as fm_group_create: offsets sample * ploidy + side, sorted, de-duplicated;
+ *               out-of-range samples and side 1 at ploidy 1 are dropped.  n = their number; output rows follow
+ *               this order and haplotype_offsets [n] (may be NULL) receives the offsets.
+ *   sites       the variants with region_start <= position <= region_end (0-based inclusive; has_region == 0:
+ *               every variant).  Over the n cells of site v: called_v, alt_v = #cells whose RAW allele value is 1
+ *               (never a rank of the LUT of matrices with values above 15), other_v = #called cells whose raw value
+ *               is neither 0 nor 1.  Site v is kept when other_v == 0, 0 < alt_v < called_v,
+ *               (n - called_v) <= max_missing * n and min(alt_v, called_v - alt_v) >= min_maf * called_v (FP64).
+ *               M = number of kept sites; kept_sites [site_capacity] (may be NULL) receives their matrix rows.
+ *   Z           p_v = alt_v / called_v, s_v = 1 / sqrt(p_v (1 - p_v)); Z[i, v] = s_v (x_iv - p_v) for a called cell,
+ *               0 for a missing one.  T = ||Z||_F^2 = sum of called_v over the kept sites (info->total_variance).
+ *   iteration   l = min(k + oversampling, n, M) <= 64.  G[v, c] = +1 when bit 63 of fm_mix(seed, v, c) is clear,
+ *               else -1 (v = the site's matrix row, c < l).  Y = Z G, Q = orth(Y); power_iterations times
+ *               W = Z^T Q, Y = Z W, Q = orth(Y); then W = Z^T Q and C = W^T W = E diag(lambda) E^T (descending).
+ *   outputs     singular_values [k] = sqrt(max(lambda, 0)), explained_variance_ratio [k] = sigma^2 / T,
+ *               scores [n][k] = Q E[:, :k] diag(sigma), loadings [site_capacity][k] (may be NULL) =
+ *               W E[:, :k] diag(1 / sigma).  Each component is flipped so that its score of largest |value| (the
+ *               first on ties) is positive.
+ * All arithmetic is FP64; every sum runs in a fixed order, so equal inputs give bit-identical outputs (also from
+ * several threads at once).  FM_ERR_INVALID_ARG, with n and M in the message, for k == 0, k > min(n, M), l > 64,
+ * min_maf outside [0, 0.5] and max_missing outside [0, 1); when kept_sites or loadings is given and M >
+ * site_capacity, info is filled in (n_haplotypes, n_sites) and the call returns FM_ERR_INVALID_ARG so that the
+ * caller can retry.  FM_ERR_UNSUPPORTED for ploidy > 2 and a matrix streamed as u8 rows.  info also receives the
+ * stage times of the call (device events; small_ms is host time of the orthonormalizations and the eigenproblem). */
+typedef struct {
+    uint32_t k, oversampling, power_iterations;
+    double min_maf, max_missing;
+    uint64_t seed;
+    int has_region;
+    int64_t region_start, region_end;
+} fm_pca_params;
+typedef struct {
+    uint64_t n_haplotypes, n_sites, rank; /* n, M, l */
+    double total_variance;                /* T */
+    float stats_ms, planes_ms, zt_q_ms, z_r_ms, gram_ms, small_ms, total_ms;
+    uint32_t zt_q_launches, z_r_launches;
+} fm_pca_info;
+fm_status fm_haplotype_pca(fm_matrix *m, const uint64_t *sample_idx, const uint8_t *side, size_t n,
+                           const fm_pca_params *params, uint32_t *haplotype_offsets_or_null, double *scores,
+                           double *singular_values, double *explained_variance_ratio, uint64_t *kept_sites_or_null,
+                           double *loadings_or_null, size_t site_capacity, fm_pca_info *info);
+
 /* ---- synthetic cohorts for benchmarks and full-size parity tests ----
  * Fills a device-resident u8 matrix (reference layout) and, when d_missing != NULL, its packed
  * missing bitmap with a counter-based generator: entry (site, column) is a pure integer function

@@ -24,6 +24,20 @@ pub struct fm_fst_estimate { pub state: i32, pub value: f64, pub sum_a: f64, pub
 pub struct fm_hudson_sums { pub num: f64, pub den: f64, pub dxy: f64, pub pi1: f64, pub pi2: f64,
                             pub dxy_uncallable: u64, pub unc1: u64, pub unc2: u64 }
 
+#[repr(C)]
+pub struct fm_pca_params {
+    pub k: u32, pub oversampling: u32, pub power_iterations: u32,
+    pub min_maf: f64, pub max_missing: f64, pub seed: u64,
+    pub has_region: c_int, pub region_start: i64, pub region_end: i64,
+}
+#[repr(C)]
+#[derive(Default)]
+pub struct fm_pca_info {
+    pub n_haplotypes: u64, pub n_sites: u64, pub rank: u64, pub total_variance: f64,
+    pub stats_ms: f32, pub planes_ms: f32, pub zt_q_ms: f32, pub z_r_ms: f32, pub gram_ms: f32, pub small_ms: f32,
+    pub total_ms: f32, pub zt_q_launches: u32, pub z_r_launches: u32,
+}
+
 extern "C" {
     pub fn fm_last_error() -> *const c_char;
     pub fn fm_device_count(count: *mut c_int) -> c_int;
@@ -81,6 +95,11 @@ extern "C" {
     pub fn fm_pairwise_differences(m: *mut fm_matrix, n_samples: usize, differences: *mut u32,
         comparable: *mut u32, pair_start: *mut u64, positions: *mut i64, positions_capacity: usize,
         n_positions_out: *mut usize) -> c_int;
+    // haplotype PCA (new entry point, not a drop-in for pca.rs; estimator in include/ferromic_gpu.h)
+    pub fn fm_haplotype_pca(m: *mut fm_matrix, sample_idx: *const u64, side: *const u8, n: usize,
+        params: *const fm_pca_params, haplotype_offsets: *mut u32, scores: *mut f64, singular_values: *mut f64,
+        explained_variance_ratio: *mut f64, kept_sites: *mut u64, loadings: *mut f64, site_capacity: usize,
+        info: *mut fm_pca_info) -> c_int;
     // BGZF (.vcf.gz as bgzip writes it) inflated on the device; fm_vcf_parse_bgzf parses from data_offset on
     pub fn fm_bgzf_inflate(gz: *const u8, n_gz: usize, out: *mut u8, capacity: usize, total_out: *mut u64) -> c_int;
     pub fn fm_vcf_parse_bgzf(gz: *const u8, n_gz: usize, data_offset: u64, chr: *const c_char, regions: *const i64,
