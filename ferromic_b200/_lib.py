@@ -74,6 +74,18 @@ class PcaInfo(C.Structure):
         ("zt_q_launches", C.c_uint32), ("z_r_launches", C.c_uint32)]
 
 
+class LdParams(C.Structure):
+    _fields_ = [("window", C.c_uint32), ("max_distance", C.c_int64), ("min_maf", C.c_double),
+                ("max_missing", C.c_double), ("has_region", C.c_int), ("region_start", C.c_int64),
+                ("region_end", C.c_int64)]
+
+
+class LdInfo(C.Structure):
+    _fields_ = [("n_haplotypes", C.c_uint64), ("n_sites", C.c_uint64), ("pairs", C.c_uint64),
+                ("called_plane", C.c_uint32), ("slabs", C.c_uint32), ("band_launches", C.c_uint32)] + [
+        (f, C.c_float) for f in ("stats_ms", "planes_ms", "band_ms", "copy_ms", "total_ms")]
+
+
 EXPORTS = [
     "fm_last_error", "fm_version", "fm_device_count", "fm_set_device", "fm_set_devices", "fm_get_devices", "fm_synchronize", "fm_trim_pool",
     "fm_matrix_create", "fm_matrix_create_inband", "fm_matrix_create_device", "fm_matrix_retain", "fm_matrix_release",
@@ -89,7 +101,7 @@ EXPORTS = [
     "fm_vcf_batch_variants", "fm_vcf_batch_genotypes", "fm_vcf_batch_positions", "fm_vcf_batch_errors", "fm_vcf_batch_matrix", "fm_vcf_batch_matrix_packed",
     "fm_vcf_batch_release", "fm_synth_fill", "fm_timings_reset", "fm_timings_get", "fm_bench_diversity",
     "fm_pairwise_differences", "fm_bgzf_inflate", "fm_vcf_parse_bgzf", "fm_bgzf_deflate_bound", "fm_bgzf_deflate",
-    "fm_falsta_tracks_bgzf", "fm_haplotype_pca",
+    "fm_falsta_tracks_bgzf", "fm_haplotype_pca", "fm_haplotype_ld",
 ]
 
 _lib = None
@@ -204,6 +216,7 @@ def lib() -> C.CDLL:
     L.fm_pairwise_differences.argtypes = [vp, sz, vp, vp, vp, vp, sz, C.POINTER(sz)]
     L.fm_haplotype_pca.argtypes = [vp, vp, vp, sz, C.POINTER(PcaParams), vp, vp, vp, vp, vp, vp, sz,
                                    C.POINTER(PcaInfo)]
+    L.fm_haplotype_ld.argtypes = [vp, vp, vp, sz, C.POINTER(LdParams), vp, vp, sz, vp, vp, sz, C.POINTER(LdInfo)]
     for name in EXPORTS:
         fn = getattr(L, name)
         if name not in ("fm_last_error", "fm_version"):

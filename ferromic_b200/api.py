@@ -1006,6 +1006,81 @@ def haplotype_pca(variants, haplotypes=None, n_components=10, region=None, min_m
                               r["loadings"])
 
 
+class HaplotypeLdResult:
+    """Windowed r^2 and D' between kept sites of a haplotype set (fm_haplotype_ld).  `r2[i, d - 1]` is the pair of
+    kept sites i and i + d (positions[i], positions[i + d]); NaN where that is not a pair or a site is monomorphic
+    among the haplotypes called at both.  `dprime` has the same layout, or is None."""
+    __slots__ = ("haplotypes", "positions", "r2", "dprime")
+
+    def __init__(self, haplotypes, positions, r2, dprime):
+        self.haplotypes = haplotypes
+        self.positions = positions
+        self.r2 = r2
+        self.dprime = dprime
+
+    def __repr__(self):
+        return (f"HaplotypeLdResult(n_haplotypes={len(self.haplotypes)}, n_sites={len(self.positions)}, "
+                f"window={self.r2.shape[1]})")
+
+
+def _matrix_ld(m: _Matrix, haplotypes, window=100, max_distance=None, region=None, min_maf=0.0, max_missing=0.0,
+               dprime=False):
+    """fm_haplotype_ld on a device matrix: dict of offsets, kept (matrix rows), r2 [M, window], dprime [M, window] or
+    None, and the call's info struct.  A size query learns M first, so the outputs take M * window cells."""
+    if not 1 <= int(window) < 2 ** 32:
+        raise ValueError("window must lie in [1, 2^32)")
+    idx = np.asarray([h[0] for h in haplotypes], dtype=np.uint64)
+    side = np.asarray([h[1] for h in haplotypes], dtype=np.uint8)
+    n_in = len(haplotypes)
+    w = int(window)
+    prm = _lib.LdParams(w, -1 if max_distance is None else int(max_distance), float(min_maf), float(max_missing),
+                        0 if region is None else 1, 0 if region is None else int(region[0]),
+                        0 if region is None else int(region[1]))
+    info = _lib.LdInfo()
+    L = lib()
+    st = L.fm_haplotype_ld(m.handle, _ptr(idx), _ptr(side), n_in, C.byref(prm), None, None, 0, None, None, 0,
+                           C.byref(info))
+    if st != _lib.FM_OK and not (st == _lib.FM_ERR_INVALID_ARG and b"capacity too small" in L.fm_last_error()):
+        check(st)
+    M = int(info.n_sites)
+    off = np.zeros(max(n_in, 1), dtype=np.uint32)
+    kept = np.zeros(max(M, 1), dtype=np.uint64)
+    r2 = np.empty(max(M * w, 1), dtype=np.float32)
+    dp = np.empty(max(M * w, 1), dtype=np.float32) if dprime else None
+    check(L.fm_haplotype_ld(m.handle, _ptr(idx), _ptr(side), n_in, C.byref(prm), _ptr(off), _ptr(kept), M, _ptr(r2),
+                            _ptr(dp), M * w, C.byref(info)))
+    n = int(info.n_haplotypes)
+    return dict(offsets=off[:n].copy(), kept=kept[:M].astype(np.int64), r2=r2[:M * w].reshape(M, w),
+                dprime=None if dp is None else dp[:M * w].reshape(M, w), info=info)
+
+
+def haplotype_ld(variants, haplotypes=None, window=100, max_distance=None, region=None, min_maf=0.0, max_missing=0.0,
+                 dprime=False) -> HaplotypeLdResult:
+    """r^2 (and D' when `dprime`) between each kept site and the next `window` kept sites, computed on the GPU
+    (definition in include/ferromic_gpu.h, fm_haplotype_ld).  haplotypes: (sample, side) pairs, None = every cell of
+    every sample, as haplotype_pca; max_distance: pairs further apart in position are NaN, None = no limit; region:
+    0-based inclusive (start, end) over positions, None = every variant.  Sites are filtered as haplotype_pca filters
+    them; missing cells follow from_variants semantics and only the haplotypes called at both sites count."""
+    vs = _parse_variants(variants)
+    if region is not None:
+        region = (int(region[0]), int(region[1]))
+        if region[1] < region[0]:
+            raise ValueError("region end must be greater than or equal to region start")
+    if vs.n_variants == 0 or vs.n_samples == 0:
+        raise ValueError("haplotype LD needs at least one variant and one sample")
+    if haplotypes is None:
+        valid = np.logical_and.accumulate(vs.gt != MISSING, axis=2)
+        sides = min(2, max(1, int(valid.sum(axis=2).max())))
+        haps = [(s, h) for s in range(vs.n_samples) for h in range(sides)]
+    else:
+        haps = _parse_haplotypes(haplotypes)
+    m = _sparse_matrix(vs)
+    r = _matrix_ld(m, haps, window, max_distance, region, min_maf, max_missing, dprime)
+    P = m.P
+    return HaplotypeLdResult([(int(o) // P, int(o) % P) for o in r["offsets"]], vs.positions[r["kept"]], r["r2"],
+                             r["dprime"])
+
+
 def _opt(value: float, some: int, bit: int):
     return value if (some >> bit) & 1 else None
 

@@ -12,6 +12,7 @@
 #include "fm_bgzf.cuh"
 #include "fm_deflate.cuh"
 #include "fm_pca.cuh"
+#include "fm_ld.cuh"
 
 #include <nvtx3/nvToolsExt.h>
 
@@ -6053,6 +6054,207 @@ fm_status fm_haplotype_pca(fm_matrix *m, const uint64_t *sample_idx, const uint8
                 }
         }
         CK(cudaStreamSynchronize(stream()));
+        info->total_ms = (float)ms_since(t_call);
+    });
+}
+
+// ------------------------------------------------------------------------------------ haplotype LD
+// Output rows go to the device in slabs of whole 64-site row blocks of at most this many bytes (r^2 and D' together;
+// a single row block may exceed it).  Two slab buffers alternate: while the band kernel fills one, the other is
+// copied to the caller on a side stream, so device memory is the planes plus two slabs whatever M * window is.
+constexpr size_t kLdSlabBytes = (size_t)64 << 20;
+
+fm_status fm_haplotype_ld(fm_matrix *m, const uint64_t *sample_idx, const uint8_t *side, size_t n_in,
+                          const fm_ld_params *prm, uint32_t *hap_off_out, uint64_t *kept_out, size_t site_capacity,
+                          float *r2, float *dprime, size_t pair_capacity, fm_ld_info *info) {
+    return guarded([&] {
+        FM_NVTX("fm_haplotype_ld");
+        const auto t_call = std::chrono::steady_clock::now();
+        require_device();
+        if (!m || !prm || !info) fail(FM_ERR_INVALID_ARG, "matrix, params or info is NULL");
+        std::memset(info, 0, sizeof(*info));
+        if (n_in && (!sample_idx || !side)) fail(FM_ERR_INVALID_ARG, "haplotype arrays are NULL");
+        if (prm->window == 0) fail(FM_ERR_INVALID_ARG, "window must be at least 1");
+        if (!(prm->min_maf >= 0.0 && prm->min_maf <= 0.5)) fail(FM_ERR_INVALID_ARG, "min_maf must lie in [0, 0.5]");
+        if (!(prm->max_missing >= 0.0 && prm->max_missing < 1.0)) fail(FM_ERR_INVALID_ARG, "max_missing must lie in [0, 1)");
+        require_cell_rows(m, "haplotype LD calls");
+        if (prm->max_distance >= 0 && !m->sorted)
+            fail(FM_ERR_UNSUPPORTED, "max_distance needs variant positions sorted ascending");
+        set_dev(m);
+        const std::vector<uint32_t> off = membership_offsets(m, sample_idx, side, n_in);
+        const uint32_t n = (uint32_t)off.size();
+        if (n >= (1u << 26)) fail(FM_ERR_INVALID_ARG, "haplotype LD supports fewer than 2^26 haplotypes");
+        uint32_t v_lo = 0, v_hi = (uint32_t)m->V;
+        if (prm->has_region) site_range(m, prm->region_start, prm->region_end, v_lo, v_hi);
+        const uint32_t R = v_hi - v_lo;
+        const uint64_t window = prm->window;
+        fm::PcaCells cells{m->d_data, m->d_missing, !m->has_missing ? 0u : (m->in_band ? 2u : 1u), (uint64_t)m->stride,
+                           m->packed ? m->d_abits : nullptr, m->packed ? m->d_cbits : nullptr, m->rw};
+
+        // 1. site statistics and kept-site list (the filters of haplotype PCA), the kept sites' alt counts and
+        // positions, and whether any kept site has a missing cell
+        DevBuf<uint32_t> d_off(std::max<uint32_t>(n, 1)), d_alt(std::max<uint32_t>(R, 1)), d_called(std::max<uint32_t>(R, 1)),
+            d_kept(std::max<uint32_t>(R, 1)), d_nsel(1), d_inc(1), d_kalt;
+        DevBuf<uint8_t> d_keep(std::max<uint32_t>(R, 1));
+        DevBuf<int64_t> d_kpos;
+        uint32_t M = 0, incomplete = 0;
+        {
+            FM_NVTX("fm_haplotype_ld: site statistics");
+            Timer tm;
+            tm.start();
+            d_off.upload(off.data(), n);
+            if (n && R) {
+                fm::fm_k_pca_site_stats<<<(R + 7) / 8, 256, 0, stream()>>>(cells, d_off.p, n, v_lo, R, prm->min_maf,
+                                                                          prm->max_missing, d_alt.p, d_called.p, d_keep.p);
+                CK(cudaGetLastError());
+                g_launches++;
+                thrust::counting_iterator<uint32_t> rows(v_lo);
+                size_t tmp_bytes = 0;
+                CK(cub::DeviceSelect::Flagged(nullptr, tmp_bytes, rows, d_keep.p, d_kept.p, d_nsel.p, (int64_t)R, stream()));
+                DevBuf<uint8_t> d_tmp(std::max<size_t>(tmp_bytes, 16));
+                CK(cub::DeviceSelect::Flagged(d_tmp.p, tmp_bytes, rows, d_keep.p, d_kept.p, d_nsel.p, (int64_t)R, stream()));
+                CK(cudaMemcpyAsync(&M, d_nsel.p, 4, cudaMemcpyDeviceToHost, stream()));
+                CK(cudaStreamSynchronize(stream()));
+            }
+            d_kalt.alloc(std::max<uint32_t>(M, 1));
+            d_kpos.alloc(std::max<uint32_t>(M, 1));
+            if (M) {
+                CK(cudaMemsetAsync(d_inc.p, 0, 4, stream()));
+                fm::fm_k_ld_sites<<<(M + 255) / 256, 256, 0, stream()>>>(d_kept.p, M, v_lo, d_alt.p, d_called.p, n, m->d_pos,
+                                                                       d_kalt.p, d_kpos.p, d_inc.p);
+                CK(cudaGetLastError());
+                g_launches++;
+                CK(cudaMemcpyAsync(&incomplete, d_inc.p, 4, cudaMemcpyDeviceToHost, stream()));
+            }
+            tm.stop();
+            info->stats_ms = tm.ms();
+        }
+        std::vector<uint32_t> kh(M);
+        d_kept.download(kh.data(), M);
+        CK(cudaStreamSynchronize(stream()));
+        // pairs under the rule: (i, i + d), 1 <= d <= window, i + d < M, within max_distance when it is set
+        uint64_t pairs = 0;
+        if (prm->max_distance < 0) {
+            for (uint64_t i = 0; i < M; ++i) pairs += std::min<uint64_t>(window, M - 1 - i);
+        } else {
+            uint64_t j = 0;
+            for (uint64_t i = 0; i < M; ++i) {
+                j = std::max(j, i);
+                while (j + 1 < M && j + 1 - i <= window && m->pos[kh[j + 1]] - m->pos[kh[i]] <= prm->max_distance) ++j;
+                pairs += j - i;
+            }
+        }
+        info->n_haplotypes = n;
+        info->n_sites = M;
+        info->pairs = pairs;
+        info->called_plane = incomplete != 0;
+        if (hap_off_out && n) std::memcpy(hap_off_out, off.data(), (size_t)n * 4);
+
+        // 2. capacities (a too small one leaves the counts in info so that the caller can retry)
+        char where[96];
+        snprintf(where, sizeof(where), " (n = %u haplotypes, M = %u kept sites)", n, M);
+        if (kept_out && M > site_capacity)
+            fail(FM_ERR_INVALID_ARG, std::string("site capacity too small: info->n_sites holds the number needed") + where);
+        if ((uint64_t)M * window > pair_capacity)
+            fail(FM_ERR_INVALID_ARG, std::string("pair capacity too small: n_sites * window cells are needed") + where);
+        if (M && !r2) fail(FM_ERR_INVALID_ARG, "r2 is required");
+        if (kept_out)
+            for (uint32_t j = 0; j < M; ++j) kept_out[j] = kh[j];
+        if (M == 0) {
+            info->total_ms = (float)ms_since(t_call);
+            return;
+        }
+
+        // 3. site-major planes of the kept sites (a called plane only when some kept site has a missing cell)
+        const bool hc = incomplete != 0;
+        const uint32_t n_words = (n + 31) / 32, n_chunks = (n_words + fm::kPwKT - 1) / fm::kPwKT;
+        const fm::PwLayout L{(M + fm::kPwBlk - 1) / fm::kPwBlk, hc ? 2u : 1u};
+        const size_t plane_words = (size_t)n_chunks * L.n_blk * L.tile_words();
+        DevBuf<uint32_t> d_planes(std::max<size_t>(plane_words, 1));
+        {
+            FM_NVTX("fm_haplotype_ld: planes");
+            Timer tm;
+            tm.start();
+            if (plane_words) {
+                CK(cudaMemsetAsync(d_planes.p, 0, plane_words * 4, stream()));
+                const uint64_t tasks = (uint64_t)((M + 31) / 32) * n_words;
+                const uint32_t grid = (uint32_t)std::min<uint64_t>((tasks + 7) / 8, 64ull * sm_count(m->device));
+                fm::fm_k_ld_planes<<<grid, 256, 0, stream()>>>(cells, d_off.p, n, d_kept.p, M, n_words, L, d_planes.p);
+                CK(cudaGetLastError());
+                g_launches++;
+            }
+            tm.stop();
+            info->planes_ms = tm.ms();
+        }
+
+        // 4. banded tiles, slab by slab; slab s + 1 is computed while slab s is copied out
+        const uint32_t outs = dprime ? 2u : 1u;
+        const uint64_t tpr = (window + fm::kPwBlk - 1) / fm::kPwBlk + 1;
+        const uint64_t rb_bytes = (uint64_t)fm::kPwBlk * window * 4 * outs;
+        const uint32_t rb_per_slab = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(L.n_blk, kLdSlabBytes / rb_bytes));
+        if (tpr * rb_per_slab >= (1ull << 31)) fail(FM_ERR_UNSUPPORTED, std::string("window too large for one launch") + where);
+        const uint32_t n_slabs = (L.n_blk + rb_per_slab - 1) / rb_per_slab;
+        const size_t slab_cells = (size_t)std::min<uint64_t>(M, (uint64_t)rb_per_slab * fm::kPwBlk) * window;
+        const size_t smem = (size_t)fm::kPwStages * 2 * L.tile_words() * 4 + 2 * fm::kPwStages * 8;
+        auto kern = hc ? fm::fm_k_ld_band<true> : fm::fm_k_ld_band<false>;
+        CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        DevBuf<float> d_slab[2];
+        for (int b = 0; b < (n_slabs > 1 ? 2 : 1); ++b) d_slab[b].alloc(slab_cells * outs);
+        EventPairs evs;
+        std::vector<cudaEvent_t> band0(n_slabs), band1(n_slabs), copy0(n_slabs), copy1(n_slabs);
+        for (uint32_t s = 0; s < n_slabs; ++s) {
+            band0[s] = evs.next();
+            band1[s] = evs.next();
+            copy0[s] = evs.next();
+            copy1[s] = evs.next();
+        }
+        cudaStream_t cs = t_side_streams.get(m->device);
+        struct DrainOnExit {  // the side stream reads the slab buffers: let it finish before they are released
+            cudaStream_t s;
+            ~DrainOnExit() { cudaStreamSynchronize(s); }
+        } drain{cs};
+        auto rows_of = [&](uint32_t s, uint32_t &r0, uint32_t &r1) {
+            r0 = s * rb_per_slab * fm::kPwBlk;
+            r1 = (uint32_t)std::min<uint64_t>(M, (uint64_t)(s + 1) * rb_per_slab * fm::kPwBlk);
+        };
+        auto band = [&](uint32_t s) {
+            FM_NVTX("fm_haplotype_ld: band");
+            if (s >= 2) CK(cudaStreamWaitEvent(stream(), copy1[s - 2], 0));  // the buffer's previous slab is out
+            const uint32_t rb0 = s * rb_per_slab, nrb = std::min(rb_per_slab, L.n_blk - rb0);
+            float *buf = d_slab[s % 2].p;
+            CK(cudaEventRecord(band0[s], stream()));
+            kern<<<(uint32_t)(nrb * tpr), (fm::kLdConsumerWarps + 1) * 32, smem, stream()>>>(
+                d_planes.p, L, n_chunks, n, M, (uint32_t)window, prm->max_distance, rb0, (uint32_t)tpr, d_kalt.p, d_kpos.p,
+                buf, dprime ? buf + slab_cells : nullptr);
+            CK(cudaGetLastError());
+            g_launches++;
+            CK(cudaEventRecord(band1[s], stream()));
+            info->band_launches++;
+        };
+        band(0);
+        for (uint32_t s = 0; s < n_slabs; ++s) {
+            if (s + 1 < n_slabs) band(s + 1);  // queued before the copy below, which may block the host (pageable)
+            FM_NVTX("fm_haplotype_ld: copy");
+            uint32_t r0, r1;
+            rows_of(s, r0, r1);
+            const size_t cells_s = (size_t)(r1 - r0) * window;
+            const float *buf = d_slab[s % 2].p;
+            CK(cudaStreamWaitEvent(cs, band1[s], 0));
+            CK(cudaEventRecord(copy0[s], cs));
+            CK(cudaMemcpyAsync(r2 + (size_t)r0 * window, buf, cells_s * 4, cudaMemcpyDeviceToHost, cs));
+            if (dprime) CK(cudaMemcpyAsync(dprime + (size_t)r0 * window, buf + slab_cells, cells_s * 4, cudaMemcpyDeviceToHost, cs));
+            CK(cudaEventRecord(copy1[s], cs));
+        }
+        info->slabs = n_slabs;
+        CK(cudaStreamSynchronize(cs));
+        CK(cudaStreamSynchronize(stream()));
+        for (uint32_t s = 0; s < n_slabs; ++s) {
+            float t = 0.f;
+            CK(cudaEventElapsedTime(&t, band0[s], band1[s]));
+            info->band_ms += t;
+            CK(cudaEventElapsedTime(&t, copy0[s], copy1[s]));
+            info->copy_ms += t;
+        }
         info->total_ms = (float)ms_since(t_call);
     });
 }

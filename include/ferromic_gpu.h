@@ -617,6 +617,56 @@ fm_status fm_haplotype_pca(fm_matrix *m, const uint64_t *sample_idx, const uint8
                            double *singular_values, double *explained_variance_ratio, uint64_t *kept_sites_or_null,
                            double *loadings_or_null, size_t site_capacity, fm_pca_info *info);
 
+/* ---- haplotype LD (this project's estimator; DESIGN.md §0 row f9, §3, §4 "Haplotype LD") ----
+ * r^2 and D' between nearby kept sites of a haplotype set.
+ *   haplotypes  (sample_idx, side) as fm_group_create / fm_haplotype_pca: offsets sample * ploidy + side, sorted and
+ *               de-duplicated; out-of-range samples and side 1 at ploidy 1 are dropped.  n = their number;
+ *               haplotype_offsets [n] (may be NULL) receives the offsets.
+ *   sites       the variants in the region (has_region == 0: every variant), filtered exactly as fm_haplotype_pca
+ *               filters them.  Counts are over RAW allele values: other_v == 0, 0 < alt_v < called_v,
+ *               (n - called_v) <= max_missing * n, min(alt_v, called_v - alt_v) >= min_maf * called_v (FP64).
+ *               M = number of kept sites, in matrix-row order; kept_sites [site_capacity] (may be NULL) receives
+ *               their matrix rows.  On a kept site a called cell is 0 or 1.
+ *   pairs       the kept-site pairs (i, i + d) with 1 <= d <= window, i + d < M and, when max_distance >= 0,
+ *               pos[i + d] - pos[i] <= max_distance.
+ *   counts      per pair, over the n haplotypes (integers): c = called at both sites; a = alt at i among the c;
+ *               b = alt at j among the c; ab = alt at both.
+ *   statistics  Dn = c ab - a b (int64; D = Dn / c^2).
+ *               r2 = ((double)Dn * (double)Dn) / ((double)(a (c - a)) * (double)(b (c - b))), in exactly this order.
+ *               D' = Dn / min(a (c - b), (c - a) b) when Dn > 0, Dn / min(a b, (c - a)(c - b)) when Dn < 0 and 0 when
+ *               Dn == 0 (signed, FP64 division of the exact integers).  Both are stored as float, the FP64 value
+ *               rounded to nearest.  Both are NaN (0x7fc00000) when c == 0, when a is 0 or c or b is 0 or c
+ *               (monomorphic among the jointly called), and for every (i, d) that is not a pair under the rule above.
+ *   layout      r2 [i * window + (d - 1)] for i < M and 1 <= d <= window (pair_capacity >= M * window), so
+ *               window >= M - 1 gives the full upper triangle.  dprime (may be NULL) uses the same layout.
+ * n < 2^26, so every integer above is exact in int64 and converts exactly to FP64; with the fixed operation order
+ * the outputs are bit-identical to a plain FP64 restatement and across calls and threads.
+ * FM_ERR_INVALID_ARG for window == 0, min_maf outside [0, 0.5], max_missing outside [0, 1) and n >= 2^26.  When
+ * kept_sites is given and M > site_capacity, or M * window > pair_capacity, info is filled in (n_haplotypes,
+ * n_sites, pairs, called_plane) and the call returns FM_ERR_INVALID_ARG so that the caller can retry; r2 may be NULL
+ * on such a size query.  M == 0 is not an error: info says so and nothing is written.  FM_ERR_UNSUPPORTED for
+ * ploidy > 2, a matrix streamed as u8 rows, and max_distance >= 0 or a region on a matrix with unsorted positions.
+ * info: pairs = number of pairs under the rule; called_plane = 1 when some kept site has a missing cell; slabs and
+ * band_launches = output slabs (at most 64 MB of device output each, or one 64-site row block) and kernel launches;
+ * the stage times are device events (band_ms and copy_ms summed over the slabs, which overlap), total_ms the host
+ * time of the whole call. */
+typedef struct {
+    uint32_t window;
+    int64_t max_distance; /* < 0: none */
+    double min_maf, max_missing;
+    int has_region;
+    int64_t region_start, region_end;
+} fm_ld_params;
+typedef struct {
+    uint64_t n_haplotypes, n_sites, pairs; /* n, M, pairs under the rule */
+    uint32_t called_plane, slabs, band_launches;
+    float stats_ms, planes_ms, band_ms, copy_ms, total_ms;
+} fm_ld_info;
+fm_status fm_haplotype_ld(fm_matrix *m, const uint64_t *sample_idx, const uint8_t *side, size_t n,
+                          const fm_ld_params *params, uint32_t *haplotype_offsets_or_null,
+                          uint64_t *kept_sites_or_null, size_t site_capacity,
+                          float *r2, float *dprime_or_null, size_t pair_capacity, fm_ld_info *info);
+
 /* ---- synthetic cohorts for benchmarks and full-size parity tests ----
  * Fills a device-resident u8 matrix (reference layout) and, when d_missing != NULL, its packed
  * missing bitmap with a counter-based generator: entry (site, column) is a pure integer function

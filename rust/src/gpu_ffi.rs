@@ -37,6 +37,19 @@ pub struct fm_pca_info {
     pub stats_ms: f32, pub planes_ms: f32, pub zt_q_ms: f32, pub z_r_ms: f32, pub gram_ms: f32, pub small_ms: f32,
     pub total_ms: f32, pub zt_q_launches: u32, pub z_r_launches: u32,
 }
+#[repr(C)]
+pub struct fm_ld_params {
+    pub window: u32, pub max_distance: i64, /* < 0: none */
+    pub min_maf: f64, pub max_missing: f64,
+    pub has_region: c_int, pub region_start: i64, pub region_end: i64,
+}
+#[repr(C)]
+#[derive(Default)]
+pub struct fm_ld_info {
+    pub n_haplotypes: u64, pub n_sites: u64, pub pairs: u64,
+    pub called_plane: u32, pub slabs: u32, pub band_launches: u32,
+    pub stats_ms: f32, pub planes_ms: f32, pub band_ms: f32, pub copy_ms: f32, pub total_ms: f32,
+}
 
 extern "C" {
     pub fn fm_last_error() -> *const c_char;
@@ -100,6 +113,10 @@ extern "C" {
         params: *const fm_pca_params, haplotype_offsets: *mut u32, scores: *mut f64, singular_values: *mut f64,
         explained_variance_ratio: *mut f64, kept_sites: *mut u64, loadings: *mut f64, site_capacity: usize,
         info: *mut fm_pca_info) -> c_int;
+    // haplotype LD (new entry point; estimator in include/ferromic_gpu.h); r2 may be NULL on a size query
+    pub fn fm_haplotype_ld(m: *mut fm_matrix, sample_idx: *const u64, side: *const u8, n: usize,
+        params: *const fm_ld_params, haplotype_offsets: *mut u32, kept_sites: *mut u64, site_capacity: usize,
+        r2: *mut f32, dprime: *mut f32, pair_capacity: usize, info: *mut fm_ld_info) -> c_int;
     // BGZF (.vcf.gz as bgzip writes it) inflated on the device; fm_vcf_parse_bgzf parses from data_offset on
     pub fn fm_bgzf_inflate(gz: *const u8, n_gz: usize, out: *mut u8, capacity: usize, total_out: *mut u64) -> c_int;
     pub fn fm_vcf_parse_bgzf(gz: *const u8, n_gz: usize, data_offset: u64, chr: *const c_char, regions: *const i64,
