@@ -926,6 +926,38 @@ def pairwise_differences(variants, sample_count):  # stats.rs:4106-4231
     return out
 
 
+def _haplotype_call(what, variants, haplotypes, region):
+    """Shared front of haplotype_pca and haplotype_ld (`what` names the call in messages): the parsed variants,
+    their device matrix, the (sample, side) list (None = every cell of every sample) and the region as two ints."""
+    vs = _parse_variants(variants)
+    if region is not None:
+        region = (int(region[0]), int(region[1]))
+        if region[1] < region[0]:
+            raise ValueError("region end must be greater than or equal to region start")
+    if vs.n_variants == 0 or vs.n_samples == 0:
+        raise ValueError(f"{what} needs at least one variant and one sample")
+    if haplotypes is None:
+        valid = np.logical_and.accumulate(vs.gt != MISSING, axis=2)
+        sides = min(2, max(1, int(valid.sum(axis=2).max())))
+        haps = [(s, h) for s in range(vs.n_samples) for h in range(sides)]
+    else:
+        haps = _parse_haplotypes(haplotypes)
+    return vs, _sparse_matrix(vs), haps, region
+
+
+def _haplotype_args(haplotypes, region):
+    """The sample index and side arrays of a (sample, side) list and the (has_region, region_start, region_end)
+    fields of fm_pca_params / fm_ld_params."""
+    idx = np.asarray([h[0] for h in haplotypes], dtype=np.uint64)
+    side = np.asarray([h[1] for h in haplotypes], dtype=np.uint8)
+    return idx, side, (0, 0, 0) if region is None else (1, int(region[0]), int(region[1]))
+
+
+def _offset_haplotypes(m: _Matrix, offsets):
+    """Cell offsets of `m` -> (sample, side) pairs."""
+    return [(int(o) // m.P, int(o) % m.P) for o in offsets]
+
+
 class HaplotypePcaResult:
     """Top principal components of the standardized haplotype x site matrix (fm_haplotype_pca).  Rows follow
     `haplotypes` ((sample, side), sorted and de-duplicated); columns of `loadings` follow `positions`."""
@@ -955,13 +987,11 @@ def _matrix_pca(m: _Matrix, haplotypes, n_components=10, region=None, min_maf=0.
                     ("power_iterations", power_iterations)):
         if int(x) < 0 or int(x) >= 2 ** 32:
             raise ValueError(f"{name} must lie in [0, 2^32)")
-    idx = np.asarray([h[0] for h in haplotypes], dtype=np.uint64)
-    side = np.asarray([h[1] for h in haplotypes], dtype=np.uint8)
+    idx, side, reg = _haplotype_args(haplotypes, region)
     n_in = len(haplotypes)
     k = int(n_components)
     prm = _lib.PcaParams(k, int(oversampling), int(power_iterations), float(min_maf), float(max_missing),
-                         int(seed) & 0xFFFFFFFFFFFFFFFF, 0 if region is None else 1,
-                         0 if region is None else int(region[0]), 0 if region is None else int(region[1]))
+                         int(seed) & 0xFFFFFFFFFFFFFFFF, *reg)
     info = _lib.PcaInfo()
     off = np.zeros(max(n_in, 1), dtype=np.uint32)
     scores = np.zeros(max(n_in * k, 1), dtype=np.float64)
@@ -984,24 +1014,10 @@ def haplotype_pca(variants, haplotypes=None, n_components=10, region=None, min_m
     randomized subspace iteration (definition in include/ferromic_gpu.h, fm_haplotype_pca).  haplotypes: (sample,
     side) pairs, None = every cell of every sample; region: 0-based inclusive (start, end) over positions, None =
     every variant.  Missing cells follow from_variants semantics and are mean-imputed (Z = 0)."""
-    vs = _parse_variants(variants)
-    if region is not None:
-        region = (int(region[0]), int(region[1]))
-        if region[1] < region[0]:
-            raise ValueError("region end must be greater than or equal to region start")
-    if vs.n_variants == 0 or vs.n_samples == 0:
-        raise ValueError("haplotype PCA needs at least one variant and one sample")
-    if haplotypes is None:
-        valid = np.logical_and.accumulate(vs.gt != MISSING, axis=2)
-        sides = min(2, max(1, int(valid.sum(axis=2).max())))
-        haps = [(s, h) for s in range(vs.n_samples) for h in range(sides)]
-    else:
-        haps = _parse_haplotypes(haplotypes)
-    m = _sparse_matrix(vs)
+    vs, m, haps, region = _haplotype_call("haplotype PCA", variants, haplotypes, region)
     r = _matrix_pca(m, haps, n_components, region, min_maf, max_missing, oversampling, power_iterations, seed,
                     loadings)
-    P = m.P
-    return HaplotypePcaResult([(int(o) // P, int(o) % P) for o in r["offsets"]], r["scores"], r["singular_values"],
+    return HaplotypePcaResult(_offset_haplotypes(m, r["offsets"]), r["scores"], r["singular_values"],
                               r["explained_variance_ratio"], r["total_variance"], vs.positions[r["kept"]],
                               r["loadings"])
 
@@ -1029,13 +1045,10 @@ def _matrix_ld(m: _Matrix, haplotypes, window=100, max_distance=None, region=Non
     None, and the call's info struct.  A size query learns M first, so the outputs take M * window cells."""
     if not 1 <= int(window) < 2 ** 32:
         raise ValueError("window must lie in [1, 2^32)")
-    idx = np.asarray([h[0] for h in haplotypes], dtype=np.uint64)
-    side = np.asarray([h[1] for h in haplotypes], dtype=np.uint8)
+    idx, side, reg = _haplotype_args(haplotypes, region)
     n_in = len(haplotypes)
     w = int(window)
-    prm = _lib.LdParams(w, -1 if max_distance is None else int(max_distance), float(min_maf), float(max_missing),
-                        0 if region is None else 1, 0 if region is None else int(region[0]),
-                        0 if region is None else int(region[1]))
+    prm = _lib.LdParams(w, -1 if max_distance is None else int(max_distance), float(min_maf), float(max_missing), *reg)
     info = _lib.LdInfo()
     L = lib()
     st = L.fm_haplotype_ld(m.handle, _ptr(idx), _ptr(side), n_in, C.byref(prm), None, None, 0, None, None, 0,
@@ -1061,24 +1074,9 @@ def haplotype_ld(variants, haplotypes=None, window=100, max_distance=None, regio
     every sample, as haplotype_pca; max_distance: pairs further apart in position are NaN, None = no limit; region:
     0-based inclusive (start, end) over positions, None = every variant.  Sites are filtered as haplotype_pca filters
     them; missing cells follow from_variants semantics and only the haplotypes called at both sites count."""
-    vs = _parse_variants(variants)
-    if region is not None:
-        region = (int(region[0]), int(region[1]))
-        if region[1] < region[0]:
-            raise ValueError("region end must be greater than or equal to region start")
-    if vs.n_variants == 0 or vs.n_samples == 0:
-        raise ValueError("haplotype LD needs at least one variant and one sample")
-    if haplotypes is None:
-        valid = np.logical_and.accumulate(vs.gt != MISSING, axis=2)
-        sides = min(2, max(1, int(valid.sum(axis=2).max())))
-        haps = [(s, h) for s in range(vs.n_samples) for h in range(sides)]
-    else:
-        haps = _parse_haplotypes(haplotypes)
-    m = _sparse_matrix(vs)
+    vs, m, haps, region = _haplotype_call("haplotype LD", variants, haplotypes, region)
     r = _matrix_ld(m, haps, window, max_distance, region, min_maf, max_missing, dprime)
-    P = m.P
-    return HaplotypeLdResult([(int(o) // P, int(o) % P) for o in r["offsets"]], vs.positions[r["kept"]], r["r2"],
-                             r["dprime"])
+    return HaplotypeLdResult(_offset_haplotypes(m, r["offsets"]), vs.positions[r["kept"]], r["r2"], r["dprime"])
 
 
 def _opt(value: float, some: int, bit: int):

@@ -48,6 +48,25 @@ __device__ __forceinline__ void fm_mbar_wait(uint64_t *bar, uint32_t parity) {
     while (!fm_mbar_try_wait(bar, parity)) {
     }
 }
+// the same wait and a plain arrival, on a shared-memory address (fm_smem_u32 of the barrier)
+__device__ __forceinline__ void fm_mbar_wait(uint32_t bar, uint32_t parity) {
+    uint32_t ok;
+    do {
+        asm volatile(
+            "{\n\t.reg .pred p;\n\t"
+            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
+            "selp.u32 %0, 1, 0, p;\n\t}"
+            : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
+    } while (!ok);
+}
+__device__ __forceinline__ void fm_mbar_arrive(uint32_t bar) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
+}
+__device__ __forceinline__ uint32_t fm_lds32(uint32_t saddr) {
+    uint32_t v;
+    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(saddr));
+    return v;
+}
 __device__ __forceinline__ uint4 fm_lds128(uint32_t saddr) {
     uint4 v;
     asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(saddr));

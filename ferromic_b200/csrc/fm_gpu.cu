@@ -5615,6 +5615,62 @@ static void require_cell_rows(const fm_matrix *m, const char *what) {
         fail(FM_ERR_UNSUPPORTED, std::string(what) + " need resident rows: this matrix was streamed as u8 rows");
 }
 
+// Grid of the plane transposes (8 warps a block, one warp task at a time, grid-strided).
+static uint32_t transpose_grid(const fm_matrix *m, uint64_t tasks) {
+    return (uint32_t)std::min<uint64_t>((tasks + 7) / 8, 64ull * sm_count(m->device));
+}
+
+// The kept sites of a haplotype set, shared by haplotype PCA and haplotype LD: the region's rows [v_lo, v_lo + R)
+// pass the site filter of include/ferromic_gpu.h on the n selected cells `off`, M of them in row order in d_kept.
+// d_alt / d_called hold the counts of every region row; incomplete is set when a kept site has a missing cell.
+struct HapSites {
+    std::vector<uint32_t> off;
+    uint32_t n = 0, v_lo = 0, R = 0, M = 0, incomplete = 0;
+    fm::HapCells cells{};
+    DevBuf<uint32_t> d_off, d_alt, d_called, d_kept;
+};
+
+// Starts `tm` at its first device work; the caller stops it after its own per-kept-site kernel.
+static void select_hap_sites(const fm_matrix *m, std::vector<uint32_t> off, int has_region, int64_t region_start,
+                             int64_t region_end, double min_maf, double max_missing, Timer &tm, HapSites &hs) {
+    hs.off = std::move(off);
+    hs.n = (uint32_t)hs.off.size();
+    uint32_t v_hi = (uint32_t)m->V;
+    if (has_region) site_range(m, region_start, region_end, hs.v_lo, v_hi);
+    hs.R = v_hi - hs.v_lo;
+    const uint32_t n = hs.n, R = hs.R;
+    hs.cells = fm::HapCells{m->d_data, m->d_missing, !m->has_missing ? 0u : (m->in_band ? 2u : 1u), (uint64_t)m->stride,
+                            m->packed ? m->d_abits : nullptr, m->packed ? m->d_cbits : nullptr, m->rw};
+    hs.d_off.alloc(std::max<uint32_t>(n, 1));
+    hs.d_alt.alloc(std::max<uint32_t>(R, 1));
+    hs.d_called.alloc(std::max<uint32_t>(R, 1));
+    hs.d_kept.alloc(std::max<uint32_t>(R, 1));
+    DevBuf<uint32_t> d_counts(2);  // M, incomplete
+    DevBuf<uint8_t> d_keep(std::max<uint32_t>(R, 1));
+    tm.start();
+    hs.d_off.upload(hs.off.data(), n);
+    if (!n || !R) return;
+    CK(cudaMemsetAsync(d_counts.p, 0, 8, stream()));
+    fm::fm_k_hap_site_stats<<<(R + 7) / 8, 256, 0, stream()>>>(hs.cells, hs.d_off.p, n, hs.v_lo, R, min_maf,
+                                                              max_missing, hs.d_alt.p, hs.d_called.p, d_keep.p,
+                                                              d_counts.p + 1);
+    CK(cudaGetLastError());
+    g_launches++;
+    size_t tmp_bytes = 0;
+    auto select = [&](void *tmp) {  // a null `tmp` only sizes it
+        CK(cub::DeviceSelect::Flagged(tmp, tmp_bytes, thrust::counting_iterator<uint32_t>(hs.v_lo), d_keep.p, hs.d_kept.p,
+                                      d_counts.p, (int64_t)R, stream()));
+    };
+    select(nullptr);
+    DevBuf<uint8_t> d_tmp(std::max<size_t>(tmp_bytes, 16));
+    select(d_tmp.p);
+    uint32_t h[2];
+    d_counts.download(h, 2);
+    CK(cudaStreamSynchronize(stream()));
+    hs.M = h[0];
+    hs.incomplete = h[1];
+}
+
 fm_status fm_pairwise_differences(fm_matrix *m, size_t n_samples, uint32_t *differences, uint32_t *comparable,
                                   uint64_t *pair_start, int64_t *positions, size_t positions_capacity,
                                   size_t *n_positions_out) {
@@ -5651,8 +5707,8 @@ fm_status fm_pairwise_differences(fm_matrix *m, size_t n_samples, uint32_t *diff
         tm.start();
         if (plane_words) {
             CK(cudaMemsetAsync(d_planes.p, 0, plane_words * 4, stream()));
-            const uint64_t tasks = m->packed ? (uint64_t)n_words * ((S * PL + 31) / 32) : (uint64_t)n_words * ((S + 31) / 32);
-            const uint32_t grid = (uint32_t)std::min<uint64_t>((tasks + 7) / 8, 64ull * sm_count(m->device));
+            const uint32_t grid =
+                transpose_grid(m, m->packed ? (uint64_t)n_words * ((S * PL + 31) / 32) : (uint64_t)n_words * ((S + 31) / 32));
             if (m->packed) {
                 const uint32_t n_cell_words = (S * PL + 31) / 32;
                 if (PL == 1)
@@ -5687,7 +5743,7 @@ fm_status fm_pairwise_differences(fm_matrix *m, size_t n_samples, uint32_t *diff
 
         // 2. upper-triangle bit-GEMM over sample pairs
         const uint64_t n_tiles = (uint64_t)L.n_blk * (L.n_blk + 1) / 2;
-        const size_t smem = (size_t)fm::kPwStages * 2 * L.tile_words() * 4 + 2 * fm::kPwStages * 8;
+        const size_t smem = L.ring_bytes();
         auto kern = hc ? fm::fm_k_pairwise_counts<true> : fm::fm_k_pairwise_counts<false>;
         CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         Timer tk;
@@ -5849,58 +5905,34 @@ fm_status fm_haplotype_pca(fm_matrix *m, const uint64_t *sample_idx, const uint8
         if (n_in && (!sample_idx || !side)) fail(FM_ERR_INVALID_ARG, "haplotype arrays are NULL");
         require_cell_rows(m, "haplotype PCA calls");
         set_dev(m);
-        const std::vector<uint32_t> off = membership_offsets(m, sample_idx, side, n_in);
-        const uint32_t n = (uint32_t)off.size();
-        uint32_t v_lo = 0, v_hi = (uint32_t)m->V;
-        if (prm->has_region) site_range(m, prm->region_start, prm->region_end, v_lo, v_hi);
-        const uint32_t R = v_hi - v_lo;
-        fm::PcaCells cells{m->d_data, m->d_missing, !m->has_missing ? 0u : (m->in_band ? 2u : 1u), (uint64_t)m->stride,
-                           m->packed ? m->d_abits : nullptr, m->packed ? m->d_cbits : nullptr, m->rw};
 
         // 1. site statistics, kept-site list, per-site scales and T
-        DevBuf<uint32_t> d_off(std::max<uint32_t>(n, 1)), d_alt(std::max<uint32_t>(R, 1)), d_called(std::max<uint32_t>(R, 1)),
-            d_kept(std::max<uint32_t>(R, 1)), d_nsel(1), d_inc(1);
-        DevBuf<uint8_t> d_keep(std::max<uint32_t>(R, 1));
+        HapSites hs;
         DevBuf<unsigned long long> d_total(1);
-        uint32_t M = 0, incomplete = 0;
         unsigned long long T = 0;
         DevBuf<double> d_u;
         {
             FM_NVTX("fm_haplotype_pca: site statistics");
             Timer tm;
-            tm.start();
-            d_off.upload(off.data(), n);
-            if (n && R) {
-                fm::fm_k_pca_site_stats<<<(R + 7) / 8, 256, 0, stream()>>>(cells, d_off.p, n, v_lo, R, prm->min_maf,
-                                                                          prm->max_missing, d_alt.p, d_called.p, d_keep.p);
-                CK(cudaGetLastError());
-                g_launches++;
-                thrust::counting_iterator<uint32_t> rows(v_lo);
-                size_t tmp_bytes = 0;
-                CK(cub::DeviceSelect::Flagged(nullptr, tmp_bytes, rows, d_keep.p, d_kept.p, d_nsel.p, (int64_t)R, stream()));
-                DevBuf<uint8_t> d_tmp(std::max<size_t>(tmp_bytes, 16));
-                CK(cub::DeviceSelect::Flagged(d_tmp.p, tmp_bytes, rows, d_keep.p, d_kept.p, d_nsel.p, (int64_t)R, stream()));
-                CK(cudaMemcpyAsync(&M, d_nsel.p, 4, cudaMemcpyDeviceToHost, stream()));
-                CK(cudaStreamSynchronize(stream()));
-            }
-            d_u.alloc(2 * (size_t)std::max<uint32_t>(M, 1));
-            if (M) {
+            select_hap_sites(m, membership_offsets(m, sample_idx, side, n_in), prm->has_region, prm->region_start,
+                             prm->region_end, prm->min_maf, prm->max_missing, tm, hs);
+            d_u.alloc(2 * (size_t)std::max<uint32_t>(hs.M, 1));
+            if (hs.M) {
                 CK(cudaMemsetAsync(d_total.p, 0, 8, stream()));
-                CK(cudaMemsetAsync(d_inc.p, 0, 4, stream()));
-                fm::fm_k_pca_scales<<<(M + 255) / 256, 256, 0, stream()>>>(d_kept.p, M, v_lo, d_alt.p, d_called.p, n, d_u.p,
-                                                                         d_total.p, d_inc.p);
+                fm::fm_k_pca_scales<<<(hs.M + 255) / 256, 256, 0, stream()>>>(hs.d_kept.p, hs.M, hs.v_lo, hs.d_alt.p,
+                                                                            hs.d_called.p, d_u.p, d_total.p);
                 CK(cudaGetLastError());
                 g_launches++;
                 CK(cudaMemcpyAsync(&T, d_total.p, 8, cudaMemcpyDeviceToHost, stream()));
-                CK(cudaMemcpyAsync(&incomplete, d_inc.p, 4, cudaMemcpyDeviceToHost, stream()));
             }
             tm.stop();
             info->stats_ms = tm.ms();
         }
+        const uint32_t n = hs.n, M = hs.M;
         info->n_haplotypes = n;
         info->n_sites = M;
         info->total_variance = (double)T;
-        if (hap_off_out && n) std::memcpy(hap_off_out, off.data(), (size_t)n * 4);
+        if (hap_off_out && n) std::memcpy(hap_off_out, hs.off.data(), (size_t)n * 4);
 
         // 2. arguments (every message names n and M)
         const uint64_t k = prm->k;
@@ -5921,7 +5953,7 @@ fm_status fm_haplotype_pca(fm_matrix *m, const uint64_t *sample_idx, const uint8
         info->rank = l;
 
         // 3. haplotype-major planes of the kept sites (a called plane only when some kept site has a missing cell)
-        const bool hc = incomplete != 0;
+        const bool hc = hs.incomplete != 0;
         const uint32_t n_words = (M + 31) / 32, n_chunks = (n_words + fm::kPwKT - 1) / fm::kPwKT;
         const fm::PwLayout L{(n + fm::kPwBlk - 1) / fm::kPwBlk, hc ? 2u : 1u};
         const size_t plane_words = (size_t)n_chunks * L.n_blk * L.tile_words();
@@ -5931,9 +5963,8 @@ fm_status fm_haplotype_pca(fm_matrix *m, const uint64_t *sample_idx, const uint8
             Timer tm;
             tm.start();
             CK(cudaMemsetAsync(d_planes.p, 0, plane_words * 4, stream()));
-            const uint64_t tasks = (uint64_t)n_words * ((n + 31) / 32);
-            const uint32_t grid = (uint32_t)std::min<uint64_t>((tasks + 7) / 8, 64ull * sm_count(m->device));
-            fm::fm_k_pca_planes<<<grid, 256, 0, stream()>>>(cells, d_off.p, n, d_kept.p, M, n_words, L, d_planes.p);
+            const uint32_t grid = transpose_grid(m, (uint64_t)n_words * ((n + 31) / 32));
+            fm::fm_k_pca_planes<<<grid, 256, 0, stream()>>>(hs.cells, hs.d_off.p, n, hs.d_kept.p, M, n_words, L, d_planes.p);
             CK(cudaGetLastError());
             g_launches++;
             tm.stop();
@@ -5960,8 +5991,8 @@ fm_status fm_haplotype_pca(fm_matrix *m, const uint64_t *sample_idx, const uint8
                 FM_NVTX("fm_haplotype_pca: Z R");
                 Timer tm;
                 tm.start();
-                kern_b<<<dim3(n_slices, n_hb), threads, smem_b, stream()>>>(d_planes.p, L, d_u.p, Rm, d_kept.p, prm->seed, n,
-                                                                           M, l, n_chunks, cps, d_part.p);
+                kern_b<<<dim3(n_slices, n_hb), threads, smem_b, stream()>>>(d_planes.p, L, d_u.p, Rm, hs.d_kept.p, prm->seed,
+                                                                           n, M, l, n_chunks, cps, d_part.p);
                 CK(cudaGetLastError());
                 const uint64_t n_el = (uint64_t)n * l;
                 fm::fm_k_pca_fold<<<(uint32_t)((n_el + 255) / 256), 256, 0, stream()>>>(d_part.p, n_slices, n_el, d_Y.p);
@@ -6038,7 +6069,7 @@ fm_status fm_haplotype_pca(fm_matrix *m, const uint64_t *sample_idx, const uint8
         info->small_ms += (float)ms_since(t0);
         if (kept_out && M) {
             std::vector<uint32_t> kh(M);
-            d_kept.download(kh.data(), M);
+            hs.d_kept.download(kh.data(), M);
             CK(cudaStreamSynchronize(stream()));
             for (uint32_t j = 0; j < M; ++j) kept_out[j] = kh[j];
         }
@@ -6081,56 +6112,34 @@ fm_status fm_haplotype_ld(fm_matrix *m, const uint64_t *sample_idx, const uint8_
         if (prm->max_distance >= 0 && !m->sorted)
             fail(FM_ERR_UNSUPPORTED, "max_distance needs variant positions sorted ascending");
         set_dev(m);
-        const std::vector<uint32_t> off = membership_offsets(m, sample_idx, side, n_in);
-        const uint32_t n = (uint32_t)off.size();
-        if (n >= (1u << 26)) fail(FM_ERR_INVALID_ARG, "haplotype LD supports fewer than 2^26 haplotypes");
-        uint32_t v_lo = 0, v_hi = (uint32_t)m->V;
-        if (prm->has_region) site_range(m, prm->region_start, prm->region_end, v_lo, v_hi);
-        const uint32_t R = v_hi - v_lo;
+        std::vector<uint32_t> off = membership_offsets(m, sample_idx, side, n_in);
+        if (off.size() >= (1u << 26)) fail(FM_ERR_INVALID_ARG, "haplotype LD supports fewer than 2^26 haplotypes");
         const uint64_t window = prm->window;
-        fm::PcaCells cells{m->d_data, m->d_missing, !m->has_missing ? 0u : (m->in_band ? 2u : 1u), (uint64_t)m->stride,
-                           m->packed ? m->d_abits : nullptr, m->packed ? m->d_cbits : nullptr, m->rw};
 
-        // 1. site statistics and kept-site list (the filters of haplotype PCA), the kept sites' alt counts and
-        // positions, and whether any kept site has a missing cell
-        DevBuf<uint32_t> d_off(std::max<uint32_t>(n, 1)), d_alt(std::max<uint32_t>(R, 1)), d_called(std::max<uint32_t>(R, 1)),
-            d_kept(std::max<uint32_t>(R, 1)), d_nsel(1), d_inc(1), d_kalt;
-        DevBuf<uint8_t> d_keep(std::max<uint32_t>(R, 1));
+        // 1. site statistics and kept-site list (the filters of haplotype PCA) and the kept sites' alt counts and
+        // positions
+        HapSites hs;
+        DevBuf<uint32_t> d_kalt;
         DevBuf<int64_t> d_kpos;
-        uint32_t M = 0, incomplete = 0;
         {
             FM_NVTX("fm_haplotype_ld: site statistics");
             Timer tm;
-            tm.start();
-            d_off.upload(off.data(), n);
-            if (n && R) {
-                fm::fm_k_pca_site_stats<<<(R + 7) / 8, 256, 0, stream()>>>(cells, d_off.p, n, v_lo, R, prm->min_maf,
-                                                                          prm->max_missing, d_alt.p, d_called.p, d_keep.p);
+            select_hap_sites(m, std::move(off), prm->has_region, prm->region_start, prm->region_end, prm->min_maf,
+                             prm->max_missing, tm, hs);
+            d_kalt.alloc(std::max<uint32_t>(hs.M, 1));
+            d_kpos.alloc(std::max<uint32_t>(hs.M, 1));
+            if (hs.M) {
+                fm::fm_k_ld_sites<<<(hs.M + 255) / 256, 256, 0, stream()>>>(hs.d_kept.p, hs.M, hs.v_lo, hs.d_alt.p, m->d_pos,
+                                                                          d_kalt.p, d_kpos.p);
                 CK(cudaGetLastError());
                 g_launches++;
-                thrust::counting_iterator<uint32_t> rows(v_lo);
-                size_t tmp_bytes = 0;
-                CK(cub::DeviceSelect::Flagged(nullptr, tmp_bytes, rows, d_keep.p, d_kept.p, d_nsel.p, (int64_t)R, stream()));
-                DevBuf<uint8_t> d_tmp(std::max<size_t>(tmp_bytes, 16));
-                CK(cub::DeviceSelect::Flagged(d_tmp.p, tmp_bytes, rows, d_keep.p, d_kept.p, d_nsel.p, (int64_t)R, stream()));
-                CK(cudaMemcpyAsync(&M, d_nsel.p, 4, cudaMemcpyDeviceToHost, stream()));
-                CK(cudaStreamSynchronize(stream()));
-            }
-            d_kalt.alloc(std::max<uint32_t>(M, 1));
-            d_kpos.alloc(std::max<uint32_t>(M, 1));
-            if (M) {
-                CK(cudaMemsetAsync(d_inc.p, 0, 4, stream()));
-                fm::fm_k_ld_sites<<<(M + 255) / 256, 256, 0, stream()>>>(d_kept.p, M, v_lo, d_alt.p, d_called.p, n, m->d_pos,
-                                                                       d_kalt.p, d_kpos.p, d_inc.p);
-                CK(cudaGetLastError());
-                g_launches++;
-                CK(cudaMemcpyAsync(&incomplete, d_inc.p, 4, cudaMemcpyDeviceToHost, stream()));
             }
             tm.stop();
             info->stats_ms = tm.ms();
         }
+        const uint32_t n = hs.n, M = hs.M;
         std::vector<uint32_t> kh(M);
-        d_kept.download(kh.data(), M);
+        hs.d_kept.download(kh.data(), M);
         CK(cudaStreamSynchronize(stream()));
         // pairs under the rule: (i, i + d), 1 <= d <= window, i + d < M, within max_distance when it is set
         uint64_t pairs = 0;
@@ -6147,8 +6156,8 @@ fm_status fm_haplotype_ld(fm_matrix *m, const uint64_t *sample_idx, const uint8_
         info->n_haplotypes = n;
         info->n_sites = M;
         info->pairs = pairs;
-        info->called_plane = incomplete != 0;
-        if (hap_off_out && n) std::memcpy(hap_off_out, off.data(), (size_t)n * 4);
+        info->called_plane = hs.incomplete != 0;
+        if (hap_off_out && n) std::memcpy(hap_off_out, hs.off.data(), (size_t)n * 4);
 
         // 2. capacities (a too small one leaves the counts in info so that the caller can retry)
         char where[96];
@@ -6166,7 +6175,7 @@ fm_status fm_haplotype_ld(fm_matrix *m, const uint64_t *sample_idx, const uint8_
         }
 
         // 3. site-major planes of the kept sites (a called plane only when some kept site has a missing cell)
-        const bool hc = incomplete != 0;
+        const bool hc = hs.incomplete != 0;
         const uint32_t n_words = (n + 31) / 32, n_chunks = (n_words + fm::kPwKT - 1) / fm::kPwKT;
         const fm::PwLayout L{(M + fm::kPwBlk - 1) / fm::kPwBlk, hc ? 2u : 1u};
         const size_t plane_words = (size_t)n_chunks * L.n_blk * L.tile_words();
@@ -6177,9 +6186,8 @@ fm_status fm_haplotype_ld(fm_matrix *m, const uint64_t *sample_idx, const uint8_
             tm.start();
             if (plane_words) {
                 CK(cudaMemsetAsync(d_planes.p, 0, plane_words * 4, stream()));
-                const uint64_t tasks = (uint64_t)((M + 31) / 32) * n_words;
-                const uint32_t grid = (uint32_t)std::min<uint64_t>((tasks + 7) / 8, 64ull * sm_count(m->device));
-                fm::fm_k_ld_planes<<<grid, 256, 0, stream()>>>(cells, d_off.p, n, d_kept.p, M, n_words, L, d_planes.p);
+                const uint32_t grid = transpose_grid(m, (uint64_t)((M + 31) / 32) * n_words);
+                fm::fm_k_ld_planes<<<grid, 256, 0, stream()>>>(hs.cells, hs.d_off.p, n, hs.d_kept.p, M, n_words, L, d_planes.p);
                 CK(cudaGetLastError());
                 g_launches++;
             }
@@ -6195,7 +6203,7 @@ fm_status fm_haplotype_ld(fm_matrix *m, const uint64_t *sample_idx, const uint8_
         if (tpr * rb_per_slab >= (1ull << 31)) fail(FM_ERR_UNSUPPORTED, std::string("window too large for one launch") + where);
         const uint32_t n_slabs = (L.n_blk + rb_per_slab - 1) / rb_per_slab;
         const size_t slab_cells = (size_t)std::min<uint64_t>(M, (uint64_t)rb_per_slab * fm::kPwBlk) * window;
-        const size_t smem = (size_t)fm::kPwStages * 2 * L.tile_words() * 4 + 2 * fm::kPwStages * 8;
+        const size_t smem = L.ring_bytes();
         auto kern = hc ? fm::fm_k_ld_band<true> : fm::fm_k_ld_band<false>;
         CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         DevBuf<float> d_slab[2];

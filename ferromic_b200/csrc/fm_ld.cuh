@@ -11,9 +11,8 @@
 // epilogue follows the header's operation order, so the outputs equal the numpy restatement bit for bit.
 #pragma once
 #include "fm_device.cuh"
-#include "fm_pairwise.cuh"  // PwLayout, kPwBlk, kPwKT, kPwStages
-#include "fm_pca.cuh"       // PcaCells
-#include "fm_wc.cuh"        // fm_mbar_wait / fm_mbar_arrive on shared-memory addresses
+#include "fm_haplotypes.cuh"  // HapCells
+#include "fm_pairwise.cuh"    // PwLayout, PwRing, kPwBlk, kPwKT
 
 namespace fm {
 
@@ -23,23 +22,15 @@ namespace fm {
 constexpr uint32_t kLdConsumerWarps = 8;
 constexpr uint32_t kLdNanBits = 0x7fc00000u;  // the quiet NaN numpy writes for float32('nan')
 
-__device__ __forceinline__ uint32_t fm_ld_lds32(uint32_t saddr) {
-    uint32_t v;
-    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(saddr));
-    return v;
-}
-
-// Per kept site j (matrix row kept[j]): its alt count and position; *incomplete |= called < n.
+// Per kept site j (matrix row kept[j]): its alt count and position.
 __global__ void __launch_bounds__(256)
 fm_k_ld_sites(const uint32_t *__restrict__ kept, uint32_t M, uint32_t v_lo, const uint32_t *__restrict__ alt,
-              const uint32_t *__restrict__ called, uint32_t n, const int64_t *__restrict__ pos,
-              uint32_t *__restrict__ kalt, int64_t *__restrict__ kpos, uint32_t *__restrict__ incomplete) {
+              const int64_t *__restrict__ pos, uint32_t *__restrict__ kalt, int64_t *__restrict__ kpos) {
     const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= M) return;
     const uint32_t v = kept[j];
     kalt[j] = alt[v - v_lo];
     kpos[j] = pos[v];
-    if (called[v - v_lo] < n) atomicOr(incomplete, 1u);
 }
 
 // Kept sites x selected haplotypes -> site-major planes of PwLayout{ceil(M / 64), planes}.  One warp per (32 kept
@@ -47,7 +38,7 @@ fm_k_ld_sites(const uint32_t *__restrict__ kept, uint32_t M, uint32_t v_lo, cons
 // t keeps for site t; the 32 site words are then one coalesced store per plane.  Padded sites and haplotypes stay
 // zero (the planes are cleared before the launch).
 __global__ void __launch_bounds__(256)
-fm_k_ld_planes(PcaCells cells, const uint32_t *__restrict__ off, uint32_t n, const uint32_t *__restrict__ kept,
+fm_k_ld_planes(HapCells cells, const uint32_t *__restrict__ off, uint32_t n, const uint32_t *__restrict__ kept,
                uint32_t M, uint32_t n_words, PwLayout L, uint32_t *__restrict__ planes) {
     constexpr uint32_t FULL = 0xffffffffu;
     const uint32_t lane = threadIdx.x & 31;
@@ -88,47 +79,24 @@ __device__ __forceinline__ void fm_ld_stats(int64_t c, int64_t a, int64_t b, int
 
 // Banded upper-triangle bit product over one slab of row blocks [rb0, rb0 + gridDim.x / tpr).  CTA t is tile
 // (bi, bj) = (rb0 + t / tpr, bi + t % tpr); tpr = ceil(window / 64) + 1 tiles per row block cover every (i, d) with
-// 1 <= d <= window exactly once.  Warp kLdConsumerWarps is the producer of fm_k_pairwise_counts' bulk-copy ring (one
-// block on diagonal tiles); a tile past the last site block has no chunks and only writes its NaN cells.  Consumer
-// thread (ti, tj) owns the sites i = 64 bi + 4 ti + {0..3} and j = 64 bj + tj + 16 {0..3}, so that for each of its
-// pairs the 16 threads of a row write 16 consecutive floats.  out_r2 / out_dp hold the slab's rows:
-// [(i - 64 rb0) * window + d - 1].
+// 1 <= d <= window exactly once.  Warp kLdConsumerWarps is the producer of the tile's PwRing; a tile past the last
+// site block has no chunks and only writes its NaN cells.  Consumer thread (ti, tj) owns the sites
+// i = 64 bi + 4 ti + {0..3} and j = 64 bj + tj + 16 {0..3}, so that for each of its pairs the 16 threads of a row
+// write 16 consecutive floats.  out_r2 / out_dp hold the slab's rows: [(i - 64 rb0) * window + d - 1].
 template <bool HC>
 __global__ void __launch_bounds__((kLdConsumerWarps + 1) * 32)
 fm_k_ld_band(const uint32_t *__restrict__ planes, PwLayout L, uint32_t n_chunks, uint32_t n, uint32_t M,
              uint32_t window, int64_t max_distance, uint32_t rb0, uint32_t tpr, const uint32_t *__restrict__ kalt,
              const int64_t *__restrict__ kpos, float *__restrict__ out_r2, float *__restrict__ out_dp) {
     extern __shared__ __align__(128) uint8_t ld_smem[];
-    const uint32_t tile_w = L.tile_words();
-    const uint32_t stage_bytes = 2u * tile_w * 4u;
-    uint64_t *bars = reinterpret_cast<uint64_t *>(ld_smem + (size_t)kPwStages * stage_bytes);
-    const uint32_t bar_full = fm_smem_u32(bars), bar_empty = bar_full + 8u * kPwStages;
+    const PwRing<kLdConsumerWarps> ring(ld_smem, L);
     const uint32_t bi = rb0 + blockIdx.x / tpr, bj = bi + blockIdx.x % tpr;
     const bool diag = bi == bj;
     const uint32_t chunks = bj < L.n_blk ? n_chunks : 0u;
-    if (threadIdx.x == 0) {
-        for (uint32_t s = 0; s < kPwStages; ++s) {
-            fm_mbar_init(bars + s, 1);
-            fm_mbar_init(bars + kPwStages + s, kLdConsumerWarps);
-        }
-        fm_fence_mbar_init();
-    }
-    __syncthreads();
+    ring.init();
     const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-
     if (warp == kLdConsumerWarps) {
-        // ------------------------------------------------------------------ producer
-        if (lane == 0) {
-            const uint32_t bytes = tile_w * 4u;
-            for (uint32_t c = 0; c < chunks; ++c) {
-                const uint32_t st = c % kPwStages;
-                if (c >= kPwStages) fm_mbar_wait(bar_empty + 8u * st, ((c / kPwStages) - 1u) & 1u);
-                uint8_t *dst = ld_smem + (size_t)st * stage_bytes;
-                fm_mbar_expect_tx(bars + st, diag ? bytes : 2u * bytes);
-                fm_bulk_g2s(dst, planes + ((size_t)c * L.n_blk + bi) * tile_w, bytes, bars + st);
-                if (!diag) fm_bulk_g2s(dst + bytes, planes + ((size_t)c * L.n_blk + bj) * tile_w, bytes, bars + st);
-            }
-        }
+        if (lane == 0) ring.produce(planes, L, chunks, bi, bj);
         return;
     }
 
@@ -140,10 +108,10 @@ fm_k_ld_band(const uint32_t *__restrict__ planes, PwLayout L, uint32_t n_chunks,
 #pragma unroll
         for (int y = 0; y < 4; ++y) acc_ab[x][y] = acc_c[x][y] = acc_a[x][y] = acc_b[x][y] = 0;
     for (uint32_t c = 0; c < chunks; ++c) {
-        const uint32_t st = c % kPwStages;
-        fm_mbar_wait(bar_full + 8u * st, (c / kPwStages) & 1u);
-        const uint32_t si = fm_smem_u32(ld_smem + (size_t)st * stage_bytes) + ti * 16u;
-        const uint32_t sj = fm_smem_u32(ld_smem + (size_t)st * stage_bytes + (diag ? 0u : tile_w * 4u)) + tj * 4u;
+        uint32_t si, sj;
+        ring.acquire(c, diag, si, sj);
+        si += ti * 16u;
+        sj += tj * 4u;
 #pragma unroll 2
         for (uint32_t k = 0; k < kPwKT; ++k) {
             const uint32_t off_a = k * kPwBlk * 4u, off_c = (kPwKT + k) * kPwBlk * 4u;
@@ -151,13 +119,13 @@ fm_k_ld_band(const uint32_t *__restrict__ planes, PwLayout L, uint32_t n_chunks,
             const uint32_t ai[4] = {ua.x, ua.y, ua.z, ua.w};
             uint32_t aj[4];
 #pragma unroll
-            for (int y = 0; y < 4; ++y) aj[y] = fm_ld_lds32(sj + off_a + 64u * y);
+            for (int y = 0; y < 4; ++y) aj[y] = fm_lds32(sj + off_a + 64u * y);
             if (HC) {
                 const uint4 uc = fm_lds128(si + off_c);
                 const uint32_t ci[4] = {uc.x, uc.y, uc.z, uc.w};
                 uint32_t cj[4];
 #pragma unroll
-                for (int y = 0; y < 4; ++y) cj[y] = fm_ld_lds32(sj + off_c + 64u * y);
+                for (int y = 0; y < 4; ++y) cj[y] = fm_lds32(sj + off_c + 64u * y);
 #pragma unroll
                 for (int x = 0; x < 4; ++x)
 #pragma unroll
@@ -174,9 +142,7 @@ fm_k_ld_band(const uint32_t *__restrict__ planes, PwLayout L, uint32_t n_chunks,
                     for (int y = 0; y < 4; ++y) acc_ab[x][y] += __popc(ai[x] & aj[y]);
             }
         }
-        // every lane's shared-memory reads of this stage precede the release
-        __syncwarp();
-        if (lane == 0) fm_mbar_arrive(bar_empty + 8u * st);
+        ring.release(c, lane);
     }
 
     // ---------------------------------------------------------------------- epilogue

@@ -21,7 +21,6 @@
 // nothing to either count.
 #pragma once
 #include "fm_device.cuh"
-#include "fm_wc.cuh"  // fm_mbar_wait / fm_mbar_arrive on shared-memory addresses
 
 namespace fm {
 
@@ -38,6 +37,69 @@ struct PwLayout {
         return ((((size_t)c * n_blk + b) * planes + p) * kPwKT + k) * kPwBlk + sl;
     }
     __host__ __device__ __forceinline__ uint32_t tile_words() const { return planes * kPwKT * kPwBlk; }
+    // dynamic shared memory of a PwRing: kPwStages stages of two tiles, then the full and empty barriers
+    __host__ __device__ __forceinline__ size_t ring_bytes() const {
+        return (size_t)kPwStages * 2 * tile_words() * 4 + 2 * kPwStages * 8;
+    }
+};
+
+// ---------------------------------------------------------------------------------------------- tile ring
+// The bulk-copy ring of the pair kernels (fm_k_pairwise_counts, fm_k_ld_band).  One CTA owns the tile (bi, bj);
+// lane 0 of the producer warp streams K-chunk c of both blocks (one block on diagonal tiles) into stage c % kPwStages
+// with 1-D bulk copies that complete on the stage's `full` mbarrier, and each of the CW consumer warps releases the
+// stage through its `empty` mbarrier once it has read it.
+template <uint32_t CW>
+struct PwRing {
+    uint8_t *smem;             // PwLayout::ring_bytes() of dynamic shared memory
+    uint32_t tile_w, stage_bytes;
+    uint64_t *bars;            // full[kPwStages], empty[kPwStages]
+    uint32_t bar_full, bar_empty;
+
+    __device__ __forceinline__ PwRing(uint8_t *s, const PwLayout &L)
+        : smem(s), tile_w(L.tile_words()), stage_bytes(2u * L.tile_words() * 4u),
+          bars(reinterpret_cast<uint64_t *>(s + (size_t)kPwStages * stage_bytes)), bar_full(fm_smem_u32(bars)),
+          bar_empty(bar_full + 8u * kPwStages) {}
+
+    // every thread of the CTA, before any other use: thread 0 initialises the barriers
+    __device__ __forceinline__ void init() const {
+        if (threadIdx.x == 0) {
+            for (uint32_t st = 0; st < kPwStages; ++st) {
+                fm_mbar_init(bars + st, 1);
+                fm_mbar_init(bars + kPwStages + st, CW);
+            }
+            fm_fence_mbar_init();
+        }
+        __syncthreads();
+    }
+
+    // the producer warp's lane 0: chunks 0 .. chunks - 1 of the blocks bi and bj of `planes`
+    __device__ __forceinline__ void produce(const uint32_t *planes, const PwLayout &L, uint32_t chunks, uint32_t bi,
+                                            uint32_t bj) const {
+        const bool diag = bi == bj;
+        const uint32_t bytes = tile_w * 4u;
+        for (uint32_t c = 0; c < chunks; ++c) {
+            const uint32_t st = c % kPwStages;
+            if (c >= kPwStages) fm_mbar_wait(bar_empty + 8u * st, ((c / kPwStages) - 1u) & 1u);
+            uint8_t *dst = smem + (size_t)st * stage_bytes;
+            fm_mbar_expect_tx(bars + st, diag ? bytes : 2u * bytes);
+            fm_bulk_g2s(dst, planes + ((size_t)c * L.n_blk + bi) * tile_w, bytes, bars + st);
+            if (!diag) fm_bulk_g2s(dst + bytes, planes + ((size_t)c * L.n_blk + bj) * tile_w, bytes, bars + st);
+        }
+    }
+
+    // a consumer: waits for chunk c; si / sj are the shared-memory addresses of its bi and bj tiles
+    __device__ __forceinline__ void acquire(uint32_t c, bool diag, uint32_t &si, uint32_t &sj) const {
+        const uint32_t st = c % kPwStages;
+        fm_mbar_wait(bar_full + 8u * st, (c / kPwStages) & 1u);
+        si = fm_smem_u32(smem + (size_t)st * stage_bytes);
+        sj = fm_smem_u32(smem + (size_t)st * stage_bytes + (diag ? 0u : tile_w * 4u));
+    }
+
+    // a consumer warp, after every lane's last read of chunk c
+    __device__ __forceinline__ void release(uint32_t c, uint32_t lane) const {
+        __syncwarp();
+        if (lane == 0) fm_mbar_arrive(bar_empty + 8u * (c % kPwStages));
+    }
 };
 
 // ---------------------------------------------------------------------------------------------- transposes
@@ -147,21 +209,16 @@ fm_k_sample_planes_packed(const uint32_t *__restrict__ abits, const uint32_t *__
 }
 
 // ---------------------------------------------------------------------------------------------- pair counts
-// Upper-triangle tiled bit-GEMM.  One CTA per 64 x 64 tile (bi <= bj) of sample pairs; warp kPwConsumerWarps is the
-// producer: its lane 0 streams the K-chunks of both sample blocks (one block on diagonal tiles) into a kPwStages ring
-// with 1-D bulk copies that complete on the stage's `full` mbarrier; the consumer warps release a stage through its
-// `empty` mbarrier.  Consumer thread (ti, tj) owns samples i = 4 ti + {0..3} and j = 4 tj + {0..3}, 32 + 4 tj +
-// {0..3} of the tile and keeps their 32 counts in registers.  Per site word and pair the cost is one LOP3 per
-// identity plane, and on top 2 LOP3 + 2 POPC with a comparability plane (1 POPC without).
+// Upper-triangle tiled bit-GEMM.  One CTA per 64 x 64 tile (bi <= bj) of sample pairs, fed by a PwRing whose
+// producer is warp kPwConsumerWarps.  Consumer thread (ti, tj) owns samples i = 4 ti + {0..3} and j = 4 tj + {0..3},
+// 32 + 4 tj + {0..3} of the tile and keeps their 32 counts in registers.  Per site word and pair the cost is one LOP3
+// per identity plane, and on top 2 LOP3 + 2 POPC with a comparability plane (1 POPC without).
 template <bool HC>
 __global__ void __launch_bounds__((kPwConsumerWarps + 1) * 32)
 fm_k_pairwise_counts(const uint32_t *__restrict__ planes, PwLayout L, uint32_t n_chunks, uint32_t n_samples,
                      uint32_t n_sites, uint32_t *__restrict__ diff_out, uint32_t *__restrict__ comp_out) {
     extern __shared__ __align__(128) uint8_t pw_smem[];
-    const uint32_t tile_w = L.tile_words();
-    const uint32_t stage_bytes = 2u * tile_w * 4u;
-    uint64_t *bars = reinterpret_cast<uint64_t *>(pw_smem + (size_t)kPwStages * stage_bytes);
-    const uint32_t bar_full = fm_smem_u32(bars), bar_empty = bar_full + 8u * kPwStages;
+    const PwRing<kPwConsumerWarps> ring(pw_smem, L);
     // blockIdx.x -> (bi, bj), row-major over the upper triangle of the block grid
     uint32_t bi = 0, rem = blockIdx.x;
     while (rem >= L.n_blk - bi) {
@@ -170,29 +227,10 @@ fm_k_pairwise_counts(const uint32_t *__restrict__ planes, PwLayout L, uint32_t n
     }
     const uint32_t bj = bi + rem;
     const bool diag = bi == bj;
-    if (threadIdx.x == 0) {
-        for (uint32_t s = 0; s < kPwStages; ++s) {
-            fm_mbar_init(bars + s, 1);
-            fm_mbar_init(bars + kPwStages + s, kPwConsumerWarps);
-        }
-        fm_fence_mbar_init();
-    }
-    __syncthreads();
+    ring.init();
     const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-
     if (warp == kPwConsumerWarps) {
-        // ------------------------------------------------------------------ producer
-        if (lane == 0) {
-            const uint32_t bytes = tile_w * 4u;
-            for (uint32_t c = 0; c < n_chunks; ++c) {
-                const uint32_t st = c % kPwStages;
-                if (c >= kPwStages) fm_mbar_wait(bar_empty + 8u * st, ((c / kPwStages) - 1u) & 1u);
-                uint8_t *dst = pw_smem + (size_t)st * stage_bytes;
-                fm_mbar_expect_tx(bars + st, diag ? bytes : 2u * bytes);
-                fm_bulk_g2s(dst, planes + ((size_t)c * L.n_blk + bi) * tile_w, bytes, bars + st);
-                if (!diag) fm_bulk_g2s(dst + bytes, planes + ((size_t)c * L.n_blk + bj) * tile_w, bytes, bars + st);
-            }
-        }
+        if (lane == 0) ring.produce(planes, L, n_chunks, bi, bj);
         return;
     }
 
@@ -205,10 +243,10 @@ fm_k_pairwise_counts(const uint32_t *__restrict__ planes, PwLayout L, uint32_t n
 #pragma unroll
         for (int b = 0; b < 8; ++b) acc_d[a][b] = acc_c[a][b] = 0;
     for (uint32_t c = 0; c < n_chunks; ++c) {
-        const uint32_t st = c % kPwStages;
-        fm_mbar_wait(bar_full + 8u * st, (c / kPwStages) & 1u);
-        const uint32_t si = fm_smem_u32(pw_smem + (size_t)st * stage_bytes) + ti * 16u;
-        const uint32_t sj = fm_smem_u32(pw_smem + (size_t)st * stage_bytes + (diag ? 0u : tile_w * 4u)) + tj * 16u;
+        uint32_t si, sj;
+        ring.acquire(c, diag, si, sj);
+        si += ti * 16u;
+        sj += tj * 16u;
 #pragma unroll 1
         for (uint32_t k = 0; k < kPwKT; ++k) {
             uint32_t x[4][8];
@@ -245,8 +283,7 @@ fm_k_pairwise_counts(const uint32_t *__restrict__ planes, PwLayout L, uint32_t n
                     for (int b = 0; b < 8; ++b) acc_d[a][b] += __popc(x[a][b]);
             }
         }
-        __syncwarp();
-        if (lane == 0) fm_mbar_arrive(bar_empty + 8u * st);
+        ring.release(c, lane);
     }
     // condensed (pdist) order: pair (i, j), i < j, sits at i (2 n - i - 1) / 2 + j - i - 1
 #pragma unroll

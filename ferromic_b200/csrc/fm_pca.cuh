@@ -1,8 +1,9 @@
 // fm_pca.cuh -- haplotype PCA by randomized subspace iteration (DESIGN.md §0 row f8, §3 and §4 "Haplotype PCA").
 //
 // Z[i, v] = s_v (x_iv - p_v) for a called cell and 0 for a missing one, over the n selected haplotypes i and the M
-// kept sites v (filters and standardization in include/ferromic_gpu.h).  The kernels here produce the site counts,
-// the haplotype-major bit planes of the kept sites and the two FP64 products every iteration needs:
+// kept sites v (filters and standardization in include/ferromic_gpu.h; site counts and filter in fm_haplotypes.cuh).
+// The kernels here produce the per-site scales, the haplotype-major bit planes of the kept sites and the two FP64
+// products every iteration needs:
 //   W = Z^T Q  (M x l, sites <- haplotypes)     and     Y = Z R  (n x l, haplotypes <- sites).
 // A cell's value is rebuilt from two bits: alt (called, raw allele 1) and called, with the per-site pair
 // u1_v = s_v (1 - p_v), u0_v = s_v (0 - p_v):  z = alt ? u1 : (called ? u0 : 0).  These are the products
@@ -11,8 +12,9 @@
 // z = alt ? u1 : u0.  Every sum runs in a fixed order (no FP64 atomics), so equal inputs give equal bits.
 #pragma once
 #include "fm_device.cuh"
-#include "fm_kernels.cuh"  // fm_mix
-#include "fm_pairwise.cuh" // PwLayout, kPwBlk, kPwKT
+#include "fm_haplotypes.cuh"  // HapCells
+#include "fm_kernels.cuh"     // fm_mix
+#include "fm_pairwise.cuh"    // PwLayout, kPwBlk, kPwKT
 
 namespace fm {
 
@@ -23,69 +25,11 @@ constexpr uint32_t kPcaHapBlocks = 4;            // haplotype blocks of 64 per C
 constexpr uint32_t kPcaMaxRank = 64;             // l <= 64
 constexpr uint32_t kPcaWordPitch = kPwBlk + 1;   // padded shared-memory pitch of a staged (plane, word) row
 
-// One cell of a resident matrix, in any of its forms: u8 rows (bitmap, in-band or no missingness) or packed rows.
-// `alt` is the RAW allele value 1 (never a rank of the LUT), `other` a called value other than 0 and 1.
-struct PcaCells {
-    const uint8_t *data;
-    const uint64_t *missing;
-    uint32_t miss_mode;  // 0 none, 1 bitmap, 2 in band (cells >= 0x80)
-    uint64_t stride;
-    const uint32_t *abits, *cbits;  // packed rows (abits != nullptr); cbits may be null
-    uint32_t rw;
-    __device__ __forceinline__ void read(uint32_t v, uint32_t col, bool &called, bool &alt, bool &other) const {
-        if (abits) {
-            const size_t w = (size_t)v * rw + (col >> 5);
-            alt = (__ldg(abits + w) >> (col & 31)) & 1u;
-            called = cbits ? ((__ldg(cbits + w) >> (col & 31)) & 1u) : true;
-            other = false;
-            return;
-        }
-        const uint64_t e = (uint64_t)v * stride + col;
-        const uint8_t x = __ldg(data + e);
-        called = miss_mode == 1 ? ((__ldg(missing + (e >> 6)) >> (e & 63)) & 1ull) == 0 : (miss_mode == 2 ? x < 0x80 : true);
-        alt = called && x == 1;
-        other = called && x > 1;
-    }
-};
-
-// Site statistics: one warp per site of [v_lo, v_lo + n_sites); counts over the n selected cells and the keep flag.
-__global__ void __launch_bounds__(256)
-fm_k_pca_site_stats(PcaCells cells, const uint32_t *__restrict__ off, uint32_t n, uint32_t v_lo, uint32_t n_sites,
-                    double min_maf, double max_missing, uint32_t *__restrict__ alt_out,
-                    uint32_t *__restrict__ called_out, uint8_t *__restrict__ keep_out) {
-    const uint32_t lane = threadIdx.x & 31;
-    const uint32_t r = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (r >= n_sites) return;
-    const uint32_t v = v_lo + r;
-    uint32_t called = 0, alt = 0, other = 0;
-    for (uint32_t i = lane; i < n; i += 32) {
-        bool c, a, o;
-        cells.read(v, __ldg(off + i), c, a, o);
-        called += c;
-        alt += a;
-        other += o;
-    }
-#pragma unroll
-    for (int d = 16; d; d >>= 1) {
-        called += __shfl_xor_sync(0xffffffffu, called, d);
-        alt += __shfl_xor_sync(0xffffffffu, alt, d);
-        other += __shfl_xor_sync(0xffffffffu, other, d);
-    }
-    if (lane) return;
-    const uint32_t minor = min(alt, called - alt);
-    const bool keep = other == 0 && alt > 0 && alt < called && (double)(n - called) <= max_missing * (double)n &&
-                      (double)minor >= min_maf * (double)called;
-    alt_out[r] = alt;
-    called_out[r] = called;
-    keep_out[r] = keep;
-}
-
 // Per kept site j (matrix row kept[j]): u[2j] = s (1 - p), u[2j + 1] = s (0 - p) with p = alt / called and
-// s = 1 / sqrt(p (1 - p)); T += called (integer); *incomplete |= called < n.
+// s = 1 / sqrt(p (1 - p)); T += called (integer).
 __global__ void __launch_bounds__(256)
 fm_k_pca_scales(const uint32_t *__restrict__ kept, uint32_t M, uint32_t v_lo, const uint32_t *__restrict__ alt,
-                const uint32_t *__restrict__ called, uint32_t n, double *__restrict__ u,
-                unsigned long long *__restrict__ total, uint32_t *__restrict__ incomplete) {
+                const uint32_t *__restrict__ called, double *__restrict__ u, unsigned long long *__restrict__ total) {
     const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= M) return;
     const uint32_t r = kept[j] - v_lo;
@@ -95,13 +39,12 @@ fm_k_pca_scales(const uint32_t *__restrict__ kept, uint32_t M, uint32_t v_lo, co
     u[2 * (size_t)j] = s * (1.0 - p);
     u[2 * (size_t)j + 1] = s * (0.0 - p);
     atomicAdd(total, (unsigned long long)c);
-    if (c < n) atomicOr(incomplete, 1u);
 }
 
 // Kept sites x selected haplotypes -> K-tiled, haplotype-major planes of PwLayout (plane 0 alt, plane 1 called when
 // present).  One warp per (kept-site word, 32 haplotypes), lane = haplotype; padded words and haplotypes stay zero.
 __global__ void __launch_bounds__(256)
-fm_k_pca_planes(PcaCells cells, const uint32_t *__restrict__ off, uint32_t n, const uint32_t *__restrict__ kept,
+fm_k_pca_planes(HapCells cells, const uint32_t *__restrict__ off, uint32_t n, const uint32_t *__restrict__ kept,
                 uint32_t M, uint32_t n_words, PwLayout L, uint32_t *__restrict__ planes) {
     const uint32_t lane = threadIdx.x & 31;
     const uint32_t groups = (n + 31) / 32;

@@ -167,20 +167,6 @@ __host__ __device__ inline size_t fm_wc_stage_bytes(uint32_t G) {
 }
 __host__ __device__ inline size_t fm_wc_pc_smem(uint32_t G) { return kWcPcStages * fm_wc_stage_bytes(G) + 2 * kWcPcStages * 8 + 16; }
 
-__device__ __forceinline__ void fm_mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t ok;
-    do {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-    } while (!ok);
-}
-__device__ __forceinline__ void fm_mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-
 // walks the sub-batches of the CTA's tasks (task = (segment, chunk of pair slots), grid-strided) in order
 struct WcCursor {
     uint32_t task, v, hi;
