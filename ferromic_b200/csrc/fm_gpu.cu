@@ -1003,82 +1003,30 @@ struct DivResult {
     uint64_t seg, unc;
 };
 
-void ensure_counts(fm_group *g);
-
-// Multi-allelic groups (fm_multi.cuh): diversity statistics of [v_lo, v_hi) from the cached
-// per-allele counts.  form: FM_MULTI_DENSE (calculate_pi_dense general) or FM_MULTI_SPARSE.
-DivResult run_multi_diversity(fm_group *g, uint32_t v_lo, uint32_t v_hi, int form, double *d_pi, double *d_theta,
-                              const int64_t *d_mask, uint32_t n_mask, const int64_t *d_filt, uint32_t n_filt) {
-    DivResult r{0.0, 0, 0};
-    const fm::PassGeom G = batch_range(v_lo, v_hi);
-    if (G.n_batches == 0) return r;
-    DevBuf<double> part_pi(G.n_batches);
-    DevBuf<uint32_t> part_u((size_t)G.n_batches * 2);
-    fm::DivEpilogue e{};
-    e.pi_out = d_pi;
-    e.theta_out = d_theta;
-    set_tables(e, g);
-    e.part_pi = part_pi.p;
-    e.part_u = part_u.p;
-    DevBuf<uint32_t> flags;
-    Timer tm;
-    tm.start();
-    if (d_pi && (d_mask || d_filt)) {
-        flags.alloc(G.n_batches);
-        launch_site_flags(g->m, v_lo, v_hi, G.b_lo, G.n_batches, d_mask, n_mask, d_filt, n_filt, flags.p);
-        e.site_flags = flags.p;
-    }
-    const uint32_t blocks = std::min<uint32_t>((G.n_batches + 7) / 8, 8u * sm_count(g->m->device));
-    fm::fm_k_multi_div_from_counts<<<blocks, 256, 0, stream()>>>(g->d_acount, g->d_cnt, 1u << g->n_bits, form, e, v_lo,
-                                                                  v_hi, G.b_lo, G.n_batches);
-    CK(cudaGetLastError());
-    g_launches++;
-    tm.stop();
-    double od[1];
-    uint64_t ou[2];
-    finish_partials(part_pi.p, 1, part_u.p, 2, G, od, ou);
-    t_tim.stats_ms += tm.ms();
-    r.pi_sum = od[0];
-    r.seg = ou[0];
-    r.unc = ou[1];
-    return r;
-}
-
-// per-allele counts of a multi-allelic group (K2m) + the general dense summary scalars
-void ensure_multi_counts_locked(fm_group *g) {
-    set_dev(g->m);
+// K2m: per-allele counts of a multi-allelic group (fm_multi.cuh) into its cache
+void allele_counts(fm_group *g) {
     const size_t V = g->m->V;
     const uint32_t A = 1u << g->n_bits;
     if (!g->d_acount) {
         g->d_acount = static_cast<uint32_t *>(dev_alloc(std::max<size_t>(V, 1) * A * sizeof(uint32_t)));
         g->d_cnt = static_cast<uint32_t *>(dev_alloc(std::max<size_t>(V, 1) * sizeof(uint32_t)));
     }
-    if (V) {
-        uint32_t lg = 0;
-        while ((1u << lg) < std::min(g->wq, 32u)) ++lg;
-        const uint32_t sps = 32u >> lg;
-        const uint64_t warps_needed = ((uint64_t)V + sps - 1) / sps;
-        const uint32_t blocks = (uint32_t)std::min<uint64_t>((warps_needed + 7) / 8, 16ull * sm_count(g->m->device));
-        const size_t ps = std::max<size_t>(V, 1) * g->wq;
-        Timer tm;
-        tm.start();
-        switch (g->n_bits) {
-            case 2: fm::fm_k_allele_counts<2><<<blocks, 256, 0, stream()>>>(g->d_allele, ps, g->d_called, g->wq, g->n, lg, 0, (uint32_t)V, g->d_acount, g->d_cnt); break;
-            case 3: fm::fm_k_allele_counts<3><<<blocks, 256, 0, stream()>>>(g->d_allele, ps, g->d_called, g->wq, g->n, lg, 0, (uint32_t)V, g->d_acount, g->d_cnt); break;
-            default: fm::fm_k_allele_counts<4><<<blocks, 256, 0, stream()>>>(g->d_allele, ps, g->d_called, g->wq, g->n, lg, 0, (uint32_t)V, g->d_acount, g->d_cnt); break;
-        }
-        CK(cudaGetLastError());
-        g_launches++;
-        t_tim.stats_launches++;
-        t_tim.stats_bytes = (uint64_t)V * g->wq * 16u * (g->n_bits + (g->d_called ? 1u : 0u));
-        tm.stop();
-        t_tim.stats_ms += tm.ms();
+    if (!V) return;
+    uint32_t lg = 0;
+    while ((1u << lg) < std::min(g->wq, 32u)) ++lg;
+    const uint32_t sps = 32u >> lg;
+    const uint64_t warps_needed = ((uint64_t)V + sps - 1) / sps;
+    const uint32_t blocks = (uint32_t)std::min<uint64_t>((warps_needed + 7) / 8, 16ull * sm_count(g->m->device));
+    const size_t ps = std::max<size_t>(V, 1) * g->wq;
+    switch (g->n_bits) {
+        case 2: fm::fm_k_allele_counts<2><<<blocks, 256, 0, stream()>>>(g->d_allele, ps, g->d_called, g->wq, g->n, lg, 0, (uint32_t)V, g->d_acount, g->d_cnt); break;
+        case 3: fm::fm_k_allele_counts<3><<<blocks, 256, 0, stream()>>>(g->d_allele, ps, g->d_called, g->wq, g->n, lg, 0, (uint32_t)V, g->d_acount, g->d_cnt); break;
+        default: fm::fm_k_allele_counts<4><<<blocks, 256, 0, stream()>>>(g->d_allele, ps, g->d_called, g->wq, g->n, lg, 0, (uint32_t)V, g->d_acount, g->d_cnt); break;
     }
-    g->have_counts = true;  // run_multi_diversity reads the cached counts
-    DivResult r = run_multi_diversity(g, 0, (uint32_t)V, FM_MULTI_DENSE, nullptr, nullptr, nullptr, 0, nullptr, 0);
-    g->seg = r.seg;
-    g->unc = r.unc;
-    g->pi_sum = r.pi_sum;
+    CK(cudaGetLastError());
+    g_launches++;
+    t_tim.stats_launches++;
+    t_tim.stats_bytes = (uint64_t)V * g->wq * 16u * (g->n_bits + (g->d_called ? 1u : 0u));
 }
 
 // segment of the row pass: group g over [v_lo, v_hi) into the diversity epilogue e
@@ -1092,149 +1040,192 @@ fm::RowSeg div_seg(const fm_group *g, const fm::DivEpilogue &e, uint32_t v_lo, u
     return s;
 }
 
-// Run the diversity statistics for sites [v_lo, v_hi): fused plane pass when counts are not
-// cached (optionally caching them when the range is the whole matrix), light kernel otherwise.
-DivResult run_diversity(fm_group *g, uint32_t v_lo, uint32_t v_hi, int pi_form, double *d_pi,
-                        double *d_theta, const int64_t *d_mask, uint32_t n_mask, const int64_t *d_filt,
-                        uint32_t n_filt, bool store_counts) {
-    if (g->n_bits > 1) {  // multi-allelic: always from the cached per-allele counts
-        if (!g->have_counts) ensure_multi_counts_locked(g);
-        return run_multi_diversity(g, v_lo, v_hi, pi_form == FM_PIFORM_COMPONENTS ? FM_MULTI_SPARSE : FM_MULTI_DENSE,
-                                   d_pi, d_theta, d_mask, n_mask, d_filt, n_filt);
+// One unit of a diversity pass: group g over the sites [v_lo, v_hi), optionally writing per-site tracks.
+struct DivUnit {
+    fm_group *g;
+    uint32_t v_lo, v_hi;
+    double *pi = nullptr, *theta = nullptr;  // [v_hi - v_lo] each, or nullptr
+    DivResult r{0.0, 0, 0};                  // totals (fold)
+};
+
+// The diversity statistics of a list of units, planned as one pass.  Units may come from different matrices of one
+// device and cover different site ranges.  Routing:
+//   multi-allelic                      -> fm_k_multi_div_from_counts (per-allele counts first when not cached)
+//   biallelic with cached counts       -> fm_k_div_from_counts
+//   otherwise, rows fit the row pass   -> ONE fm_k_plane_pass_seq launch for all of them
+//   otherwise (wider rows)             -> one column-chunked launch each
+// Every unit's per-batch partials go to one slab, folded by fold() with one kernel and one copy.  The caller holds
+// the groups' locks.
+struct DivPass {
+    std::vector<DivUnit> units;
+    int pi_form = FM_PIFORM_COUNTS;
+    // mask intervals / sorted filtered positions that drop sites from the tracks; the units then share one range
+    const int64_t *d_mask = nullptr, *d_filt = nullptr;
+    uint32_t n_mask = 0, n_filt = 0;
+    bool store_counts = false;  // units over [0, V): cache alt / called; fold() caches the summary scalars
+    const fm::HudsonEpilogue *hudson = nullptr;  // two units: ride the row pass as one pair unit with this epilogue
+    bool hudson_done = false;  // set by launch(): the Hudson partials were written (else the caller uses the counts)
+
+    void launch(Timer *tm = nullptr);  // tm: times the pass kernels
+    void fold(Timer &tm);              // units[i].r, one synchronise; tm: the launch() timer
+    void run() {                       // the pass and its totals
+        Timer tm;
+        launch(&tm);
+        fold(tm);
     }
-    const fm::PassGeom G = batch_range(v_lo, v_hi);
-    DivResult r{0.0, 0, 0};
-    if (G.n_batches == 0) return r;
-    DevBuf<double> part_pi(G.n_batches);
-    DevBuf<uint32_t> part_u((size_t)G.n_batches * 2);
-    fm::DivEpilogue e{};
-    e.pi_out = d_pi;
-    e.theta_out = d_theta;
-    set_tables(e, g);
+
+  private:
+    std::vector<size_t> off;  // first batch of each unit in the partial slab
+    DevBuf<double> part_pi;
+    DevBuf<uint32_t> part_u;
     DevBuf<uint32_t> flags;
-    Timer tm;
-    tm.start();
-    if (d_pi && (d_mask || d_filt)) {  // K5a: mask / filtered-position bits, one word per batch
-        flags.alloc(G.n_batches);
-        launch_site_flags(g->m, v_lo, v_hi, G.b_lo, G.n_batches, d_mask, n_mask, d_filt, n_filt, flags.p);
-        e.site_flags = flags.p;
+};
+
+void DivPass::launch(Timer *tm) {
+    if (units.empty()) return;
+    const int device = units[0].g->m->device;
+    off.assign(units.size(), 0);
+    size_t total = 0;
+    for (size_t i = 0; i < units.size(); ++i) {
+        off[i] = total;
+        total += batch_range(units[i].v_lo, units[i].v_hi).n_batches;
     }
-    e.pi_form = pi_form;
-    e.part_pi = part_pi.p;
-    e.part_u = part_u.p;
-    if (g->have_counts) {
-        const uint32_t blocks = std::min<uint32_t>((G.n_batches + 7) / 8, 8u * sm_count(g->m->device));
-        fm::fm_k_div_from_counts<<<blocks, 256, 0, stream()>>>(g->d_alt, g->d_cnt, e, v_lo, v_hi,
-                                                                G.b_lo, G.n_batches);
+    if (total >= (1ull << 32)) fail(FM_ERR_UNSUPPORTED, "too many sites for one batched summary call");
+    part_pi.alloc(total);
+    part_u.alloc(total * 2);
+    if (tm) tm->start();
+    const fm::PassGeom F = batch_range(units[0].v_lo, units[0].v_hi);
+    if (units[0].pi && (d_mask || d_filt) && F.n_batches) {  // K5a: mask / filtered-position bits, one word per batch
+        for (const DivUnit &u : units)
+            if (u.v_lo != F.v_lo || u.v_hi != F.v_hi) fail(FM_ERR_INVALID_ARG, "internal: site flags need one range");
+        flags.alloc(F.n_batches);
+        launch_site_flags(units[0].g->m, F.v_lo, F.v_hi, F.b_lo, F.n_batches, d_mask, n_mask, d_filt, n_filt, flags.p);
+    }
+    std::vector<fm::RowSeg> segs;
+    std::vector<fm::ChunkParams> wide;
+    for (size_t i = 0; i < units.size(); ++i) {
+        const DivUnit &u = units[i];
+        fm_group *g = u.g;
+        const bool multi = g->n_bits > 1;
+        if (multi && !g->have_counts) allele_counts(g);
+        if (!multi && !g->have_counts && store_counts) alloc_counts(g);
+        const fm::PassGeom G = batch_range(u.v_lo, u.v_hi);
+        if (!G.n_batches) continue;
+        fm::DivEpilogue e{};
+        e.pi_out = u.pi;
+        e.theta_out = u.theta;
+        set_tables(e, g);
+        e.site_flags = u.pi ? flags.p : nullptr;
+        e.pi_form = pi_form;
+        e.part_pi = part_pi.p + off[i];
+        e.part_u = part_u.p + 2 * off[i];
+        const uint32_t blocks = std::min<uint32_t>((G.n_batches + 7) / 8, 8u * sm_count(device));
+        if (multi) {
+            const int form = pi_form == FM_PIFORM_COMPONENTS ? FM_MULTI_SPARSE : FM_MULTI_DENSE;
+            fm::fm_k_multi_div_from_counts<<<blocks, 256, 0, stream()>>>(g->d_acount, g->d_cnt, 1u << g->n_bits, form, e,
+                                                                          u.v_lo, u.v_hi, G.b_lo, G.n_batches);
+        } else if (g->have_counts) {
+            fm::fm_k_div_from_counts<<<blocks, 256, 0, stream()>>>(g->d_alt, g->d_cnt, e, u.v_lo, u.v_hi, G.b_lo,
+                                                                    G.n_batches);
+        } else {
+            if (g->count_only) fail(FM_ERR_INVALID_ARG, "internal: a count-only group has no bitplanes to stream");
+            if (store_counts) {  // cache the DensePopulationSummary arrays while the planes stream by
+                e.alt_out = g->d_alt;
+                e.called_out = called_cache(g);
+            }
+            if (row_lanes_log2(g->wq) < 5)
+                segs.push_back(div_seg(g, e, u.v_lo, u.v_hi));
+            else
+                wide.push_back(fm::ChunkParams{planes_of(g), make_geom(g, u.v_lo, u.v_hi), e});
+            continue;
+        }
         CK(cudaGetLastError());
         g_launches++;
-    } else {
-        if (store_counts) {
-            e.alt_out = g->d_alt;
-            e.called_out = called_cache(g);
-        }
-        if (g->count_only) fail(FM_ERR_INVALID_ARG, "internal: a count-only group has no bitplanes to stream");
-        std::vector<fm::RowSeg> segs{div_seg(g, e, v_lo, v_hi)};
-        RowPlan plan;
-        if (row_lanes_log2(g->wq) < 5 && plan_rows(segs, nullptr, plan))
-            launch_rows(plan, g->m->device);
-        else
-            launch_chunked(fm::ChunkParams{planes_of(g), make_geom(g, v_lo, v_hi), e}, g->m->device);
     }
-    tm.stop();
-    double od[1];
-    uint64_t ou[2];
+    if (!segs.empty()) {
+        RowPlan plan;
+        if (hudson && segs.size() == 2) {
+            std::vector<fm::HudsonEpilogue> hv{*hudson};
+            hudson_done = plan_rows(segs, &hv, plan);
+        }
+        if (hudson_done || plan_rows(segs, nullptr, plan)) {
+            launch_rows(plan, device);
+        } else {
+            for (const fm::RowSeg &s : segs) {  // the set does not fit one launch: one per unit
+                std::vector<fm::RowSeg> one{s};
+                if (!plan_rows(one, nullptr, plan)) fail(FM_ERR_INVALID_ARG, "internal: a segment does not fit the row pass");
+                launch_rows(plan, device);
+            }
+        }
+    }
+    for (const fm::ChunkParams &P : wide) launch_chunked(P, device);
+    if (tm) tm->stop();
+}
+
+void DivPass::fold(Timer &tm) {
     Timer tr;
     tr.start();
-    finish_partials(part_pi.p, 1, part_u.p, 2, G, od, ou);
-    r.pi_sum = od[0];
-    r.seg = ou[0];
-    r.unc = ou[1];
+    // entry per (unit, super-batch of the GLOBAL batch grid): a unit over a sub-range folds as in finish_partials
+    std::vector<uint4> ents;
+    for (size_t i = 0; i < units.size(); ++i) {
+        const fm::PassGeom G = batch_range(units[i].v_lo, units[i].v_hi);
+        if (!G.n_batches) continue;
+        uint32_t s_lo, n_super;
+        super_range(G, s_lo, n_super);
+        for (uint32_t s = 0; s < n_super; ++s) ents.push_back(make_uint4((uint32_t)off[i], G.b_lo, G.n_batches, s_lo + s));
+    }
+    const size_t ne = ents.size();
+    std::vector<uint64_t> h(ne * 3);  // per entry the pi sum (as a double), then seg and unc of every entry
+    if (ne) {
+        DevBuf<uint4> d_ents(ne);
+        d_ents.upload(ents.data(), ne);
+        DevBuf<uint64_t> d_out(ne * 3);
+        fm::fm_k_reduce_partials_tab<<<(uint32_t)((ne + 3) / 4), 128, 0, stream()>>>(
+            part_pi.p, 1, part_u.p, 2, d_ents.p, (uint32_t)ne, reinterpret_cast<double *>(d_out.p), d_out.p + ne);
+        CK(cudaGetLastError());
+        g_launches++;
+        d_out.download(h.data(), ne * 3);
+    }
+    CK(cudaStreamSynchronize(stream()));
     tr.stop();
     t_tim.stats_ms += tm.ms();
     t_tim.reduce_ms += tr.ms();
-    return r;
+    size_t e = 0;
+    for (DivUnit &u : units) {
+        const fm::PassGeom G = batch_range(u.v_lo, u.v_hi);
+        uint32_t s_lo = 0, n_super = 0;
+        if (G.n_batches) super_range(G, s_lo, n_super);
+        u.r = DivResult{0.0, 0, 0};
+        for (uint32_t s = 0; s < n_super; ++s, ++e) {  // fixed order: independent of grid / GPU count
+            double pi;
+            std::memcpy(&pi, &h[e], sizeof(pi));
+            u.r.pi_sum += pi;
+            u.r.seg += h[ne + 2 * e];
+            u.r.unc += h[ne + 2 * e + 1];
+        }
+        if (store_counts) {
+            u.g->pi_sum = u.r.pi_sum;
+            u.g->seg = u.r.seg;
+            u.g->unc = u.r.unc;
+            u.g->have_counts = true;
+        }
+    }
 }
 
-// Diversity statistics of several groups of one matrix over [v_lo, v_hi).  Groups whose counts are not cached yet
-// and whose rows fit the row pass share ONE launch of it (fm_k_plane_pass_seq); everything else goes group by group
-// through run_diversity.
-bool run_diversity_multi(fm_group *const *gs, size_t n, uint32_t v_lo, uint32_t v_hi, int pi_form,
-                         double *const *d_pi, double *const *d_theta, const int64_t *d_mask, uint32_t n_mask,
-                         const int64_t *d_filt, uint32_t n_filt, DivResult *out, bool store_counts = false,
-                         Timer *ext_tm = nullptr) {
-    auto per_group = [&]() {
-        for (size_t i = 0; i < n; ++i) {
-            DivResult r = run_diversity(gs[i], v_lo, v_hi, pi_form, d_pi ? d_pi[i] : nullptr, d_theta ? d_theta[i] : nullptr,
-                                        d_mask, n_mask, d_filt, n_filt, store_counts);
-            if (out) out[i] = r;
-        }
-        return false;
-    };
-    bool fuse = v_hi > v_lo;
-    for (size_t i = 0; i < n && fuse; ++i)
-        fuse = !gs[i]->have_counts && gs[i]->m == gs[0]->m && gs[i]->n_bits == 1 && !gs[i]->count_only &&
-               row_lanes_log2(gs[i]->wq) < 5;
-    if (!fuse) return per_group();
-    const fm::PassGeom G = batch_range(v_lo, v_hi);
-    const bool tracks = d_pi != nullptr;
-    const bool use_flags = tracks && (d_mask || d_filt);
-    DevBuf<uint32_t> flags;
-    if (use_flags) flags.alloc(G.n_batches);
-    std::vector<DevBuf<double>> part_pi(n);
-    std::vector<DevBuf<uint32_t>> part_u(n);
-    std::vector<fm::RowSeg> segs(n);
-    for (size_t i = 0; i < n; ++i) {
-        part_pi[i].alloc(G.n_batches);
-        part_u[i].alloc((size_t)G.n_batches * 2);
-        fm::DivEpilogue e{};
-        e.pi_out = tracks ? d_pi[i] : nullptr;
-        e.theta_out = tracks ? d_theta[i] : nullptr;
-        set_tables(e, gs[i]);
-        e.site_flags = flags.p;
-        e.pi_form = pi_form;
-        e.part_pi = part_pi[i].p;
-        e.part_u = part_u[i].p;
-        if (store_counts) {  // cache the DensePopulationSummary arrays while the planes stream by
-            e.alt_out = gs[i]->d_alt;
-            e.called_out = called_cache(gs[i]);
-        }
-        segs[i] = div_seg(gs[i], e, v_lo, v_hi);
-    }
-    RowPlan plan;
-    if (!plan_rows(segs, nullptr, plan)) return per_group();
-    Timer own_tm;
-    Timer &tm = ext_tm ? *ext_tm : own_tm;
-    tm.start();
-    if (use_flags) launch_site_flags(gs[0]->m, v_lo, v_hi, G.b_lo, G.n_batches, d_mask, n_mask, d_filt, n_filt, flags.p);
-    launch_rows(plan, gs[0]->m->device);
-    tm.stop();
-    for (size_t i = 0; i < n && out; ++i) {  // out == nullptr: the caller only wants the tracks
-        double od[1];
-        uint64_t ou[2];
-        finish_partials(part_pi[i].p, 1, part_u[i].p, 2, G, od, ou);
-        out[i] = DivResult{od[0], ou[0], ou[1]};
-    }
-    if (out) t_tim.stats_ms += tm.ms();  // out == nullptr: the caller reads `ext_tm` after its own synchronise
-    return true;  // one fused launch, timed by `tm`
+// Summaries (cached counts and scalars) of groups whose counts are not cached yet, in one pass.  The caller holds
+// the groups' locks.
+void summarize_locked(const std::vector<fm_group *> &gs) {
+    if (gs.empty()) return;
+    set_dev(gs[0]->m);
+    DivPass P;
+    P.store_counts = true;
+    for (fm_group *g : gs) P.units.push_back(DivUnit{g, 0, (uint32_t)g->m->V});
+    P.run();
 }
 
 void ensure_counts(fm_group *g) {
     std::lock_guard<std::mutex> lk(g->mu);
-    if (g->have_counts) return;
-    if (g->n_bits > 1) {
-        ensure_multi_counts_locked(g);
-        return;
-    }
-    set_dev(g->m);
-    const size_t V = g->m->V;
-    alloc_counts(g);
-    DivResult r = run_diversity(g, 0, (uint32_t)V, FM_PIFORM_COUNTS, nullptr, nullptr, nullptr, 0,
-                                nullptr, 0, /*store_counts=*/true);
-    g->seg = r.seg;
-    g->unc = r.unc;
-    g->pi_sum = r.pi_sum;
-    g->have_counts = true;
+    if (!g->have_counts) summarize_locked({g});
 }
 
 struct HudsonTotals {
@@ -1296,24 +1287,156 @@ void merge_intervals(const int64_t *iv, size_t n, std::vector<int64_t> &out) {
 
 int dense_variant(const fm_matrix *m) { return m->has_missing ? FM_HV_DENSE_MISSING : FM_HV_DENSE_NOMISSING; }
 
-// 1-based output positions of sites [lo, lo + n) (stats.rs:747, 3004, 4746): small ranges are written by the host,
-// large ones come from the device copy of the positions (one kernel + one D2H instead of a million-element host
-// loop).  pos_out == NULL: the caller already knows the positions.  The copy is ordered on stream().
+// 1-based output positions of sites [lo, lo + n) (stats.rs:747, 3004, 4746): ranges of fewer than kDevicePositions
+// sites are written by the host, larger ones come from the device copy of the positions (one kernel + one D2H instead
+// of a million-element host loop).  pos_out == NULL: the caller already knows the positions.  The copy is ordered on
+// stream().
+constexpr size_t kDevicePositions = 65536;
 __global__ void fm_k_pos_plus1(const int64_t *__restrict__ pos, uint32_t lo, uint32_t n, int64_t *__restrict__ out) {
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) out[i] = pos[lo + i] + 1;
 }
+void launch_pos_plus1(const fm_matrix *m, uint32_t lo, size_t n, int64_t *out, cudaStream_t st) {
+    fm_k_pos_plus1<<<(uint32_t)std::min<size_t>((n + 255) / 256, 2048), 256, 0, st>>>(m->d_pos, lo, (uint32_t)n, out);
+    CK(cudaGetLastError());
+    g_launches++;
+}
 void download_positions_plus1(const fm_matrix *m, uint32_t lo, size_t n, int64_t *pos_out, DevBuf<int64_t> &scratch) {
     if (!pos_out || !n) return;
-    if (n < 65536) {
+    if (n < kDevicePositions) {
         for (size_t i = 0; i < n; ++i) pos_out[i] = m->pos[lo + i] + 1;
         return;
     }
     scratch.alloc(n);
-    fm_k_pos_plus1<<<(uint32_t)std::min<size_t>((n + 255) / 256, 2048), 256, 0, stream()>>>(m->d_pos, lo, (uint32_t)n, scratch.p);
-    CK(cudaGetLastError());
-    g_launches++;
+    launch_pos_plus1(m, lo, n, scratch.p, stream());
     scratch.download(pos_out, n);
 }
+
+// The per-site pi / theta tracks of a set of groups over one region (stats.rs:4693-4750), for
+// fm_per_site_diversity_multi and for the streaming ingest, which computes them chunk by chunk as the rows arrive.
+// prepare() checks the request and places the outputs, run() computes the tracks of the region's sites in a row range,
+// finish() delivers what the passes did not write straight into the caller's memory.
+struct TrackRequest {
+    fm_matrix *m = nullptr;
+    uint32_t lo = 0, hi = 0;            // site range of the region
+    std::vector<fm_group *> act;        // groups with >= 2 listed haplotypes
+    std::vector<size_t> act_idx;        // their row in the caller's arrays
+    std::vector<size_t> nan_rows;       // rows of groups with < 2 listed haplotypes: NaN (stats.rs:4675-4681)
+    size_t capacity = 0;
+    DevBuf<int64_t> d_mask, d_filt;
+    uint32_t n_mask = 0, n_filt = 0;
+    std::vector<double *> ppi, pth;     // device-visible destinations (the caller's page-locked rows or own buffers)
+    std::vector<DevBuf<double>> own_pi, own_th;
+    std::vector<char> direct;
+    int64_t *pos_out = nullptr, *pos_direct = nullptr;
+    double *pi_out = nullptr, *theta_out = nullptr;
+    bool pos_done = false;
+
+    // returns the number of sites of the region (0: nothing to compute)
+    size_t prepare(fm_matrix *mat, fm_group *const *groups, const size_t *raw_n, size_t n_groups, int64_t rs, int64_t re,
+                   const int64_t *mask_iv, size_t n_iv, const int64_t *filtered, size_t n_filtered, int64_t *pos,
+                   double *pi, double *theta, size_t cap) {
+        m = mat;
+        for (size_t i = 0; i < n_groups; ++i)
+            if (!groups[i] || groups[i]->m != m) fail(FM_ERR_INVALID_ARG, "groups must share one matrix");
+        if (region_len(rs, re) <= 0) return 0;  // stats.rs:4656-4666
+        set_dev(m);
+        site_range(m, rs, re, lo, hi);
+        const size_t n = hi - lo;
+        if (n == 0) return 0;
+        if (n > cap) fail(FM_ERR_INVALID_ARG, "output capacity too small");
+        if (!pi || !theta) fail(FM_ERR_INVALID_ARG, "output arrays are NULL");
+        capacity = cap;
+        pos_out = pos;
+        pi_out = pi;
+        theta_out = theta;
+        std::vector<int64_t> merged, fs;
+        if (mask_iv) {
+            merge_intervals(mask_iv, n_iv, merged);
+            d_mask.alloc(std::max<size_t>(merged.size(), 2));
+            d_mask.upload(merged.data(), merged.size());
+            n_mask = (uint32_t)(merged.size() / 2);
+        }
+        if (filtered && n_filtered) {
+            fs.assign(filtered, filtered + n_filtered);
+            std::sort(fs.begin(), fs.end());
+            d_filt.alloc(fs.size());
+            d_filt.upload(fs.data(), fs.size());
+            n_filt = (uint32_t)fs.size();
+        }
+        for (size_t i = 0; i < n_groups; ++i) {
+            if (raw_n[i] >= 2) {
+                act.push_back(groups[i]);
+                act_idx.push_back(i);
+            } else {
+                nan_rows.push_back(i);
+            }
+        }
+        // Page-locked output arrays take the tracks straight from the kernel's epilogue (coalesced 256-byte stores
+        // over PCIe, no HBM round trip and no copy after the pass); pageable ones get device buffers + D2H copies.
+        const size_t na = act.size();
+        ppi.resize(na);
+        pth.resize(na);
+        own_pi = std::vector<DevBuf<double>>(na);
+        own_th = std::vector<DevBuf<double>>(na);
+        direct.assign(na, 0);
+        for (size_t i = 0; i < na; ++i) {
+            double *mp = static_cast<double *>(mapped_host_range(pi_out + act_idx[i] * capacity, n * 8));
+            double *mt = static_cast<double *>(mapped_host_range(theta_out + act_idx[i] * capacity, n * 8));
+            if (mp && mt) {
+                direct[i] = 1;
+                ppi[i] = mp;
+                pth[i] = mt;
+            } else {
+                own_pi[i].alloc(n);
+                own_th[i].alloc(n);
+                ppi[i] = own_pi[i].p;
+                pth[i] = own_th[i].p;
+            }
+        }
+        if (pos_out && n >= kDevicePositions) pos_direct = static_cast<int64_t *>(mapped_host_range(pos_out, n * 8));
+        return n;
+    }
+
+    // Tracks of the region's sites in [r0, r1) on stream(); the positions kernel (once) on pos_stream.  tm: times the
+    // pass.
+    void run(size_t r0, size_t r1, cudaStream_t pos_stream, Timer *tm = nullptr) {
+        const uint32_t a = (uint32_t)std::max<size_t>(r0, lo), b = (uint32_t)std::min<size_t>(r1, hi);
+        if (a >= b) return;
+        if (pos_direct && !pos_done) {
+            launch_pos_plus1(m, lo, hi - lo, pos_direct, pos_stream);
+            pos_done = true;
+        }
+        if (act.empty()) return;
+        DivPass P;
+        P.pi_form = FM_PIFORM_COMPONENTS;
+        P.d_mask = d_mask.p;
+        P.n_mask = n_mask;
+        P.d_filt = d_filt.p;
+        P.n_filt = n_filt;
+        for (size_t i = 0; i < act.size(); ++i) P.units.push_back(DivUnit{act[i], a, b, ppi[i] + (a - lo), pth[i] + (a - lo)});
+        P.launch(tm);
+    }
+
+    void finish() {
+        const size_t n = hi - lo;
+        if (!n) return;
+        Timer tm;
+        tm.start();
+        for (size_t i = 0; i < act.size(); ++i)
+            if (!direct[i]) {
+                own_pi[i].download(pi_out + act_idx[i] * capacity, n);
+                own_th[i].download(theta_out + act_idx[i] * capacity, n);
+            }
+        DevBuf<int64_t> d_p1;
+        if (!pos_done) download_positions_plus1(m, lo, n, pos_out, d_p1);
+        tm.stop();
+        CK(cudaStreamSynchronize(stream()));
+        t_tim.d2h_ms += tm.ms();
+        const double NaN = std::numeric_limits<double>::quiet_NaN();
+        for (size_t row : nan_rows)
+            for (size_t k = 0; k < n; ++k) pi_out[row * capacity + k] = theta_out[row * capacity + k] = NaN;
+    }
+};
 
 }  // namespace
 
@@ -2140,104 +2263,26 @@ fm_status fm_group_summary(fm_group *g, uint32_t *alt_out, uint32_t *called_out,
 }
 
 // build_dense_population_summary for MANY groups -- normally one per region-sized matrix, the shape of the CLI's
-// loop over config entries (process.rs:2169 -> stats.rs:1367-1470) -- in one persistent launch: groups whose counts
-// are not cached yet become the units of one fm_k_plane_pass_seq launch, their partials
-// are folded by one kernel and come back in one copy.  Each group ends up exactly as after fm_group_summary.
+// loop over config entries (process.rs:2169 -> stats.rs:1367-1470) -- in one pass: groups whose counts are not
+// cached yet become its units (the narrow ones of one fm_k_plane_pass_seq launch), their partials are folded by one
+// kernel and come back in one copy.  Each group ends up exactly as after fm_group_summary.
 static void summarize_groups(fm_group *const *groups, size_t n_groups) {
-    {
-        if (n_groups && !groups) fail(FM_ERR_INVALID_ARG, "groups is NULL");
-        require_device();
-        if (!n_groups) return;
-        for (size_t i = 0; i < n_groups; ++i) {
-            if (!groups[i]) fail(FM_ERR_INVALID_ARG, "group is NULL");
-            if (groups[i]->m->device != groups[0]->m->device) fail(FM_ERR_INVALID_ARG, "groups must live on one device");
-        }
-        const int device = groups[0]->m->device;
-        CK(cudaSetDevice(device));
-        std::vector<fm_group *> order(groups, groups + n_groups);
-        std::sort(order.begin(), order.end());
-        order.erase(std::unique(order.begin(), order.end()), order.end());
-        std::vector<std::unique_lock<std::mutex>> locks;
-        for (fm_group *g : order) locks.emplace_back(g->mu);  // address order: no lock inversion
-        // the groups that share a launch: biallelic planes whose counts are not cached yet
-        std::vector<fm_group *> gs;
-        for (fm_group *g : order)
-            if (!g->have_counts && g->n_bits == 1 && !g->count_only && g->m->V > 0) gs.push_back(g);
-        if (!gs.empty()) {
-            std::vector<fm::RowSeg> segs(gs.size());
-            std::vector<size_t> part_off(gs.size());
-            size_t total_b = 0;
-            for (size_t i = 0; i < gs.size(); ++i) {
-                const uint32_t V = (uint32_t)gs[i]->m->V;
-                part_off[i] = total_b;
-                total_b += (V + 31) / 32;
-            }
-            DevBuf<double> ppi(total_b);
-            DevBuf<uint32_t> ppu(total_b * 2);
-            std::vector<uint4> ents;
-            for (size_t i = 0; i < gs.size(); ++i) {
-                fm_group *g = gs[i];
-                const uint32_t V = (uint32_t)g->m->V;
-                alloc_counts(g);
-                fm::DivEpilogue de{};
-                set_tables(de, g);
-                de.pi_form = FM_PIFORM_COUNTS;
-                de.part_pi = ppi.p + part_off[i];
-                de.part_u = ppu.p + 2 * part_off[i];
-                de.alt_out = g->d_alt;
-                de.called_out = called_cache(g);
-                segs[i] = div_seg(g, de, 0, V);
-                const uint32_t nb = (V + 31) / 32;
-                for (uint32_t sb = 0; sb * fm::kSuperBatches < nb; ++sb)
-                    ents.push_back(make_uint4((uint32_t)part_off[i], 0u, nb, sb));
-            }
-            if (total_b >= (1ull << 31)) fail(FM_ERR_UNSUPPORTED, "too many sites for one batched summary call");
-            RowPlan plan;
-            Timer tm;
-            tm.start();
-            if (!plan_rows(segs, nullptr, plan)) {
-                // rows wider than the row pass handles (column-chunked): one pass per group
-                locks.clear();
-                for (fm_group *g : gs) ensure_counts(g);
-                for (fm_group *g : order) locks.emplace_back(g->mu);
-            } else {
-                launch_rows(plan, device);
-                DevBuf<uint4> d_ents(ents.size());
-                d_ents.upload(ents.data(), ents.size());
-                DevBuf<double> sd(ents.size());
-                DevBuf<uint64_t> su(ents.size() * 2);
-                fm::fm_k_reduce_partials_tab<<<(uint32_t)((ents.size() + 3) / 4), 128, 0, stream()>>>(
-                    ppi.p, 1, ppu.p, 2, d_ents.p, (uint32_t)ents.size(), sd.p, su.p);
-                CK(cudaGetLastError());
-                g_launches++;
-                tm.stop();
-                std::vector<double> hd(ents.size());
-                std::vector<uint64_t> hu(ents.size() * 2);
-                sd.download(hd.data(), ents.size());
-                su.download(hu.data(), ents.size() * 2);
-                CK(cudaStreamSynchronize(stream()));
-                t_tim.stats_ms += tm.ms();
-                size_t e = 0;
-                for (size_t i = 0; i < gs.size(); ++i) {
-                    const uint32_t nb = ((uint32_t)gs[i]->m->V + 31) / 32;
-                    double pi = 0.0;
-                    uint64_t sg = 0, un = 0;
-                    for (uint32_t sb = 0; sb * fm::kSuperBatches < nb; ++sb, ++e) {  // fixed order, like finish_partials
-                        pi += hd[e];
-                        sg += hu[2 * e];
-                        un += hu[2 * e + 1];
-                    }
-                    gs[i]->pi_sum = pi;
-                    gs[i]->seg = sg;
-                    gs[i]->unc = un;
-                    gs[i]->have_counts = true;
-                }
-            }
-        }
-        locks.clear();
-        for (size_t i = 0; i < n_groups; ++i)
-            if (!groups[i]->have_counts) ensure_counts(groups[i]);  // multi-allelic / empty matrices / leftovers
+    if (n_groups && !groups) fail(FM_ERR_INVALID_ARG, "groups is NULL");
+    require_device();
+    if (!n_groups) return;
+    for (size_t i = 0; i < n_groups; ++i) {
+        if (!groups[i]) fail(FM_ERR_INVALID_ARG, "group is NULL");
+        if (groups[i]->m->device != groups[0]->m->device) fail(FM_ERR_INVALID_ARG, "groups must live on one device");
     }
+    std::vector<fm_group *> order(groups, groups + n_groups);
+    std::sort(order.begin(), order.end());
+    order.erase(std::unique(order.begin(), order.end()), order.end());
+    std::vector<std::unique_lock<std::mutex>> locks;
+    for (fm_group *g : order) locks.emplace_back(g->mu);  // address order: no lock inversion
+    std::vector<fm_group *> cold;
+    for (fm_group *g : order)
+        if (!g->have_counts) cold.push_back(g);
+    summarize_locked(cold);
 }
 
 fm_status fm_groups_summary_batch(fm_group *const *groups, size_t n_groups, uint64_t *seg_out, double *pi_sum_out,
@@ -2252,17 +2297,6 @@ fm_status fm_groups_summary_batch(fm_group *const *groups, size_t n_groups, uint
             if (unc_out) unc_out[i] = g->unc;
         }
     });
-}
-
-// summaries of the two groups of a pair: one launch when neither is cached yet
-static void ensure_counts_pair(fm_group *g1, fm_group *g2) {
-    if (g1 != g2 && !g1->have_counts && !g2->have_counts && g1->m->device == g2->m->device) {
-        fm_group *gs[2] = {g1, g2};
-        summarize_groups(gs, 2);
-        return;
-    }
-    ensure_counts(g1);
-    ensure_counts(g2);
 }
 
 fm_status fm_group_segregating_sites(fm_group *g, uint64_t *out) {
@@ -2301,11 +2335,12 @@ fm_status fm_group_pi(fm_group *g, int64_t L, int path, size_t raw_n, double *ou
             pi_sum = g->pi_sum;  // dense_pi_from_counts form
             skipped = g->unc;
         } else {
-            const int form = path == FM_PI_DENSE ? FM_PIFORM_NOMISSING : FM_PIFORM_COMPONENTS;
-            DivResult r = run_diversity(g, 0, (uint32_t)g->m->V, form, nullptr, nullptr, nullptr, 0,
-                                        nullptr, 0, false);
-            pi_sum = r.pi_sum;
-            skipped = path == FM_PI_DENSE ? 0 : r.unc;  // stats.rs:4523: (sum_pi, 0usize)
+            DivPass P;
+            P.pi_form = path == FM_PI_DENSE ? FM_PIFORM_NOMISSING : FM_PIFORM_COMPONENTS;
+            P.units.push_back(DivUnit{g, 0, (uint32_t)g->m->V});
+            P.run();
+            pi_sum = P.units[0].r.pi_sum;
+            skipped = path == FM_PI_DENSE ? 0 : P.units[0].r.unc;  // stats.rs:4523: (sum_pi, 0usize)
         }
         const int64_t eff = sat_sub(L, (int64_t)skipped);
         if (eff == 0) { *out = NaN; return; }
@@ -2363,61 +2398,11 @@ fm_status fm_per_site_diversity_multi(fm_group *const *groups, const size_t *raw
         if (!groups || !n_groups || !n_out || !raw_n) fail(FM_ERR_INVALID_ARG, "NULL argument");
         *n_out = 0;
         require_device();
-        fm_matrix *m = groups[0]->m;
-        for (size_t i = 0; i < n_groups; ++i)
-            if (!groups[i] || groups[i]->m != m) fail(FM_ERR_INVALID_ARG, "groups must share one matrix");
-        if (region_len(rs, re) <= 0) return;  // stats.rs:4656-4666
-        set_dev(m);
-        uint32_t lo, hi;
-        site_range(m, rs, re, lo, hi);
-        const size_t n = hi - lo;
+        TrackRequest T;
+        const size_t n = T.prepare(groups[0] ? groups[0]->m : nullptr, groups, raw_n, n_groups, rs, re, mask_iv, n_mask,
+                                   filtered, n_filt, pos_out, pi_out, theta_out, capacity);
         if (n == 0) return;
-        if (n > capacity) fail(FM_ERR_INVALID_ARG, "output capacity too small");
-        if (!pi_out || !theta_out) fail(FM_ERR_INVALID_ARG, "output arrays are NULL");
-        std::vector<int64_t> merged, fs;
-        DevBuf<int64_t> d_mask, d_filt;
-        if (mask_iv) {
-            merge_intervals(mask_iv, n_mask, merged);
-            d_mask.alloc(std::max<size_t>(merged.size(), 2));
-            d_mask.upload(merged.data(), merged.size());
-        }
-        if (filtered && n_filt) {
-            fs.assign(filtered, filtered + n_filt);
-            std::sort(fs.begin(), fs.end());
-            d_filt.alloc(fs.size());
-            d_filt.upload(fs.data(), fs.size());
-        }
-        // groups with fewer than two listed haplotypes yield no sites in the reference
-        // (stats.rs:4675-4681): their rows are NaN here
-        std::vector<fm_group *> act;
-        std::vector<size_t> act_idx;
-        for (size_t i = 0; i < n_groups; ++i)
-            if (raw_n[i] >= 2) {
-                act.push_back(groups[i]);
-                act_idx.push_back(i);
-            }
-        // Page-locked output arrays take the tracks straight from the kernel's epilogue (coalesced 256-byte stores
-        // over PCIe, no HBM round trip and no copy after the pass); pageable ones get device buffers + D2H copies.
-        std::vector<DevBuf<double>> d_pi(act.size()), d_th(act.size());
-        std::vector<double *> ppi(act.size()), pth(act.size());
-        std::vector<char> direct(act.size(), 0);
-        for (size_t i = 0; i < act.size(); ++i) {
-            double *mp = static_cast<double *>(mapped_host_range(pi_out + act_idx[i] * capacity, n * 8));
-            double *mt = static_cast<double *>(mapped_host_range(theta_out + act_idx[i] * capacity, n * 8));
-            if (mp && mt) {
-                direct[i] = 1;
-                ppi[i] = mp;
-                pth[i] = mt;
-            } else {
-                d_pi[i].alloc(n);
-                d_th[i].alloc(n);
-                ppi[i] = d_pi[i].p;
-                pth[i] = d_th[i].p;
-            }
-        }
         // positions + 1 (stats.rs:4746): a small kernel on a side stream underneath the pass
-        DevBuf<int64_t> d_p1;
-        int64_t *pos_direct = (pos_out && n >= 65536) ? static_cast<int64_t *>(mapped_host_range(pos_out, n * 8)) : nullptr;
         cudaStream_t side = nullptr;
         struct SideJoin {  // an early exit must not leave the side kernel writing into the caller's buffer
             cudaStream_t *s;
@@ -2426,51 +2411,32 @@ fm_status fm_per_site_diversity_multi(fm_group *const *groups, const size_t *raw
             }
         } side_join{&side};
         EventPairs evs;
-        if (pos_direct) {
-            side = t_side_streams.get(m->device);
+        if (T.pos_direct) {
+            side = t_side_streams.get(T.m->device);
             cudaEvent_t e0 = evs.next();
             CK(cudaEventRecord(e0, stream()));
             CK(cudaStreamWaitEvent(side, e0, 0));
-            fm_k_pos_plus1<<<(uint32_t)std::min<size_t>((n + 255) / 256, 2048), 256, 0, side>>>(m->d_pos, lo, (uint32_t)n, pos_direct);
-            CK(cudaGetLastError());
-            g_launches++;
         }
         Timer pass_tm;
-        bool fused = false;
         {
             std::vector<std::unique_lock<std::mutex>> locks;
-            std::vector<fm_group *> order(act);
+            std::vector<fm_group *> order(T.act);
             std::sort(order.begin(), order.end());
             order.erase(std::unique(order.begin(), order.end()), order.end());
             for (fm_group *g : order) locks.emplace_back(g->mu);  // address order: no lock inversion
-            if (!act.empty())
-                fused = run_diversity_multi(act.data(), act.size(), lo, hi, FM_PIFORM_COMPONENTS, ppi.data(), pth.data(),
-                                            mask_iv ? d_mask.p : nullptr, (uint32_t)(merged.size() / 2),
-                                            fs.empty() ? nullptr : d_filt.p, (uint32_t)fs.size(), /*out=*/nullptr, false,
-                                            &pass_tm);
+            std::vector<fm_group *> cold;  // multi-allelic tracks come from the cached per-allele counts
+            for (fm_group *g : order)
+                if (g->n_bits > 1 && !g->have_counts) cold.push_back(g);
+            summarize_locked(cold);
+            T.run(T.lo, T.hi, side, &pass_tm);
         }
-        Timer tm;
-        tm.start();
-        for (size_t i = 0; i < act.size(); ++i)
-            if (!direct[i]) {
-                d_pi[i].download(pi_out + act_idx[i] * capacity, n);
-                d_th[i].download(theta_out + act_idx[i] * capacity, n);
-            }
-        if (pos_direct) {
+        if (side) {
             cudaEvent_t e1 = evs.next();
             CK(cudaEventRecord(e1, side));
             CK(cudaStreamWaitEvent(stream(), e1, 0));
-        } else {
-            download_positions_plus1(m, lo, n, pos_out, d_p1);
         }
-        tm.stop();
-        CK(cudaStreamSynchronize(stream()));
-        t_tim.d2h_ms += tm.ms();
-        if (fused) t_tim.stats_ms += pass_tm.ms();
-        const double NaN = std::numeric_limits<double>::quiet_NaN();
-        for (size_t i = 0; i < n_groups; ++i)
-            if (raw_n[i] < 2)
-                for (size_t k = 0; k < n; ++k) pi_out[i * capacity + k] = theta_out[i * capacity + k] = NaN;
+        T.finish();
+        if (!T.act.empty()) t_tim.stats_ms += pass_tm.ms();
         *n_out = n;
     });
 }
@@ -2480,28 +2446,9 @@ fm_status fm_per_site_diversity_multi(fm_group *const *groups, const size_t *raw
 // repacked straight into the bitplanes of every declared group while the next chunk is still
 // on the PCIe bus.  The u8 rows are never resident (1.125 B/genotype of HBM and the separate
 // repack pass are saved).
-// Per-site pi / theta tracks requested for the matrix being ingested (fm_ingest_request_tracks): every chunk's
-// tracks are computed right after its repack and stored while the next chunks are still on the bus.
-struct IngestTracks {
-    std::vector<fm_group *> act;        // groups with >= 2 listed haplotypes
-    std::vector<size_t> act_idx;        // their row in the caller's arrays
-    std::vector<size_t> nan_rows;       // rows of groups with < 2 listed haplotypes: NaN (stats.rs:4675-4681)
-    uint32_t lo = 0, hi = 0;            // site range of the region
-    size_t capacity = 0;
-    DevBuf<int64_t> d_mask, d_filt;
-    uint32_t n_mask = 0, n_filt = 0;
-    bool has_mask = false;
-    std::vector<double *> ppi, pth;     // device-visible destinations (the caller's page-locked rows or own buffers)
-    std::vector<DevBuf<double>> own_pi, own_th;
-    std::vector<char> direct;
-    int64_t *pos_out = nullptr, *pos_direct = nullptr;
-    double *pi_out = nullptr, *theta_out = nullptr;
-    bool pos_done = false;
-};
-
 struct fm_ingest {
     fm_matrix *m = nullptr;
-    std::unique_ptr<IngestTracks> tracks;
+    std::unique_ptr<TrackRequest> tracks;  // fm_ingest_request_tracks: computed chunk by chunk after the repack
     cudaEvent_t pos_up = nullptr;         // the positions are on the device (recorded on copy_s)
     std::vector<fm_group *> groups;       // declared with fm_ingest_add_group (owned until finish)
     std::vector<fm_partition *> parts;    // declared with fm_ingest_add_partition
@@ -2540,34 +2487,18 @@ static void ingest_early_setup(fm_ingest *h) {
     }
 }
 
-// Tracks of the freshly repacked rows [r0, r1) on the ingest's compute stream (after launch_repack).
+// Tracks of the freshly repacked rows [r0, r1) on the ingest's compute stream (after launch_repack), stored while
+// the next chunks are still on the bus.
 static void ingest_tracks_chunk(fm_ingest *h, size_t r0, size_t r1) {
-    IngestTracks *T = h->tracks.get();
-    if (!T || T->act.empty()) return;
-    const uint32_t lo = (uint32_t)std::max<size_t>(r0, T->lo), hi = (uint32_t)std::min<size_t>(r1, T->hi);
-    if (lo >= hi) return;
+    TrackRequest *T = h->tracks.get();
+    if (!T || r1 <= T->lo || r0 >= T->hi) return;
     fm_matrix *m = h->m;
     if (!h->pos_uploaded) {  // pageable positions (small matrices): put them on the device now, ordered before the pass
         if (m->V) CK(cudaMemcpyAsync(m->d_pos, m->pos.data(), m->V * 8, cudaMemcpyHostToDevice, h->comp_s));
         h->pos_uploaded = true;
     }
     StreamScope on_comp(h->comp_s);
-    if (!T->pos_done && T->pos_direct) {
-        const size_t n = T->hi - T->lo;
-        fm_k_pos_plus1<<<(uint32_t)std::min<size_t>((n + 255) / 256, 2048), 256, 0, h->comp_s>>>(m->d_pos, T->lo, (uint32_t)n,
-                                                                                                    T->pos_direct);
-        CK(cudaGetLastError());
-        g_launches++;
-        T->pos_done = true;
-    }
-    std::vector<double *> ppi(T->act.size()), pth(T->act.size());
-    for (size_t i = 0; i < T->act.size(); ++i) {
-        ppi[i] = T->ppi[i] + (lo - T->lo);
-        pth[i] = T->pth[i] + (lo - T->lo);
-    }
-    run_diversity_multi(T->act.data(), T->act.size(), lo, hi, FM_PIFORM_COMPONENTS, ppi.data(), pth.data(),
-                        T->has_mask ? T->d_mask.p : nullptr, T->n_mask, T->n_filt ? T->d_filt.p : nullptr, T->n_filt,
-                        /*out=*/nullptr);
+    T->run(r0, r1, h->comp_s);
 }
 
 static size_t tapered_chunk(size_t rows_left, size_t chunk);
@@ -2707,81 +2638,18 @@ fm_status fm_ingest_request_tracks(fm_ingest *h, const size_t *group_index, cons
         *n_out = 0;
         if (h->rows_done) fail(FM_ERR_INVALID_ARG, "tracks must be requested before the first rows call");
         if (h->tracks) fail(FM_ERR_INVALID_ARG, "tracks were already requested for this ingest");
-        fm_matrix *m = h->m;
-        set_dev(m);
-        auto T = std::make_unique<IngestTracks>();
+        set_dev(h->m);
+        std::vector<fm_group *> gs(n_groups);
         for (size_t i = 0; i < n_groups; ++i) {
             if (group_index[i] >= h->groups.size()) fail(FM_ERR_INVALID_ARG, "group index out of range");
-            fm_group *g = h->groups[group_index[i]];
-            if (g->n_bits != 1 || g->count_only)
+            gs[i] = h->groups[group_index[i]];
+            if (gs[i]->n_bits != 1 || gs[i]->count_only)
                 fail(FM_ERR_UNSUPPORTED, "streamed tracks need biallelic bitplane groups (use fm_per_site_diversity after finish)");
-            if (raw_n[i] >= 2) {
-                T->act.push_back(g);
-                T->act_idx.push_back(i);
-            } else {
-                T->nan_rows.push_back(i);
-            }
         }
-        if (region_len(rs, re) <= 0) {  // stats.rs:4656-4666: no sites; nothing to compute while the rows arrive
-            h->tracks = std::move(T);
-            h->tracks->act.clear();
-            h->tracks->nan_rows.clear();
-            return;
-        }
-        uint32_t lo, hi;
-        site_range(m, rs, re, lo, hi);
-        const size_t n = hi - lo;
-        T->lo = lo;
-        T->hi = hi;
-        T->capacity = capacity;
-        T->pos_out = pos_out;
-        T->pi_out = pi_out;
-        T->theta_out = theta_out;
-        if (n) {
-            if (n > capacity) fail(FM_ERR_INVALID_ARG, "output capacity too small");
-            if (!pi_out || !theta_out) fail(FM_ERR_INVALID_ARG, "output arrays are NULL");
-            std::vector<int64_t> merged, fs;
-            if (mask_iv) {
-                merge_intervals(mask_iv, n_mask, merged);
-                T->d_mask.alloc(std::max<size_t>(merged.size(), 2));
-                T->d_mask.upload(merged.data(), merged.size());
-                T->n_mask = (uint32_t)(merged.size() / 2);
-                T->has_mask = true;
-            }
-            if (filtered && n_filt) {
-                fs.assign(filtered, filtered + n_filt);
-                std::sort(fs.begin(), fs.end());
-                T->d_filt.alloc(fs.size());
-                T->d_filt.upload(fs.data(), fs.size());
-                T->n_filt = (uint32_t)fs.size();
-            }
-            const size_t na = T->act.size();
-            T->ppi.resize(na);
-            T->pth.resize(na);
-            T->own_pi = std::vector<DevBuf<double>>(na);
-            T->own_th = std::vector<DevBuf<double>>(na);
-            T->direct.assign(na, 0);
-            for (size_t i = 0; i < na; ++i) {
-                double *mp = static_cast<double *>(mapped_host_range(pi_out + T->act_idx[i] * capacity, n * 8));
-                double *mt = static_cast<double *>(mapped_host_range(theta_out + T->act_idx[i] * capacity, n * 8));
-                if (mp && mt) {
-                    T->direct[i] = 1;
-                    T->ppi[i] = mp;
-                    T->pth[i] = mt;
-                } else {
-                    T->own_pi[i].alloc(n);
-                    T->own_th[i].alloc(n);
-                    T->ppi[i] = T->own_pi[i].p;
-                    T->pth[i] = T->own_th[i].p;
-                }
-            }
-            if (pos_out) T->pos_direct = static_cast<int64_t *>(mapped_host_range(pos_out, n * 8));
-            CK(cudaStreamSynchronize(stream()));  // the interval lists are host temporaries; buffers usable on comp_s
-        } else {
-            T->act.clear();
-            T->nan_rows.clear();
-        }
-        *n_out = n;
+        auto T = std::make_unique<TrackRequest>();
+        *n_out = T->prepare(h->m, gs.data(), raw_n, n_groups, rs, re, mask_iv, n_mask, filtered, n_filt, pos_out, pi_out,
+                            theta_out, capacity);
+        CK(cudaStreamSynchronize(stream()));  // the uploads and buffers are used on comp_s
         h->tracks = std::move(T);
     });
 }
@@ -3223,22 +3091,7 @@ fm_status fm_ingest_finish(fm_ingest *h, fm_matrix **matrix_out, fm_group **grou
         set_dev(h->m);
         ingest_late_setup(h);
         CK(cudaStreamSynchronize(h->comp_s));
-        if (IngestTracks *T = h->tracks.get()) {  // requested tracks: everything was computed as the rows arrived
-            const size_t n = T->hi - T->lo;
-            DevBuf<int64_t> d_p1;
-            if (n) {
-                for (size_t i = 0; i < T->act.size(); ++i)
-                    if (!T->direct[i]) {  // pageable output rows: copy them out now
-                        T->own_pi[i].download(T->pi_out + T->act_idx[i] * T->capacity, n);
-                        T->own_th[i].download(T->theta_out + T->act_idx[i] * T->capacity, n);
-                    }
-                if (!T->pos_done) download_positions_plus1(h->m, T->lo, n, T->pos_out, d_p1);  // stats.rs:4746
-                CK(cudaStreamSynchronize(stream()));
-                const double NaN = std::numeric_limits<double>::quiet_NaN();
-                for (size_t row : T->nan_rows)
-                    for (size_t k = 0; k < n; ++k) T->pi_out[row * T->capacity + k] = T->theta_out[row * T->capacity + k] = NaN;
-            }
-        }
+        if (h->tracks) h->tracks->finish();  // requested tracks: computed as the rows arrived
         if (h->timing_started) {
             float a = 0.f, b = 0.f;
             CK(cudaEventElapsedTime(&a, h->t_copy0, h->t_copy1));
@@ -3297,7 +3150,8 @@ fm_status fm_hudson_dxy(fm_group *g1, fm_group *g2, int64_t L1, int64_t L2, int 
         check_pair(g1, g2, path == FM_HUDSON_SUMMARIES);
         require_device();
         if (raw_n1 == 0 || raw_n2 == 0) return;
-        ensure_counts_pair(g1, g2);
+        fm_group *pair[2] = {g1, g2};
+        summarize_groups(pair, 2);
         set_dev(g1->m);
         const int variant = path == FM_HUDSON_SUMMARIES ? -1
                             : path == FM_HUDSON_DENSE   ? dense_variant(g1->m)
@@ -3376,76 +3230,39 @@ fm_status fm_hudson_pair(fm_group *g1, fm_group *g2, int64_t L1, int64_t L2, int
         }
         // counts: fused two-group sweep when nothing is cached yet and the main pass covers the
         // whole matrix; otherwise per-group plane passes (cached) + light kernels on the counts.
-        bool fused = false;
+        bool swept = false;  // the Hudson partials came out of the pass that cached the counts
         if (g1 != g2 && g1->m == g2->m && lo == 0 && hi == V && V > 0 && g1->n_bits == 1) {
             std::unique_lock<std::mutex> l1(g1->mu, std::defer_lock), l2(g2->mu, std::defer_lock);
             std::lock(l1, l2);
             if (!g1->have_counts && !g2->have_counts) {
-                for (fm_group *g : {g1, g2}) alloc_counts(g);
                 // ONE sweep of both groups' planes (fm_k_plane_pass_seq, pair units): every warp streams a batch of
                 // group 1, then the same batch of group 2, and evaluates the Hudson components in place -- the
                 // groups' counts and summary scalars are cached for later calls AND the Hudson partials (plus the
                 // optional per-site values) come out of the same pass (stats.rs:3179-3278).
-                fm_group *pair[2] = {g1, g2};
                 const uint32_t nb = (V + 31) / 32;
-                DevBuf<double> ppi[2], pd((size_t)nb * 5);
-                DevBuf<uint32_t> ppu[2], pu((size_t)nb * 3);
-                std::vector<fm::RowSeg> segs(2);
-                for (int k = 0; k < 2; ++k) {
-                    ppi[k].alloc(nb);
-                    ppu[k].alloc((size_t)nb * 2);
-                    fm::DivEpilogue de{};
-                    set_tables(de, pair[k]);
-                    de.pi_form = FM_PIFORM_COUNTS;
-                    de.part_pi = ppi[k].p;
-                    de.part_u = ppu[k].p;
-                    de.alt_out = pair[k]->d_alt;
-                    de.called_out = called_cache(pair[k]);
-                    segs[k] = div_seg(pair[k], de, 0, V);
-                }
+                DevBuf<double> pd((size_t)nb * 5);
+                DevBuf<uint32_t> pu((size_t)nb * 3);
                 fm::HudsonEpilogue he = e;
                 he.variant = site_variant;
                 he.part_d = pd.p;
                 he.part_u = pu.p;
-                std::vector<fm::HudsonEpilogue> hv{he};
-                RowPlan plan;
-                Timer tm;
-                tm.start();
-                const bool ok = plan_rows(segs, &hv, plan);
-                if (ok) launch_rows(plan, m->device);
-                tm.stop();
-                if (ok) {
-                    const fm::PassGeom G = batch_range(0, V);
-                    for (int k = 0; k < 2; ++k) {
-                        double od[1];
-                        uint64_t ou[2];
-                        finish_partials(ppi[k].p, 1, ppu[k].p, 2, G, od, ou);
-                        pair[k]->pi_sum = od[0];
-                        pair[k]->seg = ou[0];
-                        pair[k]->unc = ou[1];
-                        pair[k]->have_counts = true;
-                    }
+                DivPass P;
+                P.store_counts = true;
+                P.hudson = &he;
+                P.units = {DivUnit{g1, 0, V}, DivUnit{g2, 0, V}};
+                P.run();
+                swept = P.hudson_done;
+                if (swept) {
                     double od[5];
                     uint64_t ou[3];
-                    finish_partials(pd.p, 5, pu.p, 3, G, od, ou);
+                    finish_partials(pd.p, 5, pu.p, 3, batch_range(0, V), od, ou);
                     main_t = HudsonTotals{od[0], od[1], od[2], od[3], od[4], ou[0], ou[1], ou[2]};
-                    t_tim.stats_ms += tm.ms();
-                } else {  // rows too wide for the row pass: two chunked passes, then the light kernel
-                    DivResult r[2];
-                    run_diversity_multi(pair, 2, 0, V, FM_PIFORM_COUNTS, nullptr, nullptr, nullptr, 0, nullptr, 0, r, true);
-                    for (int k = 0; k < 2; ++k) {
-                        pair[k]->seg = r[k].seg;
-                        pair[k]->unc = r[k].unc;
-                        pair[k]->pi_sum = r[k].pi_sum;
-                        pair[k]->have_counts = true;
-                    }
-                    main_t = run_hudson_counts(g1, g2, lo, hi, site_variant, e);
                 }
-                fused = true;
             }
         }
-        if (!fused) {
-            ensure_counts_pair(g1, g2);
+        if (!swept) {  // rows too wide for the row pass, or counts cached before: the light kernel on the counts
+            fm_group *pair[2] = {g1, g2};
+            summarize_groups(pair, 2);
             main_t = run_hudson_counts(g1, g2, lo, hi, site_variant, e);
         }
         if (!has_region || (lo == 0 && hi == V && site_variant == aux_variant)) {
@@ -4029,7 +3846,8 @@ fm_status fm_hudson_window_sums(fm_group *g1, fm_group *g2, const int64_t *windo
         if (n_windows && !windows) fail(FM_ERR_INVALID_ARG, "NULL argument");
         require_device();
         if (!n_windows) return;
-        ensure_counts_pair(g1, g2);
+        fm_group *pair[2] = {g1, g2};
+        summarize_groups(pair, 2);
         set_dev(g1->m);
         std::vector<uint32_t> lo, hi;
         window_ranges(g1->m, windows, n_windows, lo, hi);
@@ -4387,7 +4205,8 @@ fm_status fm_hudson_pair_sharded(fm_group *g1, fm_group *g2, int64_t sequence_le
                 if (done) launch_rows(plan, m->device);
             }
             if (!done) {  // cached counts, count-only groups or rows wider than the row pass: from the counts
-                ensure_counts_pair(g1, g2);
+                fm_group *pair[2] = {g1, g2};
+                summarize_groups(pair, 2);
                 const uint32_t blocks = std::min<uint32_t>((nb + 7) / 8, 8u * sm_count(m->device));
                 fm::fm_k_hudson_from_counts<<<blocks, 256, 0, stream()>>>(g1->d_alt, g1->d_cnt, g2->d_alt, g2->d_cnt, he, 0,
                                                                            V, 0, nb);

@@ -829,6 +829,62 @@ def test_wide_rows(wide, form):
     check_pair(m, ref, lists[129], lists[16320], pos)
 
 
+@pytest.mark.gpu
+def test_wide_mixed_set(wide):
+    """A set that mixes kinds -- a group too wide for the row pass, two fresh narrow groups and a narrow group whose
+    summary is cached -- through fm_per_site_diversity_multi and fm_groups_summary_batch: the fresh narrow groups
+    share one row launch (two stats launches in all) and every output equals the per-group calls bit for bit."""
+    from ferromic_b200.api import _Matrix
+    L = _L()
+    pos, lists, ref = wide["pos"], wide["lists"], wide["ref"]
+    m = _Matrix(wide["data"], wide["miss"], pos, max_allele=1, always_bitmap=True, ingest="u8")
+    haps = [lists[114689], lists[129], lists[16320], random_haps(np.random.default_rng(22), WIDE_S, 2, 1000)]
+    k = len(haps)
+
+    def mixed_set():
+        gs = [fresh(m, h) for h in haps]
+        gs[-1].summary()
+        return gs
+
+    def stats_launches(call):
+        L.check(L.lib().fm_timings_reset())
+        L.check(call())
+        t = L.Timings()
+        L.check(L.lib().fm_timings_get(C.byref(t)))
+        return t.stats_launches
+
+    lo, hi = 1, WIDE_V
+    cap = hi - lo
+    mask, filt = [(int(pos[10]), int(pos[20]))], [int(pos[5]), int(pos[40])]
+    mk = np.ascontiguousarray(mask, dtype=np.int64).reshape(-1)
+    fl = np.ascontiguousarray(filt, dtype=np.int64)
+    raw = (C.c_size_t * k)(*[len(h) for h in haps])
+    pi, th, out_p, nout = np.zeros((k, cap)), np.zeros((k, cap)), np.zeros(cap, dtype=np.int64), C.c_size_t()
+    gs = mixed_set()
+    assert stats_launches(lambda: L.lib().fm_per_site_diversity_multi(
+        handles(gs), raw, k, int(pos[lo]), int(pos[hi - 1]), mk.ctypes.data, mk.size // 2, fl.ctypes.data, fl.size,
+        out_p.ctypes.data, pi.ctypes.data, th.ctypes.data, cap, C.byref(nout))) == 2
+    assert nout.value == cap and np.array_equal(out_p, pos[lo:hi] + 1)
+    dropped = dropped_sites(pos, lo, hi, mask, filt)
+    for i, h in enumerate(haps):
+        n, a = ref(h)
+        assert_tracks(pi[i], th[i], n[lo:hi], a[lo:hi], dropped)
+        _, _, spi, sth = per_site(fresh(m, h), len(h), pos, lo, hi, mask, filt)
+        assert same_bits(spi, pi[i]) and same_bits(sth, th[i]), len(h)
+
+    gs = mixed_set()
+    seg, unc, pis = np.zeros(k, dtype=np.uint64), np.zeros(k, dtype=np.uint64), np.zeros(k)
+    assert stats_launches(lambda: L.lib().fm_groups_summary_batch(handles(gs), k, seg.ctypes.data, pis.ctypes.data,
+                                                                  unc.ctypes.data)) == 2
+    for i, h in enumerate(haps):
+        single = fresh(m, h).summary(want_arrays=True)
+        got = gs[i].summary(want_arrays=True)
+        assert (int(seg[i]), int(unc[i])) == (single["segregating_sites"], single["uncallable_lt2"]), len(h)
+        assert pis[i] == single["pi_sum"] == got["pi_sum"], len(h)
+        assert np.array_equal(got["alt"], single["alt"]) and np.array_equal(got["called"], single["called"]), len(h)
+        check_summary(gs[i], ref, h)
+
+
 # ------------------------------------------------------------------ GPU: multi-allelic counts
 MULTI_V, MULTI_S = 300, 28673
 MULTI_SIZES = (1, 31, 33, 127, 129, 1000, 16320, 57345)
