@@ -64,7 +64,8 @@ class VcfInfo(C.Structure):
 class PcaParams(C.Structure):
     _fields_ = [("k", C.c_uint32), ("oversampling", C.c_uint32), ("power_iterations", C.c_uint32),
                 ("min_maf", C.c_double), ("max_missing", C.c_double), ("seed", C.c_uint64), ("has_region", C.c_int),
-                ("region_start", C.c_int64), ("region_end", C.c_int64)]
+                ("region_start", C.c_int64), ("region_end", C.c_int64), ("site_list", C.c_void_p),
+                ("site_list_len", C.c_uint64)]
 
 
 class PcaInfo(C.Structure):
@@ -77,13 +78,19 @@ class PcaInfo(C.Structure):
 class LdParams(C.Structure):
     _fields_ = [("window", C.c_uint32), ("max_distance", C.c_int64), ("min_maf", C.c_double),
                 ("max_missing", C.c_double), ("has_region", C.c_int), ("region_start", C.c_int64),
-                ("region_end", C.c_int64)]
+                ("region_end", C.c_int64), ("site_list", C.c_void_p), ("site_list_len", C.c_uint64)]
 
 
 class LdInfo(C.Structure):
     _fields_ = [("n_haplotypes", C.c_uint64), ("n_sites", C.c_uint64), ("pairs", C.c_uint64),
                 ("called_plane", C.c_uint32), ("slabs", C.c_uint32), ("band_launches", C.c_uint32)] + [
         (f, C.c_float) for f in ("stats_ms", "planes_ms", "band_ms", "copy_ms", "total_ms")]
+
+
+class LdPruneInfo(C.Structure):
+    _fields_ = [(f, C.c_uint64) for f in ("n_haplotypes", "n_sites", "pairs", "linked_pairs", "n_retained")] + [
+        ("called_plane", C.c_uint32), ("band_launches", C.c_uint32)] + [
+        (f, C.c_float) for f in ("stats_ms", "planes_ms", "band_ms", "scan_ms", "total_ms")]
 
 
 EXPORTS = [
@@ -102,6 +109,7 @@ EXPORTS = [
     "fm_vcf_batch_release", "fm_synth_fill", "fm_timings_reset", "fm_timings_get", "fm_bench_diversity",
     "fm_pairwise_differences", "fm_bgzf_inflate", "fm_vcf_parse_bgzf", "fm_bgzf_deflate_bound", "fm_bgzf_deflate",
     "fm_falsta_tracks_bgzf", "fm_haplotype_pca", "fm_haplotype_ld",
+    "fm_haplotype_ld_prune",
 ]
 
 _lib = None
@@ -217,6 +225,8 @@ def lib() -> C.CDLL:
     L.fm_haplotype_pca.argtypes = [vp, vp, vp, sz, C.POINTER(PcaParams), vp, vp, vp, vp, vp, vp, sz,
                                    C.POINTER(PcaInfo)]
     L.fm_haplotype_ld.argtypes = [vp, vp, vp, sz, C.POINTER(LdParams), vp, vp, sz, vp, vp, sz, C.POINTER(LdInfo)]
+    L.fm_haplotype_ld_prune.argtypes = [vp, vp, vp, sz, C.POINTER(LdParams), dbl, vp, vp, vp, sz,
+                                        C.POINTER(LdPruneInfo)]
     for name in EXPORTS:
         fn = getattr(L, name)
         if name not in ("fm_last_error", "fm_version"):

@@ -945,12 +945,31 @@ def _haplotype_call(what, variants, haplotypes, region):
     return vs, _sparse_matrix(vs), haps, region
 
 
-def _haplotype_args(haplotypes, region):
-    """The sample index and side arrays of a (sample, side) list and the (has_region, region_start, region_end)
-    fields of fm_pca_params / fm_ld_params."""
+def _haplotype_args(haplotypes, region, sites=None):
+    """The sample index and side arrays of a (sample, side) list, the (has_region, region_start, region_end) fields
+    of fm_pca_params / fm_ld_params and, for a site list (matrix rows), the array that backs its (site_list,
+    site_list_len) fields, which the caller keeps alive across the call (None: no list)."""
     idx = np.asarray([h[0] for h in haplotypes], dtype=np.uint64)
     side = np.asarray([h[1] for h in haplotypes], dtype=np.uint8)
-    return idx, side, (0, 0, 0) if region is None else (1, int(region[0]), int(region[1]))
+    reg = (0, 0, 0) if region is None else (1, int(region[0]), int(region[1]))
+    if sites is None:
+        return idx, side, reg, None
+    rows = np.asarray(sites)
+    if rows.ndim != 1 or not (rows.size == 0 or np.issubdtype(rows.dtype, np.integer)):
+        raise ValueError("sites must be a 1-D list of variant indices")
+    if rows.size and rows.min() < 0:
+        raise ValueError("sites holds a negative variant index")
+    return idx, side, reg, np.ascontiguousarray(rows, dtype=np.uint64)
+
+
+_NO_SITES = np.zeros(1, dtype=np.uint64)  # a non-NULL site_list for an empty list
+
+
+def _site_list(rows):
+    """(site_list, site_list_len) fields for the array of _haplotype_args."""
+    if rows is None:
+        return None, 0
+    return (rows if rows.size else _NO_SITES).ctypes.data, rows.size
 
 
 def _offset_haplotypes(m: _Matrix, offsets):
@@ -980,18 +999,18 @@ class HaplotypePcaResult:
 
 
 def _matrix_pca(m: _Matrix, haplotypes, n_components=10, region=None, min_maf=0.0, max_missing=0.0, oversampling=10,
-                power_iterations=4, seed=0, loadings=False):
+                power_iterations=4, seed=0, loadings=False, sites=None):
     """fm_haplotype_pca on a device matrix: dict of offsets, scores, singular_values, explained_variance_ratio,
-    total_variance, kept (matrix rows), loadings and the call's info struct."""
+    total_variance, kept (matrix rows), loadings and the call's info struct.  sites: matrix rows, None = every row."""
     for name, x in (("n_components", n_components), ("oversampling", oversampling),
                     ("power_iterations", power_iterations)):
         if int(x) < 0 or int(x) >= 2 ** 32:
             raise ValueError(f"{name} must lie in [0, 2^32)")
-    idx, side, reg = _haplotype_args(haplotypes, region)
+    idx, side, reg, rows = _haplotype_args(haplotypes, region, sites)
     n_in = len(haplotypes)
     k = int(n_components)
     prm = _lib.PcaParams(k, int(oversampling), int(power_iterations), float(min_maf), float(max_missing),
-                         int(seed) & 0xFFFFFFFFFFFFFFFF, *reg)
+                         int(seed) & 0xFFFFFFFFFFFFFFFF, *reg, *_site_list(rows))
     info = _lib.PcaInfo()
     off = np.zeros(max(n_in, 1), dtype=np.uint32)
     scores = np.zeros(max(n_in * k, 1), dtype=np.float64)
@@ -1009,14 +1028,16 @@ def _matrix_pca(m: _Matrix, haplotypes, n_components=10, region=None, min_maf=0.
 
 
 def haplotype_pca(variants, haplotypes=None, n_components=10, region=None, min_maf=0.0, max_missing=0.0,
-                  oversampling=10, power_iterations=4, seed=0, loadings=False) -> HaplotypePcaResult:
+                  oversampling=10, power_iterations=4, seed=0, loadings=False, sites=None) -> HaplotypePcaResult:
     """Top `n_components` principal components of the standardized haplotype x site matrix, computed on the GPU by
     randomized subspace iteration (definition in include/ferromic_gpu.h, fm_haplotype_pca).  haplotypes: (sample,
     side) pairs, None = every cell of every sample; region: 0-based inclusive (start, end) over positions, None =
-    every variant.  Missing cells follow from_variants semantics and are mean-imputed (Z = 0)."""
+    every variant; sites: strictly ascending indices into `variants` that may be kept (the region and filters apply
+    on top), None = every variant -- e.g. `haplotype_ld_prune(variants).sites`.  Missing cells follow from_variants
+    semantics and are mean-imputed (Z = 0)."""
     vs, m, haps, region = _haplotype_call("haplotype PCA", variants, haplotypes, region)
     r = _matrix_pca(m, haps, n_components, region, min_maf, max_missing, oversampling, power_iterations, seed,
-                    loadings)
+                    loadings, sites)
     return HaplotypePcaResult(_offset_haplotypes(m, r["offsets"]), r["scores"], r["singular_values"],
                               r["explained_variance_ratio"], r["total_variance"], vs.positions[r["kept"]],
                               r["loadings"])
@@ -1039,16 +1060,24 @@ class HaplotypeLdResult:
                 f"window={self.r2.shape[1]})")
 
 
-def _matrix_ld(m: _Matrix, haplotypes, window=100, max_distance=None, region=None, min_maf=0.0, max_missing=0.0,
-               dprime=False):
-    """fm_haplotype_ld on a device matrix: dict of offsets, kept (matrix rows), r2 [M, window], dprime [M, window] or
-    None, and the call's info struct.  A size query learns M first, so the outputs take M * window cells."""
+def _ld_params(haplotypes, window, max_distance, region, min_maf, max_missing, sites):
+    """(idx, side, fm_ld_params, the array backing its site list) of _matrix_ld / _matrix_ld_prune."""
     if not 1 <= int(window) < 2 ** 32:
         raise ValueError("window must lie in [1, 2^32)")
-    idx, side, reg = _haplotype_args(haplotypes, region)
+    idx, side, reg, rows = _haplotype_args(haplotypes, region, sites)
+    prm = _lib.LdParams(int(window), -1 if max_distance is None else int(max_distance), float(min_maf),
+                        float(max_missing), *reg, *_site_list(rows))
+    return idx, side, prm, rows
+
+
+def _matrix_ld(m: _Matrix, haplotypes, window=100, max_distance=None, region=None, min_maf=0.0, max_missing=0.0,
+               dprime=False, sites=None):
+    """fm_haplotype_ld on a device matrix: dict of offsets, kept (matrix rows), r2 [M, window], dprime [M, window] or
+    None, and the call's info struct.  A size query learns M first, so the outputs take M * window cells.  sites:
+    matrix rows, None = every row."""
+    idx, side, prm, rows = _ld_params(haplotypes, window, max_distance, region, min_maf, max_missing, sites)
     n_in = len(haplotypes)
     w = int(window)
-    prm = _lib.LdParams(w, -1 if max_distance is None else int(max_distance), float(min_maf), float(max_missing), *reg)
     info = _lib.LdInfo()
     L = lib()
     st = L.fm_haplotype_ld(m.handle, _ptr(idx), _ptr(side), n_in, C.byref(prm), None, None, 0, None, None, 0,
@@ -1068,15 +1097,66 @@ def _matrix_ld(m: _Matrix, haplotypes, window=100, max_distance=None, region=Non
 
 
 def haplotype_ld(variants, haplotypes=None, window=100, max_distance=None, region=None, min_maf=0.0, max_missing=0.0,
-                 dprime=False) -> HaplotypeLdResult:
+                 dprime=False, sites=None) -> HaplotypeLdResult:
     """r^2 (and D' when `dprime`) between each kept site and the next `window` kept sites, computed on the GPU
     (definition in include/ferromic_gpu.h, fm_haplotype_ld).  haplotypes: (sample, side) pairs, None = every cell of
     every sample, as haplotype_pca; max_distance: pairs further apart in position are NaN, None = no limit; region:
     0-based inclusive (start, end) over positions, None = every variant.  Sites are filtered as haplotype_pca filters
-    them; missing cells follow from_variants semantics and only the haplotypes called at both sites count."""
+    them, and limited to `sites` (strictly ascending indices into `variants`) when given; missing cells follow
+    from_variants semantics and only the haplotypes called at both sites count."""
     vs, m, haps, region = _haplotype_call("haplotype LD", variants, haplotypes, region)
-    r = _matrix_ld(m, haps, window, max_distance, region, min_maf, max_missing, dprime)
+    r = _matrix_ld(m, haps, window, max_distance, region, min_maf, max_missing, dprime, sites)
     return HaplotypeLdResult(_offset_haplotypes(m, r["offsets"]), vs.positions[r["kept"]], r["r2"], r["dprime"])
+
+
+class HaplotypeLdPruneResult:
+    """Greedy r^2 pruning of the kept sites of a haplotype set (fm_haplotype_ld_prune).  `sites` are the retained
+    variants' indices into the input (int64, ascending) and `positions` their positions; `n_kept` is the number of
+    sites that passed the filters, `pairs` the site pairs under the window rule and `linked_pairs` those whose r^2
+    exceeds the threshold."""
+    __slots__ = ("haplotypes", "sites", "positions", "n_kept", "pairs", "linked_pairs")
+
+    def __init__(self, haplotypes, sites, positions, n_kept, pairs, linked_pairs):
+        self.haplotypes = haplotypes
+        self.sites = sites
+        self.positions = positions
+        self.n_kept = n_kept
+        self.pairs = pairs
+        self.linked_pairs = linked_pairs
+
+    def __repr__(self):
+        return (f"HaplotypeLdPruneResult(n_haplotypes={len(self.haplotypes)}, n_kept={self.n_kept}, "
+                f"n_retained={len(self.sites)}, linked_pairs={self.linked_pairs})")
+
+
+def _matrix_ld_prune(m: _Matrix, haplotypes, r2_threshold=0.2, window=100, max_distance=None, region=None, min_maf=0.0,
+                     max_missing=0.0, sites=None):
+    """fm_haplotype_ld_prune on a device matrix: dict of offsets, kept and retained (matrix rows) and the call's info
+    struct.  The site capacity is the matrix's variant count, which bounds M."""
+    idx, side, prm, rows = _ld_params(haplotypes, window, max_distance, region, min_maf, max_missing, sites)
+    n_in = len(haplotypes)
+    info = _lib.LdPruneInfo()
+    cap = m.V
+    off = np.zeros(max(n_in, 1), dtype=np.uint32)
+    kept = np.zeros(max(cap, 1), dtype=np.uint64)
+    ret = np.zeros(max(cap, 1), dtype=np.uint64)
+    check(lib().fm_haplotype_ld_prune(m.handle, _ptr(idx), _ptr(side), n_in, C.byref(prm), float(r2_threshold),
+                                      _ptr(off), _ptr(kept), _ptr(ret), cap, C.byref(info)))
+    n, M, R = int(info.n_haplotypes), int(info.n_sites), int(info.n_retained)
+    return dict(offsets=off[:n].copy(), kept=kept[:M].astype(np.int64), retained=ret[:R].astype(np.int64), info=info)
+
+
+def haplotype_ld_prune(variants, haplotypes=None, r2_threshold=0.2, window=100, max_distance=None, region=None,
+                       min_maf=0.0, max_missing=0.0, sites=None) -> HaplotypeLdPruneResult:
+    """Greedy r^2 pruning on the GPU (definition in include/ferromic_gpu.h, fm_haplotype_ld_prune): walking the kept
+    sites of haplotype_ld in order, a site is retained unless a retained earlier site within `window` kept sites
+    (and `max_distance`) has r^2 > r2_threshold with it.  Arguments as haplotype_ld.  The result's `sites` go straight
+    into haplotype_pca(variants, sites=...) or haplotype_ld(variants, sites=...)."""
+    vs, m, haps, region = _haplotype_call("haplotype LD pruning", variants, haplotypes, region)
+    r = _matrix_ld_prune(m, haps, r2_threshold, window, max_distance, region, min_maf, max_missing, sites)
+    info = r["info"]
+    return HaplotypeLdPruneResult(_offset_haplotypes(m, r["offsets"]), r["retained"], vs.positions[r["retained"]],
+                                  int(info.n_sites), int(info.pairs), int(info.linked_pairs))
 
 
 def _opt(value: float, some: int, bit: int):

@@ -5439,8 +5439,9 @@ static uint32_t transpose_grid(const fm_matrix *m, uint64_t tasks) {
     return (uint32_t)std::min<uint64_t>((tasks + 7) / 8, 64ull * sm_count(m->device));
 }
 
-// The kept sites of a haplotype set, shared by haplotype PCA and haplotype LD: the region's rows [v_lo, v_lo + R)
-// pass the site filter of include/ferromic_gpu.h on the n selected cells `off`, M of them in row order in d_kept.
+// The kept sites of a haplotype set, shared by haplotype PCA, LD and LD pruning: the region's rows [v_lo, v_lo + R)
+// that are in the site list (when one is given) pass the site filter of include/ferromic_gpu.h on the n selected
+// cells `off`, M of them in row order in d_kept.
 // d_alt / d_called hold the counts of every region row; incomplete is set when a kept site has a missing cell.
 struct HapSites {
     std::vector<uint32_t> off;
@@ -5451,7 +5452,13 @@ struct HapSites {
 
 // Starts `tm` at its first device work; the caller stops it after its own per-kept-site kernel.
 static void select_hap_sites(const fm_matrix *m, std::vector<uint32_t> off, int has_region, int64_t region_start,
-                             int64_t region_end, double min_maf, double max_missing, Timer &tm, HapSites &hs) {
+                             int64_t region_end, double min_maf, double max_missing, const uint64_t *site_list,
+                             uint64_t site_list_len, Timer &tm, HapSites &hs) {
+    if (site_list)
+        for (uint64_t i = 0; i < site_list_len; ++i) {
+            if (site_list[i] >= m->V) fail(FM_ERR_INVALID_ARG, "site_list holds a row beyond the matrix's variants");
+            if (i && site_list[i] <= site_list[i - 1]) fail(FM_ERR_INVALID_ARG, "site_list must be strictly ascending");
+        }
     hs.off = std::move(off);
     hs.n = (uint32_t)hs.off.size();
     uint32_t v_hi = (uint32_t)m->V;
@@ -5465,14 +5472,25 @@ static void select_hap_sites(const fm_matrix *m, std::vector<uint32_t> off, int 
     hs.d_called.alloc(std::max<uint32_t>(R, 1));
     hs.d_kept.alloc(std::max<uint32_t>(R, 1));
     DevBuf<uint32_t> d_counts(2);  // M, incomplete
-    DevBuf<uint8_t> d_keep(std::max<uint32_t>(R, 1));
+    DevBuf<uint8_t> d_keep(std::max<uint32_t>(R, 1)), d_allow(site_list ? std::max<uint32_t>(R, 1) : 0);
+    DevBuf<uint64_t> d_list(site_list ? std::max<uint64_t>(site_list_len, 1) : 0);
     tm.start();
     hs.d_off.upload(hs.off.data(), n);
     if (!n || !R) return;
     CK(cudaMemsetAsync(d_counts.p, 0, 8, stream()));
+    if (site_list) {
+        CK(cudaMemsetAsync(d_allow.p, 0, R, stream()));
+        if (site_list_len) {
+            d_list.upload(site_list, site_list_len);
+            fm::fm_k_hap_allow<<<(uint32_t)((site_list_len + 255) / 256), 256, 0, stream()>>>(d_list.p, site_list_len,
+                                                                                             hs.v_lo, R, d_allow.p);
+            CK(cudaGetLastError());
+            g_launches++;
+        }
+    }
     fm::fm_k_hap_site_stats<<<(R + 7) / 8, 256, 0, stream()>>>(hs.cells, hs.d_off.p, n, hs.v_lo, R, min_maf,
-                                                              max_missing, hs.d_alt.p, hs.d_called.p, d_keep.p,
-                                                              d_counts.p + 1);
+                                                              max_missing, site_list ? d_allow.p : nullptr, hs.d_alt.p,
+                                                              hs.d_called.p, d_keep.p, d_counts.p + 1);
     CK(cudaGetLastError());
     g_launches++;
     size_t tmp_bytes = 0;
@@ -5734,7 +5752,7 @@ fm_status fm_haplotype_pca(fm_matrix *m, const uint64_t *sample_idx, const uint8
             FM_NVTX("fm_haplotype_pca: site statistics");
             Timer tm;
             select_hap_sites(m, membership_offsets(m, sample_idx, side, n_in), prm->has_region, prm->region_start,
-                             prm->region_end, prm->min_maf, prm->max_missing, tm, hs);
+                             prm->region_end, prm->min_maf, prm->max_missing, prm->site_list, prm->site_list_len, tm, hs);
             d_u.alloc(2 * (size_t)std::max<uint32_t>(hs.M, 1));
             if (hs.M) {
                 CK(cudaMemsetAsync(d_total.p, 0, 8, stream()));
@@ -5914,6 +5932,97 @@ fm_status fm_haplotype_pca(fm_matrix *m, const uint64_t *sample_idx, const uint8
 // copied to the caller on a side stream, so device memory is the planes plus two slabs whatever M * window is.
 constexpr size_t kLdSlabBytes = (size_t)64 << 20;
 
+// Argument checks shared by fm_haplotype_ld and fm_haplotype_ld_prune (same order and messages); returns the
+// haplotype offsets.
+static std::vector<uint32_t> ld_arguments(fm_matrix *m, const uint64_t *sample_idx, const uint8_t *side, size_t n_in,
+                                          const fm_ld_params *prm) {
+    if (n_in && (!sample_idx || !side)) fail(FM_ERR_INVALID_ARG, "haplotype arrays are NULL");
+    if (prm->window == 0) fail(FM_ERR_INVALID_ARG, "window must be at least 1");
+    if (!(prm->min_maf >= 0.0 && prm->min_maf <= 0.5)) fail(FM_ERR_INVALID_ARG, "min_maf must lie in [0, 0.5]");
+    if (!(prm->max_missing >= 0.0 && prm->max_missing < 1.0)) fail(FM_ERR_INVALID_ARG, "max_missing must lie in [0, 1)");
+    require_cell_rows(m, "haplotype LD calls");
+    if (prm->max_distance >= 0 && !m->sorted)
+        fail(FM_ERR_UNSUPPORTED, "max_distance needs variant positions sorted ascending");
+    set_dev(m);
+    std::vector<uint32_t> off = membership_offsets(m, sample_idx, side, n_in);
+    if (off.size() >= (1u << 26)) fail(FM_ERR_INVALID_ARG, "haplotype LD supports fewer than 2^26 haplotypes");
+    return off;
+}
+
+// Step 1 of haplotype LD and LD pruning: site statistics and kept-site list (the filters of haplotype PCA), the kept
+// sites' alt counts and positions (stats_ms), the kept rows on the host and the number of pairs under the rule.
+struct LdSites {
+    HapSites hs;
+    DevBuf<uint32_t> d_kalt;
+    DevBuf<int64_t> d_kpos;
+    std::vector<uint32_t> kh;
+    uint64_t pairs = 0;
+};
+
+static void ld_sites(const fm_matrix *m, std::vector<uint32_t> off, const fm_ld_params *prm, LdSites &ls,
+                     float &stats_ms) {
+    HapSites &hs = ls.hs;
+    {
+        FM_NVTX("haplotype LD: site statistics");
+        Timer tm;
+        select_hap_sites(m, std::move(off), prm->has_region, prm->region_start, prm->region_end, prm->min_maf,
+                         prm->max_missing, prm->site_list, prm->site_list_len, tm, hs);
+        ls.d_kalt.alloc(std::max<uint32_t>(hs.M, 1));
+        ls.d_kpos.alloc(std::max<uint32_t>(hs.M, 1));
+        if (hs.M) {
+            fm::fm_k_ld_sites<<<(hs.M + 255) / 256, 256, 0, stream()>>>(hs.d_kept.p, hs.M, hs.v_lo, hs.d_alt.p, m->d_pos,
+                                                                      ls.d_kalt.p, ls.d_kpos.p);
+            CK(cudaGetLastError());
+            g_launches++;
+        }
+        tm.stop();
+        stats_ms = tm.ms();
+    }
+    const uint32_t M = hs.M;
+    const uint64_t window = prm->window;
+    ls.kh.resize(M);
+    hs.d_kept.download(ls.kh.data(), M);
+    CK(cudaStreamSynchronize(stream()));
+    // pairs under the rule: (i, i + d), 1 <= d <= window, i + d < M, within max_distance when it is set
+    uint64_t pairs = 0;
+    if (prm->max_distance < 0) {
+        for (uint64_t i = 0; i < M; ++i) pairs += std::min<uint64_t>(window, M - 1 - i);
+    } else {
+        uint64_t j = 0;
+        for (uint64_t i = 0; i < M; ++i) {
+            j = std::max(j, i);
+            while (j + 1 < M && j + 1 - i <= window && m->pos[ls.kh[j + 1]] - m->pos[ls.kh[i]] <= prm->max_distance) ++j;
+            pairs += j - i;
+        }
+    }
+    ls.pairs = pairs;
+}
+
+// Step 3: site-major planes of the kept sites (a called plane only when some kept site has a missing cell), M >= 1.
+static fm::PwLayout ld_planes(const fm_matrix *m, const LdSites &ls, DevBuf<uint32_t> &d_planes, uint32_t &n_chunks,
+                              float &planes_ms) {
+    const HapSites &hs = ls.hs;
+    const uint32_t n = hs.n, M = hs.M;
+    const uint32_t n_words = (n + 31) / 32;
+    n_chunks = (n_words + fm::kPwKT - 1) / fm::kPwKT;
+    const fm::PwLayout L{(M + fm::kPwBlk - 1) / fm::kPwBlk, hs.incomplete ? 2u : 1u};
+    const size_t plane_words = (size_t)n_chunks * L.n_blk * L.tile_words();
+    d_planes.alloc(std::max<size_t>(plane_words, 1));
+    FM_NVTX("haplotype LD: planes");
+    Timer tm;
+    tm.start();
+    if (plane_words) {
+        CK(cudaMemsetAsync(d_planes.p, 0, plane_words * 4, stream()));
+        const uint32_t grid = transpose_grid(m, (uint64_t)((M + 31) / 32) * n_words);
+        fm::fm_k_ld_planes<<<grid, 256, 0, stream()>>>(hs.cells, hs.d_off.p, n, hs.d_kept.p, M, n_words, L, d_planes.p);
+        CK(cudaGetLastError());
+        g_launches++;
+    }
+    tm.stop();
+    planes_ms = tm.ms();
+    return L;
+}
+
 fm_status fm_haplotype_ld(fm_matrix *m, const uint64_t *sample_idx, const uint8_t *side, size_t n_in,
                           const fm_ld_params *prm, uint32_t *hap_off_out, uint64_t *kept_out, size_t site_capacity,
                           float *r2, float *dprime, size_t pair_capacity, fm_ld_info *info) {
@@ -5923,58 +6032,18 @@ fm_status fm_haplotype_ld(fm_matrix *m, const uint64_t *sample_idx, const uint8_
         require_device();
         if (!m || !prm || !info) fail(FM_ERR_INVALID_ARG, "matrix, params or info is NULL");
         std::memset(info, 0, sizeof(*info));
-        if (n_in && (!sample_idx || !side)) fail(FM_ERR_INVALID_ARG, "haplotype arrays are NULL");
-        if (prm->window == 0) fail(FM_ERR_INVALID_ARG, "window must be at least 1");
-        if (!(prm->min_maf >= 0.0 && prm->min_maf <= 0.5)) fail(FM_ERR_INVALID_ARG, "min_maf must lie in [0, 0.5]");
-        if (!(prm->max_missing >= 0.0 && prm->max_missing < 1.0)) fail(FM_ERR_INVALID_ARG, "max_missing must lie in [0, 1)");
-        require_cell_rows(m, "haplotype LD calls");
-        if (prm->max_distance >= 0 && !m->sorted)
-            fail(FM_ERR_UNSUPPORTED, "max_distance needs variant positions sorted ascending");
-        set_dev(m);
-        std::vector<uint32_t> off = membership_offsets(m, sample_idx, side, n_in);
-        if (off.size() >= (1u << 26)) fail(FM_ERR_INVALID_ARG, "haplotype LD supports fewer than 2^26 haplotypes");
+        std::vector<uint32_t> off = ld_arguments(m, sample_idx, side, n_in, prm);
         const uint64_t window = prm->window;
 
-        // 1. site statistics and kept-site list (the filters of haplotype PCA) and the kept sites' alt counts and
-        // positions
-        HapSites hs;
-        DevBuf<uint32_t> d_kalt;
-        DevBuf<int64_t> d_kpos;
-        {
-            FM_NVTX("fm_haplotype_ld: site statistics");
-            Timer tm;
-            select_hap_sites(m, std::move(off), prm->has_region, prm->region_start, prm->region_end, prm->min_maf,
-                             prm->max_missing, tm, hs);
-            d_kalt.alloc(std::max<uint32_t>(hs.M, 1));
-            d_kpos.alloc(std::max<uint32_t>(hs.M, 1));
-            if (hs.M) {
-                fm::fm_k_ld_sites<<<(hs.M + 255) / 256, 256, 0, stream()>>>(hs.d_kept.p, hs.M, hs.v_lo, hs.d_alt.p, m->d_pos,
-                                                                          d_kalt.p, d_kpos.p);
-                CK(cudaGetLastError());
-                g_launches++;
-            }
-            tm.stop();
-            info->stats_ms = tm.ms();
-        }
+        // 1. site statistics, kept-site list, pairs
+        LdSites ls;
+        ld_sites(m, std::move(off), prm, ls, info->stats_ms);
+        const HapSites &hs = ls.hs;
         const uint32_t n = hs.n, M = hs.M;
-        std::vector<uint32_t> kh(M);
-        hs.d_kept.download(kh.data(), M);
-        CK(cudaStreamSynchronize(stream()));
-        // pairs under the rule: (i, i + d), 1 <= d <= window, i + d < M, within max_distance when it is set
-        uint64_t pairs = 0;
-        if (prm->max_distance < 0) {
-            for (uint64_t i = 0; i < M; ++i) pairs += std::min<uint64_t>(window, M - 1 - i);
-        } else {
-            uint64_t j = 0;
-            for (uint64_t i = 0; i < M; ++i) {
-                j = std::max(j, i);
-                while (j + 1 < M && j + 1 - i <= window && m->pos[kh[j + 1]] - m->pos[kh[i]] <= prm->max_distance) ++j;
-                pairs += j - i;
-            }
-        }
+        const std::vector<uint32_t> &kh = ls.kh;
         info->n_haplotypes = n;
         info->n_sites = M;
-        info->pairs = pairs;
+        info->pairs = ls.pairs;
         info->called_plane = hs.incomplete != 0;
         if (hap_off_out && n) std::memcpy(hap_off_out, hs.off.data(), (size_t)n * 4);
 
@@ -5993,26 +6062,11 @@ fm_status fm_haplotype_ld(fm_matrix *m, const uint64_t *sample_idx, const uint8_
             return;
         }
 
-        // 3. site-major planes of the kept sites (a called plane only when some kept site has a missing cell)
+        // 3. site-major planes of the kept sites
         const bool hc = hs.incomplete != 0;
-        const uint32_t n_words = (n + 31) / 32, n_chunks = (n_words + fm::kPwKT - 1) / fm::kPwKT;
-        const fm::PwLayout L{(M + fm::kPwBlk - 1) / fm::kPwBlk, hc ? 2u : 1u};
-        const size_t plane_words = (size_t)n_chunks * L.n_blk * L.tile_words();
-        DevBuf<uint32_t> d_planes(std::max<size_t>(plane_words, 1));
-        {
-            FM_NVTX("fm_haplotype_ld: planes");
-            Timer tm;
-            tm.start();
-            if (plane_words) {
-                CK(cudaMemsetAsync(d_planes.p, 0, plane_words * 4, stream()));
-                const uint32_t grid = transpose_grid(m, (uint64_t)((M + 31) / 32) * n_words);
-                fm::fm_k_ld_planes<<<grid, 256, 0, stream()>>>(hs.cells, hs.d_off.p, n, hs.d_kept.p, M, n_words, L, d_planes.p);
-                CK(cudaGetLastError());
-                g_launches++;
-            }
-            tm.stop();
-            info->planes_ms = tm.ms();
-        }
+        DevBuf<uint32_t> d_planes;
+        uint32_t n_chunks = 0;
+        const fm::PwLayout L = ld_planes(m, ls, d_planes, n_chunks, info->planes_ms);
 
         // 4. banded tiles, slab by slab; slab s + 1 is computed while slab s is copied out
         const uint32_t outs = dprime ? 2u : 1u;
@@ -6023,7 +6077,7 @@ fm_status fm_haplotype_ld(fm_matrix *m, const uint64_t *sample_idx, const uint8_
         const uint32_t n_slabs = (L.n_blk + rb_per_slab - 1) / rb_per_slab;
         const size_t slab_cells = (size_t)std::min<uint64_t>(M, (uint64_t)rb_per_slab * fm::kPwBlk) * window;
         const size_t smem = L.ring_bytes();
-        auto kern = hc ? fm::fm_k_ld_band<true> : fm::fm_k_ld_band<false>;
+        auto kern = hc ? fm::fm_k_ld_band<true, false> : fm::fm_k_ld_band<false, false>;
         CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         DevBuf<float> d_slab[2];
         for (int b = 0; b < (n_slabs > 1 ? 2 : 1); ++b) d_slab[b].alloc(slab_cells * outs);
@@ -6051,8 +6105,8 @@ fm_status fm_haplotype_ld(fm_matrix *m, const uint64_t *sample_idx, const uint8_
             float *buf = d_slab[s % 2].p;
             CK(cudaEventRecord(band0[s], stream()));
             kern<<<(uint32_t)(nrb * tpr), (fm::kLdConsumerWarps + 1) * 32, smem, stream()>>>(
-                d_planes.p, L, n_chunks, n, M, (uint32_t)window, prm->max_distance, rb0, (uint32_t)tpr, d_kalt.p, d_kpos.p,
-                buf, dprime ? buf + slab_cells : nullptr);
+                d_planes.p, L, n_chunks, n, M, (uint32_t)window, prm->max_distance, rb0, (uint32_t)tpr, ls.d_kalt.p,
+                ls.d_kpos.p, buf, dprime ? buf + slab_cells : nullptr, fm::LdBits{});
             CK(cudaGetLastError());
             g_launches++;
             CK(cudaEventRecord(band1[s], stream()));
@@ -6082,6 +6136,124 @@ fm_status fm_haplotype_ld(fm_matrix *m, const uint64_t *sample_idx, const uint8_
             CK(cudaEventElapsedTime(&t, copy0[s], copy1[s]));
             info->copy_ms += t;
         }
+        info->total_ms = (float)ms_since(t_call);
+    });
+}
+
+// ------------------------------------------------------------------------------------ haplotype LD pruning
+// The forward bit rows of all kept sites stay resident at once; beyond this many bytes the call fails loudly.
+constexpr uint64_t kLdPruneBitBytes = 8ull << 30;
+
+fm_status fm_haplotype_ld_prune(fm_matrix *m, const uint64_t *sample_idx, const uint8_t *side, size_t n_in,
+                                const fm_ld_params *prm, double r2_threshold, uint32_t *hap_off_out, uint64_t *kept_out,
+                                uint64_t *retained_out, size_t site_capacity, fm_ld_prune_info *info) {
+    return guarded([&] {
+        FM_NVTX("fm_haplotype_ld_prune");
+        const auto t_call = std::chrono::steady_clock::now();
+        require_device();
+        if (!m || !prm || !info) fail(FM_ERR_INVALID_ARG, "matrix, params or info is NULL");
+        std::memset(info, 0, sizeof(*info));
+        std::vector<uint32_t> off = ld_arguments(m, sample_idx, side, n_in, prm);
+        if (!(r2_threshold >= 0.0 && r2_threshold <= 1.0)) fail(FM_ERR_INVALID_ARG, "r2_threshold must lie in [0, 1]");
+        const uint64_t window = prm->window;
+
+        // 1. site statistics, kept-site list, pairs (those of fm_haplotype_ld)
+        LdSites ls;
+        ld_sites(m, std::move(off), prm, ls, info->stats_ms);
+        const HapSites &hs = ls.hs;
+        const uint32_t n = hs.n, M = hs.M;
+        info->n_haplotypes = n;
+        info->n_sites = M;
+        info->pairs = ls.pairs;
+        info->called_plane = hs.incomplete != 0;
+        if (hap_off_out && n) std::memcpy(hap_off_out, hs.off.data(), (size_t)n * 4);
+
+        // 2. capacity (a too small one leaves the counts in info so that the caller can retry) and the bit-row limit
+        char where[112];
+        snprintf(where, sizeof(where), " (n = %u haplotypes, M = %u kept sites, window = %llu)", n, M,
+                 (unsigned long long)window);
+        if (M > site_capacity)
+            fail(FM_ERR_INVALID_ARG, std::string("site capacity too small: info->n_sites holds the number needed") + where);
+        if (M && !retained_out) fail(FM_ERR_INVALID_ARG, "retained_sites is required");
+        if (kept_out)
+            for (uint32_t j = 0; j < M; ++j) kept_out[j] = ls.kh[j];
+        if (M == 0) {
+            info->total_ms = (float)ms_since(t_call);
+            return;
+        }
+        const uint64_t w = std::min<uint64_t>(window, M - 1);
+        const uint32_t row_words = (uint32_t)std::max<uint64_t>(1, (w + 31) / 32);
+        if ((uint64_t)M * row_words * 4 > kLdPruneBitBytes)
+            fail(FM_ERR_UNSUPPORTED, std::string("the linked-pair bit rows of all kept sites exceed 8 GiB") + where);
+        const uint64_t tpr = (window + fm::kPwBlk - 1) / fm::kPwBlk + 1;
+        const uint32_t n_blk = (M + fm::kPwBlk - 1) / fm::kPwBlk;
+        if (tpr * n_blk >= (1ull << 31)) fail(FM_ERR_UNSUPPORTED, std::string("window too large for one launch") + where);
+
+        // 3. site-major planes of the kept sites
+        const bool hc = hs.incomplete != 0;
+        DevBuf<uint32_t> d_planes;
+        uint32_t n_chunks = 0;
+        const fm::PwLayout L = ld_planes(m, ls, d_planes, n_chunks, info->planes_ms);
+
+        // 4. banded tiles, all at once, into the forward bit rows of every kept site
+        const size_t bit_words = (size_t)M * row_words;
+        DevBuf<uint32_t> d_bits(bit_words), d_nret(1);
+        DevBuf<unsigned long long> d_linked(1);
+        const size_t smem = L.ring_bytes();
+        auto kern = hc ? fm::fm_k_ld_band<true, true> : fm::fm_k_ld_band<false, true>;
+        CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        {
+            FM_NVTX("fm_haplotype_ld_prune: band");
+            Timer tm;
+            CK(cudaMemsetAsync(d_bits.p, 0, bit_words * 4, stream()));
+            CK(cudaMemsetAsync(d_linked.p, 0, 8, stream()));
+            tm.start();
+            kern<<<(uint32_t)(n_blk * tpr), (fm::kLdConsumerWarps + 1) * 32, smem, stream()>>>(
+                d_planes.p, L, n_chunks, n, M, (uint32_t)window, prm->max_distance, 0u, (uint32_t)tpr, ls.d_kalt.p,
+                ls.d_kpos.p, nullptr, nullptr, fm::LdBits{r2_threshold, row_words, d_bits.p, d_linked.p});
+            CK(cudaGetLastError());
+            g_launches++;
+            tm.stop();
+            info->band_launches = 1;
+            info->band_ms = tm.ms();
+        }
+
+        // 5. the greedy scan (one CTA) and the compaction of the retained matrix rows
+        uint32_t ring_words = 32;
+        while (ring_words < row_words + 1) ring_words *= 2;
+        const size_t scan_smem = (size_t)ring_words * 4;
+        CK(cudaFuncSetAttribute(fm::fm_k_ld_prune_scan, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)scan_smem));
+        DevBuf<uint8_t> d_flags(M);
+        DevBuf<uint32_t> d_ret(M);
+        {
+            FM_NVTX("fm_haplotype_ld_prune: scan");
+            Timer tm;
+            tm.start();
+            fm::fm_k_ld_prune_scan<<<1, fm::kLdScanThreads, scan_smem, stream()>>>(d_bits.p, M, row_words, ring_words - 1,
+                                                                                 d_flags.p, d_nret.p);
+            CK(cudaGetLastError());
+            g_launches++;
+            tm.stop();
+            info->scan_ms = tm.ms();
+        }
+        size_t tmp_bytes = 0;
+        auto select = [&](void *tmp) {  // a null `tmp` only sizes it
+            CK(cub::DeviceSelect::Flagged(tmp, tmp_bytes, hs.d_kept.p, d_flags.p, d_ret.p, d_nret.p, (int64_t)M, stream()));
+        };
+        select(nullptr);
+        DevBuf<uint8_t> d_tmp(std::max<size_t>(tmp_bytes, 16));
+        select(d_tmp.p);
+        uint32_t n_ret = 0;
+        unsigned long long linked = 0;
+        d_nret.download(&n_ret, 1);
+        d_linked.download(&linked, 1);
+        CK(cudaStreamSynchronize(stream()));
+        std::vector<uint32_t> rh(n_ret);
+        d_ret.download(rh.data(), n_ret);
+        CK(cudaStreamSynchronize(stream()));
+        for (uint32_t j = 0; j < n_ret; ++j) retained_out[j] = rh[j];
+        info->linked_pairs = linked;
+        info->n_retained = n_ret;
         info->total_ms = (float)ms_since(t_call);
     });
 }

@@ -31,10 +31,11 @@ struct HapCells {
 };
 
 // Site statistics: one warp per site of [v_lo, v_lo + n_sites); counts over the n selected cells and the keep flag.
-// *incomplete |= 1 when a kept site has a missing cell among the n (the callers then build a called plane).
+// *incomplete |= 1 when a kept site has a missing cell among the n (the callers then build a called plane).  `allow`
+// (nullable, one flag per site of the range) limits the kept sites to a caller's site list.
 __global__ void __launch_bounds__(256)
 fm_k_hap_site_stats(HapCells cells, const uint32_t *__restrict__ off, uint32_t n, uint32_t v_lo, uint32_t n_sites,
-                    double min_maf, double max_missing, uint32_t *__restrict__ alt_out,
+                    double min_maf, double max_missing, const uint8_t *__restrict__ allow, uint32_t *__restrict__ alt_out,
                     uint32_t *__restrict__ called_out, uint8_t *__restrict__ keep_out, uint32_t *__restrict__ incomplete) {
     const uint32_t lane = threadIdx.x & 31;
     const uint32_t r = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -57,11 +58,21 @@ fm_k_hap_site_stats(HapCells cells, const uint32_t *__restrict__ off, uint32_t n
     if (lane) return;
     const uint32_t minor = min(alt, called - alt);
     const bool keep = other == 0 && alt > 0 && alt < called && (double)(n - called) <= max_missing * (double)n &&
-                      (double)minor >= min_maf * (double)called;
+                      (double)minor >= min_maf * (double)called && (!allow || allow[r]);
     alt_out[r] = alt;
     called_out[r] = called;
     keep_out[r] = keep;
     if (keep && called < n) atomicOr(incomplete, 1u);
+}
+
+// allow[list[i] - v_lo] = 1 for the entries of a site list that fall in [v_lo, v_lo + n_sites) (allow cleared first).
+__global__ void __launch_bounds__(256)
+fm_k_hap_allow(const uint64_t *__restrict__ list, uint64_t len, uint32_t v_lo, uint32_t n_sites,
+               uint8_t *__restrict__ allow) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= len) return;
+    const uint64_t v = list[i];
+    if (v >= v_lo && v - v_lo < n_sites) allow[v - v_lo] = 1;
 }
 
 }  // namespace fm

@@ -584,6 +584,9 @@ fm_status fm_pairwise_differences(fm_matrix *m, size_t n_samples, uint32_t *diff
  *               is neither 0 nor 1.  Site v is kept when other_v == 0, 0 < alt_v < called_v,
  *               (n - called_v) <= max_missing * n and min(alt_v, called_v - alt_v) >= min_maf * called_v (FP64).
  *               M = number of kept sites; kept_sites [site_capacity] (may be NULL) receives their matrix rows.
+ *   site list   site_list (NULL: none) of site_list_len matrix rows, strictly ascending and each < n_variants
+ *               (else FM_ERR_INVALID_ARG): only the listed rows are candidates, the region and the filters apply on
+ *               top.  G is keyed by matrix row, so a list gives the PCA of that subset of rows.
  *   Z           p_v = alt_v / called_v, s_v = 1 / sqrt(p_v (1 - p_v)); Z[i, v] = s_v (x_iv - p_v) for a called cell,
  *               0 for a missing one.  T = ||Z||_F^2 = sum of called_v over the kept sites (info->total_variance).
  *   iteration   l = min(k + oversampling, n, M) <= 64.  G[v, c] = +1 when bit 63 of fm_mix(seed, v, c) is clear,
@@ -605,6 +608,8 @@ typedef struct {
     uint64_t seed;
     int has_region;
     int64_t region_start, region_end;
+    const uint64_t *site_list; /* NULL: every row (see "site list" above) */
+    uint64_t site_list_len;
 } fm_pca_params;
 typedef struct {
     uint64_t n_haplotypes, n_sites, rank; /* n, M, l */
@@ -626,7 +631,8 @@ fm_status fm_haplotype_pca(fm_matrix *m, const uint64_t *sample_idx, const uint8
  *               filters them.  Counts are over RAW allele values: other_v == 0, 0 < alt_v < called_v,
  *               (n - called_v) <= max_missing * n, min(alt_v, called_v - alt_v) >= min_maf * called_v (FP64).
  *               M = number of kept sites, in matrix-row order; kept_sites [site_capacity] (may be NULL) receives
- *               their matrix rows.  On a kept site a called cell is 0 or 1.
+ *               their matrix rows.  On a kept site a called cell is 0 or 1.  site_list / site_list_len limit the
+ *               candidates to listed matrix rows exactly as for fm_haplotype_pca.
  *   pairs       the kept-site pairs (i, i + d) with 1 <= d <= window, i + d < M and, when max_distance >= 0,
  *               pos[i + d] - pos[i] <= max_distance.
  *   counts      per pair, over the n haplotypes (integers): c = called at both sites; a = alt at i among the c;
@@ -656,6 +662,8 @@ typedef struct {
     double min_maf, max_missing;
     int has_region;
     int64_t region_start, region_end;
+    const uint64_t *site_list; /* NULL: every row; else strictly ascending matrix rows, as fm_pca_params */
+    uint64_t site_list_len;
 } fm_ld_params;
 typedef struct {
     uint64_t n_haplotypes, n_sites, pairs; /* n, M, pairs under the rule */
@@ -666,6 +674,39 @@ fm_status fm_haplotype_ld(fm_matrix *m, const uint64_t *sample_idx, const uint8_
                           const fm_ld_params *params, uint32_t *haplotype_offsets_or_null,
                           uint64_t *kept_sites_or_null, size_t site_capacity,
                           float *r2, float *dprime_or_null, size_t pair_capacity, fm_ld_info *info);
+
+/* ---- haplotype LD pruning (this project's estimator; DESIGN.md §0 row f10, §3, §4 "LD pruning") ----
+ * Greedy r^2 pruning of the kept sites of fm_haplotype_ld, so that a PCA is not pulled toward LD blocks.  Haplotypes,
+ * kept sites (M, in matrix-row order), pairs, counts and r^2 are exactly those of fm_haplotype_ld for the same params.
+ *   linked      a pair (i, i + d) under the pair rule is linked when its FP64 r^2 -- the value before the float
+ *               rounding, in the operation order above -- is greater than r2_threshold.  A NaN r^2 (c == 0, or a
+ *               site monomorphic among the jointly called) is never linked; equality is not linked.
+ *   greedy      walk the kept sites in order: site j is retained unless some RETAINED site i < j forms a linked pair
+ *               with it (if A-B and B-C are linked and A-C is not, A and C are retained).  This is a sequential
+ *               greedy rule, not plink's --indep-pairwise (which removes by MAF inside sliding windows with a step).
+ *   outputs     retained_sites [site_capacity] receives the n_retained matrix rows of the retained sites, ascending;
+ *               kept_sites [site_capacity] (may be NULL) the M kept rows; haplotype_offsets [n] (may be NULL) the
+ *               haplotype offsets.
+ * r2_threshold must lie in [0, 1] (NaN rejected).  Every decision rests on exact integer counts and one fixed FP64
+ * expression, so the retained set is bit-for-bit reproducible across calls, threads and a plain restatement.
+ * The argument checks, messages and error codes of fm_haplotype_ld apply, then FM_ERR_INVALID_ARG for r2_threshold
+ * outside [0, 1].  When M > site_capacity, info is filled in (n_haplotypes, n_sites, pairs, called_plane) and the
+ * call returns FM_ERR_INVALID_ARG ("capacity too small") so that the caller can retry; retained_sites may be NULL on
+ * such a query.  M == 0 is not an error.  The forward bit rows of all kept sites (ceil(w / 32) u32 words a site,
+ * w = min(window, M - 1)) are resident at once: when M * ceil(w / 32) * 4 bytes exceed 8 GiB the call fails with
+ * FM_ERR_UNSUPPORTED before any band launch.
+ * info: pairs under the rule, linked_pairs, n_retained; called_plane as fm_ld_info; band_launches (1, or 0 when M == 0
+ * or the call failed before the band); stats_ms, planes_ms, band_ms and scan_ms are device events, total_ms the host
+ * time of the whole call. */
+typedef struct {
+    uint64_t n_haplotypes, n_sites, pairs, linked_pairs, n_retained; /* n, M, pairs under the rule, linked, retained */
+    uint32_t called_plane, band_launches;
+    float stats_ms, planes_ms, band_ms, scan_ms, total_ms;
+} fm_ld_prune_info;
+fm_status fm_haplotype_ld_prune(fm_matrix *m, const uint64_t *sample_idx, const uint8_t *side, size_t n,
+                                const fm_ld_params *params, double r2_threshold, uint32_t *haplotype_offsets_or_null,
+                                uint64_t *kept_sites_or_null, uint64_t *retained_sites, size_t site_capacity,
+                                fm_ld_prune_info *info);
 
 /* ---- synthetic cohorts for benchmarks and full-size parity tests ----
  * Fills a device-resident u8 matrix (reference layout) and, when d_missing != NULL, its packed

@@ -29,6 +29,7 @@ pub struct fm_pca_params {
     pub k: u32, pub oversampling: u32, pub power_iterations: u32,
     pub min_maf: f64, pub max_missing: f64, pub seed: u64,
     pub has_region: c_int, pub region_start: i64, pub region_end: i64,
+    pub site_list: *const u64, pub site_list_len: u64, /* null: every row; else strictly ascending matrix rows */
 }
 #[repr(C)]
 #[derive(Default)]
@@ -42,6 +43,7 @@ pub struct fm_ld_params {
     pub window: u32, pub max_distance: i64, /* < 0: none */
     pub min_maf: f64, pub max_missing: f64,
     pub has_region: c_int, pub region_start: i64, pub region_end: i64,
+    pub site_list: *const u64, pub site_list_len: u64, /* as fm_pca_params */
 }
 #[repr(C)]
 #[derive(Default)]
@@ -49,6 +51,13 @@ pub struct fm_ld_info {
     pub n_haplotypes: u64, pub n_sites: u64, pub pairs: u64,
     pub called_plane: u32, pub slabs: u32, pub band_launches: u32,
     pub stats_ms: f32, pub planes_ms: f32, pub band_ms: f32, pub copy_ms: f32, pub total_ms: f32,
+}
+#[repr(C)]
+#[derive(Default)]
+pub struct fm_ld_prune_info {
+    pub n_haplotypes: u64, pub n_sites: u64, pub pairs: u64, pub linked_pairs: u64, pub n_retained: u64,
+    pub called_plane: u32, pub band_launches: u32,
+    pub stats_ms: f32, pub planes_ms: f32, pub band_ms: f32, pub scan_ms: f32, pub total_ms: f32,
 }
 
 extern "C" {
@@ -117,6 +126,11 @@ extern "C" {
     pub fn fm_haplotype_ld(m: *mut fm_matrix, sample_idx: *const u64, side: *const u8, n: usize,
         params: *const fm_ld_params, haplotype_offsets: *mut u32, kept_sites: *mut u64, site_capacity: usize,
         r2: *mut f32, dprime: *mut f32, pair_capacity: usize, info: *mut fm_ld_info) -> c_int;
+    // greedy r^2 pruning of the kept sites of fm_haplotype_ld (new entry point; estimator in include/ferromic_gpu.h);
+    // retained_sites may be NULL on a size query
+    pub fn fm_haplotype_ld_prune(m: *mut fm_matrix, sample_idx: *const u64, side: *const u8, n: usize,
+        params: *const fm_ld_params, r2_threshold: f64, haplotype_offsets: *mut u32, kept_sites: *mut u64,
+        retained_sites: *mut u64, site_capacity: usize, info: *mut fm_ld_prune_info) -> c_int;
     // BGZF (.vcf.gz as bgzip writes it) inflated on the device; fm_vcf_parse_bgzf parses from data_offset on
     pub fn fm_bgzf_inflate(gz: *const u8, n_gz: usize, out: *mut u8, capacity: usize, total_out: *mut u64) -> c_int;
     pub fn fm_vcf_parse_bgzf(gz: *const u8, n_gz: usize, data_offset: u64, chr: *const c_char, regions: *const i64,

@@ -30,12 +30,12 @@ def card():
 
 
 def band_popc(so):
-    """POPC instructions of each fm_k_ld_band instantiation (all in the main loop, unrolled over 2 haplotype words)."""
+    """POPC instructions of each float fm_k_ld_band instantiation (all in the main loop, unrolled over 2 haplotype words)."""
     sass = subprocess.run(["/usr/local/cuda/bin/cuobjdump", "-sass", so], capture_output=True, text=True).stdout
     out = {}
     for part in re.split(r"\n\s*Function : ", sass):
         name = part.split("\n", 1)[0].strip()
-        if name.startswith("_ZN2fm12fm_k_ld_bandILb"):
+        if name.startswith("_ZN2fm12fm_k_ld_bandILb") and "ELb0EEE" in name:  # the float forms, not the bit forms
             out["called_plane" if "ILb1E" in name else "no_called_plane"] = len(re.findall(r"\bPOPC\b", part))
     return out
 
