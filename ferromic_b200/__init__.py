@@ -1,6 +1,6 @@
 """ferromic_b200 -- B200 (sm_100a) implementation of ferromic's per-site population-genetics
 estimators (segregating sites, pi, Watterson theta, per-site pi/theta tracks, Hudson FST/Dxy,
-Weir & Cockerham FST, pairwise sample differences, haplotype PCA, haplotype LD and LD pruning) behind the reference's own Python surface (`import ferromic_b200 as fm`).
+Weir & Cockerham FST, pairwise sample differences, haplotype PCA, haplotype LD, LD pruning and site frequency spectra) behind the reference's own Python surface (`import ferromic_b200 as fm`).
 
 All estimator arithmetic runs in hand-written CUDA kernels through the C-ABI library
 `libferromic_gpu.so` (include/ferromic_gpu.h); there is no CPU fallback."""
@@ -14,7 +14,9 @@ from .api import (  # noqa: F401
     HudsonDxyResult,
     HudsonFstResult,
     HudsonFstSite,
+    JointSiteFrequencySpectrumResult,
     Population,
+    SiteFrequencySpectrumResult,
     WcFstResult,
     WcFstSite,
     adjusted_sequence_length,
@@ -26,12 +28,14 @@ from .api import (  # noqa: F401
     hudson_fst_sites,
     hudson_fst_with_sites,
     inversion_allele_frequency,
+    joint_site_frequency_spectrum,
     pairwise_difference_arrays,
     pairwise_differences,
     nucleotide_diversity,
     per_site_diversity,
     per_site_diversity_arrays,
     segregating_sites,
+    site_frequency_spectrum,
     watterson_theta,
     wc_fst,
     wc_fst_components,

@@ -93,6 +93,29 @@ class LdPruneInfo(C.Structure):
         (f, C.c_float) for f in ("stats_ms", "planes_ms", "band_ms", "scan_ms", "total_ms")]
 
 
+class SfsParams(C.Structure):
+    _fields_ = [("projection", C.c_uint32), ("folded", C.c_int), ("has_region", C.c_int), ("region_start", C.c_int64),
+                ("region_end", C.c_int64), ("site_list", C.c_void_p), ("site_list_len", C.c_uint64)]
+
+
+class SfsInfo(C.Structure):
+    _fields_ = [(f, C.c_uint64) for f in ("n_haplotypes", "projection", "candidates", "n_sites", "projected_out",
+                                          "non_biallelic")] + [
+        (f, C.c_float) for f in ("counts_ms", "spectrum_ms", "total_ms")]
+
+
+class JointSfsParams(C.Structure):
+    _fields_ = [("projection1", C.c_uint32), ("projection2", C.c_uint32), ("folded", C.c_int), ("has_region", C.c_int),
+                ("region_start", C.c_int64), ("region_end", C.c_int64), ("site_list", C.c_void_p),
+                ("site_list_len", C.c_uint64)]
+
+
+class JointSfsInfo(C.Structure):
+    _fields_ = [(f, C.c_uint64) for f in ("n_haplotypes1", "n_haplotypes2", "projection1", "projection2", "candidates",
+                                          "n_sites", "projected_out", "non_biallelic", "incidences")] + [
+        ("passes", C.c_uint32)] + [(f, C.c_float) for f in ("counts_ms", "spectrum_ms", "total_ms")]
+
+
 EXPORTS = [
     "fm_last_error", "fm_version", "fm_device_count", "fm_set_device", "fm_set_devices", "fm_get_devices", "fm_synchronize", "fm_trim_pool",
     "fm_matrix_create", "fm_matrix_create_inband", "fm_matrix_create_device", "fm_matrix_retain", "fm_matrix_release",
@@ -109,7 +132,7 @@ EXPORTS = [
     "fm_vcf_batch_release", "fm_synth_fill", "fm_timings_reset", "fm_timings_get", "fm_bench_diversity",
     "fm_pairwise_differences", "fm_bgzf_inflate", "fm_vcf_parse_bgzf", "fm_bgzf_deflate_bound", "fm_bgzf_deflate",
     "fm_falsta_tracks_bgzf", "fm_haplotype_pca", "fm_haplotype_ld",
-    "fm_haplotype_ld_prune",
+    "fm_haplotype_ld_prune", "fm_site_frequency_spectrum", "fm_joint_site_frequency_spectrum",
 ]
 
 _lib = None
@@ -227,6 +250,10 @@ def lib() -> C.CDLL:
     L.fm_haplotype_ld.argtypes = [vp, vp, vp, sz, C.POINTER(LdParams), vp, vp, sz, vp, vp, sz, C.POINTER(LdInfo)]
     L.fm_haplotype_ld_prune.argtypes = [vp, vp, vp, sz, C.POINTER(LdParams), dbl, vp, vp, vp, sz,
                                         C.POINTER(LdPruneInfo)]
+    L.fm_site_frequency_spectrum.argtypes = [vp, vp, vp, sz, C.POINTER(SfsParams), vp, sz, vp, vp, sz, vp, vp, vp, vp,
+                                             vp, C.POINTER(SfsInfo)]
+    L.fm_joint_site_frequency_spectrum.argtypes = [vp, vp, vp, sz, vp, vp, sz, C.POINTER(JointSfsParams), vp, sz,
+                                                   C.POINTER(JointSfsInfo)]
     for name in EXPORTS:
         fn = getattr(L, name)
         if name not in ("fm_last_error", "fm_version"):

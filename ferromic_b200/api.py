@@ -1159,6 +1159,146 @@ def haplotype_ld_prune(variants, haplotypes=None, r2_threshold=0.2, window=100, 
                                   int(info.n_sites), int(info.pairs), int(info.linked_pairs))
 
 
+class SiteFrequencySpectrumResult:
+    """Projected site frequency spectrum of a haplotype set (fm_site_frequency_spectrum).  `spectrum` has m + 1 bins
+    (`projection` = m), or shape [n_windows, m + 1] with windows; `n_sites`, `segregating_sites`, `theta_pi`,
+    `theta_watterson` and `tajimas_d` are scalars without windows and per-window arrays with them.  θ_π and θ_W are
+    window totals (divide by a length for per-bp values); `projected_out` and `non_biallelic` count the candidate
+    rows left out."""
+    __slots__ = ("haplotypes", "projection", "spectrum", "n_sites", "projected_out", "non_biallelic",
+                 "segregating_sites", "theta_pi", "theta_watterson", "tajimas_d")
+
+    def __init__(self, haplotypes, projection, spectrum, n_sites, projected_out, non_biallelic, segregating_sites,
+                 theta_pi, theta_watterson, tajimas_d):
+        self.haplotypes = haplotypes
+        self.projection = projection
+        self.spectrum = spectrum
+        self.n_sites = n_sites
+        self.projected_out = projected_out
+        self.non_biallelic = non_biallelic
+        self.segregating_sites = segregating_sites
+        self.theta_pi = theta_pi
+        self.theta_watterson = theta_watterson
+        self.tajimas_d = tajimas_d
+
+    def __repr__(self):
+        return (f"SiteFrequencySpectrumResult(n_haplotypes={len(self.haplotypes)}, projection={self.projection}, "
+                f"n_sites={self.n_sites}, tajimas_d={self.tajimas_d})")
+
+
+class JointSiteFrequencySpectrumResult:
+    """Joint site frequency spectrum of two haplotype sets (fm_joint_site_frequency_spectrum): `spectrum` [m1 + 1,
+    m2 + 1] with `projection` = (m1, m2)."""
+    __slots__ = ("haplotypes1", "haplotypes2", "projection", "spectrum", "n_sites", "projected_out", "non_biallelic")
+
+    def __init__(self, haplotypes1, haplotypes2, projection, spectrum, n_sites, projected_out, non_biallelic):
+        self.haplotypes1 = haplotypes1
+        self.haplotypes2 = haplotypes2
+        self.projection = projection
+        self.spectrum = spectrum
+        self.n_sites = n_sites
+        self.projected_out = projected_out
+        self.non_biallelic = non_biallelic
+
+    def __repr__(self):
+        return (f"JointSiteFrequencySpectrumResult(projection={self.projection}, n_sites={self.n_sites})")
+
+
+def _projection(x):
+    if x is None:
+        return 0
+    if not 1 <= int(x) < 2 ** 32:
+        raise ValueError("projection must lie in [1, 2^32)")
+    return int(x)
+
+
+def _matrix_sfs(m: _Matrix, haplotypes, projection=None, region=None, windows=None, folded=False, sites=None):
+    """fm_site_frequency_spectrum on a device matrix: dict of offsets, spectrum [n_windows, m + 1] (one row without
+    windows), window_sites, segregating, theta_pi, theta_w, tajimas_d (arrays over the windows) and the call's info
+    struct.  A size query learns m first.  windows: [k, 2] 0-based inclusive position pairs."""
+    idx, side, reg, rows = _haplotype_args(haplotypes, region, sites)
+    n_in = len(haplotypes)
+    prm = _lib.SfsParams(_projection(projection), int(bool(folded)), *reg, *_site_list(rows))
+    win = None if windows is None else np.ascontiguousarray(np.asarray(windows, dtype=np.int64).reshape(-1, 2))
+    nw = 0 if win is None else len(win)
+    info = _lib.SfsInfo()
+    L = lib()
+    st = L.fm_site_frequency_spectrum(m.handle, _ptr(idx), _ptr(side), n_in, C.byref(prm), _ptr(win), nw, None, None,
+                                      0, None, None, None, None, None, C.byref(info))
+    if st != _lib.FM_OK and not (st == _lib.FM_ERR_INVALID_ARG and b"capacity too small" in L.fm_last_error()):
+        check(st)
+    bins, k = int(info.projection) + 1, max(nw, 1)
+    off = np.zeros(max(n_in, 1), dtype=np.uint32)
+    spec = np.zeros(k * bins, dtype=np.float64)
+    ws = np.zeros(k, dtype=np.uint64)
+    seg, tp, tw, td = (np.zeros(k, dtype=np.float64) for _ in range(4))
+    check(L.fm_site_frequency_spectrum(m.handle, _ptr(idx), _ptr(side), n_in, C.byref(prm), _ptr(win), nw, _ptr(off),
+                                       _ptr(spec), spec.size, _ptr(ws), _ptr(seg), _ptr(tp), _ptr(tw), _ptr(td),
+                                       C.byref(info)))
+    n = int(info.n_haplotypes)
+    return dict(offsets=off[:n].copy(), spectrum=spec.reshape(k, bins), window_sites=ws.astype(np.int64),
+                segregating=seg, theta_pi=tp, theta_w=tw, tajimas_d=td, info=info)
+
+
+def _matrix_joint_sfs(m: _Matrix, haplotypes1, haplotypes2, projection=None, region=None, folded=False, sites=None):
+    """fm_joint_site_frequency_spectrum on a device matrix: dict of spectrum [m1 + 1, m2 + 1] and the call's info
+    struct.  projection: None (each set's n) or a pair whose entries may be None."""
+    p1, p2 = (None, None) if projection is None else projection
+    idx1, side1, reg, rows = _haplotype_args(haplotypes1, region, sites)
+    idx2, side2, _, _ = _haplotype_args(haplotypes2, region)
+    prm = _lib.JointSfsParams(_projection(p1), _projection(p2), int(bool(folded)), *reg, *_site_list(rows))
+    info = _lib.JointSfsInfo()
+    L = lib()
+    args = (m.handle, _ptr(idx1), _ptr(side1), len(haplotypes1), _ptr(idx2), _ptr(side2), len(haplotypes2),
+            C.byref(prm))
+    st = L.fm_joint_site_frequency_spectrum(*args, None, 0, C.byref(info))
+    if st != _lib.FM_OK and not (st == _lib.FM_ERR_INVALID_ARG and b"capacity too small" in L.fm_last_error()):
+        check(st)
+    m1, m2 = int(info.projection1), int(info.projection2)
+    spec = np.zeros((m1 + 1) * (m2 + 1), dtype=np.float64)
+    check(L.fm_joint_site_frequency_spectrum(*args, _ptr(spec), spec.size, C.byref(info)))
+    return dict(spectrum=spec.reshape(m1 + 1, m2 + 1), info=info)
+
+
+def site_frequency_spectrum(variants, haplotypes=None, projection=None, region=None, windows=None, folded=False,
+                            sites=None) -> SiteFrequencySpectrumResult:
+    """Allele frequency spectrum of a haplotype set on the GPU, every site with at least `projection` called
+    haplotypes projected to that sample size by the hypergeometric distribution (definition in
+    include/ferromic_gpu.h, fm_site_frequency_spectrum), with S, θ_π, θ_W and Tajima's D of the projected spectrum.
+    haplotypes: (sample, side) pairs, None = every cell of every sample, as haplotype_pca; projection: None = the
+    set's size; region: 0-based inclusive (start, end), None = every variant; windows: 0-based inclusive (start, end)
+    pairs (not with a region); sites: strictly ascending indices into `variants`.  Sites with an allele value other
+    than 0 and 1 among the set's called cells are left out (`non_biallelic`)."""
+    if windows is not None and region is not None:
+        raise ValueError("windows and region are exclusive")
+    vs, m, haps, region = _haplotype_call("site frequency spectrum", variants, haplotypes, region)
+    r = _matrix_sfs(m, haps, projection, region, windows, folded, sites)
+    info = r["info"]
+    one = windows is None
+    pick = (lambda a: a[0]) if one else (lambda a: a)  # noqa: E731
+    return SiteFrequencySpectrumResult(
+        _offset_haplotypes(m, r["offsets"]), int(info.projection), pick(r["spectrum"]),
+        int(r["window_sites"][0]) if one else r["window_sites"], int(info.projected_out), int(info.non_biallelic),
+        float(pick(r["segregating"])) if one else r["segregating"], float(pick(r["theta_pi"])) if one else r["theta_pi"],
+        float(pick(r["theta_w"])) if one else r["theta_w"], float(pick(r["tajimas_d"])) if one else r["tajimas_d"])
+
+
+def joint_site_frequency_spectrum(variants, haplotypes1, haplotypes2, projection=None, region=None, folded=False,
+                                  sites=None) -> JointSiteFrequencySpectrumResult:
+    """Joint allele frequency spectrum of two haplotype sets of the same variants on the GPU (definition in
+    include/ferromic_gpu.h, fm_joint_site_frequency_spectrum): entry [j1, j2] sums, over the sites with at least
+    (m1, m2) called haplotypes in the two sets, the product of the two projected weights.  projection: None or
+    (m1, m2), an entry None = that set's size.  region and sites as site_frequency_spectrum."""
+    vs, m, haps1, region = _haplotype_call("joint site frequency spectrum", variants, haplotypes1, region)
+    haps2 = _parse_haplotypes(haplotypes2)
+    r = _matrix_joint_sfs(m, haps1, haps2, projection, region, folded, sites)
+    info = r["info"]
+    return JointSiteFrequencySpectrumResult(
+        *(sorted({(s, h) for s, h in hs if s < vs.n_samples and (h == 0 or m.P > 1)}) for hs in (haps1, haps2)),
+        (int(info.projection1), int(info.projection2)), r["spectrum"], int(info.n_sites), int(info.projected_out),
+        int(info.non_biallelic))
+
+
 def _opt(value: float, some: int, bit: int):
     return value if (some >> bit) & 1 else None
 

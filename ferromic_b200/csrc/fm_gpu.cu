@@ -13,9 +13,11 @@
 #include "fm_deflate.cuh"
 #include "fm_pca.cuh"
 #include "fm_ld.cuh"
+#include "fm_sfs.cuh"
 
 #include <nvtx3/nvToolsExt.h>
 
+#include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 #include <cub/device/device_select.cuh>
 #include <thrust/iterator/counting_iterator.h>
@@ -5451,14 +5453,31 @@ struct HapSites {
 };
 
 // Starts `tm` at its first device work; the caller stops it after its own per-kept-site kernel.
-static void select_hap_sites(const fm_matrix *m, std::vector<uint32_t> off, int has_region, int64_t region_start,
-                             int64_t region_end, double min_maf, double max_missing, const uint64_t *site_list,
-                             uint64_t site_list_len, Timer &tm, HapSites &hs) {
+// A site list of the haplotype calls: strictly ascending matrix rows, each below the variant count.
+static void check_site_list(const fm_matrix *m, const uint64_t *site_list, uint64_t site_list_len) {
     if (site_list)
         for (uint64_t i = 0; i < site_list_len; ++i) {
             if (site_list[i] >= m->V) fail(FM_ERR_INVALID_ARG, "site_list holds a row beyond the matrix's variants");
             if (i && site_list[i] <= site_list[i - 1]) fail(FM_ERR_INVALID_ARG, "site_list must be strictly ascending");
         }
+}
+
+// d_allow [R] = 1 for the rows of [v_lo, v_lo + R) in the site list (R >= 1), 0 for the others.
+static void site_list_allow(const uint64_t *site_list, uint64_t site_list_len, uint32_t v_lo, uint32_t R,
+                            DevBuf<uint64_t> &d_list, DevBuf<uint8_t> &d_allow) {
+    CK(cudaMemsetAsync(d_allow.p, 0, R, stream()));
+    if (!site_list_len) return;
+    d_list.upload(site_list, site_list_len);
+    fm::fm_k_hap_allow<<<(uint32_t)((site_list_len + 255) / 256), 256, 0, stream()>>>(d_list.p, site_list_len, v_lo, R,
+                                                                                     d_allow.p);
+    CK(cudaGetLastError());
+    g_launches++;
+}
+
+static void select_hap_sites(const fm_matrix *m, std::vector<uint32_t> off, int has_region, int64_t region_start,
+                             int64_t region_end, double min_maf, double max_missing, const uint64_t *site_list,
+                             uint64_t site_list_len, Timer &tm, HapSites &hs) {
+    check_site_list(m, site_list, site_list_len);
     hs.off = std::move(off);
     hs.n = (uint32_t)hs.off.size();
     uint32_t v_hi = (uint32_t)m->V;
@@ -5478,16 +5497,7 @@ static void select_hap_sites(const fm_matrix *m, std::vector<uint32_t> off, int 
     hs.d_off.upload(hs.off.data(), n);
     if (!n || !R) return;
     CK(cudaMemsetAsync(d_counts.p, 0, 8, stream()));
-    if (site_list) {
-        CK(cudaMemsetAsync(d_allow.p, 0, R, stream()));
-        if (site_list_len) {
-            d_list.upload(site_list, site_list_len);
-            fm::fm_k_hap_allow<<<(uint32_t)((site_list_len + 255) / 256), 256, 0, stream()>>>(d_list.p, site_list_len,
-                                                                                             hs.v_lo, R, d_allow.p);
-            CK(cudaGetLastError());
-            g_launches++;
-        }
-    }
+    if (site_list) site_list_allow(site_list, site_list_len, hs.v_lo, R, d_list, d_allow);
     fm::fm_k_hap_site_stats<<<(R + 7) / 8, 256, 0, stream()>>>(hs.cells, hs.d_off.p, n, hs.v_lo, R, min_maf,
                                                               max_missing, site_list ? d_allow.p : nullptr, hs.d_alt.p,
                                                               hs.d_called.p, d_keep.p, d_counts.p + 1);
@@ -6254,6 +6264,377 @@ fm_status fm_haplotype_ld_prune(fm_matrix *m, const uint64_t *sample_idx, const 
         for (uint32_t j = 0; j < n_ret; ++j) retained_out[j] = rh[j];
         info->linked_pairs = linked;
         info->n_retained = n_ret;
+        info->total_ms = (float)ms_since(t_call);
+    });
+}
+
+// ------------------------------------------------------------------------------------ site frequency spectra
+// The joint pass sorts at most this many (tile, row) incidences at once; rows beyond it take further passes, each
+// adding to the entries the previous one left, so the sums keep their row order.
+constexpr uint64_t kSfsIncidenceChunk = 1ull << 27;
+
+// Offsets of a haplotype set of a spectrum call (`which` names the set in messages) and its projection m.
+static std::vector<uint32_t> sfs_set(const fm_matrix *m, const uint64_t *sample_idx, const uint8_t *side, size_t n_in,
+                                     uint32_t projection, const char *which, uint32_t &proj) {
+    if (n_in && (!sample_idx || !side)) fail(FM_ERR_INVALID_ARG, std::string(which) + "haplotype arrays are NULL");
+    std::vector<uint32_t> off = membership_offsets(m, sample_idx, side, n_in);
+    const size_t n = off.size();
+    char where[96];
+    snprintf(where, sizeof(where), " (n = %zu haplotypes, projection = %u)", n, projection);
+    if (n == 0) fail(FM_ERR_INVALID_ARG, std::string(which) + "haplotype set is empty after de-duplication" + where);
+    if (n >= (1u << 26)) fail(FM_ERR_INVALID_ARG, std::string("site frequency spectra support fewer than 2^26 haplotypes") + where);
+    if (projection > n) fail(FM_ERR_INVALID_ARG, std::string(which) + "projection exceeds the number of haplotypes" + where);
+    proj = projection ? projection : (uint32_t)n;
+    return off;
+}
+
+// Step 1 of both spectrum calls: the per-set cell membership, the counting pass over the candidate rows [v_lo, v_lo
+// + R) (one read of each row for one or two sets), the compaction of the contributing rows and their counts.
+struct SfsRows {
+    uint32_t v_lo = 0, R = 0, n_sites = 0;
+    unsigned long long tot[3] = {0, 0, 0};  // candidates, projected_out, non_biallelic
+    DevBuf<uint32_t> d_ci;                  // contributing rows (relative to v_lo), ascending
+    DevBuf<uint2> d_c1, d_c2;               // their (called, alt) per set
+};
+
+static void sfs_rows(const fm_matrix *m, const std::vector<uint32_t> *const *offs, int n_sets, const uint32_t *proj,
+                     const uint64_t *site_list, uint64_t site_list_len, SfsRows &sr, float &counts_ms) {
+    const bool two = n_sets == 2;
+    fm::SfsCells cells{};
+    cells.c = fm::HapCells{m->d_data, m->d_missing, !m->has_missing ? 0u : (m->in_band ? 2u : 1u), (uint64_t)m->stride,
+                           m->packed ? m->d_abits : nullptr, m->packed ? m->d_cbits : nullptr, m->rw};
+    DevBuf<uint8_t> d_memb;
+    DevBuf<uint32_t> d_mask;
+    if (m->packed) {
+        std::vector<uint32_t> mask((size_t)n_sets * m->rw, 0);
+        for (int s = 0; s < n_sets; ++s)
+            for (uint32_t o : *offs[s]) mask[(size_t)s * m->rw + (o >> 5)] |= 1u << (o & 31);
+        d_mask.alloc(std::max<size_t>(mask.size(), 1));
+        d_mask.upload(mask.data(), mask.size());
+        cells.mask = d_mask.p;
+    } else {
+        // 16 copies, one per alignment s of a row start: byte 16 b + t of copy s is the cell 16 b + t - s of the row
+        const uint32_t Lb = (uint32_t)((m->stride + 30) / 16);
+        std::vector<uint8_t> memb((size_t)16 * Lb * 16, 0);
+        for (uint32_t s = 0; s < 16; ++s)
+            for (int k = 0; k < n_sets; ++k)
+                for (uint32_t o : *offs[k]) memb[(size_t)s * Lb * 16 + o + s] |= (uint8_t)(1u << k);
+        d_memb.alloc(memb.size());
+        d_memb.upload(memb.data(), memb.size());
+        cells.memb = d_memb.p;
+        cells.memb_blocks = Lb;
+    }
+    const uint32_t R = sr.R;
+    DevBuf<uint2> d_cnt1(std::max<uint32_t>(R, 1)), d_cnt2(two ? std::max<uint32_t>(R, 1) : 0);
+    DevBuf<uint8_t> d_flag(std::max<uint32_t>(R, 1)), d_allow(site_list ? std::max<uint32_t>(R, 1) : 0);
+    DevBuf<uint64_t> d_list(site_list ? std::max<uint64_t>(site_list_len, 1) : 0);
+    DevBuf<unsigned long long> d_tot(3);
+    DevBuf<uint32_t> d_nsel(1);
+    sr.d_ci.alloc(std::max<uint32_t>(R, 1));
+    Timer tm;
+    tm.start();
+    CK(cudaMemsetAsync(d_tot.p, 0, 3 * 8, stream()));
+    CK(cudaMemsetAsync(d_nsel.p, 0, 4, stream()));
+    if (R) {
+        if (site_list) site_list_allow(site_list, site_list_len, sr.v_lo, R, d_list, d_allow);
+        const uint32_t blocks = (uint32_t)std::min<uint64_t>((R + 7) / 8, 16ull * sm_count(m->device));
+        auto kern = two ? fm::fm_k_sfs_counts<true> : fm::fm_k_sfs_counts<false>;
+        kern<<<blocks, fm::kSfsCountThreads, 0, stream()>>>(cells, sr.v_lo, R, site_list ? d_allow.p : nullptr, proj[0],
+                                                            two ? proj[1] : 0u, d_cnt1.p, d_cnt2.p, d_flag.p, d_tot.p);
+        CK(cudaGetLastError());
+        g_launches++;
+        size_t tmp_bytes = 0;
+        auto select = [&](void *tmp) {  // a null `tmp` only sizes it
+            CK(cub::DeviceSelect::Flagged(tmp, tmp_bytes, thrust::counting_iterator<uint32_t>(0), d_flag.p, sr.d_ci.p,
+                                          d_nsel.p, (int64_t)R, stream()));
+        };
+        select(nullptr);
+        DevBuf<uint8_t> d_tmp(std::max<size_t>(tmp_bytes, 16));
+        select(d_tmp.p);
+        d_nsel.download(&sr.n_sites, 1);
+        d_tot.download(sr.tot, 3);
+        CK(cudaStreamSynchronize(stream()));
+    }
+    const uint32_t n = sr.n_sites;
+    sr.d_c1.alloc(std::max<uint32_t>(n, 1));
+    sr.d_c2.alloc(two ? std::max<uint32_t>(n, 1) : 0);
+    if (n) {
+        fm::fm_k_sfs_gather<<<(n + 255) / 256, 256, 0, stream()>>>(sr.d_ci.p, n, d_cnt1.p, two ? d_cnt2.p : nullptr,
+                                                                   sr.d_c1.p, sr.d_c2.p);
+        CK(cudaGetLastError());
+        g_launches++;
+    }
+    tm.stop();
+    counts_ms = tm.ms();
+}
+
+// The statistics of include/ferromic_gpu.h from an unfolded spectrum xi [m + 1], in the header's operation order.
+static void sfs_statistics(const double *xi, uint32_t m, double &S, double &theta_pi, double &theta_w, double &D) {
+    double s = 0.0, num = 0.0, a1 = 0.0, a2 = 0.0;
+    for (uint32_t j = 1; j < m; ++j) {
+        s += xi[j];
+        num += (double)((uint64_t)j * (m - j)) * xi[j];
+    }
+    for (uint32_t i = 1; i < m; ++i) {
+        a1 += 1.0 / (double)i;
+        a2 += 1.0 / (double)((uint64_t)i * i);
+    }
+    S = s;
+    theta_pi = num / (double)((uint64_t)m * (m - 1) / 2);
+    theta_w = s / a1;
+    D = std::numeric_limits<double>::quiet_NaN();
+    if (m < 4) return;
+    const double fm_ = (double)m;
+    const double b1 = (fm_ + 1.0) / (3.0 * (fm_ - 1.0));
+    const double b2 = 2.0 * (fm_ * fm_ + fm_ + 3.0) / (9.0 * fm_ * (fm_ - 1.0));
+    const double c1 = b1 - 1.0 / a1;
+    const double c2 = b2 - (fm_ + 2.0) / (a1 * fm_) + a2 / (a1 * a1);
+    const double e1 = c1 / a1, e2 = c2 / (a1 * a1 + a2);
+    const double rad = e1 * s + e2 * s * (s - 1.0);
+    if (rad > 0.0 && std::isfinite(rad)) D = (theta_pi - theta_w) / std::sqrt(rad);
+}
+
+// The fold rule of include/ferromic_gpu.h, in place on x [m1 + 1][m2 + 1] (a 1-D spectrum: m2 = 0).
+static void sfs_fold(double *x, uint32_t m1, uint32_t m2) {
+    const uint64_t M = (uint64_t)m1 + m2, w = (uint64_t)m2 + 1;
+    for (uint64_t j1 = 0; j1 <= m1; ++j1)
+        for (uint64_t j2 = 0; j2 <= m2; ++j2) {
+            const uint64_t s = 2 * (j1 + j2), c1 = m1 - j1, c2 = m2 - j2;
+            if (s < M || (s == M && 2 * j1 < m1)) {  // (j, c(j)) with c(j) in the zeroed half
+                x[j1 * w + j2] += x[c1 * w + c2];
+                x[c1 * w + c2] = 0.0;
+            }
+        }
+}
+
+fm_status fm_site_frequency_spectrum(fm_matrix *m, const uint64_t *sample_idx, const uint8_t *side, size_t n_in,
+                                     const fm_sfs_params *prm, const int64_t *windows, size_t n_windows,
+                                     uint32_t *hap_off_out, double *spectrum, size_t spectrum_capacity,
+                                     uint64_t *window_sites, double *seg_out, double *theta_pi_out,
+                                     double *theta_w_out, double *tajimas_d_out, fm_sfs_info *info) {
+    return guarded([&] {
+        FM_NVTX("fm_site_frequency_spectrum");
+        const auto t_call = std::chrono::steady_clock::now();
+        require_device();
+        if (!m || !prm || !info) fail(FM_ERR_INVALID_ARG, "matrix, params or info is NULL");
+        std::memset(info, 0, sizeof(*info));
+        if (n_windows && !windows) fail(FM_ERR_INVALID_ARG, "windows is NULL");
+        require_cell_rows(m, "site frequency spectra");
+        if (n_windows && prm->has_region) fail(FM_ERR_INVALID_ARG, "windows and a region are exclusive");
+        set_dev(m);
+        uint32_t mp = 0;
+        const std::vector<uint32_t> off = sfs_set(m, sample_idx, side, n_in, prm->projection, "", mp);
+        const uint32_t n = (uint32_t)off.size();
+        info->n_haplotypes = n;
+        info->projection = mp;
+        if (hap_off_out) std::memcpy(hap_off_out, off.data(), (size_t)n * 4);
+        check_site_list(m, prm->site_list, prm->site_list_len);
+        SfsRows sr;
+        uint32_t v_hi = (uint32_t)m->V;
+        if (prm->has_region) site_range(m, prm->region_start, prm->region_end, sr.v_lo, v_hi);
+        sr.R = v_hi - sr.v_lo;
+        std::vector<uint32_t> lo, hi;
+        if (n_windows) window_ranges(m, windows, n_windows, lo, hi);
+        const size_t nw = std::max<size_t>(n_windows, 1), bins = (size_t)mp + 1;
+        char where[96];
+        snprintf(where, sizeof(where), " (n = %u haplotypes, m = %u, %zu windows)", n, mp, nw);
+        if (nw * bins > spectrum_capacity)
+            fail(FM_ERR_INVALID_ARG, std::string("spectrum capacity too small: max(n_windows, 1) * (m + 1) values are needed") + where);
+        if (!spectrum) fail(FM_ERR_INVALID_ARG, "spectrum is NULL");
+        const uint32_t tiles = (uint32_t)((bins + fm::kSfsTile1 - 1) / fm::kSfsTile1);
+        if ((uint64_t)tiles * nw >= (1ull << 31)) fail(FM_ERR_UNSUPPORTED, std::string("too many windows for one launch") + where);
+
+        // 1. counting pass and compaction
+        const std::vector<uint32_t> *offs[1] = {&off};
+        {
+            FM_NVTX("fm_site_frequency_spectrum: counts");
+            sfs_rows(m, offs, 1, &mp, prm->site_list, prm->site_list_len, sr, info->counts_ms);
+        }
+        info->candidates = sr.tot[0];
+        info->projected_out = sr.tot[1];
+        info->non_biallelic = sr.tot[2];
+        info->n_sites = sr.n_sites;
+
+        // 2. each window's contributing rows, then one CTA per (window, bin tile)
+        DevBuf<uint32_t> d_ws(nw), d_we(nw);
+        DevBuf<double> d_spec(nw * bins);
+        {
+            FM_NVTX("fm_site_frequency_spectrum: spectrum");
+            Timer tm;
+            tm.start();
+            if (n_windows) {
+                DevBuf<uint32_t> d_lo(nw), d_hi(nw);
+                d_lo.upload(lo.data(), nw);
+                d_hi.upload(hi.data(), nw);
+                fm::fm_k_sfs_window_bounds<<<(uint32_t)((nw + 255) / 256), 256, 0, stream()>>>(
+                    sr.d_ci.p, sr.n_sites, d_lo.p, d_hi.p, (uint32_t)nw, d_ws.p, d_we.p);
+                CK(cudaGetLastError());
+                g_launches++;
+            } else {
+                const uint32_t se[2] = {0, sr.n_sites};
+                d_ws.upload(se, 1);
+                d_we.upload(se + 1, 1);
+            }
+            fm::fm_k_sfs_spectrum<fm::kSfsTile1, 1><<<(uint32_t)(tiles * nw), fm::kSfsTile1, 0, stream()>>>(
+                sr.d_c1.p, nullptr, mp, 0u, nullptr, d_ws.p, d_we.p, tiles, 1u, d_spec.p, bins, 0);
+            CK(cudaGetLastError());
+            g_launches++;
+            tm.stop();
+            info->spectrum_ms = tm.ms();
+        }
+        std::vector<uint32_t> ws(nw), we(nw);
+        d_ws.download(ws.data(), nw);
+        d_we.download(we.data(), nw);
+        d_spec.download(spectrum, nw * bins);
+        CK(cudaStreamSynchronize(stream()));
+
+        // 3. statistics from the unfolded spectra, then the fold
+        for (size_t w = 0; w < nw; ++w) {
+            double *xi = spectrum + w * bins;
+            double S, tp, tw, D;
+            sfs_statistics(xi, mp, S, tp, tw, D);
+            if (window_sites) window_sites[w] = we[w] - ws[w];
+            if (seg_out) seg_out[w] = S;
+            if (theta_pi_out) theta_pi_out[w] = tp;
+            if (theta_w_out) theta_w_out[w] = tw;
+            if (tajimas_d_out) tajimas_d_out[w] = D;
+            if (prm->folded) sfs_fold(xi, mp, 0);
+        }
+        info->total_ms = (float)ms_since(t_call);
+    });
+}
+
+fm_status fm_joint_site_frequency_spectrum(fm_matrix *m, const uint64_t *sample_idx1, const uint8_t *side1, size_t n1,
+                                           const uint64_t *sample_idx2, const uint8_t *side2, size_t n2,
+                                           const fm_joint_sfs_params *prm, double *spectrum, size_t spectrum_capacity,
+                                           fm_joint_sfs_info *info) {
+    return guarded([&] {
+        FM_NVTX("fm_joint_site_frequency_spectrum");
+        const auto t_call = std::chrono::steady_clock::now();
+        require_device();
+        if (!m || !prm || !info) fail(FM_ERR_INVALID_ARG, "matrix, params or info is NULL");
+        std::memset(info, 0, sizeof(*info));
+        require_cell_rows(m, "site frequency spectra");
+        set_dev(m);
+        uint32_t mp[2] = {0, 0};
+        const std::vector<uint32_t> off1 = sfs_set(m, sample_idx1, side1, n1, prm->projection1, "set 1: ", mp[0]);
+        const std::vector<uint32_t> off2 = sfs_set(m, sample_idx2, side2, n2, prm->projection2, "set 2: ", mp[1]);
+        info->n_haplotypes1 = off1.size();
+        info->n_haplotypes2 = off2.size();
+        info->projection1 = mp[0];
+        info->projection2 = mp[1];
+        check_site_list(m, prm->site_list, prm->site_list_len);
+        SfsRows sr;
+        uint32_t v_hi = (uint32_t)m->V;
+        if (prm->has_region) site_range(m, prm->region_start, prm->region_end, sr.v_lo, v_hi);
+        sr.R = v_hi - sr.v_lo;
+        const uint64_t w2 = (uint64_t)mp[1] + 1, entries = ((uint64_t)mp[0] + 1) * w2;
+        char where[96];
+        snprintf(where, sizeof(where), " (m1 = %u, m2 = %u: %llu entries)", mp[0], mp[1], (unsigned long long)entries);
+        if (entries > (1ull << 28)) fail(FM_ERR_UNSUPPORTED, std::string("the joint spectrum exceeds 2^28 entries") + where);
+        if (entries > spectrum_capacity)
+            fail(FM_ERR_INVALID_ARG, std::string("spectrum capacity too small: (m1 + 1) * (m2 + 1) values are needed") + where);
+        if (!spectrum) fail(FM_ERR_INVALID_ARG, "spectrum is NULL");
+
+        // 1. one counting pass for both sets, compaction
+        const std::vector<uint32_t> *offs[2] = {&off1, &off2};
+        {
+            FM_NVTX("fm_joint_site_frequency_spectrum: counts");
+            sfs_rows(m, offs, 2, mp, prm->site_list, prm->site_list_len, sr, info->counts_ms);
+        }
+        info->candidates = sr.tot[0];
+        info->projected_out = sr.tot[1];
+        info->non_biallelic = sr.tot[2];
+        info->n_sites = sr.n_sites;
+
+        // 2. (tile, row) incidences, stably sorted by tile in passes of at most kSfsIncidenceChunk, and one CTA per
+        //    tile walking its rows in order
+        constexpr uint32_t T = fm::kSfsJointTile;
+        const uint32_t tiles1 = (mp[0] + T) / T, tiles2 = (mp[1] + T) / T, n_tiles = tiles1 * tiles2;
+        const uint32_t n = sr.n_sites;
+        DevBuf<double> d_spec(entries);
+        {
+            FM_NVTX("fm_joint_site_frequency_spectrum: spectrum");
+            Timer tm;
+            tm.start();
+            CK(cudaMemsetAsync(d_spec.p, 0, entries * 8, stream()));
+            DevBuf<unsigned long long> d_cnt(std::max<uint32_t>(n, 1)), d_off(std::max<uint32_t>(n, 1));
+            uint64_t total = 0;
+            if (n) {
+                fm::fm_k_sfs_incidence_count<<<(n + 255) / 256, 256, 0, stream()>>>(sr.d_c1.p, sr.d_c2.p, n, mp[0], mp[1],
+                                                                                   d_cnt.p);
+                CK(cudaGetLastError());
+                g_launches++;
+                size_t tmp_bytes = 0;
+                auto scan = [&](void *tmp) {  // a null `tmp` only sizes it
+                    CK(cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, d_cnt.p, d_off.p, (int64_t)n, stream()));
+                };
+                scan(nullptr);
+                DevBuf<uint8_t> d_tmp(std::max<size_t>(tmp_bytes, 16));
+                scan(d_tmp.p);
+                unsigned long long last_off = 0, last_cnt = 0;
+                CK(cudaMemcpyAsync(&last_off, d_off.p + n - 1, 8, cudaMemcpyDeviceToHost, stream()));
+                CK(cudaMemcpyAsync(&last_cnt, d_cnt.p + n - 1, 8, cudaMemcpyDeviceToHost, stream()));
+                CK(cudaStreamSynchronize(stream()));
+                total = last_off + last_cnt;
+            }
+            info->incidences = total;
+            // pass boundaries: rows [i0, i1) whose incidences fit one sort
+            std::vector<uint32_t> cuts{0};
+            if (total > kSfsIncidenceChunk) {
+                std::vector<unsigned long long> h_off(n);
+                d_off.download(h_off.data(), n);
+                CK(cudaStreamSynchronize(stream()));
+                uint64_t base = 0;
+                for (uint32_t i = 0; i < n; ++i)
+                    if (h_off[i] - base > kSfsIncidenceChunk - n_tiles) {  // one row adds at most n_tiles
+                        cuts.push_back(i);
+                        base = h_off[i];
+                    }
+            }
+            cuts.push_back(n);
+            const uint64_t cap = std::min<uint64_t>(total, kSfsIncidenceChunk);
+            DevBuf<uint32_t> d_keys(std::max<uint64_t>(cap, 1)), d_rows(std::max<uint64_t>(cap, 1)),
+                d_keys2(std::max<uint64_t>(cap, 1)), d_rows2(std::max<uint64_t>(cap, 1)), d_seg(n_tiles + 1);
+            int key_bits = 1;
+            while (key_bits < 32 && (1ull << key_bits) < n_tiles) ++key_bits;
+            for (size_t c = 0; c + 1 < cuts.size(); ++c) {
+                const uint32_t i0 = cuts[c], i1 = cuts[c + 1];
+                if (i0 == i1) continue;
+                unsigned long long o0 = 0, o1 = total;
+                CK(cudaMemcpyAsync(&o0, d_off.p + i0, 8, cudaMemcpyDeviceToHost, stream()));
+                if (i1 < n) CK(cudaMemcpyAsync(&o1, d_off.p + i1, 8, cudaMemcpyDeviceToHost, stream()));
+                CK(cudaStreamSynchronize(stream()));
+                const uint64_t cnt = o1 - o0;
+                fm::fm_k_sfs_incidence_emit<<<(i1 - i0 + 255) / 256, 256, 0, stream()>>>(
+                    sr.d_c1.p, sr.d_c2.p, i0, i1, mp[0], mp[1], tiles2, d_off.p, d_keys.p, d_rows.p);
+                CK(cudaGetLastError());
+                g_launches++;
+                size_t tmp_bytes = 0;
+                auto sort = [&](void *tmp) {  // LSD radix sort: stable, so each tile's rows stay in row order
+                    CK(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, d_keys.p, d_keys2.p, d_rows.p, d_rows2.p,
+                                                       (int64_t)cnt, 0, key_bits, stream()));
+                };
+                sort(nullptr);
+                DevBuf<uint8_t> d_tmp(std::max<size_t>(tmp_bytes, 16));
+                sort(d_tmp.p);
+                fm::fm_k_sfs_segments<<<(n_tiles + 1 + 255) / 256, 256, 0, stream()>>>(d_keys2.p, cnt, n_tiles, d_seg.p);
+                CK(cudaGetLastError());
+                g_launches++;
+                fm::fm_k_sfs_spectrum<T, T><<<n_tiles, T * T, 0, stream()>>>(
+                    sr.d_c1.p, sr.d_c2.p, mp[0], mp[1], d_rows2.p, d_seg.p, d_seg.p + 1, n_tiles, tiles2, d_spec.p,
+                    entries, info->passes > 0);
+                CK(cudaGetLastError());
+                g_launches++;
+                info->passes++;
+                CK(cudaStreamSynchronize(stream()));  // the buffers of this pass are reused by the next
+            }
+            tm.stop();
+            info->spectrum_ms = tm.ms();
+        }
+        d_spec.download(spectrum, entries);
+        CK(cudaStreamSynchronize(stream()));
+        if (prm->folded) sfs_fold(spectrum, mp[0], mp[1]);
         info->total_ms = (float)ms_since(t_call);
     });
 }

@@ -708,6 +708,97 @@ fm_status fm_haplotype_ld_prune(fm_matrix *m, const uint64_t *sample_idx, const 
                                 uint64_t *kept_sites_or_null, uint64_t *retained_sites, size_t site_capacity,
                                 fm_ld_prune_info *info);
 
+/* ---- site frequency spectra (this project's estimator; DESIGN.md §0 row f11, §3, §4 "Site frequency spectra") ----
+ * The allele frequency spectrum of a haplotype set, projected to a fixed sample size, per window; and the joint
+ * spectrum of two sets.
+ *   haplotypes  (sample_idx, side) as fm_haplotype_pca: offsets sample * ploidy + side, sorted and de-duplicated;
+ *               out-of-range samples and side 1 at ploidy 1 are dropped.  n = their number, 1 <= n < 2^26;
+ *               haplotype_offsets [n] (may be NULL) receives the offsets.
+ *   counts      over the set's cells at matrix row v: called_v; alt_v = called cells whose RAW value is 1 (never a rank
+ *               of the LUT); other_v = called cells whose raw value is neither 0 nor 1 (packed rows: 0).
+ *   candidates  without windows the region's rows (has_region == 0: every row); with windows every row.  A site list
+ *               (site_list, site_list_len: strictly ascending rows, each < n_variants) keeps only the listed rows.
+ *   projection  m = projection, 1 <= m <= n; projection == 0 means m = n.
+ *   classes     each candidate row, in this order: other_v > 0 -> non_biallelic; called_v < m -> projected_out;
+ *               otherwise it contributes (n_sites).  Monomorphic rows contribute to bins 0 and m; no MAF filter.
+ *   weights     a contributing row with (N, a) = (called_v, alt_v) adds h(j; N, a, m) = C(a, j) C(N - a, m - j) / C(N, m)
+ *               to bin j, for j in [max(0, m - (N - a)), min(a, m)] only.  A one-bin support (N == m among others)
+ *               has weight exactly 1.0.  Otherwise, FP64: h at the mode md = clamp(floor((m + 1)(a + 1) / (N + 2))) is
+ *               Loader's saddle-point form (R's dhyper: dbinom_raw(md, a) * dbinom_raw(m - md, N - a) /
+ *               dbinom_raw(m, N) at p = m / N, with stirlerr and bd0); then h(j + 1) = h(j) * ((a - j)(m - j) /
+ *               ((j + 1)(N - a - m + j + 1))) upward and h(j - 1) = h(j) * (j (N - a - m + j) / ((a - j + 1)(m - j + 1)))
+ *               downward, each ratio one FP64 division of two exact integer products.  Each weight is within 1e-12
+ *               relative of the exact rational for N <= 2^20; an exact value below 1e-290 may come out as 0.
+ *   sums        bin j of a window is the FP64 sum of its weights over the window's contributing rows in row order, so
+ *               outputs are bit-identical across calls, threads and launch geometry (no floating-point atomics).
+ *   windows     windows_or_null: n_windows 0-based inclusive (start, end) position pairs as fm_group_window_sums; they
+ *               may overlap, be empty or lie outside the data.  Without windows there is one window.
+ *   statistics  per window from the UNFOLDED spectrum xi with sample size m, in this FP64 order:
+ *               S = sum_{j=1}^{m-1} xi_j (ascending j); theta_pi = (sum_{j=1}^{m-1} (double)(j (m - j)) * xi_j) /
+ *               (double)(m (m - 1) / 2); a1 = sum_{i=1}^{m-1} 1.0 / i, a2 = sum_{i=1}^{m-1} 1.0 / (double)(i i);
+ *               theta_W = S / a1; b1 = (m + 1) / (3 (m - 1)), b2 = 2 (m^2 + m + 3) / (9 m (m - 1)), c1 = b1 - 1 / a1,
+ *               c2 = b2 - (m + 2) / (a1 m) + a2 / (a1 a1), e1 = c1 / a1, e2 = c2 / (a1 a1 + a2);
+ *               D = (theta_pi - theta_W) / sqrt(e1 S + e2 S (S - 1)), NaN when m < 4 or the radicand is <= 0 or not
+ *               finite (so also S == 0).  theta_pi and theta_W are window totals (divide by a length as
+ *               with the pi sums); at m == 1 both are 0 / 0 = NaN.
+ *   folding     folded != 0 folds the output spectrum (the statistics still come from xi).  With c(j) = (m1 - j1,
+ *               m2 - j2) and M = m1 + m2: 2(j1 + j2) < M -> xi[j] + xi[c(j)]; 2(j1 + j2) == M -> xi[j] when j == c(j),
+ *               else xi[j] + xi[c(j)] when 2 j1 < m1, else 0; 2(j1 + j2) > M -> 0.  A 1-D spectrum is m2 = 0.  The
+ *               rule keeps the total mass; it is this project's rule, not dadi's.
+ * Outputs: spectrum [max(n_windows, 1)][m + 1]; window_sites [max(n_windows, 1)] (may be NULL) the contributing rows
+ * of each window; segregating / theta_pi / theta_w / tajimas_d [max(n_windows, 1)] (each may be NULL).  info counts
+ * the candidate rows once each (not per window).
+ * FM_ERR_INVALID_ARG for a NULL argument, n == 0, m > n, n >= 2^26, a bad site list and windows together with
+ * has_region.  When spectrum_capacity < max(n_windows, 1) * (m + 1), info is filled in (n_haplotypes, projection)
+ * and the call returns FM_ERR_INVALID_ARG ("capacity too small"); spectrum may be NULL on such a query.
+ * FM_ERR_UNSUPPORTED for ploidy > 2, a matrix streamed as u8 rows, and windows or a region on unsorted positions.
+ * info: counts_ms (counting pass and compaction) and spectrum_ms (spectrum pass) are device events, total_ms the
+ * host time of the whole call. */
+typedef struct {
+    uint32_t projection; /* m; 0: m = n */
+    int folded;
+    int has_region;
+    int64_t region_start, region_end;
+    const uint64_t *site_list; /* NULL: every row */
+    uint64_t site_list_len;
+} fm_sfs_params;
+typedef struct {
+    uint64_t n_haplotypes, projection, candidates, n_sites, projected_out, non_biallelic; /* n, m, rows */
+    float counts_ms, spectrum_ms, total_ms;
+} fm_sfs_info;
+fm_status fm_site_frequency_spectrum(fm_matrix *m, const uint64_t *sample_idx, const uint8_t *side, size_t n,
+                                     const fm_sfs_params *params, const int64_t *windows_or_null, size_t n_windows,
+                                     uint32_t *haplotype_offsets_or_null, double *spectrum, size_t spectrum_capacity,
+                                     uint64_t *window_sites_or_null, double *segregating_or_null,
+                                     double *theta_pi_or_null, double *theta_w_or_null, double *tajimas_d_or_null,
+                                     fm_sfs_info *info);
+
+/* Joint spectrum of two haplotype sets of one matrix (they may overlap), each as above with its own projection
+ * (m1, m2).  One region (or every row) and an optional site list; no windows.  A candidate row is non_biallelic when
+ * either set has other > 0, projected_out when called1 < m1 or called2 < m2, and otherwise adds h1(j1) * h2(j2) (one
+ * FP64 multiply of the weights above) to entry [j1][j2], entries summed in row order.  spectrum [m1 + 1][m2 + 1]
+ * row-major, folded by the rule above when folded != 0.  The errors of fm_site_frequency_spectrum apply to each set;
+ * the size query fills n_haplotypes1/2 and projection1/2.  More than 2^28 entries fail with FM_ERR_UNSUPPORTED before
+ * any launch.  info: passes = spectrum passes (the (tile, row) incidences are sorted at most 2^27 at a time). */
+typedef struct {
+    uint32_t projection1, projection2; /* 0: the set's n */
+    int folded;
+    int has_region;
+    int64_t region_start, region_end;
+    const uint64_t *site_list;
+    uint64_t site_list_len;
+} fm_joint_sfs_params;
+typedef struct {
+    uint64_t n_haplotypes1, n_haplotypes2, projection1, projection2, candidates, n_sites, projected_out, non_biallelic;
+    uint64_t incidences; /* (tile, row) pairs of the joint pass */
+    uint32_t passes;
+    float counts_ms, spectrum_ms, total_ms;
+} fm_joint_sfs_info;
+fm_status fm_joint_site_frequency_spectrum(fm_matrix *m, const uint64_t *sample_idx1, const uint8_t *side1, size_t n1,
+                                           const uint64_t *sample_idx2, const uint8_t *side2, size_t n2,
+                                           const fm_joint_sfs_params *params, double *spectrum,
+                                           size_t spectrum_capacity, fm_joint_sfs_info *info);
+
 /* ---- synthetic cohorts for benchmarks and full-size parity tests ----
  * Fills a device-resident u8 matrix (reference layout) and, when d_missing != NULL, its packed
  * missing bitmap with a counter-based generator: entry (site, column) is a pure integer function

@@ -59,6 +59,31 @@ pub struct fm_ld_prune_info {
     pub called_plane: u32, pub band_launches: u32,
     pub stats_ms: f32, pub planes_ms: f32, pub band_ms: f32, pub scan_ms: f32, pub total_ms: f32,
 }
+#[repr(C)]
+pub struct fm_sfs_params {
+    pub projection: u32, pub folded: c_int, pub has_region: c_int, pub region_start: i64, pub region_end: i64,
+    pub site_list: *const u64, pub site_list_len: u64,
+}
+#[repr(C)]
+#[derive(Default)]
+pub struct fm_sfs_info {
+    pub n_haplotypes: u64, pub projection: u64, pub candidates: u64, pub n_sites: u64, pub projected_out: u64,
+    pub non_biallelic: u64,
+    pub counts_ms: f32, pub spectrum_ms: f32, pub total_ms: f32,
+}
+#[repr(C)]
+pub struct fm_joint_sfs_params {
+    pub projection1: u32, pub projection2: u32, pub folded: c_int, pub has_region: c_int, pub region_start: i64,
+    pub region_end: i64, pub site_list: *const u64, pub site_list_len: u64,
+}
+#[repr(C)]
+#[derive(Default)]
+pub struct fm_joint_sfs_info {
+    pub n_haplotypes1: u64, pub n_haplotypes2: u64, pub projection1: u64, pub projection2: u64, pub candidates: u64,
+    pub n_sites: u64, pub projected_out: u64, pub non_biallelic: u64, pub incidences: u64,
+    pub passes: u32,
+    pub counts_ms: f32, pub spectrum_ms: f32, pub total_ms: f32,
+}
 
 extern "C" {
     pub fn fm_last_error() -> *const c_char;
@@ -131,6 +156,16 @@ extern "C" {
     pub fn fm_haplotype_ld_prune(m: *mut fm_matrix, sample_idx: *const u64, side: *const u8, n: usize,
         params: *const fm_ld_params, r2_threshold: f64, haplotype_offsets: *mut u32, kept_sites: *mut u64,
         retained_sites: *mut u64, site_capacity: usize, info: *mut fm_ld_prune_info) -> c_int;
+    // projected site frequency spectrum per window, with S, theta_pi, theta_W and Tajima's D (new entry point;
+    // estimator in include/ferromic_gpu.h); spectrum may be NULL on a size query
+    pub fn fm_site_frequency_spectrum(m: *mut fm_matrix, sample_idx: *const u64, side: *const u8, n: usize,
+        params: *const fm_sfs_params, windows: *const i64, n_windows: usize, haplotype_offsets: *mut u32,
+        spectrum: *mut f64, spectrum_capacity: usize, window_sites: *mut u64, segregating: *mut f64,
+        theta_pi: *mut f64, theta_w: *mut f64, tajimas_d: *mut f64, info: *mut fm_sfs_info) -> c_int;
+    // joint spectrum of two haplotype sets [m1 + 1][m2 + 1] (new entry point)
+    pub fn fm_joint_site_frequency_spectrum(m: *mut fm_matrix, sample_idx1: *const u64, side1: *const u8, n1: usize,
+        sample_idx2: *const u64, side2: *const u8, n2: usize, params: *const fm_joint_sfs_params, spectrum: *mut f64,
+        spectrum_capacity: usize, info: *mut fm_joint_sfs_info) -> c_int;
     // BGZF (.vcf.gz as bgzip writes it) inflated on the device; fm_vcf_parse_bgzf parses from data_offset on
     pub fn fm_bgzf_inflate(gz: *const u8, n_gz: usize, out: *mut u8, capacity: usize, total_out: *mut u64) -> c_int;
     pub fn fm_vcf_parse_bgzf(gz: *const u8, n_gz: usize, data_offset: u64, chr: *const c_char, regions: *const i64,
