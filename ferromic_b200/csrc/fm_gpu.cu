@@ -3458,10 +3458,25 @@ void run_wc(fm_partition *p, const std::vector<uint32_t> &wlo, const std::vector
     wseg[nw] = (uint32_t)seg_lo.size();
     const uint32_t n_seg = (uint32_t)seg_lo.size();
     if (n_seg == 0) return;
-    for (fm_group *g : p->groups) ensure_counts(g);
-    set_dev(m);
     const bool multi = p->groups[0]->n_bits > 1;
     const uint32_t A = multi ? 1u << p->groups[0]->n_bits : 2u;
+    // multi-allelic kernel geometry: pair warps (lane = pair, KP pairs per lane in registers) + one overall warp per
+    // CTA, one CTA per segment; the biallelic path has its own pairs / overall kernels (below).  Population limits are
+    // refused here, before the count pass of bitplane groups launches anything (tests/test_gpu_wc_geometry.py,
+    // test_population_limit_refused_without_a_launch).
+    static const uint32_t kp_pref = env_u32("FM_WC_KP", 1);
+    uint32_t n_pw = std::max(1u, std::min<uint32_t>(fm::kWcMaxPairWarps, (n_pairs + 32 * kp_pref - 1) / (32 * kp_pref)));
+    const uint32_t kp_need = std::max(1u, (n_pairs + n_pw * 32 - 1) / (n_pw * 32));
+    const size_t smem = multi ? fm::fm_wc_multi_cta_smem(G, A) : 0;
+    const size_t psm = fm::fm_wc_pc_smem(G);
+    if (multi) {
+        if (kp_need > fm::kWcMaxKP) fail(FM_ERR_UNSUPPORTED, "too many populations for the W&C kernel (pairs per lane)");
+        if (smem > 200 * 1024) fail(FM_ERR_UNSUPPORTED, "too many populations for the W&C kernel's staging");
+    } else if (n_pairs && psm > 200 * 1024) {
+        fail(FM_ERR_UNSUPPORTED, "too many populations for the W&C kernel's staging");
+    }
+    for (fm_group *g : p->groups) ensure_counts(g);
+    set_dev(m);
     std::vector<const uint32_t *> h_alt(G + 1), h_cnt(G + 1);
     for (uint32_t g = 0; g <= G; ++g) {
         h_alt[g] = multi ? p->groups[g]->d_acount : p->groups[g]->d_alt;
@@ -3521,16 +3536,6 @@ void run_wc(fm_partition *p, const std::vector<uint32_t> &wlo, const std::vector
     W.part_pair = d_pp.p;
     W.part_pair_n = d_pn.p;
 
-    // multi-allelic kernel geometry: pair warps (lane = pair, KP pairs per lane in registers) + one overall warp per
-    // CTA, one CTA per segment; the biallelic path has its own pairs / overall kernels (below)
-    static const uint32_t kp_pref = env_u32("FM_WC_KP", 1);
-    uint32_t n_pw = std::max(1u, std::min<uint32_t>(fm::kWcMaxPairWarps, (n_pairs + 32 * kp_pref - 1) / (32 * kp_pref)));
-    const uint32_t kp_need = std::max(1u, (n_pairs + n_pw * 32 - 1) / (n_pw * 32));
-    const size_t smem = multi ? fm::fm_wc_multi_cta_smem(G, A) : 0;
-    if (multi) {
-        if (kp_need > fm::kWcMaxKP) fail(FM_ERR_UNSUPPORTED, "too many populations for the W&C kernel (pairs per lane)");
-        if (smem > 200 * 1024) fail(FM_ERR_UNSUPPORTED, "too many populations for the W&C kernel's staging");
-    }
     W.n_pair_warps = n_pw;
     const uint32_t blocks = std::max<uint32_t>(1, std::min<uint32_t>(n_seg, 8u * sm_count(m->device)));
     Timer tm;
@@ -3555,8 +3560,6 @@ void run_wc(fm_partition *p, const std::vector<uint32_t> &wlo, const std::vector
         if (n_pairs) {
             // producer / consumer pairs kernel: task = (segment, chunk of 352 pair slots), grid-strided over a
             // persistent grid of two CTAs per SM
-            const size_t psm = fm::fm_wc_pc_smem(G);
-            if (psm > 200 * 1024) fail(FM_ERR_UNSUPPORTED, "too many populations for the W&C kernel's staging");
             const uint32_t n_chunks = (n_pairs + fm::kWcPcPairWarps * 32 - 1) / (fm::kWcPcPairWarps * 32);
             static const uint32_t su = env_u32("FM_WC_SITES_PER_STEP", 1);
             auto launch = [&](auto kern) {
