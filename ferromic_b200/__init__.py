@@ -1,6 +1,6 @@
 """ferromic_b200 -- B200 (sm_100a) implementation of ferromic's per-site population-genetics
 estimators (segregating sites, pi, Watterson theta, per-site pi/theta tracks, Hudson FST/Dxy,
-Weir & Cockerham FST, pairwise sample differences, haplotype PCA, haplotype LD, LD pruning and site frequency spectra) behind the reference's own Python surface (`import ferromic_b200 as fm`).
+Weir & Cockerham FST, pairwise sample differences, haplotype PCA, haplotype LD, LD pruning, site frequency spectra and haplotype frequencies) behind the reference's own Python surface (`import ferromic_b200 as fm`).
 
 All estimator arithmetic runs in hand-written CUDA kernels through the C-ABI library
 `libferromic_gpu.so` (include/ferromic_gpu.h); there is no CPU fallback."""
@@ -8,6 +8,7 @@ from ._lib import FerromicGpuError, SO_PATH, lib  # noqa: F401
 from .api import (  # noqa: F401
     DiversitySite,
     FstEstimate,
+    HaplotypeFrequencyResult,
     HaplotypeLdPruneResult,
     HaplotypeLdResult,
     HaplotypePcaResult,
@@ -20,6 +21,7 @@ from .api import (  # noqa: F401
     WcFstResult,
     WcFstSite,
     adjusted_sequence_length,
+    haplotype_frequencies,
     haplotype_ld,
     haplotype_ld_prune,
     haplotype_pca,

@@ -116,6 +116,25 @@ class JointSfsInfo(C.Structure):
         ("passes", C.c_uint32)] + [(f, C.c_float) for f in ("counts_ms", "spectrum_ms", "total_ms")]
 
 
+class HapfreqParams(C.Structure):
+    _fields_ = [("size", C.c_uint32), ("step", C.c_uint32), ("min_maf", C.c_double), ("max_missing", C.c_double),
+                ("has_region", C.c_int), ("region_start", C.c_int64), ("region_end", C.c_int64),
+                ("site_list", C.c_void_p), ("site_list_len", C.c_uint64)]
+
+
+class HapfreqOut(C.Structure):
+    _fields_ = [("window_capacity", C.c_size_t)] + [
+        (f, C.c_void_p) for f in ("window_first", "window_sites", "n_used", "distinct", "top_counts", "sum_sq", "h1",
+                                  "h12", "h123", "h2_h1", "diversity", "count_offsets", "counts")] + [
+        ("counts_capacity", C.c_size_t)]
+
+
+class HapfreqInfo(C.Structure):
+    _fields_ = [(f, C.c_uint64) for f in ("n_haplotypes", "n_sites", "n_windows", "classes", "collisions")] + [
+        ("called_plane", C.c_uint32)] + [
+        (f, C.c_float) for f in ("stats_ms", "planes_ms", "hash_ms", "sort_ms", "count_ms", "total_ms")]
+
+
 EXPORTS = [
     "fm_last_error", "fm_version", "fm_device_count", "fm_set_device", "fm_set_devices", "fm_get_devices", "fm_synchronize", "fm_trim_pool",
     "fm_matrix_create", "fm_matrix_create_inband", "fm_matrix_create_device", "fm_matrix_retain", "fm_matrix_release",
@@ -133,6 +152,7 @@ EXPORTS = [
     "fm_pairwise_differences", "fm_bgzf_inflate", "fm_vcf_parse_bgzf", "fm_bgzf_deflate_bound", "fm_bgzf_deflate",
     "fm_falsta_tracks_bgzf", "fm_haplotype_pca", "fm_haplotype_ld",
     "fm_haplotype_ld_prune", "fm_site_frequency_spectrum", "fm_joint_site_frequency_spectrum",
+    "fm_haplotype_frequencies",
 ]
 
 _lib = None
@@ -254,6 +274,8 @@ def lib() -> C.CDLL:
                                              vp, C.POINTER(SfsInfo)]
     L.fm_joint_site_frequency_spectrum.argtypes = [vp, vp, vp, sz, vp, vp, sz, C.POINTER(JointSfsParams), vp, sz,
                                                    C.POINTER(JointSfsInfo)]
+    L.fm_haplotype_frequencies.argtypes = [vp, vp, vp, sz, C.POINTER(HapfreqParams), vp, sz, vp, vp, sz,
+                                           C.POINTER(HapfreqOut), C.POINTER(HapfreqInfo)]
     for name in EXPORTS:
         fn = getattr(L, name)
         if name not in ("fm_last_error", "fm_version"):

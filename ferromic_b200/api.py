@@ -1299,6 +1299,140 @@ def joint_site_frequency_spectrum(variants, haplotypes1, haplotypes2, projection
         int(info.non_biallelic))
 
 
+class HaplotypeFrequencyResult:
+    """Distinct haplotypes per window of kept sites with Garud's H statistics and the haplotype diversity
+    (fm_haplotype_frequencies).  `positions` are the kept sites' positions; `start` / `end` the positions of each
+    window's first and last kept site (-1 for a window without kept sites), `n_sites` its kept-site count.  `n_used`
+    (haplotypes without a missing cell in the window), `distinct`, `top_counts` ([3] per window: the three largest
+    class sizes), `sum_sq`, `h1`, `h12`, `h123`, `h2_h1` and `diversity` are scalars without windows and per-window
+    arrays with them; `counts` holds each window's class sizes in descending order (an array, or a list of arrays
+    with windows) when requested, else None."""
+    __slots__ = ("haplotypes", "positions", "start", "end", "n_sites", "n_used", "distinct", "top_counts", "sum_sq",
+                 "h1", "h12", "h123", "h2_h1", "diversity", "counts")
+
+    def __init__(self, haplotypes, positions, start, end, n_sites, n_used, distinct, top_counts, sum_sq, h1, h12, h123,
+                 h2_h1, diversity, counts):
+        self.haplotypes = haplotypes
+        self.positions = positions
+        self.start = start
+        self.end = end
+        self.n_sites = n_sites
+        self.n_used = n_used
+        self.distinct = distinct
+        self.top_counts = top_counts
+        self.sum_sq = sum_sq
+        self.h1 = h1
+        self.h12 = h12
+        self.h123 = h123
+        self.h2_h1 = h2_h1
+        self.diversity = diversity
+        self.counts = counts
+
+    def __repr__(self):
+        return (f"HaplotypeFrequencyResult(n_haplotypes={len(self.haplotypes)}, n_sites={len(self.positions)}, "
+                f"distinct={self.distinct}, h12={self.h12})")
+
+
+_HAPFREQ_OUT = (("window_first", np.uint64), ("window_sites", np.uint64), ("n_used", np.uint32),
+                ("distinct", np.uint32), ("sum_sq", np.uint64), ("h1", np.float64), ("h12", np.float64),
+                ("h123", np.float64), ("h2_h1", np.float64), ("diversity", np.float64))
+
+
+def _matrix_hapfreq(m: _Matrix, haplotypes, size=None, step=None, windows=None, region=None, min_maf=0.0,
+                    max_missing=0.0, sites=None, counts=False):
+    """fm_haplotype_frequencies on a device matrix: dict of offsets, kept (matrix rows), window_first, window_sites,
+    n_used, distinct, top_counts [k, 3], sum_sq, h1, h12, h123, h2_h1, diversity (arrays over the k windows),
+    count_offsets and counts (class sizes, CSR) or None, and the call's info struct.  A size query learns M and the
+    window count first; with counts a further query learns the number of classes.  windows: [k, 2] 0-based inclusive
+    position pairs; size / step: count windows of kept sites."""
+    if size is not None and not 1 <= int(size) < 2 ** 32:
+        raise ValueError("size must lie in [1, 2^32)")
+    if step is not None and not 1 <= int(step) < 2 ** 32:
+        raise ValueError("step must lie in [1, 2^32)")
+    if step is not None and size is None:
+        raise ValueError("step needs size")
+    if windows is not None and size is not None:
+        raise ValueError("windows and size are exclusive")
+    if windows is not None and region is not None:
+        raise ValueError("windows and region are exclusive")
+    idx, side, reg, rows = _haplotype_args(haplotypes, region, sites)
+    n_in = len(haplotypes)
+    prm = _lib.HapfreqParams(0 if size is None else int(size), 0 if step is None else int(step), float(min_maf),
+                             float(max_missing), *reg, *_site_list(rows))
+    win = None if windows is None else np.ascontiguousarray(np.asarray(windows, dtype=np.int64).reshape(-1, 2))
+    nw_in = 0 if win is None else len(win)
+    info = _lib.HapfreqInfo()
+    L = lib()
+
+    def call(out, off=None, kept=None, cap=0):
+        return L.fm_haplotype_frequencies(m.handle, _ptr(idx), _ptr(side), n_in, C.byref(prm), _ptr(win), nw_in,
+                                          _ptr(off), _ptr(kept), cap, C.byref(out), C.byref(info))
+
+    def sized(st):
+        if st != _lib.FM_OK and not (st == _lib.FM_ERR_INVALID_ARG and b"capacity too small" in L.fm_last_error()):
+            check(st)
+        return st
+
+    sized(call(_lib.HapfreqOut()))
+    M, nw = int(info.n_sites), int(info.n_windows)
+    k = max(nw, 1)
+    arrays = {name: np.zeros(k, dtype=dt) for name, dt in _HAPFREQ_OUT}
+    arrays["top_counts"] = np.zeros(3 * k, dtype=np.uint32)
+    coff = np.zeros(k + 1, dtype=np.uint64) if counts else None
+    cls = None
+    off = np.zeros(max(n_in, 1), dtype=np.uint32)
+    kept = np.zeros(max(M, 1), dtype=np.uint64)
+
+    def out_struct():
+        return _lib.HapfreqOut(k, *(_ptr(arrays[f]) for f in ("window_first", "window_sites", "n_used", "distinct",
+                                                              "top_counts", "sum_sq", "h1", "h12", "h123", "h2_h1",
+                                                              "diversity")), _ptr(coff), _ptr(cls),
+                            0 if cls is None else cls.size)
+
+    st = sized(call(out_struct(), off, kept, M))
+    if st != _lib.FM_OK:  # only the class sizes did not fit
+        cls = np.zeros(max(int(info.classes), 1), dtype=np.uint32)
+        check(call(out_struct(), off, kept, M))
+    n = int(info.n_haplotypes)
+    res = {name: arrays[name][:nw] for name, _ in _HAPFREQ_OUT}
+    res.update(offsets=off[:n].copy(), kept=kept[:M].astype(np.int64), top_counts=arrays["top_counts"][:3 * nw]
+               .reshape(nw, 3), count_offsets=None if coff is None else coff[:nw + 1].astype(np.int64),
+               counts=None if coff is None else (np.zeros(0, np.uint32) if cls is None else cls[:int(info.classes)]),
+               info=info)
+    return res
+
+
+def haplotype_frequencies(variants, haplotypes=None, size=None, step=None, windows=None, region=None, min_maf=0.0,
+                          max_missing=0.0, sites=None, counts=False) -> HaplotypeFrequencyResult:
+    """Distinct haplotypes over windows of kept sites on the GPU, with Garud's H1, H12, H123 and H2/H1 and the
+    haplotype diversity (definition in include/ferromic_gpu.h, fm_haplotype_frequencies).  haplotypes: (sample,
+    side) pairs, None = every cell of every sample, as haplotype_pca; sites are the kept sites of haplotype_ld (min_maf,
+    max_missing, region, `sites`).  Windows: `size` kept sites every `step` (None = size; a last partial window is
+    dropped), or `windows` as 0-based inclusive (start, end) position pairs (not with size or region), or neither for
+    one window of every kept site.  A haplotype with a missing cell in a window is left out of that window.  counts:
+    also return each window's class sizes, descending."""
+    vs, m, haps, region = _haplotype_call("haplotype frequencies", variants, haplotypes, region)
+    r = _matrix_hapfreq(m, haps, size, step, windows, region, min_maf, max_missing, sites, counts)
+    positions = vs.positions[r["kept"]]
+    first, cnt = r["window_first"].astype(np.int64), r["window_sites"].astype(np.int64)
+    has = cnt > 0
+    start = np.where(has, positions[np.where(has, first, 0)] if len(positions) else -1, -1).astype(np.int64)
+    end = np.where(has, positions[np.where(has, first + cnt - 1, 0)] if len(positions) else -1, -1).astype(np.int64)
+    cls = None
+    if counts:
+        co = r["count_offsets"]
+        cls = [r["counts"][co[w]:co[w + 1]] for w in range(len(co) - 1)]
+    if size is None and windows is None:
+        one = lambda a: a[0].item()  # noqa: E731
+        return HaplotypeFrequencyResult(
+            _offset_haplotypes(m, r["offsets"]), positions, int(start[0]), int(end[0]), int(cnt[0]),
+            one(r["n_used"]), one(r["distinct"]), r["top_counts"][0], one(r["sum_sq"]), one(r["h1"]), one(r["h12"]),
+            one(r["h123"]), one(r["h2_h1"]), one(r["diversity"]), None if cls is None else cls[0])
+    return HaplotypeFrequencyResult(
+        _offset_haplotypes(m, r["offsets"]), positions, start, end, cnt, r["n_used"], r["distinct"], r["top_counts"],
+        r["sum_sq"], r["h1"], r["h12"], r["h123"], r["h2_h1"], r["diversity"], cls)
+
+
 def _opt(value: float, some: int, bit: int):
     return value if (some >> bit) & 1 else None
 

@@ -14,11 +14,13 @@
 #include "fm_pca.cuh"
 #include "fm_ld.cuh"
 #include "fm_sfs.cuh"
+#include "fm_hapfreq.cuh"
 
 #include <nvtx3/nvToolsExt.h>
 
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
+#include <cub/device/device_segmented_sort.cuh>
 #include <cub/device/device_select.cuh>
 #include <thrust/iterator/counting_iterator.h>
 #include <thrust/iterator/transform_iterator.h>
@@ -6638,6 +6640,252 @@ fm_status fm_joint_site_frequency_spectrum(fm_matrix *m, const uint64_t *sample_
         d_spec.download(spectrum, entries);
         CK(cudaStreamSynchronize(stream()));
         if (prm->folded) sfs_fold(spectrum, mp[0], mp[1]);
+        info->total_ms = (float)ms_since(t_call);
+    });
+}
+
+// ------------------------------------------------------------------------------------ haplotype frequencies
+// (window, haplotype) entries hashed, sorted and counted at once; windows beyond it take further batches.
+constexpr uint64_t kHapfreqBatch = 1ull << 27;
+// The haplotype-major key (and called) bits of all kept sites are resident at once; beyond this the call fails.
+constexpr uint64_t kHapfreqKeyBytes = 8ull << 30;
+
+fm_status fm_haplotype_frequencies(fm_matrix *m, const uint64_t *sample_idx, const uint8_t *side, size_t n_in,
+                                   const fm_hapfreq_params *prm, const int64_t *windows, size_t n_windows,
+                                   uint32_t *hap_off_out, uint64_t *kept_out, size_t site_capacity,
+                                   const fm_hapfreq_out *out, fm_hapfreq_info *info) {
+    return guarded([&] {
+        FM_NVTX("fm_haplotype_frequencies");
+        const auto t_call = std::chrono::steady_clock::now();
+        require_device();
+        if (!m || !prm || !out || !info) fail(FM_ERR_INVALID_ARG, "matrix, params, out or info is NULL");
+        std::memset(info, 0, sizeof(*info));
+        if (n_in && (!sample_idx || !side)) fail(FM_ERR_INVALID_ARG, "haplotype arrays are NULL");
+        if (n_windows && !windows) fail(FM_ERR_INVALID_ARG, "windows is NULL");
+        if (!(prm->min_maf >= 0.0 && prm->min_maf <= 0.5)) fail(FM_ERR_INVALID_ARG, "min_maf must lie in [0, 0.5]");
+        if (!(prm->max_missing >= 0.0 && prm->max_missing < 1.0)) fail(FM_ERR_INVALID_ARG, "max_missing must lie in [0, 1)");
+        if (prm->step && !prm->size) fail(FM_ERR_INVALID_ARG, "step needs size");
+        if (n_windows && prm->size) fail(FM_ERR_INVALID_ARG, "windows and size are exclusive");
+        if (n_windows && prm->has_region) fail(FM_ERR_INVALID_ARG, "windows and a region are exclusive");
+        require_cell_rows(m, "haplotype frequencies");
+        set_dev(m);
+        std::vector<uint32_t> off = membership_offsets(m, sample_idx, side, n_in);
+        if (off.empty()) fail(FM_ERR_INVALID_ARG, "haplotype set is empty after de-duplication");
+        if (off.size() >= (1u << 26)) fail(FM_ERR_INVALID_ARG, "haplotype frequencies support fewer than 2^26 haplotypes");
+        std::vector<uint32_t> lo, hi;
+        if (n_windows) window_ranges(m, windows, n_windows, lo, hi);
+
+        // 1. site statistics and kept sites (those of fm_haplotype_ld)
+        HapSites hs;
+        {
+            FM_NVTX("haplotype frequencies: site statistics");
+            Timer tm;
+            select_hap_sites(m, std::move(off), prm->has_region, prm->region_start, prm->region_end, prm->min_maf,
+                             prm->max_missing, prm->site_list, prm->site_list_len, tm, hs);
+            tm.stop();
+            info->stats_ms = tm.ms();
+        }
+        const uint32_t n = hs.n, M = hs.M;
+        std::vector<uint32_t> kh(M);
+        hs.d_kept.download(kh.data(), M);
+        CK(cudaStreamSynchronize(stream()));
+
+        // 2. windows as (first kept site, kept-site count)
+        std::vector<uint32_t> wf, ws;
+        if (prm->size) {
+            const uint32_t step = prm->step ? prm->step : prm->size;
+            for (uint64_t f = 0; f + prm->size <= M; f += step) {
+                wf.push_back((uint32_t)f);
+                ws.push_back(prm->size);
+            }
+        } else if (n_windows) {
+            for (size_t w = 0; w < n_windows; ++w) {
+                const uint32_t a = (uint32_t)(std::lower_bound(kh.begin(), kh.end(), lo[w]) - kh.begin());
+                const uint32_t b = (uint32_t)(std::lower_bound(kh.begin(), kh.end(), hi[w]) - kh.begin());
+                wf.push_back(a);
+                ws.push_back(b - a);
+            }
+        } else {
+            wf.push_back(0);
+            ws.push_back(M);
+        }
+        const uint32_t nw = (uint32_t)wf.size();
+        info->n_haplotypes = n;
+        info->n_sites = M;
+        info->n_windows = nw;
+        info->called_plane = hs.incomplete != 0;
+        if (hap_off_out) std::memcpy(hap_off_out, hs.off.data(), (size_t)n * 4);
+
+        // 3. capacities (a too small one leaves the counts in info so that the caller can retry) and the key limit
+        char where[112];
+        snprintf(where, sizeof(where), " (n = %u haplotypes, M = %u kept sites, %u windows)", n, M, nw);
+        if (kept_out && M > site_capacity)
+            fail(FM_ERR_INVALID_ARG, std::string("site capacity too small: info->n_sites holds the number needed") + where);
+        if (std::max<uint32_t>(nw, 1) > out->window_capacity)
+            fail(FM_ERR_INVALID_ARG, std::string("window capacity too small: info->n_windows holds the number needed") + where);
+        const uint32_t KW = (M + 63) / 64;
+        const uint64_t key_bytes = (uint64_t)n * (KW + 1) * 8 * (hs.incomplete ? 2 : 1);
+        if (key_bytes > kHapfreqKeyBytes)
+            fail(FM_ERR_UNSUPPORTED, std::string("the haplotype-major key bits of the kept sites exceed 8 GiB") + where);
+        if (kept_out)
+            for (uint32_t j = 0; j < M; ++j) kept_out[j] = kh[j];
+        for (uint32_t w = 0; w < nw; ++w) {
+            if (out->window_first) out->window_first[w] = wf[w];
+            if (out->window_sites) out->window_sites[w] = ws[w];
+        }
+        const bool csr = out->count_offsets != nullptr;
+        if (csr) out->count_offsets[0] = 0;
+        if (nw == 0) {
+            info->total_ms = (float)ms_since(t_call);
+            return;
+        }
+
+        // 4. haplotype-major key rows [KW + 1][n] (the last row zero, read by the funnel shift) and called rows
+        DevBuf<uint64_t> d_keys((size_t)(KW + 1) * n), d_called(hs.incomplete ? (size_t)(KW + 1) * n : 0);
+        {
+            FM_NVTX("haplotype frequencies: planes");
+            Timer tm;
+            tm.start();
+            CK(cudaMemsetAsync(d_keys.p + (size_t)KW * n, 0, (size_t)n * 8, stream()));
+            if (hs.incomplete) CK(cudaMemsetAsync(d_called.p + (size_t)KW * n, 0, (size_t)n * 8, stream()));
+            if (KW) {
+                fm::fm_k_hapfreq_planes<<<transpose_grid(m, (uint64_t)KW * ((n + 31) / 32)), 256, 0, stream()>>>(
+                    hs.cells, hs.d_off.p, n, hs.d_kept.p, M, KW, d_keys.p, hs.incomplete ? d_called.p : nullptr);
+                CK(cudaGetLastError());
+                g_launches++;
+            }
+            tm.stop();
+            info->planes_ms = tm.ms();
+        }
+
+        // 5. per batch of windows: hash, segmented sort, count (and the class sizes when requested)
+        const uint32_t per_batch = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(nw, kHapfreqBatch / n));
+        const size_t cap = (size_t)per_batch * n;
+        DevBuf<uint32_t> d_wf(nw), d_ws(nw), d_used(nw), d_k(nw), d_top(3 * (size_t)nw);
+        DevBuf<unsigned long long> d_s2(nw), d_coll(1);
+        DevBuf<double> d_stat(5 * (size_t)nw);
+        DevBuf<uint64_t> d_hk(cap), d_hk2(cap);
+        DevBuf<uint32_t> d_hv(cap), d_hv2(cap), d_rep(cap), d_aux(cap), d_seg(per_batch + 1);
+        DevBuf<uint32_t> d_cls(csr ? cap : 0), d_clsk(csr ? per_batch + 1 : 0), d_coff(csr ? per_batch + 1 : 0);
+        DevBuf<uint32_t> d_csr(csr ? cap : 0), d_csr2(csr ? cap : 0);
+        DevBuf<uint8_t> d_tmp;
+        auto cub_run = [&d_tmp](auto f) {  // sizes d_tmp for a cub call (it only grows) and runs it
+            size_t bytes = 0;
+            f(nullptr, bytes);
+            if (bytes > d_tmp.n) d_tmp.alloc(bytes);
+            f(d_tmp.p, bytes);
+        };
+        d_wf.upload(wf.data(), nw);
+        d_ws.upload(ws.data(), nw);
+        {
+            std::vector<uint32_t> seg(per_batch + 1);
+            for (uint32_t w = 0; w <= per_batch; ++w) seg[w] = w * n;
+            d_seg.upload(seg.data(), per_batch + 1);
+        }
+        CK(cudaMemsetAsync(d_coll.p, 0, 8, stream()));
+        const fm::HapfreqDev dev{d_used.p, d_k.p, d_top.p, d_s2.p, d_stat.p, d_stat.p + nw, d_stat.p + 2 * (size_t)nw,
+                                 d_stat.p + 3 * (size_t)nw, d_stat.p + 4 * (size_t)nw, csr ? d_cls.p : nullptr,
+                                 csr ? d_clsk.p : nullptr};
+        uint64_t classes = 0;
+        for (uint32_t w0 = 0; w0 < nw; w0 += per_batch) {
+            const uint32_t bw = std::min(per_batch, nw - w0);
+            const uint64_t elems = (uint64_t)bw * n;
+            {
+                FM_NVTX("haplotype frequencies: hash");
+                Timer tm;
+                tm.start();
+                fm::fm_k_hapfreq_hash<<<(uint32_t)((elems + 255) / 256), 256, 0, stream()>>>(
+                    d_keys.p, hs.incomplete ? d_called.p : nullptr, n, d_wf.p, d_ws.p, w0, elems, d_hk.p, d_hv.p);
+                CK(cudaGetLastError());
+                g_launches++;
+                tm.stop();
+                info->hash_ms += tm.ms();
+            }
+            {
+                FM_NVTX("haplotype frequencies: sort");
+                Timer tm;
+                tm.start();
+                cub_run([&](void *tmp, size_t &bytes) {
+                    CK(cub::DeviceSegmentedSort::SortPairs(tmp, bytes, d_hk.p, d_hk2.p, d_hv.p, d_hv2.p, (int64_t)elems,
+                                                           (int64_t)bw, d_seg.p, d_seg.p + 1, stream()));
+                });
+                tm.stop();
+                info->sort_ms += tm.ms();
+            }
+            {
+                FM_NVTX("haplotype frequencies: count");
+                Timer tm;
+                tm.start();
+                CK(cudaMemsetAsync(d_aux.p, 0, elems * 4, stream()));
+                fm::fm_k_hapfreq_count<<<bw, fm::kHapfreqCountThreads, 0, stream()>>>(
+                    d_keys.p, n, d_wf.p, d_ws.p, w0, d_hk2.p, d_hv2.p, d_rep.p, d_aux.p, dev, d_coll.p);
+                CK(cudaGetLastError());
+                g_launches++;
+                tm.stop();
+                info->count_ms += tm.ms();
+            }
+            if (!csr) continue;
+            {
+                FM_NVTX("haplotype frequencies: class sizes");
+                Timer tm;
+                tm.start();
+                CK(cudaMemsetAsync(d_clsk.p + bw, 0, 4, stream()));
+                cub_run([&](void *tmp, size_t &bytes) {
+                    CK(cub::DeviceScan::ExclusiveSum(tmp, bytes, d_clsk.p, d_coff.p, (int64_t)bw + 1, stream()));
+                });
+                fm::fm_k_hapfreq_gather<<<(uint32_t)((elems + 255) / 256), 256, 0, stream()>>>(d_cls.p, n, elems, d_clsk.p,
+                                                                                              d_coff.p, d_csr.p);
+                CK(cudaGetLastError());
+                g_launches++;
+                uint32_t total = 0;
+                CK(cudaMemcpyAsync(&total, d_coff.p + bw, 4, cudaMemcpyDeviceToHost, stream()));
+                CK(cudaStreamSynchronize(stream()));
+                if (total)
+                    cub_run([&](void *tmp, size_t &bytes) {
+                        CK(cub::DeviceSegmentedSort::SortKeysDescending(tmp, bytes, d_csr.p, d_csr2.p, (int64_t)total,
+                                                                        (int64_t)bw, d_coff.p, d_coff.p + 1, stream()));
+                    });
+                tm.stop();
+                info->sort_ms += tm.ms();
+                if (total && out->counts && classes + total <= out->counts_capacity) {
+                    d_csr2.download(out->counts + classes, total);
+                    CK(cudaStreamSynchronize(stream()));
+                }
+                classes += total;
+            }
+        }
+
+        // 6. per-window results
+        std::vector<uint32_t> h_used(nw), h_k(nw), h_top(3 * (size_t)nw);
+        std::vector<unsigned long long> h_s2(nw);
+        std::vector<double> h_stat(5 * (size_t)nw);
+        unsigned long long coll = 0;
+        d_used.download(h_used.data(), nw);
+        d_k.download(h_k.data(), nw);
+        d_top.download(h_top.data(), 3 * (size_t)nw);
+        d_s2.download(h_s2.data(), nw);
+        d_stat.download(h_stat.data(), 5 * (size_t)nw);
+        d_coll.download(&coll, 1);
+        CK(cudaStreamSynchronize(stream()));
+        info->collisions = coll;
+        for (uint32_t w = 0; w < nw; ++w) {
+            if (out->n_used) out->n_used[w] = h_used[w];
+            if (out->distinct) out->distinct[w] = h_k[w];
+            if (out->top_counts)
+                for (int q = 0; q < 3; ++q) out->top_counts[3 * (size_t)w + q] = h_top[3 * (size_t)w + q];
+            if (out->sum_sq) out->sum_sq[w] = h_s2[w];
+            double *dst[5] = {out->h1, out->h12, out->h123, out->h2_h1, out->diversity};
+            for (int q = 0; q < 5; ++q)
+                if (dst[q]) dst[q][w] = h_stat[(size_t)q * nw + w];
+        }
+        uint64_t total_k = 0;
+        for (uint32_t w = 0; w < nw; ++w) {
+            total_k += h_k[w];
+            if (csr) out->count_offsets[w + 1] = total_k;
+        }
+        info->classes = total_k;
+        if (csr && total_k > out->counts_capacity)
+            fail(FM_ERR_INVALID_ARG, std::string("counts capacity too small: info->classes holds the number needed") + where);
         info->total_ms = (float)ms_since(t_call);
     });
 }

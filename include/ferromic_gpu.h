@@ -799,6 +799,82 @@ fm_status fm_joint_site_frequency_spectrum(fm_matrix *m, const uint64_t *sample_
                                            const fm_joint_sfs_params *params, double *spectrum,
                                            size_t spectrum_capacity, fm_joint_sfs_info *info);
 
+/* ---- haplotype frequencies (this project's estimator; DESIGN.md §0 row f12, §3, §4 "Haplotype frequencies") ----
+ * Distinct haplotypes per window of kept sites, with the haplotype homozygosity statistics of Garud et al. (2015)
+ * and the haplotype diversity (scikit-allel's garud_h, moving_garud_h and haplotype_diversity).
+ *   haplotypes  (sample_idx, side) as fm_haplotype_pca: offsets sample * ploidy + side, sorted and de-duplicated;
+ *               out-of-range samples and side 1 at ploidy 1 are dropped.  n = their number, 1 <= n < 2^26;
+ *               haplotype_offsets [n] (may be NULL) receives the offsets.
+ *   sites       the kept sites of fm_haplotype_ld for the same min_maf, max_missing, region and site list; M of them
+ *               in matrix-row order; kept_sites [site_capacity] (may be NULL) receives their rows.
+ *   windows     count windows (size >= 1): window w is kept sites [w step, w step + size) for every w with
+ *               w step + size <= M (a last partial window is dropped, as allel.moving_statistic drops it); step == 0
+ *               means step = size; a region is allowed.  Position windows (windows_or_null, n_windows 0-based
+ *               inclusive (start, end) pairs as fm_site_frequency_spectrum; not with a region or size): window w takes
+ *               the kept sites whose position lies in it, and may be empty, overlap others or lie outside the data.
+ *               Neither: one window of all M kept sites.
+ *   key         a haplotype's key in a window is its allele bits (raw value 1 = 1) at the window's kept sites, in site
+ *               order.  A haplotype with a missing cell at any kept site of the window is left out of that window
+ *               (only possible with max_missing > 0).  scikit-allel instead treats -1 as one more allele value.
+ *   counts      N = haplotypes used; K = distinct keys among them; c1 >= c2 >= c3 the three largest class sizes (0
+ *               where there are fewer classes); s2 = sum of c^2 over the classes (exact).  A window without kept sites
+ *               has K = 1 when N > 0.
+ *   statistics  each one FP64 division of exact integers (N^2 < 2^52), so correctly rounded:
+ *               h1 = (double)s2 / (double)(N N); h12 = (double)(s2 + 2 c1 c2) / (double)(N N);
+ *               h123 = (double)(s2 + 2 (c1 c2 + c1 c3 + c2 c3)) / (double)(N N); h2_h1 = (double)(s2 - c1 c1) /
+ *               (double)s2; diversity = (double)(N N - s2) / (double)(N (N - 1)).  All are NaN when N == 0, and
+ *               diversity also when N == 1.  These equal scikit-allel's (p1 + p2)^2 + sum_{i>=3} p_i^2 (H12) and
+ *               (1 - sum p^2) n / (n - 1) (haplotype diversity) algebraically.
+ *   hash        keys are grouped by a 64-bit hash and then compared exactly, so the result does not depend on it:
+ *               x_0, ..., x_{L-1} are the window's key words (bit b of x_i = kept site first + 64 i + b, the last
+ *               word holding the remaining bits), h = 0, h = h * 0x9e3779b97f4a7c15 + x_i (mod 2^64) for each word in
+ *               order, and the hash is MurmurHash3's fmix64(h).  Two keys that hash alike but differ are split into
+ *               exact classes; info->collisions counts the hash runs that held more than one key.
+ * Outputs (out; each pointer may be NULL) are indexed by window, window_capacity entries each: window_first (index of
+ * the window's first kept site, for an empty window the number of kept sites before it) and window_sites; n_used,
+ * distinct, top_counts [3 per window] and sum_sq; h1, h12, h123, h2_h1 and diversity.  count_offsets [n_windows + 1]
+ * with counts [counts_capacity] give each window's class sizes in descending order (CSR; requested by
+ * count_offsets != NULL).  Outputs are bit-identical across calls and threads.
+ * FM_ERR_INVALID_ARG for a NULL argument, n == 0 or n >= 2^26 after de-duplication, min_maf outside [0, 0.5],
+ * max_missing outside [0, 1), a bad site list, step without size, and windows together with size or a region.  When
+ * kept_sites is given and M > site_capacity, or max(n_windows, 1) > window_capacity, or the class sizes exceed
+ * counts_capacity, info is filled in (n_haplotypes, n_sites, n_windows, called_plane; classes and count_offsets too
+ * in the last case) and the call returns FM_ERR_INVALID_ARG ("capacity too small") so that the caller can retry.
+ * FM_ERR_UNSUPPORTED for ploidy > 2, a matrix streamed as u8 rows, windows or a region on unsorted positions, and,
+ * before any launch, haplotype-major key bits above 8 GiB (n * (ceil(M / 64) + 1) * 8 bytes, twice that when some
+ * kept site has a missing cell).
+ * info: n_windows (count windows: the number that fit; else max(n_windows, 1)), classes = sum of K, collisions;
+ * called_plane = 1 when some kept site has a missing cell; stats_ms, planes_ms, hash_ms, sort_ms (hash sort, and the
+ * class-size sort when counts are requested) and count_ms are device events summed over the batches of at most 2^27
+ * (window, haplotype) entries, total_ms the host time of the whole call. */
+typedef struct {
+    uint32_t size, step; /* count windows of `size` kept sites (0: none); step 0 = size */
+    double min_maf, max_missing;
+    int has_region;
+    int64_t region_start, region_end;
+    const uint64_t *site_list; /* NULL: every row; else strictly ascending matrix rows, as fm_pca_params */
+    uint64_t site_list_len;
+} fm_hapfreq_params;
+typedef struct {
+    size_t window_capacity;
+    uint64_t *window_first, *window_sites;
+    uint32_t *n_used, *distinct, *top_counts; /* top_counts [window_capacity][3] */
+    uint64_t *sum_sq;
+    double *h1, *h12, *h123, *h2_h1, *diversity;
+    uint64_t *count_offsets; /* [window_capacity + 1] */
+    uint32_t *counts;
+    size_t counts_capacity;
+} fm_hapfreq_out;
+typedef struct {
+    uint64_t n_haplotypes, n_sites, n_windows, classes, collisions; /* n, M, windows, sum of K, split hash runs */
+    uint32_t called_plane;
+    float stats_ms, planes_ms, hash_ms, sort_ms, count_ms, total_ms;
+} fm_hapfreq_info;
+fm_status fm_haplotype_frequencies(fm_matrix *m, const uint64_t *sample_idx, const uint8_t *side, size_t n,
+                                   const fm_hapfreq_params *params, const int64_t *windows_or_null, size_t n_windows,
+                                   uint32_t *haplotype_offsets_or_null, uint64_t *kept_sites_or_null,
+                                   size_t site_capacity, const fm_hapfreq_out *out, fm_hapfreq_info *info);
+
 /* ---- synthetic cohorts for benchmarks and full-size parity tests ----
  * Fills a device-resident u8 matrix (reference layout) and, when d_missing != NULL, its packed
  * missing bitmap with a counter-based generator: entry (site, column) is a pure integer function

@@ -84,6 +84,26 @@ pub struct fm_joint_sfs_info {
     pub passes: u32,
     pub counts_ms: f32, pub spectrum_ms: f32, pub total_ms: f32,
 }
+#[repr(C)]
+pub struct fm_hapfreq_params {
+    pub size: u32, pub step: u32, pub min_maf: f64, pub max_missing: f64, pub has_region: c_int, pub region_start: i64,
+    pub region_end: i64, pub site_list: *const u64, pub site_list_len: u64,
+}
+#[repr(C)]
+pub struct fm_hapfreq_out {
+    pub window_capacity: usize,
+    pub window_first: *mut u64, pub window_sites: *mut u64,
+    pub n_used: *mut u32, pub distinct: *mut u32, pub top_counts: *mut u32, pub sum_sq: *mut u64,
+    pub h1: *mut f64, pub h12: *mut f64, pub h123: *mut f64, pub h2_h1: *mut f64, pub diversity: *mut f64,
+    pub count_offsets: *mut u64, pub counts: *mut u32, pub counts_capacity: usize,
+}
+#[repr(C)]
+#[derive(Default)]
+pub struct fm_hapfreq_info {
+    pub n_haplotypes: u64, pub n_sites: u64, pub n_windows: u64, pub classes: u64, pub collisions: u64,
+    pub called_plane: u32,
+    pub stats_ms: f32, pub planes_ms: f32, pub hash_ms: f32, pub sort_ms: f32, pub count_ms: f32, pub total_ms: f32,
+}
 
 extern "C" {
     pub fn fm_last_error() -> *const c_char;
@@ -166,6 +186,11 @@ extern "C" {
     pub fn fm_joint_site_frequency_spectrum(m: *mut fm_matrix, sample_idx1: *const u64, side1: *const u8, n1: usize,
         sample_idx2: *const u64, side2: *const u8, n2: usize, params: *const fm_joint_sfs_params, spectrum: *mut f64,
         spectrum_capacity: usize, info: *mut fm_joint_sfs_info) -> c_int;
+    // distinct haplotypes per window with Garud's H1, H12, H123, H2/H1 and haplotype diversity (new entry point;
+    // estimator in include/ferromic_gpu.h); out's arrays may be NULL on a size query
+    pub fn fm_haplotype_frequencies(m: *mut fm_matrix, sample_idx: *const u64, side: *const u8, n: usize,
+        params: *const fm_hapfreq_params, windows: *const i64, n_windows: usize, haplotype_offsets: *mut u32,
+        kept_sites: *mut u64, site_capacity: usize, out: *const fm_hapfreq_out, info: *mut fm_hapfreq_info) -> c_int;
     // BGZF (.vcf.gz as bgzip writes it) inflated on the device; fm_vcf_parse_bgzf parses from data_offset on
     pub fn fm_bgzf_inflate(gz: *const u8, n_gz: usize, out: *mut u8, capacity: usize, total_out: *mut u64) -> c_int;
     pub fn fm_vcf_parse_bgzf(gz: *const u8, n_gz: usize, data_offset: u64, chr: *const c_char, regions: *const i64,
